@@ -3,6 +3,7 @@
 
   python bench.py [--gpus N] [--steps K] [--warmup W]                 # this repo's CUDA path (liborbx.so)
   python bench.py --impl reference [--gpus N] [--steps K] [--warmup W] # OpenCV (cv2) on the host cores
+  python bench.py --steps K --dump-outputs DIR                         # + the last timed step's outputs as DIR/*.npy
 
 Workload (BASELINE.json configs[1] + the front-end's call pattern, src/frontend.cpp:98-108): a batch of B = 256
 synthetic 640x480 BGR frames, ORB with 1000 features / scale 1.2 / 8 levels, then 2 brute-force Hamming matches per
@@ -228,6 +229,41 @@ def run_reference(args, cfg, rank: int, world: int):
     emit(line)
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, last_step, is_c3: bool) -> None:
+    """--dump-outputs: what the timed step's caller receives, as float32 / float64 .npy files in out_dir (at most DUMP_BYTES).
+    Frames whose largest possible output does not fit are left out: a fixed, seeded sample of frames (frames.npy) is kept,
+    chosen from the batch size and the buffer shapes only, so two builds run with the same arguments dump the same frames.
+
+      frames.npy      [F]          float64  indices of the dumped frames in the step's batch
+      counts.npy      [F]          float64  keypoints per frame                       (not for c3: its train sets are inputs)
+      keypoints.npy   [sum, 7]     float32  cv::KeyPoint records of those frames, in order: x, y, size, angle, response, octave, class_id
+      descriptors.npy [sum, 32]    float32  their ORB descriptors, one byte per column  (not for c3)
+      matches.npy     [2, F, M, 4] float32  cv::DMatch records of the step's two matches of the map: queryIdx, trainIdx, imgIdx, distance
+    """
+    cnt, kps, desc, best = last_step
+    n_match, nb, m, _ = best.shape
+    cap = kps.shape[1]
+    per_frame = n_match * m * 16 + (0 if is_c3 else 8 + cap * (7 + 32) * 4)
+    n_keep = min(nb, DUMP_BYTES // per_frame)
+    frames = np.arange(nb) if n_keep == nb else np.sort(np.random.default_rng(0).choice(nb, n_keep, replace=False))
+    out = {"frames": frames.astype(np.float64)}
+    if not is_c3:
+        rec = np.concatenate([kps[i, :cnt[i]] for i in frames]) if n_keep else np.zeros((0, 7), np.float32)
+        rec = np.concatenate([rec[:, :5], rec[:, 5:].view(np.int32).astype(np.float32)], axis=1)   # octave, class_id: int32 fields
+        out.update(counts=cnt[frames].astype(np.float64), keypoints=rec,
+                   descriptors=(np.concatenate([desc[i, :cnt[i]] for i in frames]) if n_keep else np.zeros((0, 32), np.uint8)).astype(np.float32))
+    mt = best[:, frames].copy()
+    out["matches"] = np.concatenate([mt[..., :3].astype(np.float32), mt[..., 3:].view(np.float32)], axis=-1)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+    print(f"bench.py: outputs of the last timed step ({n_keep} of {nb} frames, {sum(a.nbytes for a in out.values()) / 2**20:.1f} MiB) written to {out_dir}",
+          file=sys.stderr)
+
+
 def _load_json(rel):
     try:
         return json.load(open(os.path.join(ROOT, rel)))
@@ -287,7 +323,10 @@ def run_orbx(args, cfg, rank: int, world: int, local_rank: int):
     counts = d_cnt.cpu().numpy()
     assert counts.max() <= cap, "capacity too small for this data"
     if not is_c3:
-        map_np = synth_map_queries(d_desc[0, :counts[0]].cpu().numpy(), MAPM, 17)
+        # the map is made from frame 0's descriptors as the CPU oracle computes them (the same bytes a correct build returns),
+        # so that the matcher's inputs do not depend on the build being measured
+        from oracle import oracle as O
+        map_np = synth_map_queries(O.detect_and_compute(frames_np[0], NF, SCALE, NLEVELS, cap=cap)[1], MAPM, 17)
     d_map = torch.from_numpy(map_np).to(dev)
     torch.cuda.synchronize()
 
@@ -318,6 +357,11 @@ def run_orbx(args, cfg, rank: int, world: int, local_rank: int):
     ms = e0.elapsed_time(e1)
     launches = ctx.launch_count - launches0
     t_wall1 = time.perf_counter()
+    last_step = None
+    if args.dump_outputs and rank == 0:                  # what the last timed step left in the output buffers, before anything reuses them
+        with torch.cuda.stream(stream):
+            last_step = [t_.clone() for t_ in (d_cnt, d_kps, d_desc, d_best)]
+        torch.cuda.synchronize()
     clocks = None
     if sampler:
         note = None
@@ -593,6 +637,8 @@ def run_orbx(args, cfg, rank: int, world: int, local_rank: int):
             "roofline_match": roof_match, "stage_ms": stage_ms, "cpu_baseline": cpu, "parity": parity}
     if sweep is not None:
         line["sweep"] = sweep
+    if last_step is not None:
+        dump_outputs(args.dump_outputs, [t_.cpu().numpy() for t_ in last_step], is_c3)
     emit(line)
     if dist is not None:
         dist.destroy_process_group()
@@ -626,7 +672,14 @@ def main():
     ap.add_argument("--impl", default="orbx", choices=["orbx", "reference"])
     ap.add_argument("--config", default="c2", choices=sorted(CONFIGS), help="BASELINE.json configs[0..4]; the default c2 is the metric's configuration")
     ap.add_argument("--batch", type=int, default=0, help="frames per GPU per step (default: the config's)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the outputs of the last one as DIR/<name>.npy (float32 / float64, at most 64 MiB; "
+                         "rank 0's frames; see dump_outputs)")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "orbx":
+        ap.error("--dump-outputs writes the orbx arm's outputs")
     cfg = CONFIGS[args.config]
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

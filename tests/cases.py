@@ -37,10 +37,20 @@ ORB_CASES = {
     "heapsel_b1000": (lambda: _rolled(777 + 16, 42, 78), 1000),
 }
 
-# larger cases: checked live against cv2 / between oracle and GPU, not stored as fixtures
+# larger cases: checked between oracle and GPU, and against cv2 (live when importable, and its stored result in
+# tests/golden/, written by tools/make_golden_live.py)
 ORB_CASES_LARGE = {
     "720p1500": (lambda: synth_frame(720, 1280, 4), 1500),
     "1080p2000": (lambda: synth_frame(1080, 1920, 5), 2000),
+}
+
+# (nfeatures, scaleFactor, nlevels) other than the reference's yaml, on synth_frame(480, 640, 31): oracle vs cv2
+LIVE_PARAMS = [(300, 1.5, 4), (400, 2.0, 3), (600, 1.1, 12), (500, 1.2, 1), (250, 2.5, 2)]
+
+# name -> (query factory, train factory) of the "realistic" match cases compared with cv2 (stored as match_live_<name>.npz)
+LIVE_MATCH_CASES = {
+    "1500x2000": (lambda: synth_map_queries(synth_descriptors(2000, 30), 1500, 31), lambda: synth_descriptors(2000, 30)),
+    "3000x2000": (lambda: synth_map_queries(synth_descriptors(2000, 1), 3000, 2), lambda: synth_descriptors(2000, 1)),
 }
 
 
@@ -64,3 +74,25 @@ MATCH_CASES = {
 
 def sha(a: np.ndarray) -> str:
     return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
+
+
+def _sample_rows(n: int, k: int = 32) -> np.ndarray:
+    return np.sort(np.random.default_rng(0).choice(n, min(n, k), replace=False)).astype(np.int64)
+
+
+def stored(**arrays) -> dict:
+    """What tools/make_golden_live.py keeps of each record array of a cv2 result: its row count, the sha256 of its bytes
+    and a fixed sample of its rows (the sample only names the differing rows when a comparison fails)."""
+    out = {}
+    for name, a in arrays.items():
+        rows = _sample_rows(len(a))
+        out.update({f"{name}_n": len(a), f"{name}_sha": sha(a), f"{name}_rows": rows, f"{name}_sample": a[rows]})
+    return out
+
+
+def assert_equals_stored(g, what: str, **arrays) -> None:
+    """Every array equals, byte for byte, the cv2 result `g` holds (a stored() record loaded from tests/golden/)."""
+    for name, a in arrays.items():
+        assert len(a) == int(g[f"{name}_n"]), f"{what}: {len(a)} {name} rows vs {int(g[f'{name}_n'])} from cv2"
+        bad = [int(r) for r, s in zip(g[f"{name}_rows"], g[f"{name}_sample"]) if np.asarray(a[r]).tobytes() != np.asarray(s).tobytes()]
+        assert sha(a) == str(g[f"{name}_sha"]), f"{what}: {name} differ from cv2's (sampled rows that differ: {bad})"

@@ -48,3 +48,43 @@ def test_orbx_arm_refuses_to_run_without_a_gpu():
     assert p.returncode != 0
     assert "no CPU fallback" in (p.stderr + p.stdout)
     assert not any(ln.strip().startswith("{") for ln in p.stdout.splitlines())
+
+
+def test_dump_outputs_writes_the_step_outputs_as_float_arrays(tmp_path):
+    """--dump-outputs: the buffers of a step (counts, keypoint records, descriptors, the two match record sets) become float32 /
+    float64 .npy files holding the same values; a batch whose outputs could exceed the 64 MiB budget is cut to a seeded sample
+    of frames that depends only on the buffer shapes."""
+    sys.path.insert(0, ROOT)
+    import numpy as np
+    import bench
+    rng = np.random.default_rng(3)
+    for nb, cap, m, dumped in ((5, 40, 64, 5), (256, 1280, 2048, 253)):
+        cnt = rng.integers(0, cap + 1, nb).astype(np.int32)
+        cnt[0] = 0
+        kps = rng.random((nb, cap, 7)).astype(np.float32)
+        kps[..., 5:].view(np.int32)[:] = rng.integers(-1, 8, (nb, cap, 2))
+        desc = rng.integers(0, 256, (nb, cap, 32), dtype=np.uint8)
+        best = rng.integers(-1, cap, (2, nb, m, 4)).astype(np.int32)
+        best[..., 3].view(np.float32)[:] = rng.integers(0, 257, (2, nb, m))
+        out = tmp_path / str(nb)
+        bench.dump_outputs(str(out), [cnt, kps, desc, best], False)
+        got = {p.stem: np.load(p) for p in out.iterdir()}
+        assert sorted(got) == ["counts", "descriptors", "frames", "keypoints", "matches"]
+        assert all(a.dtype in (np.float32, np.float64) for a in got.values())
+        assert sum(a.nbytes for a in got.values()) <= 64 << 20
+        fr = got["frames"].astype(np.int64)
+        assert len(fr) == dumped and np.array_equal(fr, np.unique(fr)) and fr.max() < nb
+        assert np.array_equal(got["counts"], cnt[fr])
+        rec = np.concatenate([kps[i, :cnt[i]] for i in fr])
+        assert np.array_equal(got["keypoints"][:, :5], rec[:, :5]) and np.array_equal(got["keypoints"][:, 5:], rec[:, 5:].view(np.int32))
+        assert np.array_equal(got["descriptors"], np.concatenate([desc[i, :cnt[i]] for i in fr]))
+        bf = best[:, fr]
+        assert np.array_equal(got["matches"][..., :3], bf[..., :3]) and np.array_equal(got["matches"][..., 3], bf[..., 3].view(np.float32))
+        bench.dump_outputs(str(out), [cnt, kps, desc, best], False)
+        assert np.array_equal(np.load(out / "frames.npy"), got["frames"])
+
+
+def test_steps_must_be_positive():
+    p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "0"], capture_output=True, text=True, cwd=ROOT,
+                       timeout=120)
+    assert p.returncode != 0 and "--steps" in p.stderr and not p.stdout.strip()

@@ -1,4 +1,4 @@
-"""GPU parity tests (run with -m gpu on the B200 box): the CUDA path, called through the C-ABI of liborbx.so,
+"""GPU parity tests (run with -m gpu on a B200): the CUDA path, called through the C-ABI of liborbx.so,
 against (a) the committed cv2 golden vectors, (b) the CPU oracle on the same seeded inputs, (c) cv2 itself when
 importable, and (d) size-independent properties at BASELINE.json's full sizes.
 
@@ -10,7 +10,7 @@ import os
 import numpy as np
 import pytest
 
-from cases import MATCH_CASES, ORB_CASES, ORB_CASES_LARGE
+from cases import LIVE_MATCH_CASES, MATCH_CASES, ORB_CASES, ORB_CASES_LARGE, assert_equals_stored, sha
 
 pytestmark = pytest.mark.gpu
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
@@ -386,16 +386,28 @@ def test_frontend_pattern(orbmod, oracle):
 
 
 def test_cv2_live_if_available(orbmod):
-    cv2 = pytest.importorskip("cv2")
+    """Against cv2's stored results (tests/golden/, tools/make_golden_live.py) always, and cv2 live when importable."""
+    try:
+        import cv2
+    except ImportError:
+        cv2 = None
     from oracle import oracle as O
-    from rgbd_visualodometry_b200.synth import synth_descriptors, synth_frame, synth_map_queries
+    from rgbd_visualodometry_b200.synth import synth_frame
     img = synth_frame(480, 640, 555)
+    g = np.load(os.path.join(GOLD, "orb_live555_1000.npz"))
+    assert sha(img) == str(g["img_sha"])
     k, d = orbmod.ORB_create(1000, 1.2, 8).detectAndCompute(img, None)
-    kc, dc = cv2.ORB_create(1000, 1.2, 8).detectAndCompute(img, None)
-    _assert_kp_equal(k, d, O.cv2_keypoints_to_array(kc), dc, "cv2 live")
-    t = synth_descriptors(2000, 1); q = synth_map_queries(t, 3000, 2)
+    assert_equals_stored(g, "ORB vs stored cv2", keypoints=k, descriptors=d)
+    if cv2 is not None:
+        kc, dc = cv2.ORB_create(1000, 1.2, 8).detectAndCompute(img, None)
+        _assert_kp_equal(k, d, O.cv2_keypoints_to_array(kc), dc, "cv2 live")
+    q, t = (f() for f in LIVE_MATCH_CASES["3000x2000"])
+    gm = np.load(os.path.join(GOLD, "match_live_3000x2000.npz"))
+    assert sha(q) == str(gm["q_sha"]) and sha(t) == str(gm["t_sha"])
     m = orbmod.BFMatcher(orbmod.NORM_HAMMING).match(q, t)
-    assert m.tobytes() == O.cv2_matches_to_array(cv2.BFMatcher(cv2.NORM_HAMMING).match(q, t)).tobytes()
+    assert_equals_stored(gm, "match vs stored cv2", match=m)
+    if cv2 is not None:
+        assert m.tobytes() == O.cv2_matches_to_array(cv2.BFMatcher(cv2.NORM_HAMMING).match(q, t)).tobytes()
 
 
 def test_orb_4k_5000(orbmod, oracle):

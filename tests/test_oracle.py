@@ -1,11 +1,11 @@
-"""Pins the CPU oracle (oracle/orb_oracle.c): against the committed cv2 golden vectors, against cv2 live
-(when importable) stage by stage, and through its own invariants.  CPU only."""
+"""Pins the CPU oracle (oracle/orb_oracle.c): against the committed cv2 golden vectors, stage by stage against the stored
+cv2 results (and cv2 live when importable), and through its own invariants.  CPU only."""
 import os
 
 import numpy as np
 import pytest
 
-from cases import MATCH_CASES, ORB_CASES, ORB_CASES_LARGE, sha
+from cases import LIVE_MATCH_CASES, LIVE_PARAMS, MATCH_CASES, ORB_CASES, ORB_CASES_LARGE, assert_equals_stored, sha
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
 
@@ -105,23 +105,33 @@ def test_retain_best_semantics(oracle):
             assert sorted(r["x"]) == sorted(keep["x"])
 
 
-@pytest.mark.skipif(cv2 is None, reason="cv2 not importable")
 class TestLiveCv2:
+    """The oracle against OpenCV's own operators: against the stored cv2 results always (tests/golden/, written by
+    tools/make_golden_live.py), and against cv2 live as well when it is importable."""
+
     def test_stages(self, oracle):
         from rgbd_visualodometry_b200.synth import synth_frame
+        gs = np.load(os.path.join(GOLD, "stages_701x467.npz"))
         img = synth_frame(467, 701, 21)
+        assert sha(img) == str(gs["img_sha"]), "synthetic generator drifted from the one that made the fixtures"
         g = oracle.gray(img)
-        assert np.array_equal(g, cv2.cvtColor(img, cv2.COLOR_BGR2GRAY))
+        assert sha(g) == str(gs["gray_sha"])
+        if cv2 is not None:
+            assert np.array_equal(g, cv2.cvtColor(img, cv2.COLOR_BGR2GRAY))
         ws, hs, _ = oracle.level_geometry(701, 467)
         prev = g
         for l in range(1, 8):
             cur = oracle.resize_exact(prev, ws[l], hs[l])
-            assert np.array_equal(cur, cv2.resize(prev, (ws[l], hs[l]), interpolation=cv2.INTER_LINEAR_EXACT)), l
+            assert sha(cur) == str(gs["level_sha"][l - 1]), l
+            if cv2 is not None:
+                assert np.array_equal(cur, cv2.resize(prev, (ws[l], hs[l]), interpolation=cv2.INTER_LINEAR_EXACT)), l
             prev = cur
-        f = cv2.FastFeatureDetector_create(20, True).detect(g)
         fo = oracle.fast_nms(g)
-        assert len(f) == len(fo)
-        assert all((int(a.pt[0]), int(a.pt[1]), a.response) == (int(b["x"]), int(b["y"]), float(b["response"])) for a, b in zip(f, fo))
+        assert_equals_stored(gs, "FAST", fast=fo)
+        if cv2 is not None:
+            f = cv2.FastFeatureDetector_create(20, True).detect(g)
+            assert len(f) == len(fo)
+            assert all((int(a.pt[0]), int(a.pt[1]), a.response) == (int(b["x"]), int(b["y"]), float(b["response"])) for a, b in zip(f, fo))
 
     def test_sincos_matches_libm(self, oracle):
         """orbo_sincosf restates glibc sinf/cosf; numpy's float32 sin/cos call the same libm here."""
@@ -140,24 +150,35 @@ class TestLiveCv2:
     def test_orb_large(self, oracle, name):
         mk, n = ORB_CASES_LARGE[name]
         img = mk()
-        k, d = cv2.ORB_create(n, 1.2, 8).detectAndCompute(img, None)
+        g = np.load(os.path.join(GOLD, f"orb_{name}.npz"))
+        assert sha(img) == str(g["img_sha"]), "synthetic generator drifted from the one that made the fixtures"
         ko, do = oracle.detect_and_compute(img, n)
-        assert ko.tobytes() == oracle.cv2_keypoints_to_array(k).tobytes() and np.array_equal(d, do)
+        assert_equals_stored(g, f"oracle {name}", keypoints=ko, descriptors=do)
+        if cv2 is not None:
+            k, d = cv2.ORB_create(n, 1.2, 8).detectAndCompute(img, None)
+            assert ko.tobytes() == oracle.cv2_keypoints_to_array(k).tobytes() and np.array_equal(d, do)
 
     def test_match_live(self, oracle):
-        from rgbd_visualodometry_b200.synth import synth_descriptors, synth_map_queries
-        t = synth_descriptors(2000, 30)
-        q = synth_map_queries(t, 1500, 31)
-        m = cv2.BFMatcher(cv2.NORM_HAMMING).match(q, t)
-        assert oracle.match_hamming(q, t).tobytes() == oracle.cv2_matches_to_array(m).tobytes()
+        q, t = (f() for f in LIVE_MATCH_CASES["1500x2000"])
+        g = np.load(os.path.join(GOLD, "match_live_1500x2000.npz"))
+        assert sha(q) == str(g["q_sha"]) and sha(t) == str(g["t_sha"])
+        mo = oracle.match_hamming(q, t)
+        assert_equals_stored(g, "oracle match", match=mo)
+        if cv2 is not None:
+            m = cv2.BFMatcher(cv2.NORM_HAMMING).match(q, t)
+            assert mo.tobytes() == oracle.cv2_matches_to_array(m).tobytes()
 
 
-@pytest.mark.skipif(cv2 is None, reason="cv2 not importable")
-@pytest.mark.parametrize("params", [(300, 1.5, 4), (400, 2.0, 3), (600, 1.1, 12), (500, 1.2, 1), (250, 2.5, 2)])
+@pytest.mark.parametrize("params", LIVE_PARAMS)
 def test_oracle_other_parameters_vs_cv2_live(oracle, params):
+    """Stored cv2 result always; cv2 live as well when importable."""
     from rgbd_visualodometry_b200.synth import synth_frame
     n, sf, nl = params
     img = synth_frame(480, 640, 31)
+    g = np.load(os.path.join(GOLD, f"orb_params_{n}_{sf}_{nl}.npz"))
+    assert sha(img) == str(g["img_sha"])
     k, d = oracle.detect_and_compute(img, n, sf, nl)
-    kc, dc = cv2.ORB_create(n, sf, nl).detectAndCompute(img, None)
-    assert k.tobytes() == oracle.cv2_keypoints_to_array(kc).tobytes() and np.array_equal(d, dc)
+    assert_equals_stored(g, f"oracle ORB({n}, {sf}, {nl})", keypoints=k, descriptors=d)
+    if cv2 is not None:
+        kc, dc = cv2.ORB_create(n, sf, nl).detectAndCompute(img, None)
+        assert k.tobytes() == oracle.cv2_keypoints_to_array(kc).tobytes() and np.array_equal(d, dc)

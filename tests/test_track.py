@@ -174,8 +174,9 @@ def test_async_submit_collect_equals_sync_and_feeds_tracking(orbmod):
 @pytest.mark.gpu
 def test_tracking_loop_orbx_equals_cv2_frontend():
     """BASELINE config 1 in miniature (tools/run_vo_synth.py): the reference's tracking loop on a synthetic RGB-D sequence with
-    the hot path behind the orbx C-ABI vs the same loop with cv2's operators: identical keypoint / match / inlier counts and
-    poses frame by frame, and the trajectory within millimetres of the ground truth."""
+    the hot path behind the orbx C-ABI vs the same loop with cv2's operators (live, and as stored in tests/golden/ by
+    tools/make_golden_live.py): identical keypoint / match / inlier counts and poses frame by frame, and the trajectory
+    within millimetres of the ground truth.  Both loops solve PnP with cv2.solvePnPRansac, so this test needs cv2."""
     cv2 = pytest.importorskip("cv2")
     import importlib.util, os
     spec = importlib.util.spec_from_file_location("run_vo_synth", os.path.join(os.path.dirname(__file__), "..", "tools", "run_vo_synth.py"))
@@ -188,6 +189,10 @@ def test_tracking_loop_orbx_equals_cv2_frontend():
     for x, y in zip(a, b):
         assert x[1:4] == y[1:4], (x[:4], y[:4])
         assert np.allclose(x[4], y[4], atol=1e-9)
+    g = np.load(os.path.join(os.path.dirname(__file__), "golden", "vo_synth16_cv2.npz"))
+    assert [list(x[:4]) for x in a] == g["counts"].tolist()
+    assert np.allclose([x[5] for x in a], g["truth"], atol=1e-12)
+    assert np.allclose([x[4] for x in a], g["centre"], atol=1e-6)      # metres; PnP runs on this host's cv2 build
     err = max(np.linalg.norm(x[4] - x[5]) for x in a)
     assert err < 0.01, err                                   # metres; 1 px at 2 m is ~3.9 mm
     assert min(x[3] for x in a[1:]) >= 30                    # PnP inliers
