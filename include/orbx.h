@@ -210,8 +210,6 @@ int orbx_debug_read_fast(orbx_ctx* ctx, int frame, int level, int32_t* x, int32_
 /* Average device time (ms) of each pipeline stage over the last extraction / match call, measured with CUDA
  * events on the context's stream; names[i] are static strings.  Returns the number of stages written. */
 int orbx_debug_stage_times(orbx_ctx* ctx, const char** names, float* ms, int cap);
-/* Matcher pipeline trace (only when the environment variable ORBX_MATCH_TRACE is set): 16 tiles x 16 SM-clock stamps. */
-int orbx_debug_match_trace(orbx_ctx* ctx, long long* out);
 /* Pyramid, FAST and selection exist as two kernel families with identical results: warp-private kernels (pyramid / FAST:
  * TMA-fed, chosen for launches of about 26 VGA frames' worth of pixels and more; selection: one warp per (frame, level), chosen
  * for frames up to about 0.6 Mpixel) and CTA-cooperative kernels with the shorter critical path (smaller launches, e.g. the

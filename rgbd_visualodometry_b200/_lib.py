@@ -88,7 +88,6 @@ SYMBOLS = {
     "orbx_debug_read_level": (C.c_int, [_P, C.c_int, C.c_int, _P, C.c_size_t]),
     "orbx_debug_read_fast": (C.c_int, [_P, C.c_int, C.c_int, _P, _P, _P, C.c_int, C.POINTER(C.c_int)]),
     "orbx_debug_stage_times": (C.c_int, [_P, C.POINTER(C.c_char_p), C.POINTER(C.c_float), C.c_int]),
-    "orbx_debug_match_trace": (C.c_int, [_P, _P]),
     "orbx_debug_force_kernels": (C.c_int, [_P, C.c_int]),
     "orbx_set_profiling": (C.c_int, [_P, C.c_int]),
 }

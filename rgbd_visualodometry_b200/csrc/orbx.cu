@@ -39,10 +39,10 @@ const int8_t k_pattern_host[256 * 4] = {
 constexpr int FAST_R = 16, FAST_NT = 256;
 constexpr int FAST_NWARP = 4;             // warps per CTA of k_fast_warp (independent units; 7 CTAs per SM by shared memory)
 static_assert(FAST_R == FW_R, "band height");
-constexpr int MAX_LANES = 4;               // concurrent frame-range pipelines of one device-resident extraction call
-constexpr int HOST_MAX_LANES = 12, HOST_DEFAULT_LANES = 8;         // host-buffer calls: more, shorter ranges shrink the un-overlapped head (first upload) and tail
-constexpr int LANE_MIN_FRAMES = 64;        // a lane must still fill the GPU on its own
+constexpr int HOST_LANES = 8;              // host-buffer calls: more, shorter ranges shrink the un-overlapped head (first upload) and tail
 constexpr int HOST_LANE_MIN_FRAMES = 16;   // host-buffer batches: lanes mainly overlap PCIe copies with kernels
+constexpr long SIDE_LEVEL_MAX_PX = 100000; // pyramid levels (from level 2 on) below this many pixels run on the side stream
+constexpr size_t STAGE_WAKE_BYTES = (size_t)2 << 20;   // staged copies of at least this many bytes wake the copier threads
 constexpr int N_STAGES = 7;
 const char* const k_stage_names[N_STAGES] = {"gray", "pyramid", "fast_nms", "select_harris", "blur", "describe", "match"};
 
@@ -88,7 +88,7 @@ struct orbx_ctx {
     const uint8_t* view_desc = nullptr;      // device descriptors / counts of the frames the last host call (or collect) produced
     const int* view_counts = nullptr;
     int view_frames = 0;
-    Buf mq, mt, mbest, msecond, mkeys, mstatus, mcounts, mtrace;
+    Buf mq, mt, mbest, msecond, mkeys, mstatus, mcounts;
     int* h_small = nullptr;                  // pinned: counts[max_batch] + status[max_batch] + 1
     uint8_t* h_stage_in = nullptr; size_t h_stage_in_bytes = 0;     // pinned staging of pageable caller frames (device layout)
     uint8_t* h_stage_out = nullptr; size_t h_stage_out_bytes = 0;   // ... of results bound for pageable caller buffers
@@ -117,10 +117,10 @@ struct orbx_ctx {
     bool profiling = false;
     int force_kernels = -1;                   // orbx_debug_force_kernels: -1 by launch size, 0 warp-private TMA kernels, 1 CTA-cooperative kernels
     cudaEvent_t ev[N_STAGES + 2] = {};   // 0..6 bracket the six extraction stages, 7..8 the matcher
-    cudaStream_t lane[HOST_MAX_LANES] = {};   // extra frame-range pipelines (lane 0 is `stream`)
-    cudaStream_t side[HOST_MAX_LANES] = {};   // per lane: high-priority stream of the small pyramid levels + their FAST bands
-    cudaEvent_t ev_sfork[HOST_MAX_LANES] = {}, ev_sjoin[HOST_MAX_LANES] = {};
-    cudaEvent_t ev_fork = nullptr, ev_join[HOST_MAX_LANES] = {};
+    cudaStream_t lane[HOST_LANES] = {};   // extra frame-range pipelines (lane 0 is `stream`)
+    cudaStream_t side[HOST_LANES] = {};   // per lane: high-priority stream of the small pyramid levels + their FAST bands
+    cudaEvent_t ev_sfork[HOST_LANES] = {}, ev_sjoin[HOST_LANES] = {};
+    cudaEvent_t ev_fork = nullptr, ev_join[HOST_LANES] = {};
     float stage_ms[N_STAGES] = {};
     bool stage_valid[N_STAGES] = {};
 };
@@ -410,17 +410,14 @@ int run_extract_range(orbx_ctx* c, cudaStream_t st, int lane_id, bool marks, int
     // Kernel choice by the size of the launch: the warp-private TMA kernels (one warp walks a whole band / a stack of strips)
     // win once there are enough warps to fill the GPU; below about 26 VGA frames' worth of pixels the CTA-cooperative
     // kernels have the shorter critical path (one 640x480 frame: pyramid + FAST 0.077 ms against 0.115 ms), which is what the
-    // sequential VO loop (one frame per call, src/frontend.cpp:98-108) feels.  ORBX_*_OLD = 1 / 0 forces one or the other.
+    // sequential VO loop (one frame per call, src/frontend.cpp:98-108) feels.  orbx_debug_force_kernels pins one or the other.
     const bool small_launch = (long)nb * g.w * g.h < 8000000L;
-    static const int env_old_pyr = getenv("ORBX_PYR_OLD") ? atoi(getenv("ORBX_PYR_OLD")) : -1;
-    static const int env_old_fast = getenv("ORBX_FAST_OLD") ? atoi(getenv("ORBX_FAST_OLD")) : -1;
-    const bool old_pyr = c->force_kernels >= 0 ? c->force_kernels != 0 : env_old_pyr >= 0 ? env_old_pyr != 0 : small_launch;
-    const bool old_fast = c->force_kernels >= 0 ? c->force_kernels != 0 : env_old_fast >= 0 ? env_old_fast != 0 : small_launch;
+    const bool old_pyr_fast = c->force_kernels >= 0 ? c->force_kernels != 0 : small_launch;
     auto launch_pyr = [&](int l, cudaStream_t s) {
         if (g.L[l].w <= 0 || g.L[l].h <= 0) return;
         const int nitems = (g.L[l].pitch / 8) * ((g.L[l].h + PYR_RH - 1) / PYR_RH);     // (column octet, row strip) work items
         const dim3 grd((unsigned)((nitems + PYR_NT - 1) / PYR_NT), B);
-        if (g.L[l].pt_ok && !old_pyr)
+        if (g.L[l].pt_ok && !old_pyr_fast)
             k_pyr_tma<<<dim3((unsigned)((g.L[l].pt_ntask + PT_NWARP - 1) / PT_NWARP), B), PT_NWARP * 32,
                         PT_NWARP * pt_warp_bytes(g.L[l].pt_bw, g.L[l].pt_bh) + 128, s>>>(g, c->pmaps.m[l], l, f0, (uint8_t*)c->pyr.p, tabs, status);
         else if (g.L[l].xspan <= 7) k_pyr_down<false><<<grd, PYR_NT, 0, s>>>(g, l, pyr, tabs);
@@ -430,11 +427,10 @@ int run_extract_range(orbx_ctx* c, cudaStream_t st, int lane_id, bool marks, int
     // The blur (FMA-pipe-bound, needs only the pyramid) follows the small levels on the side stream, i.e. it also runs under the
     // large levels' FAST launch (ALU-pipe-bound): 0.959 -> 0.944 ms per 256 VGA frames.  Capping the occupancy of either kernel
     // so that both are resident in fixed proportions was measured and loses (FAST needs its 7 CTAs per SM).
-    static const int env_co = getenv("ORBX_CO") ? atoi(getenv("ORBX_CO")) : 1;
     bool blur_done = false;
     auto launch_fast = [&](int band_lo, int band_hi, cudaStream_t s) {
         if (band_hi <= band_lo) return;
-        if (old_fast) {
+        if (old_pyr_fast) {
             if (band_lo == 0) k_fast_bands<FAST_R, FAST_NT><<<dim3((unsigned)g.total_bands, B), FAST_NT, 0, s>>>(g, pyr, rowcnt, rowent);
         } else
             k_fast_warp<FAST_NWARP><<<dim3((unsigned)((band_hi - band_lo + FAST_NWARP - 1) / FAST_NWARP), B), FAST_NWARP * 32, FAST_NWARP * FW_WARP_BYTES + 128, s>>>(
@@ -446,11 +442,8 @@ int run_extract_range(orbx_ctx* c, cudaStream_t st, int lane_id, bool marks, int
     // those levels run on a HIGH-PRIORITY side stream (their few CTAs take the next free slots) underneath the FAST launch of the
     // large levels, which is issue-bound and has slots to spare for them only in time, not in space.
     int lt = g.nlevels;                                      // first level of the side chain
-    {
-        static const int tail_px = getenv("ORBX_TAIL_PX") ? atoi(getenv("ORBX_TAIL_PX")) : 100000;   // levels below this many pixels are "small"; 0: no side chain
-        for (int l = g.nlevels - 1; l >= 2 && (long)g.L[l].w * g.L[l].h < tail_px; --l) lt = l;
-        if (old_fast || g.total_bands <= 0 || marks) lt = g.nlevels;   // (stage timers on: one stream, clean per-stage times)
-    }
+    for (int l = g.nlevels - 1; l >= 2 && (long)g.L[l].w * g.L[l].h < SIDE_LEVEL_MAX_PX; --l) lt = l;
+    if (old_pyr_fast || g.total_bands <= 0 || marks) lt = g.nlevels;   // (stage timers on: one stream, clean per-stage times)
     nv.next("orbx:pyramid");
     for (int l = 1; l < lt; ++l) launch_pyr(l, st);
     if (marks) stage_mark(c, 2);
@@ -460,7 +453,7 @@ int run_extract_range(orbx_ctx* c, cudaStream_t st, int lane_id, bool marks, int
         CU(cudaStreamWaitEvent(side, side_fork, 0));
         for (int l = lt; l < g.nlevels; ++l) launch_pyr(l, side);
         launch_fast(g.L[lt].band0, g.total_bands, side);
-        if (env_co && g.total_blur > 0) {
+        if (g.total_blur > 0) {
             k_blur<<<dim3((unsigned)g.total_blur, B), BLUR_NT, 0, side>>>(g, pyr, blur);
             ++c->launches; blur_done = true;
         }
@@ -470,64 +463,41 @@ int run_extract_range(orbx_ctx* c, cudaStream_t st, int lane_id, bool marks, int
     } else if (g.total_bands > 0) launch_fast(0, g.total_bands, st);
     nv.next("orbx:select_harris");
     if (marks) stage_mark(c, 3);
-    // Experiment kept behind ORBX_OVERLAP=1 (and only when the blur did not already go to the side stream): the selection (three
-    // launches of single-warp work per (frame, level), latency-bound) on the high-priority side stream UNDER the blur, which needs
-    // only the pyramid.  Measured slower than the sequential order (0.983 ms against 0.962 ms per 256 VGA frames): the selection's
-    // dependent launches wait for slots the blur's CTAs hold.
-    static const int env_overlap = getenv("ORBX_OVERLAP") ? atoi(getenv("ORBX_OVERLAP")) : 0;
-    const bool overlap_sel = env_overlap && !marks && g.total_blur > 0 && !blur_done;
-    cudaStream_t ss = overlap_sel ? side : st;
-    if (overlap_sel) { CU(cudaEventRecord(side_fork, st)); CU(cudaStreamWaitEvent(side, side_fork, 0)); }
     {
         // Selection kernel family by problem size: one WARP per (frame, level) when the candidate lists are short and there are
         // thousands of them (256 VGA frames: 0.116 ms against 0.17 ms), one CTA per (frame, level) when the lists are long -- 512
         // threads wide there (64 frames of 1920x1080: 0.30 ms against 0.43 ms with 128 threads and 0.65 ms with warps;
         // 3840x2160: 1.21 against 1.88 and 2.57 ms).
-        static const int env_old_sel = getenv("ORBX_SELECT_OLD") ? atoi(getenv("ORBX_SELECT_OLD")) : -1;
-        const bool old_sel = c->force_kernels >= 0 ? c->force_kernels != 0 : env_old_sel >= 0 ? env_old_sel != 0 : (long)g.w * g.h > 600000L;
-        static const int env_sel_nt = getenv("ORBX_SELECT_NT") ? atoi(getenv("ORBX_SELECT_NT")) : 0;   // A/B timing only
-        const bool wide = env_sel_nt ? env_sel_nt > SEL_NT : (long)g.w * g.h > 600000L;
+        const bool wide = (long)g.w * g.h > 600000L;
+        const bool old_sel = c->force_kernels >= 0 ? c->force_kernels != 0 : wide;
         if (old_sel) {
-            if (wide) k_select<SEL_NT_WIDE><<<dim3(B, (unsigned)g.nlevels), SEL_NT_WIDE, 0, ss>>>(g, pyr, rowcnt, rowent, work, selpos, fincnt, status);
-            else      k_select<SEL_NT><<<dim3(B, (unsigned)g.nlevels), SEL_NT, 0, ss>>>(g, pyr, rowcnt, rowent, work, selpos, fincnt, status);
+            if (wide) k_select<SEL_NT_WIDE><<<dim3(B, (unsigned)g.nlevels), SEL_NT_WIDE, 0, st>>>(g, pyr, rowcnt, rowent, work, selpos, fincnt, status);
+            else      k_select<SEL_NT><<<dim3(B, (unsigned)g.nlevels), SEL_NT, 0, st>>>(g, pyr, rowcnt, rowent, work, selpos, fincnt, status);
             ++c->launches;
         }
         else {
             // (the warp going straight on to Harris and the second retainBest -- one launch instead of three -- was measured: 0.1435 ms
             //  against 0.1159 ms per 256 VGA frames; the 14 serial Harris evaluations per lane cost the level-0 warps more than the
             //  two launch gaps and the Harris kernel's tail)
-            static const int env_fused = getenv("ORBX_SELECT_FUSED") ? atoi(getenv("ORBX_SELECT_FUSED")) : 0;
-            if (env_fused) {
-                k_select_fast<true><<<dim3(B, (unsigned)g.nlevels), 32, 0, ss>>>(g, pyr, rowcnt, rowent, work, selpos, selcnt, fincnt);
-                ++c->launches;
-            } else {
-                k_select_fast<false><<<dim3(B, (unsigned)g.nlevels), 32, 0, ss>>>(g, pyr, rowcnt, rowent, work, selpos, selcnt, fincnt);
-                if (g.total_hblk > 0) k_harris<<<dim3((unsigned)g.total_hblk, B), HARRIS_NT, 0, ss>>>(g, pyr, work, selcnt);
-                k_select_harris<<<dim3(B, (unsigned)g.nlevels), 32, (size_t)g.selh_elems * 12, ss>>>(g, work, selpos, selcnt, fincnt, g.selh_elems);
-                c->launches += 3;
-            }
+            k_select_fast<<<dim3(B, (unsigned)g.nlevels), 32, 0, st>>>(g, rowcnt, rowent, work, selpos, selcnt, fincnt);
+            if (g.total_hblk > 0) k_harris<<<dim3((unsigned)g.total_hblk, B), HARRIS_NT, 0, st>>>(g, pyr, work, selcnt);
+            k_select_harris<<<dim3(B, (unsigned)g.nlevels), 32, (size_t)g.selh_elems * 12, st>>>(g, work, selpos, selcnt, fincnt, g.selh_elems);
+            c->launches += 3;
         }
     }
-    if (overlap_sel) CU(cudaEventRecord(side_join, side));
     nv.next("orbx:blur");
     if (marks) stage_mark(c, 4);
     if (g.total_blur > 0 && !blur_done) {
         k_blur<<<dim3((unsigned)g.total_blur, B), BLUR_NT, 0, st>>>(g, pyr, blur);
         ++c->launches;
     }
-    if (overlap_sel) CU(cudaStreamWaitEvent(st, side_join, 0));
     nv.next("orbx:describe");
     if (marks) stage_mark(c, 5);
-    static const int old_desc = getenv("ORBX_DESC_OLD") ? atoi(getenv("ORBX_DESC_OLD")) : 0;   // A/B timing only
-    if (old_desc)
-        k_describe<<<dim3((unsigned)((std::max(cap, 1) + DESC_KPB * DESC_KPW - 1) / (DESC_KPB * DESC_KPW)), B), DESC_NT, 0, st>>>(
-            g, pyr, blur, work, fincnt, (const float4*)c->pattern.p, d_kps, d_desc, d_counts, cap);
-    else {
+    {
         // groups of 4 slots per warp: four per warp when the batch is large (the warp's set-up is shared, and there are still
         // enough CTAs for several waves), one group per warp (lowest latency) when it is a single frame
-        static const int env_gpw = getenv("ORBX_DESC_GPW") ? atoi(getenv("ORBX_DESC_GPW")) : 0;
         const long groups = (long)nb * ((std::min(std::max(cap, 1), std::max(c->nfeatures, 1)) + DS_G - 1) / DS_G);
-        const int gpw = env_gpw > 0 ? std::min(env_gpw, DS_MAX_GPW) : (groups >= 148L * 24 * 8 ? 4 : 1);   // measured at 256 VGA frames: 1 / 2 / 4 / 8 / 16 -> 0.192 / 0.192 / 0.185 / 0.205 / 0.259 ms
+        const int gpw = groups >= 148L * 24 * 8 ? 4 : 1;   // measured at 256 VGA frames: 1 / 2 / 4 / 8 / 16 -> 0.192 / 0.192 / 0.185 / 0.205 / 0.259 ms
         const int gcap = (std::max(cap, 1) + DS_G - 1) / DS_G;
         k_describe_tma<<<dim3((unsigned)((gcap + DS_NW * gpw - 1) / (DS_NW * gpw)), B), DS_NW * 32, DS_NW * DS_WARP_BYTES + 128, st>>>(
             g, c->dmaps, f0, work, fincnt, (const float4*)c->pattern.p, d_kps, d_desc, d_counts, cap, gpw, status);
@@ -537,36 +507,16 @@ int run_extract_range(orbx_ctx* c, cudaStream_t st, int lane_id, bool marks, int
     return ORBX_OK;
 }
 
-// The extraction pipeline on device-resident frames; everything asynchronous, ordered on c->stream.
-// Large batches are cut into `lanes` frame ranges that run the same kernel sequence on their own streams: the stages
-// bound differently (FAST issue-bound, pyramid / selection / describe latency-bound), so CTAs of different stages
-// from different lanes share the SMs and fill each other's stalls.  Frames are independent, so no lane ever waits
-// for another; the lanes fork from and join back into c->stream with events.
+// The extraction pipeline on device-resident frames; everything asynchronous, ordered on c->stream.  One frame range:
+// every kernel fills the GPU on its own (cutting the batch into concurrent frame ranges measured 4 % slower with 3 ranges).
 int run_extract(orbx_ctx* c, const uint8_t* d_imgs, int batch, int w, int h, size_t step, size_t frame_stride, int channels,
                 float* d_kps, uint8_t* d_desc, int cap, int* d_counts)
 {
     int rc = set_geometry(c, w, h);
     if (rc) return rc;
     CU(cudaMemsetAsync(c->status.p, 0, sizeof(int) * (size_t)batch, c->stream));
-    static const int env_lanes = getenv("ORBX_LANES") ? atoi(getenv("ORBX_LANES")) : 1;   // 1: every kernel fills the GPU on its own now (3 lanes measured 4 % slower)
-    int lanes = std::max(1, std::min(env_lanes, MAX_LANES));
-    if (batch < lanes * LANE_MIN_FRAMES) lanes = 1;
-    if (c->profiling) lanes = 1;
-    if (lanes == 1) {
-        rc = run_extract_range(c, c->stream, 0, c->profiling, 0, batch, d_imgs, step,
-                               frame_stride, channels, d_kps, d_desc, cap, d_counts);
-        if (rc) return rc;
-    } else {
-        CU(cudaEventRecord(c->ev_fork, c->stream));
-        for (int k = 0; k < lanes; ++k) {
-            const int f0 = (int)((long)batch * k / lanes), f1 = (int)((long)batch * (k + 1) / lanes);
-            cudaStream_t st = k == 0 ? c->stream : c->lane[k];
-            if (k > 0) CU(cudaStreamWaitEvent(st, c->ev_fork, 0));
-            rc = run_extract_range(c, st, k, false, f0, f1 - f0, d_imgs, step, frame_stride, channels, d_kps, d_desc, cap, d_counts);
-            if (rc) return rc;
-            if (k > 0) { CU(cudaEventRecord(c->ev_join[k], st)); CU(cudaStreamWaitEvent(c->stream, c->ev_join[k], 0)); }
-        }
-    }
+    if ((rc = run_extract_range(c, c->stream, 0, c->profiling, 0, batch, d_imgs, step, frame_stride, channels, d_kps, d_desc, cap, d_counts)))
+        return rc;
     CU(cudaGetLastError());
     c->last_batch = batch;
     if (c->profiling) for (int i = 0; i < 6; ++i) c->stage_valid[i] = true;
@@ -624,10 +574,8 @@ int run_match(orbx_ctx* c, const uint8_t* d_q, int nq, const uint8_t* d_t, int n
     const bool knn2 = d_second != nullptr;
     // CTA-pair kernel (tcgen05 cta_group::2, query tiles in twos) whenever the (query tile, set) pairs alone fill the GPU;
     // small problems keep the single-CTA kernel, whose CTAs are independent units for the train-row split.
-    // ORBX_MATCH_2CTA = 0 / 1 forces one of them (experiments).
-    static const int pair_env = getenv("ORBX_MATCH_2CTA") ? atoi(getenv("ORBX_MATCH_2CTA")) : -1;
     const int tiles_1 = (nq + MT_QROWS - 1) / MT_QROWS, tiles_2 = (tiles_1 + 1) & ~1;
-    const bool pair = pair_env >= 0 ? pair_env != 0 : (tiles_1 >= 2 && (long)tiles_2 * nsets >= 148);
+    const bool pair = tiles_1 >= 2 && (long)tiles_2 * nsets >= 148;
     const int tiles_m = pair ? tiles_2 : tiles_1;
     const int ntile_n = (nt + MT_BN - 1) / MT_BN;
     constexpr int kSMs = 148;                                // one CTA per SM (163 KB of shared memory each)
@@ -667,12 +615,10 @@ int run_match(orbx_ctx* c, const uint8_t* d_q, int nq, const uint8_t* d_t, int n
         ++c->launches;
     }
     const dim3 grd((unsigned)tiles_m, (unsigned)nsplit, (unsigned)zgroups);
-    if (getenv("ORBX_MATCH_TRACE") && !c->mtrace.p) { if ((rc = ensure(c, c->mtrace, 16 * 16 * 8))) return rc; cudaMemset(c->mtrace.p, 0, 16 * 16 * 8); }
-    static const int dbg = getenv("ORBX_MATCH_DBG") ? atoi(getenv("ORBX_MATCH_DBG")) : 0;   // perf experiments only: skips a role's work (wrong results)
-    if (pair && knn2) k_hamming_umma2<true><<<grd, MT_THREADS, MT_SMEM_BYTES, st>>>(d_q, nq, d_t, nt, stride_rows, d_counts, nsets, rows_per_split, d_best, d_second, keys, d_status, dbg, (long long*)c->mtrace.p);
-    else if (pair) k_hamming_umma2<false><<<grd, MT_THREADS, MT_SMEM_BYTES, st>>>(d_q, nq, d_t, nt, stride_rows, d_counts, nsets, rows_per_split, d_best, d_second, keys, d_status, dbg, (long long*)c->mtrace.p);
-    else if (knn2) k_hamming_umma<true><<<grd, MT_THREADS, MT_SMEM_BYTES, st>>>(d_q, nq, d_t, nt, stride_rows, d_counts, nsets, rows_per_split, d_best, d_second, keys, d_status, dbg, (long long*)c->mtrace.p);
-    else      k_hamming_umma<false><<<grd, MT_THREADS, MT_SMEM_BYTES, st>>>(d_q, nq, d_t, nt, stride_rows, d_counts, nsets, rows_per_split, d_best, d_second, keys, d_status, dbg, (long long*)c->mtrace.p);
+    if (pair && knn2) k_hamming_umma2<true><<<grd, MT_THREADS, MT_SMEM_BYTES, st>>>(d_q, nq, d_t, nt, stride_rows, d_counts, nsets, rows_per_split, d_best, d_second, keys, d_status);
+    else if (pair) k_hamming_umma2<false><<<grd, MT_THREADS, MT_SMEM_BYTES, st>>>(d_q, nq, d_t, nt, stride_rows, d_counts, nsets, rows_per_split, d_best, d_second, keys, d_status);
+    else if (knn2) k_hamming_umma<true><<<grd, MT_THREADS, MT_SMEM_BYTES, st>>>(d_q, nq, d_t, nt, stride_rows, d_counts, nsets, rows_per_split, d_best, d_second, keys, d_status);
+    else      k_hamming_umma<false><<<grd, MT_THREADS, MT_SMEM_BYTES, st>>>(d_q, nq, d_t, nt, stride_rows, d_counts, nsets, rows_per_split, d_best, d_second, keys, d_status);
     ++c->launches;
     if (nsplit > 1) {
         k_match_finalize<<<(unsigned)((nout + 255) / 256), 256, 0, st>>>(keys, nq, nout, d_best);
@@ -738,13 +684,13 @@ int orbx_create(orbx_ctx** out, int device, int nfeatures, float scale_factor, i
     if (cudaGetDeviceProperties(&prop, device) != cudaSuccess) return bail(ORBX_E_CUDA);
     if (prop.major != 10) return bail(ORBX_E_CUDA);          // sm_100a only: no other code path exists
     if (cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking) != cudaSuccess) return bail(ORBX_E_CUDA);
-    for (int k = 0; k < HOST_MAX_LANES; ++k)
+    for (int k = 0; k < HOST_LANES; ++k)
         if ((k > 0 && cudaStreamCreateWithFlags(&c->lane[k], cudaStreamNonBlocking) != cudaSuccess) || cudaEventCreateWithFlags(&c->ev_join[k], cudaEventDisableTiming) != cudaSuccess) return bail(ORBX_E_CUDA);
     if (cudaEventCreateWithFlags(&c->ev_fork, cudaEventDisableTiming) != cudaSuccess) return bail(ORBX_E_CUDA);
     {
         int prio_lo = 0, prio_hi = 0;
         if (cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi) != cudaSuccess) return bail(ORBX_E_CUDA);
-        for (int k = 0; k < HOST_MAX_LANES; ++k)
+        for (int k = 0; k < HOST_LANES; ++k)
             if (cudaStreamCreateWithPriority(&c->side[k], cudaStreamNonBlocking, prio_hi) != cudaSuccess ||
                 cudaEventCreateWithFlags(&c->ev_sfork[k], cudaEventDisableTiming) != cudaSuccess ||
                 cudaEventCreateWithFlags(&c->ev_sjoin[k], cudaEventDisableTiming) != cudaSuccess) return bail(ORBX_E_CUDA);
@@ -761,7 +707,7 @@ int orbx_create(orbx_ctx** out, int device, int nfeatures, float scale_factor, i
     if (cudaMemset(c->mstatus.p, 0, sizeof(int) * 16) != cudaSuccess) return bail(ORBX_E_CUDA);
     {
         float pat[1024];                                     // the rBRIEF pattern as float4 (x0, y0, x1, y1) per test,
-        for (int t = 0; t < 8; ++t)                          // transposed to [t][lane]: test lane * 8 + t  (k_describe)
+        for (int t = 0; t < 8; ++t)                          // transposed to [t][lane]: test lane * 8 + t  (k_describe_tma)
             for (int lane = 0; lane < 32; ++lane)
                 for (int k = 0; k < 4; ++k) pat[(t * 32 + lane) * 4 + k] = (float)k_pattern_host[(lane * 8 + t) * 4 + k];
         if (cudaMemcpy(c->pattern.p, pat, sizeof pat, cudaMemcpyHostToDevice) != cudaSuccess) return bail(ORBX_E_CUDA);
@@ -787,7 +733,7 @@ void orbx_destroy(orbx_ctx* c)
     cudaSetDevice(c->device);
     if (c->stream) cudaStreamSynchronize(c->stream);
     Buf* bufs[] = {&c->pyr, &c->blur, &c->rowcnt, &c->rowent, &c->work, &c->selpos, &c->fincnt, &c->selcnt, &c->status, &c->tabs, &c->pattern, &c->in, &c->kps,
-                   &c->desc, &c->counts, &c->mq, &c->mt, &c->mbest, &c->msecond, &c->mkeys, &c->mstatus, &c->mcounts, &c->mtrace,
+                   &c->desc, &c->counts, &c->mq, &c->mt, &c->mbest, &c->msecond, &c->mkeys, &c->mstatus, &c->mcounts,
                    &c->t_desc, &c->t_pos, &c->t_nrm, &c->t_outl, &c->t_slots, &c->t_cand, &c->t_ncand, &c->t_q, &c->t_in, &c->t_best, &c->t_filtered,
                    &c->t_minmax, &c->t_aux};
     for (Buf* b : bufs) if (b->p) cudaFree(b->p);
@@ -803,9 +749,9 @@ void orbx_destroy(orbx_ctx* c)
         if (a.done) cudaEventDestroy(a.done);
     }
     for (int i = 0; i < N_STAGES + 2; ++i) if (c->ev[i]) cudaEventDestroy(c->ev[i]);
-    for (int k = 0; k < HOST_MAX_LANES; ++k) { if (c->ev_join[k]) cudaEventDestroy(c->ev_join[k]); if (c->lane[k]) { cudaStreamSynchronize(c->lane[k]); cudaStreamDestroy(c->lane[k]); } }
+    for (int k = 0; k < HOST_LANES; ++k) { if (c->ev_join[k]) cudaEventDestroy(c->ev_join[k]); if (c->lane[k]) { cudaStreamSynchronize(c->lane[k]); cudaStreamDestroy(c->lane[k]); } }
     if (c->ev_fork) cudaEventDestroy(c->ev_fork);
-    for (int k = 0; k < HOST_MAX_LANES; ++k) {
+    for (int k = 0; k < HOST_LANES; ++k) {
         if (c->side[k]) { cudaStreamSynchronize(c->side[k]); cudaStreamDestroy(c->side[k]); }
         if (c->ev_sfork[k]) cudaEventDestroy(c->ev_sfork[k]);
         if (c->ev_sjoin[k]) cudaEventDestroy(c->ev_sjoin[k]);
@@ -898,18 +844,15 @@ static int host_batch(orbx_ctx* c, const uint8_t* const* imgs, int batch, int w,
     if ((rc = set_geometry(c, w, h))) return rc;
 
     // ---- which caller buffers need staging
-    static const int stage_env = getenv("ORBX_STAGE") ? atoi(getenv("ORBX_STAGE")) : 1;      // 0: never stage (A/B timing only)
-    const bool stage_in = stage_env && !(host_ptr_is_pinned(imgs[0]) && host_ptr_is_pinned(imgs[batch - 1] + (size_t)(h - 1) * step + row - 1));
+    const bool stage_in = !(host_ptr_is_pinned(imgs[0]) && host_ptr_is_pinned(imgs[batch - 1] + (size_t)(h - 1) * step + row - 1));
     bool stage_out = false;
-    if (stage_env && cap > 0) stage_out = !(host_ptr_is_pinned(kps) && host_ptr_is_pinned(desc));
-    for (int j = 0; j < nmaps && stage_env && !stage_out; ++j) if (nq[j] > 0 && !host_ptr_is_pinned(best[j])) stage_out = true;
+    if (cap > 0) stage_out = !(host_ptr_is_pinned(kps) && host_ptr_is_pinned(desc));
+    for (int j = 0; j < nmaps && !stage_out; ++j) if (nq[j] > 0 && !host_ptr_is_pinned(best[j])) stage_out = true;
     const size_t o_kps = 0, o_desc = round_up(sizeof(orbx_keypoint) * capz * batch, 256), o_best = o_desc + round_up((size_t)32 * capz * batch, 256);
     if (stage_in && (rc = ensure_pinned(c, c->h_stage_in, c->h_stage_in_bytes, fstride * batch))) return rc;
     if (stage_out && (rc = ensure_pinned(c, c->h_stage_out, c->h_stage_out_bytes, o_best + mrows * 16))) return rc;
     HostStager* hs = (stage_in || stage_out) ? stager_of(c) : nullptr;
-    static const int stage_nt = getenv("ORBX_STAGE_NT") ? atoi(getenv("ORBX_STAGE_NT")) : 1;   // non-temporal stores into the pinned input staging
-    static const size_t wake_bytes = getenv("ORBX_STAGE_WAKE_BYTES") ? (size_t)atoll(getenv("ORBX_STAGE_WAKE_BYTES")) : (size_t)2 << 20;
-    const bool wake_in = fstride * batch >= wake_bytes, wake_out = (size_t)60 * capz * batch + mrows * 16 >= wake_bytes;
+    const bool wake_in = fstride * batch >= STAGE_WAKE_BYTES, wake_out = (size_t)60 * capz * batch + mrows * 16 >= STAGE_WAKE_BYTES;
     orbx_keypoint* kps_dl = stage_out ? (orbx_keypoint*)(c->h_stage_out + o_kps) : kps;       // where the D2H copies land
     uint8_t* desc_dl = stage_out ? c->h_stage_out + o_desc : desc;
 
@@ -921,14 +864,13 @@ static int host_batch(orbx_ctx* c, const uint8_t* const* imgs, int batch, int w,
             off += (size_t)nq[j];
         }
     }
-    static const int host_lanes_max = std::max(1, std::min(HOST_MAX_LANES, getenv("ORBX_HOST_LANES") ? atoi(getenv("ORBX_HOST_LANES")) : HOST_DEFAULT_LANES));
     int* h_counts = c->h_small;
     int* h_status = c->h_small + batch;
     int* h_mstatus = c->h_small + 2 * batch;
-    const int lanes = c->profiling ? 1 : std::max(1, std::min(host_lanes_max, batch / HOST_LANE_MIN_FRAMES));
+    const int lanes = c->profiling ? 1 : std::max(1, std::min(HOST_LANES, batch / HOST_LANE_MIN_FRAMES));
     // staged inputs: all pieces are queued up front, lane by lane, so the copier threads run ahead of the lane loop
-    std::atomic<int> in_done[HOST_MAX_LANES], out_done(0);
-    int in_target[HOST_MAX_LANES] = {}, out_target = 0;
+    std::atomic<int> in_done[HOST_LANES], out_done(0);
+    int in_target[HOST_LANES] = {}, out_target = 0;
     struct Drain {                                           // no queued piece may outlive the counters above, whichever way this call ends
         HostStager* hs; std::atomic<int>* in; int* in_t; int n; std::atomic<int>* out; int* out_t;
         ~Drain() { if (hs) { for (int k = 0; k < n; ++k) hs->help_until(in[k], in_t[k]); hs->help_until(*out, *out_t); } }
@@ -938,7 +880,7 @@ static int host_batch(orbx_ctx* c, const uint8_t* const* imgs, int batch, int w,
             int f0, f1;
             host_lane_range(batch, lanes, k, &f0, &f1);
             in_done[k].store(0, std::memory_order_relaxed);
-            for (int i = f0; i < f1; ++i) in_target[k] += hs->submit(c->h_stage_in + fstride * i, dstep, imgs[i], step, row, (size_t)h, &in_done[k], wake_in, stage_nt != 0);
+            for (int i = f0; i < f1; ++i) in_target[k] += hs->submit(c->h_stage_in + fstride * i, dstep, imgs[i], step, row, (size_t)h, &in_done[k], wake_in, true);
         }
     CU(cudaEventRecord(c->ev_fork, c->stream));
     for (int k = 0; k < lanes; ++k) {
@@ -1223,13 +1165,6 @@ int orbx_set_profiling(orbx_ctx* c, int enable)
     c->profiling = enable != 0;
     for (int i = 0; i < N_STAGES; ++i) c->stage_valid[i] = false;
     return ORBX_OK;
-}
-
-int orbx_debug_match_trace(orbx_ctx* c, long long* out /*256*/)
-{
-    if (!c || !out || !c->mtrace.p) return ORBX_E_ARG;
-    cudaStreamSynchronize(c->stream);
-    return cudaMemcpy(out, c->mtrace.p, 16 * 16 * 8, cudaMemcpyDeviceToHost) == cudaSuccess ? ORBX_OK : ORBX_E_CUDA;
 }
 
 int orbx_debug_stage_times(orbx_ctx* c, const char** names, float* ms, int cap)

@@ -40,7 +40,6 @@ constexpr int DS_OFF_ODESC = DS_OFF_BL + 2 * DS_BL_BYTES;
 constexpr int DS_OFF_OKPS = DS_OFF_ODESC + DS_G * 32;
 constexpr int DS_OFF_BAR = DS_OFF_OKPS + 128;
 constexpr int DS_WARP_BYTES = (DS_OFF_BAR + 4 * 8 + 127) / 128 * 128;
-constexpr int DS_MAX_GPW = 16;
 
 struct DescMaps { CUtensorMap ic[ORBX_LEVELS_MAX], bl[ORBX_LEVELS_MAX]; };   // pyramid level / blurred level as (x, y, frame)
 
@@ -105,7 +104,9 @@ __global__ void __launch_bounds__(DS_NW * 32, 5) k_describe_tma(const __grid_con
     if (has_next) nxt = locate(gi + DS_NW); else nxt.ok = false;
     if (lane < 2 && cur.ok) { load_ic(cur, (unsigned)lane); load_bl(cur, (unsigned)lane); }
 
-    // ---- this lane's 8 test pairs: (x0, x1) and (y0, y1) packs
+    // ---- this lane's 8 test pairs: (x0, x1) and (y0, y1) packs, read once with coalesced 128-bit loads (the host transposes
+    //      the pattern table to [t][lane]); a per-keypoint gather of 128-byte-strided float4s costs 32 L1 wavefronts per
+    //      load and makes the LSU the bound
     unsigned long long PX[8], PY[8];
 #pragma unroll
     for (int t = 0; t < 8; ++t) {
@@ -190,8 +191,10 @@ __global__ void __launch_bounds__(DS_NW * 32, 5) k_describe_tma(const __grid_con
             if (!mbar_wait(bar_bl + 8u * b, (m >> 1) & 1u)) { if (lane == 0) atomicOr(&status[f], 2); return; }
             const float snk = __shfl_sync(0xffffffffu, sn, k), csk = __shfl_sync(0xffffffffu, cs, k);
             const int xk = __shfl_sync(0xffffffffu, cur.x, k);
-            // (v + MAGIC) holds rint(v) in its low mantissa bits; MAGIC = 1.5 * 2^23 + 18 moves the origin to the window's
-            // corner.  addr = DS_BLW * bits(y) + bits(x) + cbase  (mod 2^32)
+            // (v + MAGIC) holds rint(v) in its low mantissa bits, exactly for |v| < 2^22; MAGIC = 1.5 * 2^23 + 18 moves the
+            // origin to the window's corner (18 is even, so ties-to-even is unchanged).  addr = DS_BLW * bits(y) + bits(x) + cbase  (mod 2^32)
+            // The rotation's products are packed FMUL2 (mul / add .f32x2 are IEEE per half); the subtraction / addition stays
+            // scalar because ptxas contracts mul.rn.f32x2 + add.rn.f32x2 into FFMA2 even under -fmad=false.
             const unsigned long long MAGIC2 = f2_pack(12582930.0f, 12582930.0f);
             const unsigned long long cs2 = f2_pack(csk, csk), sn2 = f2_pack(snk, snk);
             const unsigned cbase = base_s + DS_OFF_BL + b * DS_BL_BYTES + ((unsigned)(xk - 18) & 15u) - (unsigned)(DS_BLW + 1) * 0x4B400000u;

@@ -9,7 +9,7 @@
 //                                                                       ballot compaction, raster order kept
 //   k_select        A.4-6 retainBest(2n) -> Harris -> retainBest(n)     libstdc++ introselect order reproduced
 //   k_blur          A.8   7x7 float-FMA Gaussian of the samplable region of every level (register sliding window)
-//   k_describe      A.7-10 IC angle, steered rBRIEF-256 sampled from the blurred level, cv::KeyPoint records (warp / keypoint)
+// The descriptor stage (A.7-10) is k_describe_tma in orbx_desc.cuh.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -43,6 +43,7 @@ __device__ __forceinline__ uint2 lds_v2(unsigned addr)
 }
 __device__ __forceinline__ unsigned lds_u32(unsigned addr) { unsigned v; asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(addr) : "memory"); return v; }
 __device__ __forceinline__ unsigned lds_u16(unsigned addr) { unsigned short v; asm volatile("ld.shared.u16 %0, [%1];" : "=h"(v) : "r"(addr) : "memory"); return v; }
+__device__ __forceinline__ unsigned lds_u8(unsigned addr) { unsigned v; asm volatile("ld.shared.u8 %0, [%1];" : "=r"(v) : "r"(addr) : "memory"); return v; }
 __device__ __forceinline__ void sts_u8(unsigned addr, unsigned v) { asm volatile("st.shared.u8 [%0], %1;" :: "r"(addr), "r"(v) : "memory"); }
 __device__ __forceinline__ void sts_u16(unsigned addr, unsigned v) { asm volatile("st.shared.u16 [%0], %1;" :: "r"(addr), "h"((unsigned short)v) : "memory"); }
 __device__ __forceinline__ uint4 lds_v4(unsigned addr)
@@ -50,6 +51,12 @@ __device__ __forceinline__ uint4 lds_v4(unsigned addr)
     uint4 v;
     asm volatile("ld.shared.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(addr) : "memory");
     return v;
+}
+__device__ __forceinline__ int dp4a_us(unsigned a_u8x4, unsigned b_s8x4, int c)       // sum of u8 * s8 products + c
+{
+    int d;
+    asm("dp4a.u32.s32 %0, %1, %2, %3;" : "=r"(d) : "r"(a_u8x4), "r"(b_s8x4), "r"(c));
+    return d;
 }
 
 // ------------------------------------------------------------------------------------------------ A.1 gray
@@ -1136,204 +1143,6 @@ __global__ void __launch_bounds__(BLUR_NT) k_blur(const __grid_constant__ Geom g
 {
     __shared__ __align__(16) uint8_t s_ring[BLUR_RING_BYTES];
     blur_body(g, pyr, blur, blockIdx.x, blockIdx.y, s_ring);
-}
-
-// ------------------------------------------------------------------------------------------------ A.7 / A.9 / A.10 describe
-// One warp = DESC_KPW final keypoints, one after the other (no block-level sync), software-pipelined: while keypoint i
-// is computed, the two windows of keypoint i+1 are already streaming into the warp's other shared-memory buffer with
-// cp.async (4-byte LDGSTS: no registers, no scoreboards), so the global-load latency sits under the arithmetic.
-//   per keypoint   blurred window  rows y-18 .. y+20, 10 aligned words from (x-18)&~3   (39 x 40 B)  -> rBRIEF samples
-//                  unblurred window rows y-15 .. y+17, 9 aligned words from (x-15)&~3   (33 x 36 B)  -> IC moments
-//   (both always inside the level: keypoints keep 31 px from the border)
-//   * IC moments: lane <-> disc row v = lane - 15.  The lane reads its row as 9 words (pitch 9 words: conflict-free),
-//     realigns them with funnel shifts, masks them with the row's disc extent (lane constants) and takes
-//     sum(u * I) and sum(I) with DP4A; m01 = v * sum(I); shuffle reduction.
-//   * the lane's 8 test pairs live in REGISTERS for the whole warp lifetime (pattern table transposed on the host to
-//     [t][lane], read once with fully coalesced 128-bit loads) -- a per-keypoint gather of 128-byte-strided float4s
-//     costs 32 L1 wavefronts per load and made the LSU the bound;
-//   * the products of the rotation are packed FMUL2 (fma/mul/add .f32x2 are IEEE per half); the subtraction / addition
-//     stays scalar because ptxas contracts mul.rn.f32x2 + add.rn.f32x2 into FFMA2 even under -fmad=false;
-//   * cvRound of the rotated coordinates is the exact magic-number add (|v| < 2^22); the window origin (+18, +18: even,
-//     so ties-to-even is unchanged) rides in the magic constant, so the sample address is one IMAD + one IADD;
-//   * the level of a slot comes from a warp scan of the 8 per-level counts (ballot + popc).
-// Keypoint records and descriptors leave as coalesced stores.
-constexpr int DESC_KPB = 4;            // warps per CTA
-constexpr int DESC_KPW = 4;            // keypoints per warp
-constexpr int DESC_NT = DESC_KPB * 32;
-constexpr int DW_PITCH = 40, DW_ROWS = 39;         // blurred window: 13 steps x 3 rows, 10 words per row
-constexpr int IC_PITCH = 36, IC_ROWS = 33;         // unblurred window: 11 steps x 3 rows, 9 words per row
-constexpr int DESC_BUF = DW_PITCH * DW_ROWS + IC_PITCH * IC_ROWS;   // 2748 bytes per keypoint buffer
-constexpr int DESC_BUF_PAD = (DESC_BUF + 15) / 16 * 16;
-
-__device__ __forceinline__ int dp4a_us(unsigned a_u8x4, unsigned b_s8x4, int c)       // sum of u8 * s8 products + c
-{
-    int d;
-    asm("dp4a.u32.s32 %0, %1, %2, %3;" : "=r"(d) : "r"(a_u8x4), "r"(b_s8x4), "r"(c));
-    return d;
-}
-__device__ __forceinline__ unsigned lds_u8(unsigned addr) { unsigned v; asm volatile("ld.shared.u8 %0, [%1];" : "=r"(v) : "r"(addr) : "memory"); return v; }
-
-struct DescKp { int x, y, lvl; float response; };
-
-__global__ void __launch_bounds__(DESC_NT, 6) k_describe(const __grid_constant__ Geom g, const uint8_t* __restrict__ pyr,
-                                                      const uint8_t* __restrict__ blur, const Elem* __restrict__ work,
-                                                      const int* __restrict__ fincnt, const float4* __restrict__ pattern,
-                                                      float* __restrict__ kps_out, uint8_t* __restrict__ desc_out,
-                                                      int* __restrict__ counts_out, int cap)
-{
-    __shared__ __align__(16) uint8_t s_buf[DESC_KPB][2][DESC_BUF_PAD];
-    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5, f = blockIdx.y;
-    // ---- per-level counts -> inclusive prefix across lanes (lane l <-> level l)
-    int pre = lane < g.nlevels ? __ldg(fincnt + f * g.nlevels + lane) : 0;
-#pragma unroll
-    for (int d = 1; d < 32; d <<= 1) { const int o = __shfl_up_sync(0xffffffffu, pre, d); if (lane >= d) pre += o; }
-    const int total = __shfl_sync(0xffffffffu, pre, 31);
-    if (blockIdx.x == 0 && threadIdx.x == 0) counts_out[f] = total;
-    const int nkp = min(total, cap);
-    const int slot0 = blockIdx.x * (DESC_KPB * DESC_KPW) + wid;
-    if (slot0 >= nkp) return;                                // warp-uniform
-    const unsigned buf_s = (unsigned)__cvta_generic_to_shared(&s_buf[wid][0][0]);
-
-    // slot -> keypoint (warp-uniform result)
-    auto locate = [&](int slot) -> DescKp {
-        const int lvl = __popc(__ballot_sync(0xffffffffu, pre <= slot) & ((1u << g.nlevels) - 1u));
-        const int before = __shfl_sync(0xffffffffu, pre, max(lvl - 1, 0));
-        const int idx = slot - (lvl > 0 ? before : 0);
-        const Elem e = work[(size_t)f * g.ws_frame + g.L[lvl].ws_off + idx];
-        DescKp k;
-        k.x = (int)(e.pos & 0xffffu); k.y = (int)(e.pos >> 16); k.lvl = lvl; k.response = e.response;
-        return k;
-    };
-    // both windows of a keypoint -> buffer `b` (cp.async, asynchronous)
-    const int wr = lane / 10, wc = lane - wr * 10;           // blurred window: lanes 0..29 = 3 rows x 10 words
-    const int ir = lane / 9, ic = lane - ir * 9;             // unblurred window: lanes 0..26 = 3 rows x 9 words
-    auto stage = [&](const DescKp& k, int b) {
-        const LevelGeom& L = g.L[k.lvl];
-        const size_t base = (size_t)f * g.pyr_frame + L.img_off;
-        const int pitch = L.pitch;
-        const unsigned bs = buf_s + (unsigned)b * DESC_BUF_PAD;
-        if (lane < 30) {
-            const uint8_t* src = blur + base + (size_t)(k.y - 18 + wr) * pitch + ((k.x - 18) & ~3) + wc * 4;
-            unsigned dst = bs + wr * DW_PITCH + wc * 4;
-#pragma unroll
-            for (int j = 0; j < DW_ROWS / 3; ++j, src += 3 * pitch, dst += 3 * DW_PITCH) cp_async_4(dst, src);
-        }
-        if (lane < 27) {
-            const uint8_t* src = pyr + base + (size_t)(k.y - 15 + ir) * pitch + ((k.x - 15) & ~3) + ic * 4;
-            unsigned dst = bs + DW_PITCH * DW_ROWS + ir * IC_PITCH + ic * 4;
-#pragma unroll
-            for (int j = 0; j < IC_ROWS / 3; ++j, src += 3 * pitch, dst += 3 * IC_PITCH) cp_async_4(dst, src);
-        }
-    };
-
-    DescKp kp = locate(slot0);
-    stage(kp, 0);
-    cp_async_commit();
-
-    // ---- this lane's 8 test pairs: (x0, x1) and (y0, y1) packs
-    unsigned long long PX[8], PY[8];
-#pragma unroll
-    for (int t = 0; t < 8; ++t) {
-        const float4 pt = __ldg(pattern + t * 32 + lane);
-        PX[t] = f2_pack(pt.x, pt.z);
-        PY[t] = f2_pack(pt.y, pt.w);
-    }
-    // IC disc: lane <-> row v = lane - 15 (lane 31 idle); icmask[j] keeps the columns u = 4j-15 .. 4j-12 inside the disc
-    const int icv = min(lane, 30) - 15;
-    uint32_t icmask[8];
-    {
-        // umax[|v|] = {15, 15, 15, 15, 14, 14, 14, 13, 13, 12, 11, 10, 9, 8, 6, 3} as nibbles (no local array)
-        constexpr unsigned long long UMAXP = 0x3689ABCDDEEEFFFFull;
-        const int um = (int)((UMAXP >> (4 * (icv < 0 ? -icv : icv))) & 15ull);
-#pragma unroll
-        for (int j = 0; j < 8; ++j) {
-            uint32_t m = 0;
-#pragma unroll
-            for (int b = 0; b < 4; ++b) {
-                const int u = 4 * j + b - 15;
-                if (u <= 15 && lane < 31 && (u < 0 ? -u : u) <= um) m |= 0xFFu << (8 * b);
-            }
-            icmask[j] = m;
-        }
-    }
-
-#pragma unroll 1
-    for (int it = 0; it < DESC_KPW; ++it) {
-        const int slot = slot0 + it * DESC_KPB;
-        const bool has_next = it + 1 < DESC_KPW && slot + DESC_KPB < nkp;     // warp-uniform
-        DescKp kpn = kp;
-        if (has_next) { kpn = locate(slot + DESC_KPB); stage(kpn, (it + 1) & 1); }
-        cp_async_commit();
-        cp_async_wait<1>();                                  // this keypoint's windows have landed (this lane's copies)
-        __syncwarp();                                        // ... and every other lane's
-        const int x = kp.x, y = kp.y, lvl = kp.lvl;
-        const LevelGeom& L = g.L[lvl];
-        const unsigned bs = buf_s + (unsigned)(it & 1) * DESC_BUF_PAD;
-
-        // ---- IC moments from the unblurred window
-        int m10 = 0, m01 = 0;
-        {
-            const unsigned rowa = bs + DW_PITCH * DW_ROWS + (unsigned)min(lane, 30) * IC_PITCH;
-            const unsigned shb = (unsigned)((x - 15) & 3) * 8u;
-            uint32_t W[9];
-#pragma unroll
-            for (int j = 0; j < 9; ++j) W[j] = lds_u32(rowa + 4 * j);
-            int rowsum = 0;
-#pragma unroll
-            for (int j = 0; j < 8; ++j) {
-                const uint32_t w = __funnelshift_r(W[j], W[j + 1], shb) & icmask[j];       // columns u = 4j-15 .. 4j-12
-                const int u0 = 4 * j - 15;
-                const uint32_t coef = (uint32_t)(u0 & 255) | ((uint32_t)((u0 + 1) & 255) << 8) | ((uint32_t)((u0 + 2) & 255) << 16) | ((uint32_t)((u0 + 3) & 255) << 24);
-                m10 = dp4a_us(w, coef, m10);
-                rowsum = dp4a_us(w, 0x01010101u, rowsum);
-            }
-            m01 = icv * rowsum;
-        }
-#pragma unroll
-        for (int d = 16; d > 0; d >>= 1) { m10 += __shfl_xor_sync(0xffffffffu, m10, d); m01 += __shfl_xor_sync(0xffffffffu, m01, d); }
-        const float ang = fast_atan2_deg((float)m01, (float)m10);
-        float sn, cs;
-        glibc_sincosf(__fmul_rn(ang, __int_as_float(0x3c8efa35)), &sn, &cs);
-        // ---- steered rBRIEF: lane <-> descriptor byte
-        {
-            // (v + MAGIC) holds rint(v) in its low mantissa bits; MAGIC = 1.5 * 2^23 + 18 moves the origin to the
-            // window's corner.  addr = DW_PITCH * bits(y) + bits(x) + cbase  (mod 2^32)
-            const unsigned long long MAGIC2 = f2_pack(12582930.0f, 12582930.0f);
-            const unsigned long long cs2 = f2_pack(cs, cs), sn2 = f2_pack(sn, sn);
-            const unsigned cbase = bs + (unsigned)((x - 18) & 3) - (unsigned)(DW_PITCH + 1) * 0x4B400000u;   // the +18s stay
-            unsigned byte = 0;
-#pragma unroll
-            for (int t = 0; t < 8; ++t) {
-                const unsigned long long xc = f2_mul(PX[t], cs2), ys = f2_mul(PY[t], sn2);
-                const unsigned long long xs = f2_mul(PX[t], sn2), yc = f2_mul(PY[t], cs2);
-                const float fx0 = __fsub_rn(f2_lo(xc), f2_lo(ys)), fx1 = __fsub_rn(f2_hi(xc), f2_hi(ys));
-                const float fy0 = __fadd_rn(f2_lo(xs), f2_lo(yc)), fy1 = __fadd_rn(f2_hi(xs), f2_hi(yc));
-                const unsigned long long bx = f2_add(f2_pack(fx0, fx1), MAGIC2), by = f2_add(f2_pack(fy0, fy1), MAGIC2);
-                const unsigned a0 = (unsigned)by * (unsigned)DW_PITCH + (unsigned)bx + cbase;
-                const unsigned a1 = (unsigned)(by >> 32) * (unsigned)DW_PITCH + (unsigned)(bx >> 32) + cbase;
-                const unsigned t0 = lds_u8(a0), t1 = lds_u8(a1);
-                byte |= (unsigned)(t0 < t1) << t;
-            }
-            const size_t o = (size_t)f * cap + slot;
-            desc_out[o * 32 + lane] = (uint8_t)byte;
-            if (lane < 7) {
-                float val;
-                switch (lane) {
-                    case 0: val = __fmul_rn((float)x, L.scale); break;
-                    case 1: val = __fmul_rn((float)y, L.scale); break;
-                    case 2: val = __fmul_rn(31.0f, L.scale); break;
-                    case 3: val = ang; break;
-                    case 4: val = kp.response; break;
-                    case 5: val = __int_as_float(lvl); break;
-                    default: val = __int_as_float(-1); break;
-                }
-                kps_out[o * 7 + lane] = val;
-            }
-        }
-        if (!has_next) break;
-        __syncwarp();                                        // every lane is done with this buffer before it is refilled
-        kp = kpn;
-    }
 }
 
 }  // namespace orbx

@@ -304,7 +304,7 @@ template <bool KNN2, bool PAIR>
 __device__ __forceinline__ void
 hamming_umma_body(const uint8_t* __restrict__ query, int nq, const uint8_t* __restrict__ train, int nt, int train_stride_rows,
                const int* __restrict__ train_counts, int nsets, int rows_per_split, int4* __restrict__ best,
-               int4* __restrict__ second, int* __restrict__ keys, int* __restrict__ status, int dbg, long long* __restrict__ trace)
+               int4* __restrict__ second, int* __restrict__ keys, int* __restrict__ status)
 {
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
@@ -428,18 +428,12 @@ hamming_umma_body(const uint8_t* __restrict__ query, int nq, const uint8_t* __re
             fetch(slot);                                     // refill the slot just consumed
             const int s = t % MT_STAGES;
             const uint32_t ph = (uint32_t)(t / MT_STAGES) & 1u;
-            const bool tr_on = trace && blockIdx.x == 0 && blockIdx.y == 0 && blockIdx.z == 0 && t >= 40 && t < 56 && r == 0;
-            if (tr_on) trace[(t - 40) * 16 + 8] = clock64();
             if (!mbar_wait(bar_empty + 8 * s, ph ^ 1u)) { ok = false; break; }
-            if (tr_on) trace[(t - 40) * 16 + 9] = clock64();
-            if (!(dbg & 4)) {
-                if (PAIR) expand_half_row(smem + MT_SMEM_B + s * MT_B_BYTES, MT2_HALF, r, hk, cv);
-                else      expand_row(smem + MT_SMEM_B + s * MT_B_BYTES, MT_BN, r, cv, cv2);
-            }
+            if (PAIR) expand_half_row(smem + MT_SMEM_B + s * MT_B_BYTES, MT2_HALF, r, hk, cv);
+            else      expand_row(smem + MT_SMEM_B + s * MT_B_BYTES, MT_BN, r, cv, cv2);
             fence_proxy_async_smem();                        // every writer fences, then one lane arrives for the warp (on the leader's barrier)
             __syncwarp();
             if (lane == 0) bar_arrive_lead<PAIR>(lead_full + 8 * s);
-            if (tr_on) trace[(t - 40) * 16 + 10] = clock64();
 #pragma unroll 1
             for (int k = 0; k < MT_EXP_GROUPS; ++k) step(cur);
             t += MT_EXP_GROUPS;
@@ -472,14 +466,10 @@ hamming_umma_body(const uint8_t* __restrict__ query, int nq, const uint8_t* __re
                 const uint32_t ph = (uint32_t)(t / MT_STAGES) & 1u;
                 const int b = t & 1;
                 const uint32_t bph = (uint32_t)(t >> 1) & 1u;
-                const bool tr_on = trace && blockIdx.x == 0 && blockIdx.y == 0 && blockIdx.z == 0 && t >= 40 && t < 56 && lane == 0;
-                if (tr_on) trace[(t - 40) * 16 + 0] = clock64();
                 if (!ready_next) {
                     if (!mbar_wait(bar_tempty + 8 * b, bph ^ 1u)) { ok = false; break; }
-                    if (tr_on) trace[(t - 40) * 16 + 1] = clock64();
                     if (!mbar_wait(bar_full + 8 * s, ph)) { ok = false; break; }
                 }
-                if (tr_on) trace[(t - 40) * 16 + 2] = clock64();
                 tc_fence_after();
                 const uint32_t sb = sbu + MT_SMEM_B + s * MT_B_BYTES;
                 const uint64_t db0 = umma_desc_sw128(sb);
@@ -493,7 +483,7 @@ hamming_umma_body(const uint8_t* __restrict__ query, int nq, const uint8_t* __re
                 const uint32_t ph1 = (uint32_t)((t + 2) / MT_STAGES) & 1u, bph1 = (uint32_t)((t + 2) >> 1) & 1u;
 #pragma unroll
                 for (int a = 0; a < 2; ++a) {
-                    if (elect_one() && !(dbg & 2)) {
+                    if (elect_one()) {
                         const uint32_t d = tb + (uint32_t)((b * 2 + a) * MT_BN);
                         const uint32_t ta = tb + MT_TMEM_A + (uint32_t)a * 64u;
 #pragma unroll
@@ -513,7 +503,6 @@ hamming_umma_body(const uint8_t* __restrict__ query, int nq, const uint8_t* __re
                     umma_commit<PAIR>(bar_tfull + 8 * b);           // accumulators of this tile complete (both CTAs' barriers)
                 }
                 __syncwarp();
-                if (tr_on) trace[(t - 40) * 16 + 3] = clock64();
             }
         }
     } else if (warp >= MT_EPI_WARP0 && warp < MT_EPI_WARP0 + 8) {
@@ -530,112 +519,95 @@ hamming_umma_body(const uint8_t* __restrict__ query, int nq, const uint8_t* __re
             for (int i = 0; i < rg.ntiles; ++i, ++t) {
                 const int b = t & 1;
                 const uint32_t bph = (uint32_t)(t >> 1) & 1u;
-                const bool tr_on = trace && blockIdx.x == 0 && blockIdx.y == 0 && blockIdx.z == 0 && t >= 40 && t < 56 && warp == MT_EPI_WARP0 + 1 && lane == 0;
-                if (tr_on) trace[(t - 40) * 16 + 4] = clock64();
                 if (!mbar_wait(bar_tfull + 8 * b, bph)) { ok = false; break; }
-                if (tr_on) trace[(t - 40) * 16 + 5] = clock64();
                 tc_fence_after();
                 const int j0 = rg.n0 + i * MT_BN;
                 const bool full = (j0 + MT_BN <= rg.n1);
                 constexpr int NCH = MT_BN / 32;
                 uint32_t r[NCH][32];
-                if (!(dbg & 1)) {
-                    const uint32_t tacc = tmem_base + lane_base + (uint32_t)((b * 2 + a) * MT_BN);
-                    int k1 = INT_MIN, k2 = INT_MIN;
-                    if (!KNN2 && full) {
-                        // accumulator = 127 * dot + code lies in [-32512, 32607]: it fits in 16 bits, so the tile comes out of
-                        // tensor memory packed two columns per register (half the registers, half the max operations), and every
-                        // value of a row is distinct (distinct codes), so the packed maximum loses nothing
-                        uint32_t rp[MT_BN / 2];
-                        tc_ld32_pack16(tacc, rp);
-                        tc_ld16_pack16(tacc + 64, rp + 32);
-                        tc_wait_ld();
-                        if (tr_on) trace[(t - 40) * 16 + 6] = clock64();
-                        tc_fence_before();
-                        __syncwarp();
-                        if (lane == 0) bar_arrive_lead<PAIR>(lead_tempty + 8 * b);           // TMEM buffer back to the issuer BEFORE the reduction
-                        unsigned p[8];                           // eight independent max chains (ILP), then a short tree
+                const uint32_t tacc = tmem_base + lane_base + (uint32_t)((b * 2 + a) * MT_BN);
+                int k1 = INT_MIN, k2 = INT_MIN;
+                if (!KNN2 && full) {
+                    // accumulator = 127 * dot + code lies in [-32512, 32607]: it fits in 16 bits, so the tile comes out of
+                    // tensor memory packed two columns per register (half the registers, half the max operations), and every
+                    // value of a row is distinct (distinct codes), so the packed maximum loses nothing
+                    uint32_t rp[MT_BN / 2];
+                    tc_ld32_pack16(tacc, rp);
+                    tc_ld16_pack16(tacc + 64, rp + 32);
+                    tc_wait_ld();
+                    tc_fence_before();
+                    __syncwarp();
+                    if (lane == 0) bar_arrive_lead<PAIR>(lead_tempty + 8 * b);           // TMEM buffer back to the issuer BEFORE the reduction
+                    unsigned p[8];                           // eight independent max chains (ILP), then a short tree
 #pragma unroll
-                        for (int u = 0; u < 8; ++u) {
-                            p[u] = __vimax3_s16x2(rp[u], rp[8 + u], rp[16 + u]);
-                            p[u] = __vimax3_s16x2(p[u], rp[24 + u], rp[32 + u]);
-                            p[u] = __vmaxs2(p[u], rp[40 + u]);
+                    for (int u = 0; u < 8; ++u) {
+                        p[u] = __vimax3_s16x2(rp[u], rp[8 + u], rp[16 + u]);
+                        p[u] = __vimax3_s16x2(p[u], rp[24 + u], rp[32 + u]);
+                        p[u] = __vmaxs2(p[u], rp[40 + u]);
+                    }
+                    const unsigned pk = __vimax3_s16x2(__vimax3_s16x2(p[0], p[1], p[2]), __vimax3_s16x2(p[3], p[4], p[5]), __vmaxs2(p[6], p[7]));
+                    k1 = max((int)(pk << 16) >> 16, (int)pk >> 16);
+                } else if (!KNN2) {
+                    // a set's partial last tile was issued with N = 32, 64 (or 96) columns, its rows past the set's end are
+                    // copies of the last row (never the maximum): same packed path, 32-column chunks as far as N goes
+                    const int nch = (rg.n1 - j0 + 31) >> 5;
+                    uint32_t rp[MT_BN / 2];
+#pragma unroll
+                    for (int ch = 0; ch < NCH; ++ch) {
+                        if (ch < nch) tc_ld16_pack16(tacc + (uint32_t)(ch * 32), rp + ch * 16);
+                        else {
+#pragma unroll
+                            for (int u = 0; u < 16; ++u) rp[ch * 16 + u] = 0x80008000u;
                         }
-                        const unsigned pk = __vimax3_s16x2(__vimax3_s16x2(p[0], p[1], p[2]), __vimax3_s16x2(p[3], p[4], p[5]), __vmaxs2(p[6], p[7]));
-                        k1 = max((int)(pk << 16) >> 16, (int)pk >> 16);
-                    } else if (!KNN2) {
-                        // a set's partial last tile was issued with N = 32, 64 (or 96) columns, its rows past the set's end are
-                        // copies of the last row (never the maximum): same packed path, 32-column chunks as far as N goes
-                        const int nch = (rg.n1 - j0 + 31) >> 5;
-                        uint32_t rp[MT_BN / 2];
+                    }
+                    tc_wait_ld();
+                    tc_fence_before();
+                    __syncwarp();
+                    if (lane == 0) bar_arrive_lead<PAIR>(lead_tempty + 8 * b);
+                    unsigned p[8];
 #pragma unroll
-                        for (int ch = 0; ch < NCH; ++ch) {
-                            if (ch < nch) tc_ld16_pack16(tacc + (uint32_t)(ch * 32), rp + ch * 16);
-                            else {
-#pragma unroll
-                                for (int u = 0; u < 16; ++u) rp[ch * 16 + u] = 0x80008000u;
-                            }
-                        }
-                        tc_wait_ld();
-                        if (tr_on) trace[(t - 40) * 16 + 6] = clock64();
-                        tc_fence_before();
-                        __syncwarp();
-                        if (lane == 0) bar_arrive_lead<PAIR>(lead_tempty + 8 * b);
-                        unsigned p[8];
-#pragma unroll
-                        for (int u = 0; u < 8; ++u) {
-                            p[u] = __vimax3_s16x2(rp[u], rp[8 + u], rp[16 + u]);
-                            p[u] = __vimax3_s16x2(p[u], rp[24 + u], rp[32 + u]);
-                            p[u] = __vmaxs2(p[u], rp[40 + u]);
-                        }
-                        const unsigned pk = __vimax3_s16x2(__vimax3_s16x2(p[0], p[1], p[2]), __vimax3_s16x2(p[3], p[4], p[5]), __vmaxs2(p[6], p[7]));
-                        k1 = max((int)(pk << 16) >> 16, (int)pk >> 16);
-                    } else {
+                    for (int u = 0; u < 8; ++u) {
+                        p[u] = __vimax3_s16x2(rp[u], rp[8 + u], rp[16 + u]);
+                        p[u] = __vimax3_s16x2(p[u], rp[24 + u], rp[32 + u]);
+                        p[u] = __vmaxs2(p[u], rp[40 + u]);
+                    }
+                    const unsigned pk = __vimax3_s16x2(__vimax3_s16x2(p[0], p[1], p[2]), __vimax3_s16x2(p[3], p[4], p[5]), __vmaxs2(p[6], p[7]));
+                    k1 = max((int)(pk << 16) >> 16, (int)pk >> 16);
+                } else {
 #pragma unroll
                     for (int ch = 0; ch < NCH; ++ch) tc_ld32(tacc + (uint32_t)(ch * 32), r[ch]);
                     tc_wait_ld();
-                    if (tr_on) trace[(t - 40) * 16 + 6] = clock64();
                     // The accumulators now live in registers: hand the TMEM buffer back to the issuer BEFORE the max
                     // reduction, so the epilogue's arithmetic overlaps the MMAs of tile t + 2 instead of gating them.
                     tc_fence_before();
                     __syncwarp();
                     if (lane == 0) bar_arrive_lead<PAIR>(lead_tempty + 8 * b);
 #pragma unroll
-                        for (int ch = 0; ch < NCH; ++ch)
+                    for (int ch = 0; ch < NCH; ++ch)
 #pragma unroll
-                            for (int c = 0; c < 32; ++c)
-                                if (full || j0 + ch * 32 + c < rg.n1) {
-                                    const int k = (int)r[ch][c];
-                                    if (KNN2) k2 = max(k2, min(k1, k));
-                                    k1 = max(k1, k);
-                                }
-                    }
-                    // decode the tile winner(s) into the global key  dot << 20 | (0xFFFFF - j)
+                        for (int c = 0; c < 32; ++c)
+                            if (full || j0 + ch * 32 + c < rg.n1) {
+                                const int k = (int)r[ch][c];
+                                if (KNN2) k2 = max(k2, min(k1, k));
+                                k1 = max(k1, k);
+                            }
+                }
+                // decode the tile winner(s) into the global key  dot << 20 | (0xFFFFF - j)
 #pragma unroll
-                    for (int w = 0; w < (KNN2 ? 2 : 1); ++w) {
-                        const int k = w == 0 ? k1 : k2;
-                        if (k != INT_MIN) {
-                            const unsigned kk = (unsigned)(k + MT_ASCALE * 256);
-                            const unsigned q = kk / (unsigned)MT_ASCALE;          // dot + 256
-                            const int code = (MT_BN - 1) - (int)(kk - q * (unsigned)MT_ASCALE);   // 48 * (CTA holding the row) + local row
-                            const int nh = ((min(MT_BN, rg.n1 - j0) + 31) & ~31) >> 1;
-                            const int jl = PAIR && code >= MT2_HALF ? nh + code - MT2_HALF : code;
-                            const int gk = ((int)q - 256) * (1 << MT_KEY_SHIFT) + ((MT_MAX_TRAIN - 1) - (j0 + jl));
-                            if (KNN2) m2 = max(m2, min(m1, gk));
-                            m1 = max(m1, gk);
-                        }
+                for (int w = 0; w < (KNN2 ? 2 : 1); ++w) {
+                    const int k = w == 0 ? k1 : k2;
+                    if (k != INT_MIN) {
+                        const unsigned kk = (unsigned)(k + MT_ASCALE * 256);
+                        const unsigned q = kk / (unsigned)MT_ASCALE;          // dot + 256
+                        const int code = (MT_BN - 1) - (int)(kk - q * (unsigned)MT_ASCALE);   // 48 * (CTA holding the row) + local row
+                        const int nh = ((min(MT_BN, rg.n1 - j0) + 31) & ~31) >> 1;
+                        const int jl = PAIR && code >= MT2_HALF ? nh + code - MT2_HALF : code;
+                        const int gk = ((int)q - 256) * (1 << MT_KEY_SHIFT) + ((MT_MAX_TRAIN - 1) - (j0 + jl));
+                        if (KNN2) m2 = max(m2, min(m1, gk));
+                        m1 = max(m1, gk);
                     }
                 }
-                else {                                       // (perf-experiment mode without TMEM loads: still release the buffer)
-                    tc_fence_before();
-                    __syncwarp();
-                    if (lane == 0) bar_arrive_lead<PAIR>(lead_tempty + 8 * b);
-                }
-                if (tr_on) trace[(t - 40) * 16 + 11] = clock64() + (m1 & 1);
-                if (tr_on) trace[(t - 40) * 16 + 7] = clock64();
             }
-            const bool tr_set = trace && blockIdx.x == 0 && blockIdx.y == 0 && blockIdx.z == 0 && t > 40 && t <= 56 && warp == MT_EPI_WARP0 + 1 && lane == 0;
-            if (tr_set) trace[(t - 1 - 40) * 16 + 12] = clock64();
             if (ok && qrow < nq) {
                 const size_t o = (size_t)set * nq + qrow;
                 if (keys) {
@@ -656,7 +628,6 @@ hamming_umma_body(const uint8_t* __restrict__ query, int nq, const uint8_t* __re
                     }
                 }
             }
-            if (tr_set) trace[(t - 1 - 40) * 16 + 13] = clock64();
         }
     }
     if (!ok) atomicOr(status, 2);
@@ -671,8 +642,8 @@ hamming_umma_body(const uint8_t* __restrict__ query, int nq, const uint8_t* __re
 
 #define ORBX_MATCH_PARAMS const uint8_t* __restrict__ query, int nq, const uint8_t* __restrict__ train, int nt, int train_stride_rows, \
                const int* __restrict__ train_counts, int nsets, int rows_per_split, int4* __restrict__ best, \
-               int4* __restrict__ second, int* __restrict__ keys, int* __restrict__ status, int dbg, long long* __restrict__ trace
-#define ORBX_MATCH_ARGS query, nq, train, nt, train_stride_rows, train_counts, nsets, rows_per_split, best, second, keys, status, dbg, trace
+               int4* __restrict__ second, int* __restrict__ keys, int* __restrict__ status
+#define ORBX_MATCH_ARGS query, nq, train, nt, train_stride_rows, train_counts, nsets, rows_per_split, best, second, keys, status
 // single CTA per query tile (small problems: independent CTAs, train rows can be split across them)
 template <bool KNN2>
 __global__ void __launch_bounds__(MT_THREADS, 1) k_hamming_umma(ORBX_MATCH_PARAMS) { hamming_umma_body<KNN2, false>(ORBX_MATCH_ARGS); }

@@ -80,11 +80,7 @@ struct SelFastSmem { Elem v[SELF_SMEM_ELEMS]; uint16_t pos[2 * SELF_SMEM_ELEMS];
 
 // One warp per (frame, level): gather the per-row FAST lists (raster order) and retainBest(2 n_l) on the FAST score; survivors ->
 // the prefix of the level's global workspace, their number -> selcnt.
-// FUSED = true (experiment, ORBX_SELECT_FUSED=1; measured slower: 0.1435 against 0.1159 ms per 256 VGA frames): the same warp goes
-// straight on -- Harris responses of its own survivors (lane-strided), then retainBest(n_l) on them, final list and fincnt written --
-// so that k_harris and k_select_harris are not launched.
-template <bool FUSED>
-__global__ void __launch_bounds__(32) k_select_fast(const __grid_constant__ Geom g, const uint8_t* __restrict__ pyr, const uint32_t* __restrict__ rowcnt,
+__global__ void __launch_bounds__(32) k_select_fast(const __grid_constant__ Geom g, const uint32_t* __restrict__ rowcnt,
                                                     const uint32_t* __restrict__ rowent, Elem* __restrict__ work, uint32_t* __restrict__ selpos,
                                                     int* __restrict__ selcnt, int* __restrict__ fincnt)
 {
@@ -153,21 +149,7 @@ __global__ void __launch_bounds__(32) k_select_fast(const __grid_constant__ Geom
                            : retain_best_warp<uint32_t>(v, N, 2 * L.quota, gpos, gpos + N, lane);
     __syncwarp();
     if (lane == 0) selcnt[f * g.nlevels + l] = n1;
-    if (!FUSED) {
-        if (v != gv) for (int i = lane; i < n1; i += 32) gv[i] = v[i];
-        return;
-    }
-    const uint8_t* img = pyr + (size_t)f * g.pyr_frame + L.img_off;
-    for (int i = lane; i < n1; i += 32) {
-        const uint32_t pos = v[i].pos;
-        v[i].response = harris_response(img, L.pitch, (int)(pos & 0xffffu), (int)(pos >> 16));
-    }
-    __syncwarp();
-    const int n2 = in_smem ? retain_best_warp<uint16_t>(v, n1, L.quota, sm.pos, sm.pos + SELF_SMEM_ELEMS, lane)
-                           : retain_best_warp<uint32_t>(v, n1, L.quota, gpos, gpos + N, lane);
-    __syncwarp();
-    if (lane == 0) fincnt[f * g.nlevels + l] = n2;
-    if (v != gv) for (int i = lane; i < n2; i += 32) gv[i] = v[i];
+    if (v != gv) for (int i = lane; i < n1; i += 32) gv[i] = v[i];
 }
 
 // One thread per candidate that survived the first selection: response <- Harris (A.5) on the unblurred level.

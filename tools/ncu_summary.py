@@ -33,7 +33,7 @@ for r in data:
     kern.setdefault(name, []).append({"dram_read_bytes": to_bytes(r[ri], units[ri]), "dram_write_bytes": to_bytes(r[wi], units[wi]),
                                       "time_us": float(r[ti]) * {"us": 1, "ms": 1e3, "ns": 1e-3}.get(units[ti], 1)})
 json.dump({"note": "dram__bytes_read.sum / dram__bytes_write.sum per launch from ncu --set full --clock-control none, "
-                   "ORBX_LANES=1 tools/prof_step.py 256 2 (256 VGA frames per launch)", "kernels": kern},
+                   "tools/prof_step.py 256 2 (256 VGA frames per launch)", "kernels": kern},
           open(out + "_ncu_dram_traffic.json", "w"), indent=1)
 # one record per kernel (a kernel launched once per level: the sums over its launches) -- what bench.py quotes
 def col(name):
@@ -55,6 +55,6 @@ for r in step_rows:
     if m["launches"] == 1:                               # utilisation figures of the first (largest) launch
         for k, key in (("issue", "issue_active_pct"), ("alu", "alu_pipe_pct"), ("fma", "fma_pipe_pct"), ("tensor", "tensor_pipe_pct"), ("dram", "dram_throughput_pct"), ("regs", "registers")):
             if ci[k] is not None and r[ci[k]] != "": m[key] = float(r[ci[k]])
-json.dump({"note": "ncu --set full --clock-control none of ORBX_LANES=1 tools/prof_step.py 256 2 (256 VGA frames per launch, BASELINE config 2): per-kernel sums over "
+json.dump({"note": "ncu --set full --clock-control none of tools/prof_step.py 256 2 (256 VGA frames per launch, BASELINE config 2): per-kernel sums over "
                    "its launches inside ONE step (from the capture's last k_gray launch on); pipe / issue percentages of the kernel's first launch", "kernels": met}, open(out + "_ncu_metrics.json", "w"), indent=1)
 print(open(out + "_ncu_full_summary.csv").read())

@@ -1,8 +1,8 @@
 #!/usr/bin/env python
 """Static SASS instruction counts per source line (and per opcode) of one kernel of liborbx.so.
 
-  python tools/sass_lines.py k_describe            # per-line histogram
-  python tools/sass_lines.py k_describe --ops      # opcode histogram
+  python tools/sass_lines.py k_describe_tma            # per-line histogram
+  python tools/sass_lines.py k_describe_tma --ops      # opcode histogram
 
 Needs the library built with -lineinfo (it is) and cuobjdump / nvdisasm on PATH.  CPU-only; used to budget
 instruction counts before spending GPU time.

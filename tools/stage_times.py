@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Per-stage device times of the extraction (+ match) on B synthetic VGA frames, without the rest of bench.py.
-  python tools/stage_times.py [B] [reps]        (experiment switches such as ORBX_FAST_DBG are read by the library)"""
+  python tools/stage_times.py [B] [reps]        (ORBX_LIB=<path> times another build of the library)"""
 import os
 import sys
 

@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Device time of the whole extraction step (and of extraction + 2 matches) on B synthetic VGA frames with the library's
 normal stream layout (stage timers off, so the side-stream overlaps are active) -- wall clock over many asynchronous steps.
-  python tools/step_time.py [B] [reps]        (experiment switches such as ORBX_OVERLAP / ORBX_TAIL_PX are read by the library)"""
+  python tools/step_time.py [B] [reps]        (ORBX_LIB=<path> times another build of the library)"""
 import os
 import sys
 import time
