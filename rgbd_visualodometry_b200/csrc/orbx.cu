@@ -12,6 +12,7 @@
 #include <stdlib.h>
 #include <string.h>
 #include <algorithm>
+#include <memory>
 #include <new>
 #include <string>
 #include <vector>
@@ -45,6 +46,7 @@ constexpr long SIDE_LEVEL_MAX_PX = 100000; // pyramid levels (from level 2 on) b
 constexpr size_t STAGE_WAKE_BYTES = (size_t)2 << 20;   // staged copies of at least this many bytes wake the copier threads
 constexpr int N_STAGES = 7;
 const char* const k_stage_names[N_STAGES] = {"gray", "pyramid", "fast_nms", "select_harris", "blur", "describe", "match"};
+constexpr int MATCH_WORDS = 16;           // matcher status words (mstatus), one per slot: lane k of a host-buffer batch uses slot k
 
 size_t round_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
@@ -60,17 +62,46 @@ struct NvtxStages {                      // one open range at a time: next() clo
     ~NvtxStages() { if (open) nvtxRangePop(); }
 };
 
-struct Buf {
-    void* p = nullptr;
+// The context's CUDA resources, each released by its owner's destructor (none of these throws).
+template <class T, cudaError_t (*release)(void*)>
+struct Mem {                                 // move-only, so that a grown table column can replace the old one
+    T* p = nullptr;
     size_t bytes = 0;
+    Mem() = default;
+    Mem(Mem&& o) noexcept : p(o.p), bytes(o.bytes) { o.p = nullptr; o.bytes = 0; }
+    Mem& operator=(Mem&& o) noexcept { std::swap(p, o.p); std::swap(bytes, o.bytes); o.reset(); return *this; }
+    ~Mem() { reset(); }
+    void reset() { if (p) release(p); p = nullptr; bytes = 0; }
 };
+using Buf = Mem<void, cudaFree>;             // device memory
+using HostBuf = Mem<uint8_t, cudaFreeHost>;  // pinned host memory
+
+template <class H, cudaError_t (*destroy)(H)>
+struct Handle {                              // a stream or an event
+    H h = nullptr;
+    Handle() = default;
+    Handle(const Handle&) = delete;
+    Handle& operator=(const Handle&) = delete;
+    ~Handle() { if (h) destroy(h); }
+    operator H() const { return h; }
+};
+using Stream = Handle<cudaStream_t, cudaStreamDestroy>;
+using Event = Handle<cudaEvent_t, cudaEventDestroy>;
 
 }  // namespace
 
+// Members are released in reverse order of declaration, after orbx_destroy has synchronized every stream: the stager
+// goes first, so its threads are joined before the pinned staging they copy into is freed, and the streams go last.
 struct orbx_ctx {
+    Stream stream;
+    Stream lane[HOST_LANES];                 // extra frame-range pipelines (lane 0 is `stream`)
+    Stream side[HOST_LANES];                 // per lane: high-priority stream of the small pyramid levels + their FAST bands
+    Event ev[N_STAGES + 2];                  // 0..6 bracket the six extraction stages, 7..8 the matcher
+    Event ev_sfork[HOST_LANES], ev_sjoin[HOST_LANES];
+    Event ev_fork, ev_join[HOST_LANES];
+
     int device = 0, nfeatures = 0, nlevels = 0, max_w = 0, max_h = 0, max_batch = 0;
     float scale_factor = 1.2f;
-    cudaStream_t stream = nullptr;
     std::string err;
     uint64_t launches = 0;
 
@@ -89,10 +120,6 @@ struct orbx_ctx {
     const int* view_counts = nullptr;
     int view_frames = 0;
     Buf mq, mt, mbest, msecond, mkeys, mstatus, mcounts;
-    int* h_small = nullptr;                  // pinned: counts[max_batch] + status[max_batch] + 1
-    uint8_t* h_stage_in = nullptr; size_t h_stage_in_bytes = 0;     // pinned staging of pageable caller frames (device layout)
-    uint8_t* h_stage_out = nullptr; size_t h_stage_out_bytes = 0;   // ... of results bound for pageable caller buffers
-    HostStager* stager = nullptr;            // copier threads, created by the first call that needs them
     int last_batch = 0;
 
     // device-resident map-point table (SURVEY 8(f).1): slot-addressed columns + the host's id -> slot index
@@ -105,10 +132,10 @@ struct orbx_ctx {
     // asynchronous single-frame pipeline (orbx_submit_frame / orbx_collect_frame): two slots of pinned host staging and
     // device outputs, so the host can prepare / consume one frame while the GPU works on the other
     struct AsyncSlot {
-        uint8_t* h_in = nullptr; size_t h_in_bytes = 0;
-        uint8_t* h_out = nullptr; size_t h_out_bytes = 0;   // [counts 16 B][status 16 B][kps cap*28][desc cap*32]
+        Event done;
         Buf d_kps, d_desc, d_counts;
-        cudaEvent_t done = nullptr;
+        HostBuf h_in;
+        HostBuf h_out;                       // [counts 16 B][status 16 B][kps cap*28][desc cap*32]
         int cap = 0;
         bool busy = false;
     } aslot[2];
@@ -116,13 +143,28 @@ struct orbx_ctx {
 
     bool profiling = false;
     int force_kernels = -1;                   // orbx_debug_force_kernels: -1 by launch size, 0 warp-private TMA kernels, 1 CTA-cooperative kernels
-    cudaEvent_t ev[N_STAGES + 2] = {};   // 0..6 bracket the six extraction stages, 7..8 the matcher
-    cudaStream_t lane[HOST_LANES] = {};   // extra frame-range pipelines (lane 0 is `stream`)
-    cudaStream_t side[HOST_LANES] = {};   // per lane: high-priority stream of the small pyramid levels + their FAST bands
-    cudaEvent_t ev_sfork[HOST_LANES] = {}, ev_sjoin[HOST_LANES] = {};
-    cudaEvent_t ev_fork = nullptr, ev_join[HOST_LANES] = {};
     float stage_ms[N_STAGES] = {};
     bool stage_valid[N_STAGES] = {};
+
+    // Pinned words the synchronous entry points read back, in ints: [counts][status][match]
+    //   counts  max(max_batch, 3)  per-frame keypoint counts; orbx_track_match's candidate / match count and distance bounds
+    //   status  max_batch          per-frame device status
+    //   match   MATCH_WORDS        copies of the matcher status words
+    HostBuf h_small;
+    size_t h_small_bytes() const { return sizeof(int) * (std::max(max_batch, 3) + max_batch + MATCH_WORDS); }
+    int* h_counts() const { return (int*)h_small.p; }
+    int* h_status() const { return h_counts() + std::max(max_batch, 3); }
+    int* h_match() const { return h_status() + max_batch; }
+    HostBuf h_stage_in;                      // pinned staging of pageable caller frames (device layout)
+    HostBuf h_stage_out;                     // ... of results bound for pageable caller buffers
+    std::unique_ptr<HostStager> stager;      // copier threads, created by the first call that needs them
+
+    void synchronize_streams() const
+    {
+        cudaStreamSynchronize(stream);
+        for (int k = 1; k < HOST_LANES; ++k) cudaStreamSynchronize(lane[k]);
+        for (const Stream& s : side) cudaStreamSynchronize(s);
+    }
 };
 
 namespace {
@@ -146,10 +188,20 @@ int fail(orbx_ctx* c, int code, const char* fmt, const char* a = "", const char*
 int ensure(orbx_ctx* c, Buf& b, size_t bytes)
 {
     if (b.bytes >= bytes && b.p) return ORBX_OK;
-    if (b.p) { cudaFree(b.p); b.p = nullptr; b.bytes = 0; }
+    b.reset();
     bytes = std::max<size_t>(bytes, 256);
     cudaError_t e = cudaMalloc(&b.p, bytes);
     if (e != cudaSuccess) return fail(c, ORBX_E_NOMEM, "cudaMalloc failed: %s", cudaGetErrorString(e));
+    b.bytes = bytes;
+    return ORBX_OK;
+}
+
+int ensure(orbx_ctx* c, HostBuf& b, size_t bytes, const char* what)
+{
+    if (b.bytes >= bytes && b.p) return ORBX_OK;
+    b.reset();
+    bytes = std::max<size_t>(bytes, 4096);
+    if (cudaMallocHost((void**)&b.p, bytes) != cudaSuccess) { cudaGetLastError(); return fail(c, ORBX_E_NOMEM, "%s", what); }
     b.bytes = bytes;
     return ORBX_OK;
 }
@@ -284,12 +336,24 @@ void build_geom(const orbx_ctx* c, int w, int h, Geom* g, std::vector<uint32_t>*
     }
 }
 
-// One 3-D u8 tensor map (x = pitch, y = rows, z = frame) per pyramid level over the context's pyramid buffer: k_fast_warp's
-// image tiles are TMA boxes of FW_TP x FW_TR x 1 (out-of-range parts are zero-filled by the hardware).
+typedef CUresult (*enc_t)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*, const cuuint32_t*, const cuuint32_t*,
+                          CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+
+// A 3-D u8 tensor map (x = pitch, y = rows, z = frame) over level L of `base` (the pyramid or the blurred pyramid, one
+// frame every g.pyr_frame bytes) with boxes of bw x bh x 1; the hardware zero-fills the parts of a box outside the level.
+bool encode_level(enc_t enc, const orbx_ctx* c, CUtensorMap* m, const Buf& base, const LevelGeom& L, int bw, int bh)
+{
+    const cuuint64_t dims[3] = {(cuuint64_t)L.pitch, (cuuint64_t)L.h, (cuuint64_t)c->max_batch};
+    const cuuint64_t strides[2] = {(cuuint64_t)L.pitch, (cuuint64_t)c->geom.pyr_frame};
+    const cuuint32_t box[3] = {(cuuint32_t)bw, (cuuint32_t)bh, 1}, es[3] = {1, 1, 1};
+    return enc(m, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, (uint8_t*)base.p + L.img_off, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
+               CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+}
+
+// The tensor maps of the current geometry: k_fast_warp's image tiles (FW_TP x FW_TR boxes of every pyramid level),
+// k_pyr_tma's source boxes (each level as the source of the next) and k_describe_tma's windows (pyramid and blurred levels).
 int build_fast_maps(orbx_ctx* c)
 {
-    typedef CUresult (*enc_t)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*, const cuuint32_t*, const cuuint32_t*,
-                              CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
     static enc_t enc = nullptr;
     if (!enc) {
         void* fn = nullptr;
@@ -303,48 +367,34 @@ int build_fast_maps(orbx_ctx* c)
     for (int l = 0; l < g.nlevels; ++l) {
         const LevelGeom& L = g.L[l];
         if (L.nbands <= 0 || L.in_w <= 0) continue;
-        const cuuint64_t dims[3] = {(cuuint64_t)L.pitch, (cuuint64_t)L.h, (cuuint64_t)c->max_batch};
-        const cuuint64_t strides[2] = {(cuuint64_t)L.pitch, (cuuint64_t)g.pyr_frame};
-        const cuuint32_t box[3] = {FW_TP, FW_TR, 1}, es[3] = {1, 1, 1};
-        const CUresult r = enc(&c->fmaps.m[l], CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, (uint8_t*)c->pyr.p + L.img_off, dims, strides, box, es,
-                               CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) return fail(c, ORBX_E_CUDA, "cuTensorMapEncodeTiled failed for a pyramid level");
+        if (!encode_level(enc, c, &c->fmaps.m[l], c->pyr, L, FW_TP, FW_TR)) return fail(c, ORBX_E_CUDA, "cuTensorMapEncodeTiled failed for a pyramid level");
     }
     memset(&c->pmaps, 0, sizeof c->pmaps);
     for (int l = 1; l < g.nlevels; ++l) {
         const LevelGeom& D = g.L[l];
-        const LevelGeom& S = g.L[l - 1];
-        if (!D.pt_ok) continue;
-        const cuuint64_t dims[3] = {(cuuint64_t)S.pitch, (cuuint64_t)S.h, (cuuint64_t)c->max_batch};
-        const cuuint64_t strides[2] = {(cuuint64_t)S.pitch, (cuuint64_t)g.pyr_frame};
-        const cuuint32_t box[3] = {(cuuint32_t)D.pt_bw, (cuuint32_t)D.pt_bh, 1}, es[3] = {1, 1, 1};
-        const CUresult r = enc(&c->pmaps.m[l], CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, (uint8_t*)c->pyr.p + S.img_off, dims, strides, box, es,
-                               CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) return fail(c, ORBX_E_CUDA, "cuTensorMapEncodeTiled failed for a pyramid source level");
+        if (D.pt_ok && !encode_level(enc, c, &c->pmaps.m[l], c->pyr, g.L[l - 1], D.pt_bw, D.pt_bh))
+            return fail(c, ORBX_E_CUDA, "cuTensorMapEncodeTiled failed for a pyramid source level");
     }
     memset(&c->dmaps, 0, sizeof c->dmaps);
     for (int l = 0; l < g.nlevels; ++l) {
         const LevelGeom& L = g.L[l];
         if (L.in_w <= 0) continue;
-        const cuuint64_t dims[3] = {(cuuint64_t)L.pitch, (cuuint64_t)L.h, (cuuint64_t)c->max_batch};
-        const cuuint64_t strides[2] = {(cuuint64_t)L.pitch, (cuuint64_t)g.pyr_frame};
-        const cuuint32_t box_ic[3] = {DS_ICW, DS_ICH, 1}, box_bl[3] = {DS_BLW, DS_BLH, 1}, es[3] = {1, 1, 1};
-        if (enc(&c->dmaps.ic[l], CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, (uint8_t*)c->pyr.p + L.img_off, dims, strides, box_ic, es,
-                CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS ||
-            enc(&c->dmaps.bl[l], CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, (uint8_t*)c->blur.p + L.img_off, dims, strides, box_bl, es,
-                CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
+        if (!encode_level(enc, c, &c->dmaps.ic[l], c->pyr, L, DS_ICW, DS_ICH) || !encode_level(enc, c, &c->dmaps.bl[l], c->blur, L, DS_BLW, DS_BLH))
             return fail(c, ORBX_E_CUDA, "cuTensorMapEncodeTiled failed for a descriptor window map");
     }
     return ORBX_OK;
 }
 
+// The cached size (geom_w, geom_h) is cleared first and stored last, so a failure anywhere in between leaves a context
+// that rebuilds its geometry, tap table and tensor maps on the next call.
 int set_geometry(orbx_ctx* c, int w, int h)
 {
     if (c->geom_w == w && c->geom_h == h) return ORBX_OK;
+    c->geom_w = c->geom_h = -1;
     std::vector<uint32_t> tabs;
     build_geom(c, w, h, &c->geom, &tabs);
     for (int l = 1; l < c->nlevels; ++l)
-        if (c->geom.L[l].xspan > 11) { c->geom_w = c->geom_h = -1; return fail(c, ORBX_E_UNSUPPORTED, "scale_factor too large for the pyramid kernels (4 outputs must span <= 12 source bytes: about 2.6)"); }
+        if (c->geom.L[l].xspan > 11) return fail(c, ORBX_E_UNSUPPORTED, "scale_factor too large for the pyramid kernels (4 outputs must span <= 12 source bytes: about 2.6)");
     int rc = ensure(c, c->tabs, tabs.size() * 4);
     if (rc) return rc;
     CU(cudaMemcpyAsync(c->tabs.p, tabs.data(), tabs.size() * 4, cudaMemcpyHostToDevice, c->stream));
@@ -395,6 +445,31 @@ int run_extract_range(orbx_ctx* c, cudaStream_t st, int lane_id, bool marks, int
     cudaStream_t side = c->side[lane_id];
     cudaEvent_t side_fork = c->ev_sfork[lane_id], side_join = c->ev_sjoin[lane_id];
 
+    // ---- kernel choice for this call (orbx_debug_force_kernels: 0 pins the warp kernels, 1 the CTA-cooperative ones)
+    // Pyramid / FAST by the size of the launch: the warp-private TMA kernels (one warp walks a whole band / a stack of strips)
+    // win once there are enough warps to fill the GPU; below about 26 VGA frames' worth of pixels the CTA-cooperative
+    // kernels have the shorter critical path (one 640x480 frame: pyramid + FAST 0.077 ms against 0.115 ms), which is what the
+    // sequential VO loop (one frame per call, src/frontend.cpp:98-108) feels.
+    const bool cta_family = c->force_kernels >= 0 ? c->force_kernels != 0 : (long)nb * g.w * g.h < 8000000L;
+    // Selection by problem size: one WARP per (frame, level) when the candidate lists are short and there are thousands of
+    // them (256 VGA frames: 0.116 ms against 0.17 ms), one CTA per (frame, level) when the lists are long -- 512 threads wide
+    // there (64 frames of 1920x1080: 0.30 ms against 0.43 ms with 128 threads and 0.65 ms with warps; 3840x2160: 1.21
+    // against 1.88 and 2.57 ms).  sel_cta_threads = 0: the warp trio k_select_fast, k_harris, k_select_harris.
+    const bool wide = (long)g.w * g.h > 600000L;
+    const bool cta_select = c->force_kernels >= 0 ? c->force_kernels != 0 : wide;
+    const int sel_cta_threads = !cta_select ? 0 : wide ? SEL_NT_WIDE : SEL_NT;
+    // The small upper levels are a chain of short, latency-bound launches (at 640x480 levels 4..7 take as long as levels 1..3
+    // for a fifth of the pixels).  They leave the critical path: from level `lt` on, the pyramid chain and the FAST bands of
+    // those levels run on a HIGH-PRIORITY side stream (their few CTAs take the next free slots) underneath the FAST launch of the
+    // large levels, which is issue-bound and has slots to spare for them only in time, not in space.
+    int lt = g.nlevels;                                      // first level of the side chain
+    for (int l = g.nlevels - 1; l >= 2 && (long)g.L[l].w * g.L[l].h < SIDE_LEVEL_MAX_PX; --l) lt = l;
+    if (cta_family || g.total_bands <= 0 || marks) lt = g.nlevels;   // (stage timers on: one stream, clean per-stage times)
+    // Describe groups of 4 slots per warp: four per warp when the batch is large (the warp's set-up is shared, and there are
+    // still enough CTAs for several waves), one group per warp (lowest latency) when it is a single frame.
+    const long groups = (long)nb * ((std::min(std::max(cap, 1), std::max(c->nfeatures, 1)) + DS_G - 1) / DS_G);
+    const int gpw = groups >= 148L * 24 * 8 ? 4 : 1;   // measured at 256 VGA frames: 1 / 2 / 4 / 8 / 16 -> 0.192 / 0.192 / 0.185 / 0.205 / 0.259 ms
+
     NvtxStages nv;
     nv.next("orbx:gray");
     if (marks) stage_mark(c, 0);
@@ -407,17 +482,11 @@ int run_extract_range(orbx_ctx* c, cudaStream_t st, int lane_id, bool marks, int
         ++c->launches;
     }
     if (marks) stage_mark(c, 1);
-    // Kernel choice by the size of the launch: the warp-private TMA kernels (one warp walks a whole band / a stack of strips)
-    // win once there are enough warps to fill the GPU; below about 26 VGA frames' worth of pixels the CTA-cooperative
-    // kernels have the shorter critical path (one 640x480 frame: pyramid + FAST 0.077 ms against 0.115 ms), which is what the
-    // sequential VO loop (one frame per call, src/frontend.cpp:98-108) feels.  orbx_debug_force_kernels pins one or the other.
-    const bool small_launch = (long)nb * g.w * g.h < 8000000L;
-    const bool old_pyr_fast = c->force_kernels >= 0 ? c->force_kernels != 0 : small_launch;
     auto launch_pyr = [&](int l, cudaStream_t s) {
         if (g.L[l].w <= 0 || g.L[l].h <= 0) return;
         const int nitems = (g.L[l].pitch / 8) * ((g.L[l].h + PYR_RH - 1) / PYR_RH);     // (column octet, row strip) work items
         const dim3 grd((unsigned)((nitems + PYR_NT - 1) / PYR_NT), B);
-        if (g.L[l].pt_ok && !old_pyr_fast)
+        if (g.L[l].pt_ok && !cta_family)
             k_pyr_tma<<<dim3((unsigned)((g.L[l].pt_ntask + PT_NWARP - 1) / PT_NWARP), B), PT_NWARP * 32,
                         PT_NWARP * pt_warp_bytes(g.L[l].pt_bw, g.L[l].pt_bh) + 128, s>>>(g, c->pmaps.m[l], l, f0, (uint8_t*)c->pyr.p, tabs, status);
         else if (g.L[l].xspan <= 7) k_pyr_down<false><<<grd, PYR_NT, 0, s>>>(g, l, pyr, tabs);
@@ -430,20 +499,13 @@ int run_extract_range(orbx_ctx* c, cudaStream_t st, int lane_id, bool marks, int
     bool blur_done = false;
     auto launch_fast = [&](int band_lo, int band_hi, cudaStream_t s) {
         if (band_hi <= band_lo) return;
-        if (old_pyr_fast) {
+        if (cta_family) {
             if (band_lo == 0) k_fast_bands<FAST_R, FAST_NT><<<dim3((unsigned)g.total_bands, B), FAST_NT, 0, s>>>(g, pyr, rowcnt, rowent);
         } else
             k_fast_warp<FAST_NWARP><<<dim3((unsigned)((band_hi - band_lo + FAST_NWARP - 1) / FAST_NWARP), B), FAST_NWARP * 32, FAST_NWARP * FW_WARP_BYTES + 128, s>>>(
                 g, c->fmaps, f0, band_lo, band_hi, rowcnt, rowent, status);
         ++c->launches;
     };
-    // The small upper levels are a chain of short, latency-bound launches (at 640x480 levels 4..7 take as long as levels 1..3
-    // for a fifth of the pixels).  They leave the critical path: from level `lt` on, the pyramid chain and the FAST bands of
-    // those levels run on a HIGH-PRIORITY side stream (their few CTAs take the next free slots) underneath the FAST launch of the
-    // large levels, which is issue-bound and has slots to spare for them only in time, not in space.
-    int lt = g.nlevels;                                      // first level of the side chain
-    for (int l = g.nlevels - 1; l >= 2 && (long)g.L[l].w * g.L[l].h < SIDE_LEVEL_MAX_PX; --l) lt = l;
-    if (old_pyr_fast || g.total_bands <= 0 || marks) lt = g.nlevels;   // (stage timers on: one stream, clean per-stage times)
     nv.next("orbx:pyramid");
     for (int l = 1; l < lt; ++l) launch_pyr(l, st);
     if (marks) stage_mark(c, 2);
@@ -463,27 +525,18 @@ int run_extract_range(orbx_ctx* c, cudaStream_t st, int lane_id, bool marks, int
     } else if (g.total_bands > 0) launch_fast(0, g.total_bands, st);
     nv.next("orbx:select_harris");
     if (marks) stage_mark(c, 3);
-    {
-        // Selection kernel family by problem size: one WARP per (frame, level) when the candidate lists are short and there are
-        // thousands of them (256 VGA frames: 0.116 ms against 0.17 ms), one CTA per (frame, level) when the lists are long -- 512
-        // threads wide there (64 frames of 1920x1080: 0.30 ms against 0.43 ms with 128 threads and 0.65 ms with warps;
-        // 3840x2160: 1.21 against 1.88 and 2.57 ms).
-        const bool wide = (long)g.w * g.h > 600000L;
-        const bool old_sel = c->force_kernels >= 0 ? c->force_kernels != 0 : wide;
-        if (old_sel) {
-            if (wide) k_select<SEL_NT_WIDE><<<dim3(B, (unsigned)g.nlevels), SEL_NT_WIDE, 0, st>>>(g, pyr, rowcnt, rowent, work, selpos, fincnt, status);
-            else      k_select<SEL_NT><<<dim3(B, (unsigned)g.nlevels), SEL_NT, 0, st>>>(g, pyr, rowcnt, rowent, work, selpos, fincnt, status);
-            ++c->launches;
-        }
-        else {
-            // (the warp going straight on to Harris and the second retainBest -- one launch instead of three -- was measured: 0.1435 ms
-            //  against 0.1159 ms per 256 VGA frames; the 14 serial Harris evaluations per lane cost the level-0 warps more than the
-            //  two launch gaps and the Harris kernel's tail)
-            k_select_fast<<<dim3(B, (unsigned)g.nlevels), 32, 0, st>>>(g, rowcnt, rowent, work, selpos, selcnt, fincnt);
-            if (g.total_hblk > 0) k_harris<<<dim3((unsigned)g.total_hblk, B), HARRIS_NT, 0, st>>>(g, pyr, work, selcnt);
-            k_select_harris<<<dim3(B, (unsigned)g.nlevels), 32, (size_t)g.selh_elems * 12, st>>>(g, work, selpos, selcnt, fincnt, g.selh_elems);
-            c->launches += 3;
-        }
+    if (sel_cta_threads > 0) {
+        if (sel_cta_threads == SEL_NT_WIDE) k_select<SEL_NT_WIDE><<<dim3(B, (unsigned)g.nlevels), SEL_NT_WIDE, 0, st>>>(g, pyr, rowcnt, rowent, work, selpos, fincnt, status);
+        else                                k_select<SEL_NT><<<dim3(B, (unsigned)g.nlevels), SEL_NT, 0, st>>>(g, pyr, rowcnt, rowent, work, selpos, fincnt, status);
+        ++c->launches;
+    } else {
+        // (the warp going straight on to Harris and the second retainBest -- one launch instead of three -- was measured: 0.1435 ms
+        //  against 0.1159 ms per 256 VGA frames; the 14 serial Harris evaluations per lane cost the level-0 warps more than the
+        //  two launch gaps and the Harris kernel's tail)
+        k_select_fast<<<dim3(B, (unsigned)g.nlevels), 32, 0, st>>>(g, rowcnt, rowent, work, selpos, selcnt, fincnt);
+        if (g.total_hblk > 0) k_harris<<<dim3((unsigned)g.total_hblk, B), HARRIS_NT, 0, st>>>(g, pyr, work, selcnt);
+        k_select_harris<<<dim3(B, (unsigned)g.nlevels), 32, (size_t)g.selh_elems * 12, st>>>(g, work, selpos, selcnt, fincnt, g.selh_elems);
+        c->launches += 3;
     }
     nv.next("orbx:blur");
     if (marks) stage_mark(c, 4);
@@ -493,15 +546,9 @@ int run_extract_range(orbx_ctx* c, cudaStream_t st, int lane_id, bool marks, int
     }
     nv.next("orbx:describe");
     if (marks) stage_mark(c, 5);
-    {
-        // groups of 4 slots per warp: four per warp when the batch is large (the warp's set-up is shared, and there are still
-        // enough CTAs for several waves), one group per warp (lowest latency) when it is a single frame
-        const long groups = (long)nb * ((std::min(std::max(cap, 1), std::max(c->nfeatures, 1)) + DS_G - 1) / DS_G);
-        const int gpw = groups >= 148L * 24 * 8 ? 4 : 1;   // measured at 256 VGA frames: 1 / 2 / 4 / 8 / 16 -> 0.192 / 0.192 / 0.185 / 0.205 / 0.259 ms
-        const int gcap = (std::max(cap, 1) + DS_G - 1) / DS_G;
-        k_describe_tma<<<dim3((unsigned)((gcap + DS_NW * gpw - 1) / (DS_NW * gpw)), B), DS_NW * 32, DS_NW * DS_WARP_BYTES + 128, st>>>(
-            g, c->dmaps, f0, work, fincnt, (const float4*)c->pattern.p, d_kps, d_desc, d_counts, cap, gpw, status);
-    }
+    const int gcap = (std::max(cap, 1) + DS_G - 1) / DS_G;
+    k_describe_tma<<<dim3((unsigned)((gcap + DS_NW * gpw - 1) / (DS_NW * gpw)), B), DS_NW * 32, DS_NW * DS_WARP_BYTES + 128, st>>>(
+        g, c->dmaps, f0, work, fincnt, (const float4*)c->pattern.p, d_kps, d_desc, d_counts, cap, gpw, status);
     ++c->launches;
     if (marks) stage_mark(c, 6);
     return ORBX_OK;
@@ -557,8 +604,19 @@ int check_args_extract(orbx_ctx* c, int batch, int w, int h, int channels, int c
 // call starts clean without a per-call memset on the matcher's critical path, and report.
 int match_timed_out(orbx_ctx* c)
 {
-    cudaMemset(c->mstatus.p, 0, sizeof(int) * 16);
+    cudaMemset(c->mstatus.p, 0, sizeof(int) * MATCH_WORDS);
     return fail(c, ORBX_E_INTERNAL, "matcher pipeline timed out on an mbarrier (device status set)");
+}
+
+// Matcher status words [slot, slot + n) -> h_match(), behind everything queued on the context's stream; then wait for
+// that stream and report a timeout if any of the words is set.
+int sync_match_words(orbx_ctx* c, int slot, int n)
+{
+    int* h = c->h_match() + slot;
+    if (n > 0) CU(cudaMemcpyAsync(h, (int*)c->mstatus.p + slot, sizeof(int) * n, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    for (int i = 0; i < n; ++i) if (h[i]) return match_timed_out(c);
+    return ORBX_OK;
 }
 
 // The matcher on device-resident operands, asynchronous on `st` (default: the context's stream).  `slot` selects the
@@ -605,7 +663,6 @@ int run_match(orbx_ctx* c, const uint8_t* d_q, int nq, const uint8_t* d_t, int n
     int* keys = nullptr;
     const size_t nout = (size_t)nq * nsets;
     int rc;
-    if ((rc = ensure(c, c->mstatus, sizeof(int) * 16))) return rc;
     int* d_status = (int*)c->mstatus.p + slot;               // zero since orbx_create; re-zeroed by match_timed_out() after a failure
     if (!lane_call) stage_mark(c, 7);
     if (nsplit > 1) {
@@ -629,7 +686,36 @@ int run_match(orbx_ctx* c, const uint8_t* d_q, int nq, const uint8_t* d_t, int n
     return ORBX_OK;
 }
 
-int match_host(orbx_ctx* c, const uint8_t* query, int nq, const uint8_t* train, int nt, orbx_match* out, int* n_out, bool knn2)
+// The host-buffer matcher, synchronous on the context's stream: nq query rows against nsets train sets of stride_rows rows
+// each (all of them, or as many as the host `counts` give per set).  best and second (when not null) receive [nsets][nq]
+// records each; with `pairs` (the second-best of one set), `best` receives [nq][2] {best, second} records instead.
+int match_host(orbx_ctx* c, const uint8_t* query, int nq, const uint8_t* train, int stride_rows, const int* counts, int nsets,
+               orbx_match* best, orbx_match* second, bool pairs)
+{
+    const size_t tbytes = (size_t)nsets * stride_rows * 32, obytes = (size_t)nsets * nq * 16;
+    const bool knn2 = pairs || second;
+    int rc;
+    if ((rc = ensure(c, c->mq, (size_t)nq * 32)) || (rc = ensure(c, c->mt, tbytes)) || (rc = ensure(c, c->mbest, obytes)) ||
+        (knn2 && (rc = ensure(c, c->msecond, obytes))) || (counts && (rc = ensure(c, c->mcounts, sizeof(int) * (size_t)nsets))))
+        return rc;
+    CU(cudaMemcpyAsync(c->mq.p, query, (size_t)nq * 32, cudaMemcpyHostToDevice, c->stream));
+    CU(cudaMemcpyAsync(c->mt.p, train, tbytes, cudaMemcpyHostToDevice, c->stream));
+    if (counts) CU(cudaMemcpyAsync(c->mcounts.p, counts, sizeof(int) * (size_t)nsets, cudaMemcpyHostToDevice, c->stream));
+    if ((rc = run_match(c, (const uint8_t*)c->mq.p, nq, (const uint8_t*)c->mt.p, stride_rows, stride_rows, counts ? (const int*)c->mcounts.p : nullptr,
+                        nsets, (int4*)c->mbest.p, knn2 ? (int4*)c->msecond.p : nullptr)))
+        return rc;
+    if (pairs) {
+        CU(cudaMemcpy2DAsync(best, 32, c->mbest.p, 16, 16, (size_t)nq, cudaMemcpyDeviceToHost, c->stream));
+        CU(cudaMemcpy2DAsync(best + 1, 32, c->msecond.p, 16, 16, (size_t)nq, cudaMemcpyDeviceToHost, c->stream));
+    } else {
+        CU(cudaMemcpyAsync(best, c->mbest.p, obytes, cudaMemcpyDeviceToHost, c->stream));
+        if (second) CU(cudaMemcpyAsync(second, c->msecond.p, obytes, cudaMemcpyDeviceToHost, c->stream));
+    }
+    return sync_match_words(c, 0, 1);
+}
+
+// orbx_match_hamming / orbx_match_hamming_knn2: one train set of nt rows
+int match_one_set(orbx_ctx* c, const uint8_t* query, int nq, const uint8_t* train, int nt, orbx_match* out, int* n_out, bool knn2)
 {
     if (!c) return ORBX_E_ARG;
     if (n_out) *n_out = 0;
@@ -637,23 +723,8 @@ int match_host(orbx_ctx* c, const uint8_t* query, int nq, const uint8_t* train, 
     if (nq == 0 || nt == 0) return ORBX_OK;                 // cv: empty query or train -> no matches, no throw
     if (!query || !train || !out) return fail(c, ORBX_E_ARG, "null pointer");
     CU(cudaSetDevice(c->device));
-    int rc;
-    if ((rc = ensure(c, c->mq, (size_t)nq * 32))) return rc;
-    if ((rc = ensure(c, c->mt, (size_t)nt * 32))) return rc;
-    if ((rc = ensure(c, c->mbest, (size_t)nq * 16))) return rc;
-    if (knn2 && (rc = ensure(c, c->msecond, (size_t)nq * 16))) return rc;
-    CU(cudaMemcpyAsync(c->mq.p, query, (size_t)nq * 32, cudaMemcpyHostToDevice, c->stream));
-    CU(cudaMemcpyAsync(c->mt.p, train, (size_t)nt * 32, cudaMemcpyHostToDevice, c->stream));
-    if ((rc = run_match(c, (const uint8_t*)c->mq.p, nq, (const uint8_t*)c->mt.p, nt, nt, nullptr, 1, (int4*)c->mbest.p, knn2 ? (int4*)c->msecond.p : nullptr))) return rc;
-    if (!knn2) {
-        CU(cudaMemcpyAsync(out, c->mbest.p, (size_t)nq * 16, cudaMemcpyDeviceToHost, c->stream));
-    } else {
-        CU(cudaMemcpy2DAsync(out, 32, c->mbest.p, 16, 16, (size_t)nq, cudaMemcpyDeviceToHost, c->stream));
-        CU(cudaMemcpy2DAsync(out + 1, 32, c->msecond.p, 16, 16, (size_t)nq, cudaMemcpyDeviceToHost, c->stream));
-    }
-    CU(cudaMemcpyAsync(c->h_small, c->mstatus.p, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaStreamSynchronize(c->stream));
-    if (c->h_small[0]) return match_timed_out(c);
+    const int rc = match_host(c, query, nq, train, nt, nullptr, 1, out, nullptr, knn2);
+    if (rc) return rc;
     if (n_out) *n_out = nq;
     return ORBX_OK;
 }
@@ -674,46 +745,46 @@ int orbx_create(orbx_ctx** out, int device, int nfeatures, float scale_factor, i
         return ORBX_E_ARG;
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0 || device < 0 || device >= ndev) return ORBX_E_CUDA;
-    orbx_ctx* c = new (std::nothrow) orbx_ctx();
+    std::unique_ptr<orbx_ctx> owner(new (std::nothrow) orbx_ctx());   // a failure below deletes the partly built context
+    orbx_ctx* c = owner.get();
     if (!c) return ORBX_E_NOMEM;
     c->device = device; c->nfeatures = nfeatures; c->scale_factor = scale_factor; c->nlevels = nlevels;
     c->max_w = max_w; c->max_h = max_h; c->max_batch = max_batch;
-    auto bail = [&](int code) { orbx_destroy(c); return code; };
-    if (cudaSetDevice(device) != cudaSuccess) return bail(ORBX_E_CUDA);
+    if (cudaSetDevice(device) != cudaSuccess) return ORBX_E_CUDA;
     cudaDeviceProp prop;
-    if (cudaGetDeviceProperties(&prop, device) != cudaSuccess) return bail(ORBX_E_CUDA);
-    if (prop.major != 10) return bail(ORBX_E_CUDA);          // sm_100a only: no other code path exists
-    if (cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking) != cudaSuccess) return bail(ORBX_E_CUDA);
+    if (cudaGetDeviceProperties(&prop, device) != cudaSuccess) return ORBX_E_CUDA;
+    if (prop.major != 10) return ORBX_E_CUDA;                // sm_100a only: no other code path exists
+    int prio_lo = 0, prio_hi = 0;
+    if (cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi) != cudaSuccess) return ORBX_E_CUDA;
+    if (cudaStreamCreateWithFlags(&c->stream.h, cudaStreamNonBlocking) != cudaSuccess) return ORBX_E_CUDA;
     for (int k = 0; k < HOST_LANES; ++k)
-        if ((k > 0 && cudaStreamCreateWithFlags(&c->lane[k], cudaStreamNonBlocking) != cudaSuccess) || cudaEventCreateWithFlags(&c->ev_join[k], cudaEventDisableTiming) != cudaSuccess) return bail(ORBX_E_CUDA);
-    if (cudaEventCreateWithFlags(&c->ev_fork, cudaEventDisableTiming) != cudaSuccess) return bail(ORBX_E_CUDA);
-    {
-        int prio_lo = 0, prio_hi = 0;
-        if (cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi) != cudaSuccess) return bail(ORBX_E_CUDA);
-        for (int k = 0; k < HOST_LANES; ++k)
-            if (cudaStreamCreateWithPriority(&c->side[k], cudaStreamNonBlocking, prio_hi) != cudaSuccess ||
-                cudaEventCreateWithFlags(&c->ev_sfork[k], cudaEventDisableTiming) != cudaSuccess ||
-                cudaEventCreateWithFlags(&c->ev_sjoin[k], cudaEventDisableTiming) != cudaSuccess) return bail(ORBX_E_CUDA);
-    }
-    for (int i = 0; i < N_STAGES + 2; ++i) if (cudaEventCreate(&c->ev[i]) != cudaSuccess) return bail(ORBX_E_CUDA);
+        if ((k > 0 && cudaStreamCreateWithFlags(&c->lane[k].h, cudaStreamNonBlocking) != cudaSuccess) ||
+            cudaStreamCreateWithPriority(&c->side[k].h, cudaStreamNonBlocking, prio_hi) != cudaSuccess ||
+            cudaEventCreateWithFlags(&c->ev_join[k].h, cudaEventDisableTiming) != cudaSuccess ||
+            cudaEventCreateWithFlags(&c->ev_sfork[k].h, cudaEventDisableTiming) != cudaSuccess ||
+            cudaEventCreateWithFlags(&c->ev_sjoin[k].h, cudaEventDisableTiming) != cudaSuccess)
+            return ORBX_E_CUDA;
+    if (cudaEventCreateWithFlags(&c->ev_fork.h, cudaEventDisableTiming) != cudaSuccess) return ORBX_E_CUDA;
+    for (auto& a : c->aslot) if (cudaEventCreateWithFlags(&a.done.h, cudaEventDisableTiming) != cudaSuccess) return ORBX_E_CUDA;
+    for (Event& e : c->ev) if (cudaEventCreate(&e.h) != cudaSuccess) return ORBX_E_CUDA;
     build_geom(c, max_w, max_h, &c->geom_max, nullptr);
     const Geom& g = c->geom_max;
     const size_t B = (size_t)max_batch;
     if (ensure(c, c->pyr, g.pyr_frame * B + (size_t)(96 + 8) * g.L[0].pitch) ||   // + slack: the blur streams up to ~100 rows past a level's end (masked outputs)
         ensure(c, c->blur, g.pyr_frame * B) || ensure(c, c->rowcnt, g.cnt_frame * 4 * B) || ensure(c, c->rowent, g.ent_frame * 4 * B) ||
         ensure(c, c->work, g.ws_frame * sizeof(Elem) * B) || ensure(c, c->selpos, g.ws_frame * 8 * B) || ensure(c, c->fincnt, sizeof(int) * ORBX_LEVELS_MAX * B) || ensure(c, c->selcnt, sizeof(int) * ORBX_LEVELS_MAX * B) ||
-        ensure(c, c->status, sizeof(int) * B) || ensure(c, c->pattern, sizeof(float) * 1024) || ensure(c, c->mstatus, sizeof(int) * 16))
-        return bail(ORBX_E_NOMEM);
-    if (cudaMemset(c->mstatus.p, 0, sizeof(int) * 16) != cudaSuccess) return bail(ORBX_E_CUDA);
+        ensure(c, c->status, sizeof(int) * B) || ensure(c, c->pattern, sizeof(float) * 1024) || ensure(c, c->mstatus, sizeof(int) * MATCH_WORDS) ||
+        ensure(c, c->h_small, c->h_small_bytes(), "cudaMallocHost failed"))
+        return ORBX_E_NOMEM;
+    if (cudaMemset(c->mstatus.p, 0, sizeof(int) * MATCH_WORDS) != cudaSuccess) return ORBX_E_CUDA;
     {
         float pat[1024];                                     // the rBRIEF pattern as float4 (x0, y0, x1, y1) per test,
         for (int t = 0; t < 8; ++t)                          // transposed to [t][lane]: test lane * 8 + t  (k_describe_tma)
             for (int lane = 0; lane < 32; ++lane)
                 for (int k = 0; k < 4; ++k) pat[(t * 32 + lane) * 4 + k] = (float)k_pattern_host[(lane * 8 + t) * 4 + k];
-        if (cudaMemcpy(c->pattern.p, pat, sizeof pat, cudaMemcpyHostToDevice) != cudaSuccess) return bail(ORBX_E_CUDA);
+        if (cudaMemcpy(c->pattern.p, pat, sizeof pat, cudaMemcpyHostToDevice) != cudaSuccess) return ORBX_E_CUDA;
     }
-    if (cudaMemset(c->status.p, 0, sizeof(int) * B) != cudaSuccess) return bail(ORBX_E_CUDA);
-    if (cudaMallocHost((void**)&c->h_small, sizeof(int) * (2 * B + 16)) != cudaSuccess) return bail(ORBX_E_NOMEM);
+    if (cudaMemset(c->status.p, 0, sizeof(int) * B) != cudaSuccess) return ORBX_E_CUDA;
     if (cudaFuncSetAttribute(k_hamming_umma2<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
         cudaFuncSetAttribute(k_hamming_umma2<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
         cudaFuncSetAttribute(k_hamming_umma<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
@@ -722,8 +793,8 @@ int orbx_create(orbx_ctx** out, int device, int nfeatures, float scale_factor, i
         cudaFuncSetAttribute(k_pyr_tma, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024) != cudaSuccess ||
         cudaFuncSetAttribute(k_describe_tma, cudaFuncAttributeMaxDynamicSharedMemorySize, DS_NW * DS_WARP_BYTES + 128) != cudaSuccess ||
         cudaFuncSetAttribute(k_select_harris, cudaFuncAttributeMaxDynamicSharedMemorySize, 16384 * 12) != cudaSuccess)
-        return bail(ORBX_E_CUDA);
-    *out = c;
+        return ORBX_E_CUDA;
+    *out = owner.release();
     return ORBX_OK;
 }
 
@@ -731,32 +802,7 @@ void orbx_destroy(orbx_ctx* c)
 {
     if (!c) return;
     cudaSetDevice(c->device);
-    if (c->stream) cudaStreamSynchronize(c->stream);
-    Buf* bufs[] = {&c->pyr, &c->blur, &c->rowcnt, &c->rowent, &c->work, &c->selpos, &c->fincnt, &c->selcnt, &c->status, &c->tabs, &c->pattern, &c->in, &c->kps,
-                   &c->desc, &c->counts, &c->mq, &c->mt, &c->mbest, &c->msecond, &c->mkeys, &c->mstatus, &c->mcounts,
-                   &c->t_desc, &c->t_pos, &c->t_nrm, &c->t_outl, &c->t_slots, &c->t_cand, &c->t_ncand, &c->t_q, &c->t_in, &c->t_best, &c->t_filtered,
-                   &c->t_minmax, &c->t_aux};
-    for (Buf* b : bufs) if (b->p) cudaFree(b->p);
-    if (c->h_small) cudaFreeHost(c->h_small);
-    delete c->stager;
-    if (c->h_stage_in) cudaFreeHost(c->h_stage_in);
-    if (c->h_stage_out) cudaFreeHost(c->h_stage_out);
-    for (auto& a : c->aslot) {
-        if (a.h_in) cudaFreeHost(a.h_in);
-        if (a.h_out) cudaFreeHost(a.h_out);
-        Buf* ab[] = {&a.d_kps, &a.d_desc, &a.d_counts};
-        for (Buf* b : ab) if (b->p) cudaFree(b->p);
-        if (a.done) cudaEventDestroy(a.done);
-    }
-    for (int i = 0; i < N_STAGES + 2; ++i) if (c->ev[i]) cudaEventDestroy(c->ev[i]);
-    for (int k = 0; k < HOST_LANES; ++k) { if (c->ev_join[k]) cudaEventDestroy(c->ev_join[k]); if (c->lane[k]) { cudaStreamSynchronize(c->lane[k]); cudaStreamDestroy(c->lane[k]); } }
-    if (c->ev_fork) cudaEventDestroy(c->ev_fork);
-    for (int k = 0; k < HOST_LANES; ++k) {
-        if (c->side[k]) { cudaStreamSynchronize(c->side[k]); cudaStreamDestroy(c->side[k]); }
-        if (c->ev_sfork[k]) cudaEventDestroy(c->ev_sfork[k]);
-        if (c->ev_sjoin[k]) cudaEventDestroy(c->ev_sjoin[k]);
-    }
-    if (c->stream) cudaStreamDestroy(c->stream);
+    c->synchronize_streams();
     delete c;
 }
 
@@ -769,13 +815,11 @@ int orbx_synchronize(orbx_ctx* c)
     if (!c) return ORBX_E_ARG;
     CU(cudaSetDevice(c->device));
     const int b = c->last_batch;
-    if (b > 0) CU(cudaMemcpyAsync(c->h_small, c->status.p, sizeof(int) * (size_t)b, cudaMemcpyDeviceToHost, c->stream));
-    int* h_m = c->h_small + 2 * (size_t)c->max_batch;        // the asynchronous matcher entry points defer their status words to this call
-    CU(cudaMemcpyAsync(h_m, c->mstatus.p, sizeof(int) * 16, cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaStreamSynchronize(c->stream));
-    for (int i = 0; i < 16; ++i) if (h_m[i]) return match_timed_out(c);
+    if (b > 0) CU(cudaMemcpyAsync(c->h_status(), c->status.p, sizeof(int) * (size_t)b, cudaMemcpyDeviceToHost, c->stream));
+    const int rc = sync_match_words(c, 0, MATCH_WORDS);     // the asynchronous matcher entry points defer their status words to this call
+    if (rc) return rc;
     for (int i = 0; i < b; ++i)
-        if (c->h_small[i]) return fail(c, ORBX_E_INTERNAL, "device-side status set for a frame");
+        if (c->h_status()[i]) return fail(c, ORBX_E_INTERNAL, "device-side status set for a frame");
     return ORBX_OK;
 }
 
@@ -804,23 +848,13 @@ static bool host_ptr_is_pinned(const void* p)
     return a.type == cudaMemoryTypeHost || a.type == cudaMemoryTypeManaged;
 }
 
-static int ensure_pinned(orbx_ctx* c, uint8_t*& p, size_t& have, size_t bytes)
-{
-    if (have >= bytes && p) return ORBX_OK;
-    if (p) { cudaFreeHost(p); p = nullptr; have = 0; }
-    bytes = std::max<size_t>(bytes, 4096);
-    if (cudaMallocHost((void**)&p, bytes) != cudaSuccess) { cudaGetLastError(); return fail(c, ORBX_E_NOMEM, "cudaMallocHost failed for the pinned staging buffer"); }
-    have = bytes;
-    return ORBX_OK;
-}
-
 static HostStager* stager_of(orbx_ctx* c)
 {
     if (!c->stager) {
         int n = getenv("ORBX_STAGE_THREADS") ? atoi(getenv("ORBX_STAGE_THREADS")) : (int)std::min(8u, std::max(2u, std::thread::hardware_concurrency() / 2));
-        c->stager = new HostStager(std::max(0, std::min(n, 32)));
+        c->stager.reset(new HostStager(std::max(0, std::min(n, 32))));
     }
-    return c->stager;
+    return c->stager.get();
 }
 
 static int host_batch(orbx_ctx* c, const uint8_t* const* imgs, int batch, int w, int h, size_t step, int channels,
@@ -837,8 +871,7 @@ static int host_batch(orbx_ctx* c, const uint8_t* const* imgs, int batch, int w,
     if ((rc = ensure(c, c->in, fstride * batch)) || (rc = ensure(c, c->kps, sizeof(orbx_keypoint) * capz * batch)) ||
         (rc = ensure(c, c->desc, (size_t)32 * capz * batch)) || (rc = ensure(c, c->counts, sizeof(int) * (size_t)batch)))
         return rc;
-    if (nmaps > 0 && ((rc = ensure(c, c->mq, std::max<size_t>(qrows, 1) * 32)) || (rc = ensure(c, c->mbest, std::max<size_t>(mrows, 1) * 16)) ||
-                      (rc = ensure(c, c->mstatus, sizeof(int) * 16))))
+    if (nmaps > 0 && ((rc = ensure(c, c->mq, std::max<size_t>(qrows, 1) * 32)) || (rc = ensure(c, c->mbest, std::max<size_t>(mrows, 1) * 16))))
         return rc;
     for (int i = 0; i < batch; ++i) if (!imgs[i]) return fail(c, ORBX_E_ARG, "null frame pointer");
     if ((rc = set_geometry(c, w, h))) return rc;
@@ -849,12 +882,13 @@ static int host_batch(orbx_ctx* c, const uint8_t* const* imgs, int batch, int w,
     if (cap > 0) stage_out = !(host_ptr_is_pinned(kps) && host_ptr_is_pinned(desc));
     for (int j = 0; j < nmaps && !stage_out; ++j) if (nq[j] > 0 && !host_ptr_is_pinned(best[j])) stage_out = true;
     const size_t o_kps = 0, o_desc = round_up(sizeof(orbx_keypoint) * capz * batch, 256), o_best = o_desc + round_up((size_t)32 * capz * batch, 256);
-    if (stage_in && (rc = ensure_pinned(c, c->h_stage_in, c->h_stage_in_bytes, fstride * batch))) return rc;
-    if (stage_out && (rc = ensure_pinned(c, c->h_stage_out, c->h_stage_out_bytes, o_best + mrows * 16))) return rc;
+    const char* no_pinned = "cudaMallocHost failed for the pinned staging buffer";
+    if (stage_in && (rc = ensure(c, c->h_stage_in, fstride * batch, no_pinned))) return rc;
+    if (stage_out && (rc = ensure(c, c->h_stage_out, o_best + mrows * 16, no_pinned))) return rc;
     HostStager* hs = (stage_in || stage_out) ? stager_of(c) : nullptr;
     const bool wake_in = fstride * batch >= STAGE_WAKE_BYTES, wake_out = (size_t)60 * capz * batch + mrows * 16 >= STAGE_WAKE_BYTES;
-    orbx_keypoint* kps_dl = stage_out ? (orbx_keypoint*)(c->h_stage_out + o_kps) : kps;       // where the D2H copies land
-    uint8_t* desc_dl = stage_out ? c->h_stage_out + o_desc : desc;
+    orbx_keypoint* kps_dl = stage_out ? (orbx_keypoint*)(c->h_stage_out.p + o_kps) : kps;       // where the D2H copies land
+    uint8_t* desc_dl = stage_out ? c->h_stage_out.p + o_desc : desc;
 
     CU(cudaMemsetAsync(c->status.p, 0, sizeof(int) * (size_t)batch, c->stream));
     {
@@ -864,9 +898,8 @@ static int host_batch(orbx_ctx* c, const uint8_t* const* imgs, int batch, int w,
             off += (size_t)nq[j];
         }
     }
-    int* h_counts = c->h_small;
-    int* h_status = c->h_small + batch;
-    int* h_mstatus = c->h_small + 2 * batch;
+    int* h_counts = c->h_counts();
+    int* h_status = c->h_status();
     const int lanes = c->profiling ? 1 : std::max(1, std::min(HOST_LANES, batch / HOST_LANE_MIN_FRAMES));
     // staged inputs: all pieces are queued up front, lane by lane, so the copier threads run ahead of the lane loop
     std::atomic<int> in_done[HOST_LANES], out_done(0);
@@ -880,7 +913,7 @@ static int host_batch(orbx_ctx* c, const uint8_t* const* imgs, int batch, int w,
             int f0, f1;
             host_lane_range(batch, lanes, k, &f0, &f1);
             in_done[k].store(0, std::memory_order_relaxed);
-            for (int i = f0; i < f1; ++i) in_target[k] += hs->submit(c->h_stage_in + fstride * i, dstep, imgs[i], step, row, (size_t)h, &in_done[k], wake_in, true);
+            for (int i = f0; i < f1; ++i) in_target[k] += hs->submit(c->h_stage_in.p + fstride * i, dstep, imgs[i], step, row, (size_t)h, &in_done[k], wake_in, true);
         }
     CU(cudaEventRecord(c->ev_fork, c->stream));
     for (int k = 0; k < lanes; ++k) {
@@ -891,7 +924,7 @@ static int host_batch(orbx_ctx* c, const uint8_t* const* imgs, int batch, int w,
         if (k > 0) CU(cudaStreamWaitEvent(st, c->ev_fork, 0));
         if (stage_in) {
             hs->help_until(in_done[k], in_target[k]);        // (the pinned image has the device layout: one copy per lane)
-            CU(cudaMemcpyAsync((uint8_t*)c->in.p + fstride * f0, c->h_stage_in + fstride * f0, fstride * n, cudaMemcpyHostToDevice, st));
+            CU(cudaMemcpyAsync((uint8_t*)c->in.p + fstride * f0, c->h_stage_in.p + fstride * f0, fstride * n, cudaMemcpyHostToDevice, st));
         } else if ((rc = upload_frames(c, st, imgs, f0, f1, step, row, h, dstep, fstride))) return rc;
         if ((rc = run_extract_range(c, st, k, c->profiling, f0, f1 - f0, (const uint8_t*)c->in.p, dstep,
                                     fstride, channels, (float*)c->kps.p, (uint8_t*)c->desc.p, cap, (int*)c->counts.p)))
@@ -911,12 +944,11 @@ static int host_batch(orbx_ctx* c, const uint8_t* const* imgs, int batch, int w,
                 if ((rc = run_match(c, (const uint8_t*)c->mq.p + qoff * 32, nq[j], (const uint8_t*)c->desc.p + (size_t)f0 * cap * 32, cap, cap,
                                     (const int*)c->counts.p + f0, (int)n, d_best, nullptr, st, k)))
                     return rc;
-                orbx_match* dl = stage_out ? (orbx_match*)(c->h_stage_out + o_best) + moff + (size_t)f0 * nq[j] : best[j] + (size_t)f0 * nq[j];
+                orbx_match* dl = stage_out ? (orbx_match*)(c->h_stage_out.p + o_best) + moff + (size_t)f0 * nq[j] : best[j] + (size_t)f0 * nq[j];
                 CU(cudaMemcpyAsync(dl, d_best, (size_t)16 * nq[j] * n, cudaMemcpyDeviceToHost, st));
             }
             qoff += (size_t)nq[j]; moff += (size_t)nq[j] * batch;
         }
-        if (nmaps > 0) CU(cudaMemcpyAsync(h_mstatus + k, (int*)c->mstatus.p + k, sizeof(int), cudaMemcpyDeviceToHost, st));
         if (k > 0 || stage_out) CU(cudaEventRecord(c->ev_join[k], st));
         if (k > 0) CU(cudaStreamWaitEvent(c->stream, c->ev_join[k], 0));
     }
@@ -942,15 +974,14 @@ static int host_batch(orbx_ctx* c, const uint8_t* const* imgs, int batch, int w,
             size_t moff = 0;
             for (int j = 0; j < nmaps; ++j) {
                 if (nq[j] > 0)
-                    out_target += hs->submit(best[j] + (size_t)f0 * nq[j], 0, (orbx_match*)(c->h_stage_out + o_best) + moff + (size_t)f0 * nq[j], 0,
+                    out_target += hs->submit(best[j] + (size_t)f0 * nq[j], 0, (orbx_match*)(c->h_stage_out.p + o_best) + moff + (size_t)f0 * nq[j], 0,
                                              (size_t)16 * nq[j] * (size_t)(f1 - f0), 1, &out_done, wake_out);
                 moff += (size_t)nq[j] * batch;
             }
         }
         hs->help_until(out_done, out_target);
     }
-    CU(cudaStreamSynchronize(c->stream));
-    for (int k = 0; k < lanes; ++k) if (nmaps > 0 && h_mstatus[k]) return match_timed_out(c);
+    if ((rc = sync_match_words(c, 0, nmaps > 0 ? lanes : 0))) return rc;      // lane k's matches report in slot k
     bool over = false;
     for (int i = 0; i < batch; ++i) {
         if (h_status[i]) return fail(c, ORBX_E_INTERNAL, "device-side status set for a frame");
@@ -1025,11 +1056,11 @@ int orbx_detect_and_compute(orbx_ctx* c, const uint8_t* img, int w, int h, size_
 
 int orbx_match_hamming(orbx_ctx* c, const uint8_t* q, int nq, const uint8_t* t, int nt, orbx_match* out, int* n_out)
 {
-    return match_host(c, q, nq, t, nt, out, n_out, false);
+    return match_one_set(c, q, nq, t, nt, out, n_out, false);
 }
 int orbx_match_hamming_knn2(orbx_ctx* c, const uint8_t* q, int nq, const uint8_t* t, int nt, orbx_match* out, int* n_out)
 {
-    return match_host(c, q, nq, t, nt, out, n_out, true);
+    return match_one_set(c, q, nq, t, nt, out, n_out, true);
 }
 
 int orbx_match_hamming_device(orbx_ctx* c, const uint8_t* d_query, int nq, const uint8_t* d_train, int nt, int nsets,
@@ -1062,23 +1093,7 @@ int orbx_match_hamming_sets(orbx_ctx* c, const uint8_t* query, int nq, const uin
     if (nq == 0 || train_stride_rows == 0 || nsets == 0) return ORBX_OK;
     if (!query || !train || !best || !train_counts) return fail(c, ORBX_E_ARG, "null pointer");
     CU(cudaSetDevice(c->device));
-    const size_t tbytes = (size_t)nsets * train_stride_rows * 32, obytes = (size_t)nsets * nq * 16;
-    int rc;
-    if ((rc = ensure(c, c->mq, (size_t)nq * 32)) || (rc = ensure(c, c->mt, tbytes)) || (rc = ensure(c, c->mbest, obytes)) ||
-        (rc = ensure(c, c->mcounts, sizeof(int) * (size_t)nsets)) || (second && (rc = ensure(c, c->msecond, obytes))))
-        return rc;
-    CU(cudaMemcpyAsync(c->mq.p, query, (size_t)nq * 32, cudaMemcpyHostToDevice, c->stream));
-    CU(cudaMemcpyAsync(c->mt.p, train, tbytes, cudaMemcpyHostToDevice, c->stream));
-    CU(cudaMemcpyAsync(c->mcounts.p, train_counts, sizeof(int) * (size_t)nsets, cudaMemcpyHostToDevice, c->stream));
-    if ((rc = run_match(c, (const uint8_t*)c->mq.p, nq, (const uint8_t*)c->mt.p, train_stride_rows, train_stride_rows, (const int*)c->mcounts.p,
-                        nsets, (int4*)c->mbest.p, second ? (int4*)c->msecond.p : nullptr)))
-        return rc;
-    CU(cudaMemcpyAsync(best, c->mbest.p, obytes, cudaMemcpyDeviceToHost, c->stream));
-    if (second) CU(cudaMemcpyAsync(second, c->msecond.p, obytes, cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaMemcpyAsync(c->h_small, c->mstatus.p, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaStreamSynchronize(c->stream));
-    if (c->h_small[0]) return match_timed_out(c);
-    return ORBX_OK;
+    return match_host(c, query, nq, train, train_stride_rows, train_counts, nsets, best, second, false);
 }
 
 int orbx_filter_matches(orbx_match* m, int n, float ratio)
@@ -1194,15 +1209,15 @@ namespace {
 int grow_keep(orbx_ctx* c, Buf& b, size_t old_bytes, size_t new_bytes)
 {
     if (b.bytes >= new_bytes && b.p) return ORBX_OK;
-    void* np = nullptr;
-    if (cudaMalloc(&np, std::max<size_t>(new_bytes, 256)) != cudaSuccess) return fail(c, ORBX_E_NOMEM, "cudaMalloc failed (map table)");
-    if (cudaMemsetAsync(np, 0, std::max<size_t>(new_bytes, 256), c->stream) != cudaSuccess) { cudaFree(np); return fail(c, ORBX_E_CUDA, "memset failed"); }
-    if (b.p && old_bytes) {
-        if (cudaMemcpyAsync(np, b.p, old_bytes, cudaMemcpyDeviceToDevice, c->stream) != cudaSuccess) { cudaFree(np); return fail(c, ORBX_E_CUDA, "copy failed"); }
-    }
+    Buf nb;                                                  // freed here if anything below fails
+    const size_t bytes = std::max<size_t>(new_bytes, 256);
+    if (cudaMalloc(&nb.p, bytes) != cudaSuccess) return fail(c, ORBX_E_NOMEM, "cudaMalloc failed (map table)");
+    nb.bytes = bytes;
+    if (cudaMemsetAsync(nb.p, 0, bytes, c->stream) != cudaSuccess) return fail(c, ORBX_E_CUDA, "memset failed");
+    if (b.p && old_bytes && cudaMemcpyAsync(nb.p, b.p, old_bytes, cudaMemcpyDeviceToDevice, c->stream) != cudaSuccess)
+        return fail(c, ORBX_E_CUDA, "copy failed");
     cudaStreamSynchronize(c->stream);
-    if (b.p) cudaFree(b.p);
-    b.p = np; b.bytes = std::max<size_t>(new_bytes, 256);
+    b = std::move(nb);
     return ORBX_OK;
 }
 
@@ -1392,7 +1407,7 @@ int orbx_track_match(orbx_ctx* c, const int64_t* ids, int m, const double* pose_
     k_visibility<<<1, VIS_NT, 0, c->stream>>>((const int*)c->t_slots.p, m, T, K, cols, rows, (const double*)c->t_pos.p, (const double*)c->t_nrm.p,
                                               (const uint8_t*)c->t_outl.p, (int*)c->t_cand.p, (int*)c->t_ncand.p);
     ++c->launches;
-    int* h = c->h_small;
+    int* h = c->h_counts();
     CU(cudaMemcpyAsync(h, c->t_ncand.p, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
     CU(cudaStreamSynchronize(c->stream));                    // the candidate count sizes the matcher's grid
     const int nc = h[0];
@@ -1409,9 +1424,7 @@ int orbx_track_match(orbx_ctx* c, const int64_t* ids, int m, const double* pose_
     CU(cudaGetLastError());
     CU(cudaMemcpyAsync(h, (int*)c->t_ncand.p + 1, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
     CU(cudaMemcpyAsync(h + 1, c->t_minmax.p, 2 * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaMemcpyAsync(h + 3, c->mstatus.p, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaStreamSynchronize(c->stream));
-    if (h[3]) return match_timed_out(c);
+    if ((rc = sync_match_words(c, 0, 1))) return rc;
     const int nm = h[0];
     if (nm > 0) CU(cudaMemcpy(matches, c->t_filtered.p, (size_t)nm * 16, cudaMemcpyDeviceToHost));
     *n_matches = nm;
@@ -1457,30 +1470,16 @@ int orbx_submit_frame(orbx_ctx* c, const uint8_t* img, int w, int h, size_t step
 {
     if (!c) return ORBX_E_ARG;
     if (!img || w <= 0 || h <= 0) return fail(c, ORBX_E_ARG, "empty or null image (use the synchronous call for empty frames)");
-    if (w > c->max_w || h > c->max_h) return fail(c, ORBX_E_ARG, "frame larger than the context maximum");
-    if (channels != 1 && channels != 3) return fail(c, ORBX_E_UNSUPPORTED, "channels must be 1 (gray) or 3 (BGR)");
+    int rc = check_args_extract(c, 1, w, h, channels, 0);
+    if (rc) return rc;
     if (step < (size_t)w * channels) return fail(c, ORBX_E_ARG, "step smaller than a row");
     if (c->a_inflight >= 2) return fail(c, ORBX_E_BUSY, "two frames already in flight: collect one first");
     CU(cudaSetDevice(c->device));
     orbx_ctx::AsyncSlot& a = c->aslot[(c->a_head + c->a_inflight) & 1];
     const int cap = std::max(2 * c->nfeatures, 64);
     const size_t row = (size_t)w * channels, dstep = round_up(row, 16), fstride = dstep * h;
-    const size_t out_bytes = 32 + (size_t)cap * 60;
-    int rc;
-    if (a.h_in_bytes < fstride) {
-        if (a.h_in) cudaFreeHost(a.h_in);
-        a.h_in = nullptr; a.h_in_bytes = 0;
-        if (cudaMallocHost((void**)&a.h_in, fstride) != cudaSuccess) return fail(c, ORBX_E_NOMEM, "pinned allocation failed");
-        a.h_in_bytes = fstride;
-    }
-    if (a.h_out_bytes < out_bytes) {
-        if (a.h_out) cudaFreeHost(a.h_out);
-        a.h_out = nullptr; a.h_out_bytes = 0;
-        if (cudaMallocHost((void**)&a.h_out, out_bytes) != cudaSuccess) return fail(c, ORBX_E_NOMEM, "pinned allocation failed");
-        a.h_out_bytes = out_bytes;
-    }
-    if (!a.done && cudaEventCreateWithFlags(&a.done, cudaEventDisableTiming) != cudaSuccess) return fail(c, ORBX_E_CUDA, "event creation failed");
-    if ((rc = ensure(c, c->in, fstride)) || (rc = ensure(c, a.d_kps, sizeof(orbx_keypoint) * (size_t)cap)) || (rc = ensure(c, a.d_desc, (size_t)32 * cap)) ||
+    if ((rc = ensure(c, a.h_in, fstride, "pinned allocation failed")) || (rc = ensure(c, a.h_out, 32 + (size_t)cap * 60, "pinned allocation failed")) ||
+        (rc = ensure(c, c->in, fstride)) || (rc = ensure(c, a.d_kps, sizeof(orbx_keypoint) * (size_t)cap)) || (rc = ensure(c, a.d_desc, (size_t)32 * cap)) ||
         (rc = ensure(c, a.d_counts, 32)))
         return rc;
     a.cap = cap;
@@ -1488,17 +1487,17 @@ int orbx_submit_frame(orbx_ctx* c, const uint8_t* img, int w, int h, size_t step
         c->view_desc = nullptr; c->view_counts = nullptr; c->view_frames = 0;   // overwritten, so "frame 0 of the last extraction" no longer exists
     }
     if ((rc = set_geometry(c, w, h))) return rc;
-    for (int y = 0; y < h; ++y) memcpy(a.h_in + (size_t)y * dstep, img + (size_t)y * step, row);     // the caller's buffer is free on return
+    for (int y = 0; y < h; ++y) memcpy(a.h_in.p + (size_t)y * dstep, img + (size_t)y * step, row);     // the caller's buffer is free on return
     // everything below is stream-ordered behind the previous frame: the shared per-frame workspace is reused safely
-    CU(cudaMemcpyAsync(c->in.p, a.h_in, fstride, cudaMemcpyHostToDevice, c->stream));
+    CU(cudaMemcpyAsync(c->in.p, a.h_in.p, fstride, cudaMemcpyHostToDevice, c->stream));
     CU(cudaMemsetAsync(c->status.p, 0, sizeof(int), c->stream));
     if ((rc = run_extract_range(c, c->stream, 0, false, 0, 1, (const uint8_t*)c->in.p, dstep, fstride, channels, (float*)a.d_kps.p,
                                 (uint8_t*)a.d_desc.p, cap, (int*)a.d_counts.p)))
         return rc;
-    CU(cudaMemcpyAsync(a.h_out, a.d_counts.p, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaMemcpyAsync(a.h_out + 16, c->status.p, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaMemcpyAsync(a.h_out + 32, a.d_kps.p, sizeof(orbx_keypoint) * (size_t)cap, cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaMemcpyAsync(a.h_out + 32 + (size_t)cap * 28, a.d_desc.p, (size_t)32 * cap, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaMemcpyAsync(a.h_out.p, a.d_counts.p, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaMemcpyAsync(a.h_out.p + 16, c->status.p, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaMemcpyAsync(a.h_out.p + 32, a.d_kps.p, sizeof(orbx_keypoint) * (size_t)cap, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaMemcpyAsync(a.h_out.p + 32 + (size_t)cap * 28, a.d_desc.p, (size_t)32 * cap, cudaMemcpyDeviceToHost, c->stream));
     CU(cudaEventRecord(a.done, c->stream));
     CU(cudaGetLastError());
     a.busy = true;
@@ -1516,8 +1515,8 @@ int orbx_collect_frame(orbx_ctx* c, orbx_keypoint* kps, uint8_t* desc, int cap, 
     orbx_ctx::AsyncSlot& a = c->aslot[c->a_head];
     CU(cudaEventSynchronize(a.done));
     int n, status;
-    memcpy(&n, a.h_out, sizeof n);
-    memcpy(&status, a.h_out + 16, sizeof status);
+    memcpy(&n, a.h_out.p, sizeof n);
+    memcpy(&status, a.h_out.p + 16, sizeof status);
     *n_out = n;
     if (n > a.cap) {                                          // more ties than the internal capacity: redo synchronously is the caller's fallback
         a.busy = false; c->a_head ^= 1; --c->a_inflight;
@@ -1529,8 +1528,8 @@ int orbx_collect_frame(orbx_ctx* c, orbx_keypoint* kps, uint8_t* desc, int cap, 
         return fail(c, ORBX_E_INTERNAL, "device-side status set for the collected frame");
     }
     if (n > cap) return fail(c, ORBX_E_CAPACITY, "output capacity too small; n_out holds the needed count (frame still in flight)");
-    memcpy(kps, a.h_out + 32, sizeof(orbx_keypoint) * (size_t)n);
-    memcpy(desc, a.h_out + 32 + (size_t)a.cap * 28, (size_t)32 * n);
+    memcpy(kps, a.h_out.p + 32, sizeof(orbx_keypoint) * (size_t)n);
+    memcpy(desc, a.h_out.p + 32 + (size_t)a.cap * 28, (size_t)32 * n);
     // the collected frame becomes "frame 0 of the last extraction" for orbx_track_match / orbx_map_upsert_from_frame
     c->view_desc = (const uint8_t*)a.d_desc.p; c->view_counts = (const int*)a.d_counts.p; c->view_frames = 1; c->out_cap = a.cap;
     a.busy = false;
