@@ -143,6 +143,19 @@ int orbx_match_hamming_device_ragged(orbx_ctx* ctx, const uint8_t* d_query, int 
  * ([nsets][train_stride_rows][32] with train_counts[nsets]); best / second are [nsets][nq] (second may be NULL). */
 int orbx_match_hamming_sets(orbx_ctx* ctx, const uint8_t* query, int nq, const uint8_t* train, int train_stride_rows,
                             const int* train_counts, int nsets, orbx_match* best, orbx_match* second);
+/* BFMatcher(NORM_HAMMING, crossCheck = true).match(query, train), HOST buffers.  out: capacity nq records;
+ * *n_out = number of mutual pairs, ascending queryIdx.  Empty query or train -> ORBX_OK, 0 (cv2 raises on an empty train).
+ * A pair (i, j) is kept when j is query i's nearest train row and i is train row j's nearest query, the lowest index
+ * winning ties in both directions.  nq >= 2^20 -> ORBX_E_UNSUPPORTED. */
+int orbx_match_hamming_crosscheck(orbx_ctx* ctx, const uint8_t* query, int nq, const uint8_t* train, int nt,
+                                  orbx_match* out, int* n_out);
+/* DEVICE-resident, asynchronous, ragged batch (d_train / d_train_counts exactly as orbx_match_hamming_device_ragged):
+ * set s's mutual pairs compacted to d_out + s*nq (ascending queryIdx), their count in d_n_out[s].  The reverse direction
+ * (each train row's nearest query) comes out of the same distance tiles, with no second pass.  nq = 0 or
+ * train_stride_rows = 0 zeroes d_n_out[0 .. nsets). */
+int orbx_match_hamming_device_crosscheck(orbx_ctx* ctx, const uint8_t* d_query, int nq, const uint8_t* d_train,
+                                         int train_stride_rows, const int* d_train_counts, int nsets,
+                                         orbx_match* d_out, int* d_n_out);
 /* The front-end's whole per-frame pattern on HOST frames in one call (src/frontend.cpp:98-108: one detectAndCompute,
  * then match() of map-point candidates against the frame's descriptors, src/frontend.cpp:153 + :187), for a batch:
  * extraction as orbx_detect_and_compute_batch, then for each of the `nmaps` query sets (queries[j]: nq[j] x 32 host

@@ -120,6 +120,7 @@ struct orbx_ctx {
     const int* view_counts = nullptr;
     int view_frames = 0;
     Buf mq, mt, mbest, msecond, mkeys, mstatus, mcounts;
+    Buf mcolkeys, mxcount;                   // cross-check: column keys [nsets][stride_rows], the host form's pair count
     int last_batch = 0;
 
     // device-resident map-point table (SURVEY 8(f).1): slot-addressed columns + the host's id -> slot index
@@ -622,13 +623,17 @@ int sync_match_words(orbx_ctx* c, int slot, int n)
 // The matcher on device-resident operands, asynchronous on `st` (default: the context's stream).  `slot` selects the
 // status word (one per lane, so concurrent lanes never reset each other's); lanes never take the split-train path,
 // whose key scratch is shared.
+// Cross-check (d_xc_count set, d_second null, not a lane call): set s's mutual pairs are compacted in place to d_best + s * nq,
+// their count to d_xc_count[s].
 int run_match(orbx_ctx* c, const uint8_t* d_q, int nq, const uint8_t* d_t, int nt, int stride_rows, const int* d_counts, int nsets,
-              int4* d_best, int4* d_second, cudaStream_t st = nullptr, int slot = 0)
+              int4* d_best, int4* d_second, cudaStream_t st = nullptr, int slot = 0, int* d_xc_count = nullptr)
 {
     NvtxRange nvr("orbx:match_hamming");
     const bool lane_call = st != nullptr;
     if (!st) st = c->stream;
     if (nt >= MT_MAX_TRAIN) return fail(c, ORBX_E_UNSUPPORTED, "train set larger than 2^20 - 1 rows");
+    const bool xchk = d_xc_count != nullptr;
+    if (xchk && nq >= MT_MAX_QUERY_XC) return fail(c, ORBX_E_UNSUPPORTED, "cross-check query set larger than 2^20 - 1 rows");
     const bool knn2 = d_second != nullptr;
     // CTA-pair kernel (tcgen05 cta_group::2, query tiles in twos) whenever the (query tile, set) pairs alone fill the GPU;
     // small problems keep the single-CTA kernel, whose CTAs are independent units for the train-row split.
@@ -671,14 +676,28 @@ int run_match(orbx_ctx* c, const uint8_t* d_q, int nq, const uint8_t* d_t, int n
         k_match_keys_init<<<(unsigned)((nout + 255) / 256), 256, 0, st>>>(keys, nout);
         ++c->launches;
     }
+    int* col_keys = nullptr;
+    if (xchk) {
+        const size_t ncol = (size_t)nsets * stride_rows;
+        if ((rc = ensure(c, c->mcolkeys, ncol * sizeof(int)))) return rc;
+        col_keys = (int*)c->mcolkeys.p;
+        k_match_keys_init<<<(unsigned)((ncol + 255) / 256), 256, 0, st>>>(col_keys, ncol);
+        ++c->launches;
+    }
     const dim3 grd((unsigned)tiles_m, (unsigned)nsplit, (unsigned)zgroups);
-    if (pair && knn2) k_hamming_umma2<true><<<grd, MT_THREADS, MT_SMEM_BYTES, st>>>(d_q, nq, d_t, nt, stride_rows, d_counts, nsets, rows_per_split, d_best, d_second, keys, d_status);
+    if (pair && xchk) k_hamming_umma2_xc<><<<grd, MT_THREADS, MT_SMEM_BYTES_XC, st>>>(d_q, nq, d_t, nt, stride_rows, d_counts, nsets, rows_per_split, d_best, d_second, keys, d_status, col_keys);
+    else if (xchk) k_hamming_umma_xc<><<<grd, MT_THREADS, MT_SMEM_BYTES_XC, st>>>(d_q, nq, d_t, nt, stride_rows, d_counts, nsets, rows_per_split, d_best, d_second, keys, d_status, col_keys);
+    else if (pair && knn2) k_hamming_umma2<true><<<grd, MT_THREADS, MT_SMEM_BYTES, st>>>(d_q, nq, d_t, nt, stride_rows, d_counts, nsets, rows_per_split, d_best, d_second, keys, d_status);
     else if (pair) k_hamming_umma2<false><<<grd, MT_THREADS, MT_SMEM_BYTES, st>>>(d_q, nq, d_t, nt, stride_rows, d_counts, nsets, rows_per_split, d_best, d_second, keys, d_status);
     else if (knn2) k_hamming_umma<true><<<grd, MT_THREADS, MT_SMEM_BYTES, st>>>(d_q, nq, d_t, nt, stride_rows, d_counts, nsets, rows_per_split, d_best, d_second, keys, d_status);
     else      k_hamming_umma<false><<<grd, MT_THREADS, MT_SMEM_BYTES, st>>>(d_q, nq, d_t, nt, stride_rows, d_counts, nsets, rows_per_split, d_best, d_second, keys, d_status);
     ++c->launches;
     if (nsplit > 1) {
         k_match_finalize<<<(unsigned)((nout + 255) / 256), 256, 0, st>>>(keys, nq, nout, d_best);
+        ++c->launches;
+    }
+    if (xchk) {                                              // reads the finalised row winners
+        k_crosscheck_compact<><<<(unsigned)nsets, XC_NT, 0, st>>>(d_best, nq, col_keys, stride_rows, d_best, d_xc_count);
         ++c->launches;
     }
     if (!lane_call) { stage_mark(c, 8); if (c->profiling) c->stage_valid[6] = true; }
@@ -689,21 +708,24 @@ int run_match(orbx_ctx* c, const uint8_t* d_q, int nq, const uint8_t* d_t, int n
 // The host-buffer matcher, synchronous on the context's stream: nq query rows against nsets train sets of stride_rows rows
 // each (all of them, or as many as the host `counts` give per set).  best and second (when not null) receive [nsets][nq]
 // records each; with `pairs` (the second-best of one set), `best` receives [nq][2] {best, second} records instead.
+// With `xc_count` (cross-check of one set), `best` receives the mutual pairs and *xc_count their number.
 int match_host(orbx_ctx* c, const uint8_t* query, int nq, const uint8_t* train, int stride_rows, const int* counts, int nsets,
-               orbx_match* best, orbx_match* second, bool pairs)
+               orbx_match* best, orbx_match* second, bool pairs, int* xc_count = nullptr)
 {
     const size_t tbytes = (size_t)nsets * stride_rows * 32, obytes = (size_t)nsets * nq * 16;
     const bool knn2 = pairs || second;
     int rc;
     if ((rc = ensure(c, c->mq, (size_t)nq * 32)) || (rc = ensure(c, c->mt, tbytes)) || (rc = ensure(c, c->mbest, obytes)) ||
-        (knn2 && (rc = ensure(c, c->msecond, obytes))) || (counts && (rc = ensure(c, c->mcounts, sizeof(int) * (size_t)nsets))))
+        (knn2 && (rc = ensure(c, c->msecond, obytes))) || (counts && (rc = ensure(c, c->mcounts, sizeof(int) * (size_t)nsets))) ||
+        (xc_count && (rc = ensure(c, c->mxcount, sizeof(int) * (size_t)nsets))))
         return rc;
     CU(cudaMemcpyAsync(c->mq.p, query, (size_t)nq * 32, cudaMemcpyHostToDevice, c->stream));
     CU(cudaMemcpyAsync(c->mt.p, train, tbytes, cudaMemcpyHostToDevice, c->stream));
     if (counts) CU(cudaMemcpyAsync(c->mcounts.p, counts, sizeof(int) * (size_t)nsets, cudaMemcpyHostToDevice, c->stream));
     if ((rc = run_match(c, (const uint8_t*)c->mq.p, nq, (const uint8_t*)c->mt.p, stride_rows, stride_rows, counts ? (const int*)c->mcounts.p : nullptr,
-                        nsets, (int4*)c->mbest.p, knn2 ? (int4*)c->msecond.p : nullptr)))
+                        nsets, (int4*)c->mbest.p, knn2 ? (int4*)c->msecond.p : nullptr, nullptr, 0, xc_count ? (int*)c->mxcount.p : nullptr)))
         return rc;
+    if (xc_count) CU(cudaMemcpyAsync(xc_count, c->mxcount.p, sizeof(int) * (size_t)nsets, cudaMemcpyDeviceToHost, c->stream));
     if (pairs) {
         CU(cudaMemcpy2DAsync(best, 32, c->mbest.p, 16, 16, (size_t)nq, cudaMemcpyDeviceToHost, c->stream));
         CU(cudaMemcpy2DAsync(best + 1, 32, c->msecond.p, 16, 16, (size_t)nq, cudaMemcpyDeviceToHost, c->stream));
@@ -789,6 +811,8 @@ int orbx_create(orbx_ctx** out, int device, int nfeatures, float scale_factor, i
         cudaFuncSetAttribute(k_hamming_umma2<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
         cudaFuncSetAttribute(k_hamming_umma<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
         cudaFuncSetAttribute(k_hamming_umma<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
+        cudaFuncSetAttribute(k_hamming_umma2_xc<>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES_XC) != cudaSuccess ||
+        cudaFuncSetAttribute(k_hamming_umma_xc<>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES_XC) != cudaSuccess ||
         cudaFuncSetAttribute(k_fast_warp<FAST_NWARP>, cudaFuncAttributeMaxDynamicSharedMemorySize, FAST_NWARP * FW_WARP_BYTES + 128) != cudaSuccess ||
         cudaFuncSetAttribute(k_pyr_tma, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024) != cudaSuccess ||
         cudaFuncSetAttribute(k_describe_tma, cudaFuncAttributeMaxDynamicSharedMemorySize, DS_NW * DS_WARP_BYTES + 128) != cudaSuccess ||
@@ -1094,6 +1118,40 @@ int orbx_match_hamming_sets(orbx_ctx* c, const uint8_t* query, int nq, const uin
     if (!query || !train || !best || !train_counts) return fail(c, ORBX_E_ARG, "null pointer");
     CU(cudaSetDevice(c->device));
     return match_host(c, query, nq, train, train_stride_rows, train_counts, nsets, best, second, false);
+}
+
+int orbx_match_hamming_crosscheck(orbx_ctx* c, const uint8_t* q, int nq, const uint8_t* t, int nt, orbx_match* out, int* n_out)
+{
+    if (!c) return ORBX_E_ARG;
+    if (!n_out) return fail(c, ORBX_E_ARG, "null n_out");
+    *n_out = 0;
+    if (nq < 0 || nt < 0) return fail(c, ORBX_E_ARG, "negative row count");
+    if (nq >= MT_MAX_QUERY_XC) return fail(c, ORBX_E_UNSUPPORTED, "cross-check query set larger than 2^20 - 1 rows");
+    if (nq == 0 || nt == 0) return ORBX_OK;                 // empty query or train -> no pairs (cv2 raises on an empty train)
+    if (!q || !t || !out) return fail(c, ORBX_E_ARG, "null pointer");
+    CU(cudaSetDevice(c->device));
+    int n = 0;
+    const int rc = match_host(c, q, nq, t, nt, nullptr, 1, out, nullptr, false, &n);
+    if (rc) return rc;
+    *n_out = n;
+    return ORBX_OK;
+}
+
+int orbx_match_hamming_device_crosscheck(orbx_ctx* c, const uint8_t* d_query, int nq, const uint8_t* d_train, int train_stride_rows,
+                                         const int* d_train_counts, int nsets, orbx_match* d_out, int* d_n_out)
+{
+    if (!c) return ORBX_E_ARG;
+    if (nq < 0 || train_stride_rows < 0 || nsets < 0 || nsets > 65535) return fail(c, ORBX_E_ARG, "bad sizes");
+    if (nq >= MT_MAX_QUERY_XC) return fail(c, ORBX_E_UNSUPPORTED, "cross-check query set larger than 2^20 - 1 rows");
+    if (nsets == 0) return ORBX_OK;
+    if (!d_n_out) return fail(c, ORBX_E_ARG, "null pointer");
+    CU(cudaSetDevice(c->device));
+    if (nq == 0 || train_stride_rows == 0) {                 // no pairs in any set
+        CU(cudaMemsetAsync(d_n_out, 0, sizeof(int) * (size_t)nsets, c->stream));
+        return ORBX_OK;
+    }
+    if (!d_query || !d_train || !d_out || !d_train_counts) return fail(c, ORBX_E_ARG, "null pointer");
+    return run_match(c, d_query, nq, d_train, train_stride_rows, train_stride_rows, d_train_counts, nsets, (int4*)d_out, nullptr, nullptr, 0, d_n_out);
 }
 
 int orbx_filter_matches(orbx_match* m, int n, float ratio)

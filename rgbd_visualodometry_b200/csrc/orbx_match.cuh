@@ -62,6 +62,11 @@ constexpr uint32_t MT_TMEM_A = 4 * MT_BN;                  // first column of th
 constexpr int MT_KEY_SHIFT = 20;
 constexpr int MT_MAX_TRAIN = 1 << MT_KEY_SHIFT;            // train rows per set representable in the packed key
 static_assert(4 * MT_BN + 128 <= 512, "TMEM budget");
+// cross-check kernels only: every epilogue warp's column maxima of a tile, [accumulator buffer][epilogue warp][MT_BN] ints,
+// behind the barrier block (the other kernels' layout and launch size stay as they are)
+constexpr int MT_SMEM_XC = MT_SMEM_BAR + 128;
+constexpr int MT_SMEM_BYTES_XC = MT_SMEM_XC + 2 * 8 * MT_BN * 4 + 1024;
+constexpr int MT_MAX_QUERY_XC = 1 << MT_KEY_SHIFT;         // query rows representable in the column key dot << 20 | (0xFFFFF - q)
 
 // ---- PTX wrappers ------------------------------------------------------------------------------------------
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -300,12 +305,41 @@ template <bool PAIR> __device__ __forceinline__ void umma_i8(uint32_t d, uint64_
 }
 template <bool PAIR> __device__ __forceinline__ void umma_commit(uint32_t bar) { if (PAIR) tc_commit2(bar); else tc_commit(bar); }
 
-template <bool KNN2, bool PAIR>
+// ---- cross-check (XCHK): column maxima from the same accumulators ----------------------------------------------------
+// Every column of a tile holds one train row, and all its values carry that row's code, so the column maximum of the
+// accumulator is the row's largest dot.  Widened to (v << 8) | (255 - row of the CTA), its plain maximum is "largest
+// dot, lowest query row".  One PRMT widens a packed half (the selector's msb replicates the sign of the selected byte).
+__device__ __forceinline__ int xc_widen(uint32_t packed, uint32_t c, uint32_t sel)
+{
+    uint32_t r;
+    asm("prmt.b32 %0, %1, %2, %3;" : "=r"(r) : "r"(packed), "r"(c), "r"(sel));
+    return (int)r;
+}
+// This warp's 96 column maxima over its 32 query rows -> xc[0 .. MT_BN) (slot 2u + h = half h of packed register u, the
+// same slot in every warp).  A padded query row (q >= nq) counts as v = -32768, below every accumulator (>= -32512).
+__device__ __forceinline__ void xc_warp_columns(const uint32_t* rp, bool valid, int row_cta, int* xc)
+{
+    const uint32_t c = 255u - (uint32_t)row_cta;
+#pragma unroll
+    for (int u = 0; u < MT_BN / 2; u += 2) {
+        const uint32_t r0 = valid ? rp[u] : 0x80008000u, r1 = valid ? rp[u + 1] : 0x80008000u;
+        int4 m;
+        m.x = __reduce_max_sync(0xffffffffu, xc_widen(r0, c, 0x9104u));
+        m.y = __reduce_max_sync(0xffffffffu, xc_widen(r0, c, 0xB324u));
+        m.z = __reduce_max_sync(0xffffffffu, xc_widen(r1, c, 0x9104u));
+        m.w = __reduce_max_sync(0xffffffffu, xc_widen(r1, c, 0xB324u));
+        *reinterpret_cast<int4*>(xc + 2 * u) = m;
+    }
+}
+__device__ __forceinline__ void xc_epilogue_sync() { asm volatile("bar.sync 1, 256;" ::: "memory"); }   // the 8 epilogue warps only
+
+template <bool KNN2, bool PAIR, bool XCHK>
 __device__ __forceinline__ void
 hamming_umma_body(const uint8_t* __restrict__ query, int nq, const uint8_t* __restrict__ train, int nt, int train_stride_rows,
                const int* __restrict__ train_counts, int nsets, int rows_per_split, int4* __restrict__ best,
-               int4* __restrict__ second, int* __restrict__ keys, int* __restrict__ status)
+               int4* __restrict__ second, int* __restrict__ keys, int* __restrict__ status, int* __restrict__ col_keys)
 {
+    static_assert(!(KNN2 && XCHK), "cross-check keeps the best match only");
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
     const uint32_t sbase = smem_u32(smem);
@@ -512,14 +546,21 @@ hamming_umma_body(const uint8_t* __restrict__ query, int nq, const uint8_t* __re
         const uint32_t lane_base = (uint32_t)((warp & 3) * 32) << 16;
         int t = 0;
         int cnt_next = match_set_count(train_counts, min((int)blockIdx.z, nsets - 1), nt);
-        for (int set = blockIdx.z; set < nsets && ok; set += gridDim.z) {
+        // XCHK: the epilogue warps meet at a named barrier once per tile, so after a timeout a warp keeps walking the tiles
+        // (without waiting on the pipeline) and never leaves the others at that barrier
+        for (int set = blockIdx.z; set < nsets && (XCHK || ok); set += gridDim.z) {
             const MatchSetRange rg = match_set_range_n(cnt_next, nt, split, rows_per_split);   // (next set's row count loaded a set ahead, as in the issuer)
             if (set + (int)gridDim.z < nsets) cnt_next = match_set_count(train_counts, set + (int)gridDim.z, nt);
             int m1 = INT_MIN, m2 = INT_MIN;
             for (int i = 0; i < rg.ntiles; ++i, ++t) {
                 const int b = t & 1;
                 const uint32_t bph = (uint32_t)(t >> 1) & 1u;
-                if (!mbar_wait(bar_tfull + 8 * b, bph)) { ok = false; break; }
+                if constexpr (XCHK) {
+                    if (ok && !mbar_wait(bar_tfull + 8 * b, bph)) ok = false;
+                    if (!ok) { xc_epilogue_sync(); continue; }
+                } else {
+                    if (!mbar_wait(bar_tfull + 8 * b, bph)) { ok = false; break; }
+                }
                 tc_fence_after();
                 const int j0 = rg.n0 + i * MT_BN;
                 const bool full = (j0 + MT_BN <= rg.n1);
@@ -547,6 +588,8 @@ hamming_umma_body(const uint8_t* __restrict__ query, int nq, const uint8_t* __re
                     }
                     const unsigned pk = __vimax3_s16x2(__vimax3_s16x2(p[0], p[1], p[2]), __vimax3_s16x2(p[3], p[4], p[5]), __vmaxs2(p[6], p[7]));
                     k1 = max((int)(pk << 16) >> 16, (int)pk >> 16);
+                    if constexpr (XCHK)
+                        xc_warp_columns(rp, qrow < nq, qrow - q0, reinterpret_cast<int*>(smem + MT_SMEM_XC) + (b * 8 + warp - MT_EPI_WARP0) * MT_BN);
                 } else if (!KNN2) {
                     // a set's partial last tile was issued with N = 32, 64 (or 96) columns, its rows past the set's end are
                     // copies of the last row (never the maximum): same packed path, 32-column chunks as far as N goes
@@ -573,6 +616,8 @@ hamming_umma_body(const uint8_t* __restrict__ query, int nq, const uint8_t* __re
                     }
                     const unsigned pk = __vimax3_s16x2(__vimax3_s16x2(p[0], p[1], p[2]), __vimax3_s16x2(p[3], p[4], p[5]), __vmaxs2(p[6], p[7]));
                     k1 = max((int)(pk << 16) >> 16, (int)pk >> 16);
+                    if constexpr (XCHK)                      // (chunks past N hold -32768: no column there)
+                        xc_warp_columns(rp, qrow < nq, qrow - q0, reinterpret_cast<int*>(smem + MT_SMEM_XC) + (b * 8 + warp - MT_EPI_WARP0) * MT_BN);
                 } else {
 #pragma unroll
                     for (int ch = 0; ch < NCH; ++ch) tc_ld32(tacc + (uint32_t)(ch * 32), r[ch]);
@@ -605,6 +650,30 @@ hamming_umma_body(const uint8_t* __restrict__ query, int nq, const uint8_t* __re
                         const int gk = ((int)q - 256) * (1 << MT_KEY_SHIFT) + ((MT_MAX_TRAIN - 1) - (j0 + jl));
                         if (KNN2) m2 = max(m2, min(m1, gk));
                         m1 = max(m1, gk);
+                    }
+                }
+                if constexpr (XCHK) {
+                    // the 8 warps' maxima of a column -> the CTA's, decoded like a row winner (the code names the train row,
+                    // whatever the column's slot) into the column key  dot << 20 | (0xFFFFF - q); one atomicMax per column.
+                    // Slots of buffer b are written again at tile t + 2, behind the next tile's barrier.
+                    xc_epilogue_sync();
+                    const int e = tid - MT_EPI_WARP0 * 32;
+                    if (e < MT_BN) {
+                        const int* xcs = reinterpret_cast<const int*>(smem + MT_SMEM_XC) + b * 8 * MT_BN + e;
+                        int kx = xcs[0];
+#pragma unroll
+                        for (int w = 1; w < 8; ++w) kx = max(kx, xcs[w * MT_BN]);
+                        const int v = kx >> 8;
+                        if (v != -32768) {                   // (only padded query rows, or a chunk past the tile's N)
+                            const unsigned kk = (unsigned)(v + MT_ASCALE * 256);
+                            const unsigned q = kk / (unsigned)MT_ASCALE;      // dot + 256
+                            const int code = (MT_BN - 1) - (int)(kk - q * (unsigned)MT_ASCALE);
+                            const int nh = ((min(MT_BN, rg.n1 - j0) + 31) & ~31) >> 1;
+                            const int j = j0 + (PAIR && code >= MT2_HALF ? nh + code - MT2_HALF : code);
+                            if (j < rg.n1)                   // columns past the set's end are copies of its last row
+                                atomicMax(&col_keys[(size_t)set * train_stride_rows + j],
+                                          ((int)q - 256) * (1 << MT_KEY_SHIFT) + ((MT_MAX_QUERY_XC - 1) - (q0 + 255 - (kx & 255))));
+                        }
                     }
                 }
             }
@@ -646,12 +715,58 @@ hamming_umma_body(const uint8_t* __restrict__ query, int nq, const uint8_t* __re
 #define ORBX_MATCH_ARGS query, nq, train, nt, train_stride_rows, train_counts, nsets, rows_per_split, best, second, keys, status
 // single CTA per query tile (small problems: independent CTAs, train rows can be split across them)
 template <bool KNN2>
-__global__ void __launch_bounds__(MT_THREADS, 1) k_hamming_umma(ORBX_MATCH_PARAMS) { hamming_umma_body<KNN2, false>(ORBX_MATCH_ARGS); }
+__global__ void __launch_bounds__(MT_THREADS, 1) k_hamming_umma(ORBX_MATCH_PARAMS) { hamming_umma_body<KNN2, false, false>(ORBX_MATCH_ARGS, nullptr); }
 // CTA pair on the two SMs of a TPC (tcgen05 cta_group::2): blockIdx.x = 2 * pair + rank
 template <bool KNN2>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(MT_THREADS, 1) k_hamming_umma2(ORBX_MATCH_PARAMS) { hamming_umma_body<KNN2, true>(ORBX_MATCH_ARGS); }
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(MT_THREADS, 1) k_hamming_umma2(ORBX_MATCH_PARAMS) { hamming_umma_body<KNN2, true, false>(ORBX_MATCH_ARGS, nullptr); }
+// cross-check (BFMatcher crossCheck = true): the best-match kernels above plus every train row's nearest query, merged into
+// col_keys[set][train_stride_rows] (INT_MIN-initialised) by atomicMax; launched with MT_SMEM_BYTES_XC.
+// The cross-check kernels are templates (instantiated with <>) only so that they are emitted after the kernels instantiated
+// earlier in orbx.cu: as plain __global__ functions they change the module's function order, and with it NVVM's code for
+// k_select<512>, which they do not touch.
+template <int = 0> __global__ void __launch_bounds__(MT_THREADS, 1) k_hamming_umma_xc(ORBX_MATCH_PARAMS, int* __restrict__ col_keys)
+{
+    hamming_umma_body<false, false, true>(ORBX_MATCH_ARGS, col_keys);
+}
+template <int = 0> __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(MT_THREADS, 1) k_hamming_umma2_xc(ORBX_MATCH_PARAMS, int* __restrict__ col_keys)
+{
+    hamming_umma_body<false, true, true>(ORBX_MATCH_ARGS, col_keys);
+}
 #undef ORBX_MATCH_PARAMS
 #undef ORBX_MATCH_ARGS
+
+// ONE CTA per set: query i keeps its best match (i, j) iff column j's key names i, i.e. i is also train row j's nearest
+// query (lowest index on ties); the kept records are compacted stably in query order to out[set][0 .. n_out[set]).
+// best and out may be the same buffer: a record only moves to a lower or equal index, and a chunk is read before it is written.
+constexpr int XC_NT = 1024;
+template <int = 0> __global__ void __launch_bounds__(XC_NT) k_crosscheck_compact(const int4* best, int nq, const int* __restrict__ col_keys, int stride_rows,
+                                                              int4* out, int* __restrict__ n_out)
+{
+    __shared__ int s_warp[XC_NT / 32];
+    __shared__ int s_base;
+    const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
+    const size_t set = blockIdx.x;
+    best += set * nq; out += set * nq; col_keys += set * stride_rows;
+    if (tid == 0) s_base = 0;
+    __syncthreads();
+    for (int base = 0; base < nq; base += XC_NT) {
+        const int i = base + tid;
+        int4 r = make_int4(0, -1, 0, 0);
+        if (i < nq) r = best[i];
+        const bool keep = r.y >= 0 && (MT_MAX_QUERY_XC - 1) - (col_keys[r.y] & (MT_MAX_QUERY_XC - 1)) == i;
+        const unsigned bal = __ballot_sync(0xffffffffu, keep);
+        if (lane == 0) s_warp[wid] = __popc(bal);
+        __syncthreads();
+        int before = 0, total = 0;
+        for (int w = 0; w < XC_NT / 32; ++w) { const int c = s_warp[w]; if (w < wid) before += c; total += c; }
+        const int out0 = s_base;
+        if (keep) out[out0 + before + __popc(bal & ((1u << lane) - 1u))] = r;
+        __syncthreads();
+        if (tid == 0) s_base = out0 + total;
+        __syncthreads();
+    }
+    if (tid == 0) n_out[set] = s_base;
+}
 
 __global__ void k_match_keys_init(int* __restrict__ keys, size_t n)
 {

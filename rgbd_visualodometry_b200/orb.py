@@ -7,7 +7,7 @@
   orb_->detectAndCompute(color_, Mat(), kps, desc)            ORB.detectAndCompute(image, None) -> (kps, desc)
       src/frontend.cpp:153
   matcher.match(query, train, matches)                        BFMatcher(NORM_HAMMING).match(query, train)
-      src/frontend.cpp:187                                    (+ knnMatch(query, train, k=2))
+      src/frontend.cpp:187                                    (+ knnMatch(query, train, k=2), crossCheck=True)
   max(min_dis * match_ratio, 30) filter                       filter_matches(matches, match_ratio)
       src/frontend.cpp:190-211
 
@@ -158,6 +158,21 @@ class Context:
         n = C.c_int(0)
         self._check(self.lib.orbx_match_hamming_knn2(self.h, _ptr(q), len(q), _ptr(t), len(t), _ptr(out), C.byref(n)))
         return out[:n.value]
+
+    def match_crosscheck(self, query: np.ndarray, train: np.ndarray) -> np.ndarray:
+        """BFMatcher(NORM_HAMMING, crossCheck=True).match: the mutual nearest pairs, ascending queryIdx."""
+        q = np.ascontiguousarray(query, np.uint8).reshape(-1, 32)
+        t = np.ascontiguousarray(train, np.uint8).reshape(-1, 32)
+        out = np.zeros(max(len(q), 1), DMATCH_DTYPE)
+        n = C.c_int(0)
+        self._check(self.lib.orbx_match_hamming_crosscheck(self.h, _ptr(q), len(q), _ptr(t), len(t), _ptr(out), C.byref(n)))
+        return out[:n.value]
+
+    def match_device_crosscheck(self, d_query_ptr: int, nq: int, d_train_ptr: int, stride_rows: int, d_counts_ptr: int, nsets: int,
+                                d_out_ptr: int, d_n_out_ptr: int):
+        """Asynchronous, device-resident, ragged batch: set s's mutual pairs to d_out[s, :d_n_out[s]] ([nsets, nq] records)."""
+        self._check(self.lib.orbx_match_hamming_device_crosscheck(self.h, d_query_ptr, nq, d_train_ptr, stride_rows, d_counts_ptr, nsets,
+                                                                  d_out_ptr, d_n_out_ptr))
 
     def match_device(self, d_query_ptr: int, nq: int, d_train_ptr: int, nt: int, nsets: int, d_best_ptr: int, d_second_ptr: int = 0):
         self._check(self.lib.orbx_match_hamming_device(self.h, d_query_ptr, nq, d_train_ptr, nt, nsets, d_best_ptr,
@@ -331,19 +346,26 @@ def ORB_create(nfeatures=500, scaleFactor=1.2, nlevels=8, device=0, kernels=-1) 
 
 
 class BFMatcher:
-    """cv::BFMatcher(NORM_HAMMING) stand-in on the tcgen05 int8 tensor cores."""
+    """cv::BFMatcher(NORM_HAMMING[, crossCheck]) stand-in on the tcgen05 int8 tensor cores.  With crossCheck, match keeps
+    only the mutual nearest pairs (the reverse direction comes out of the same distance tiles); an empty train set gives
+    no matches where cv2 raises."""
 
     def __init__(self, normType=NORM_HAMMING, crossCheck=False, device=0):
-        if normType != NORM_HAMMING or crossCheck:
-            raise OrbxError(E_UNSUPPORTED, "only NORM_HAMMING without crossCheck is implemented (what the hot path uses)")
+        if normType != NORM_HAMMING:
+            raise OrbxError(E_UNSUPPORTED, "only NORM_HAMMING is implemented (what the hot path uses)")
+        self.crossCheck = bool(crossCheck)
         self._ctx = Context(1, 1.2, 1, 64, 64, 1, device)
 
     def match(self, queryDescriptors, trainDescriptors):
         if queryDescriptors is None or trainDescriptors is None:
             return np.zeros(0, DMATCH_DTYPE)
+        if self.crossCheck:
+            return self._ctx.match_crosscheck(queryDescriptors, trainDescriptors)
         return self._ctx.match(queryDescriptors, trainDescriptors)
 
     def knnMatch(self, queryDescriptors, trainDescriptors, k=2):
+        if self.crossCheck:
+            raise OrbxError(E_UNSUPPORTED, "knnMatch with crossCheck is not implemented")
         if k != 2:
             raise OrbxError(E_UNSUPPORTED, "knnMatch is implemented for k = 2")
         if queryDescriptors is None or trainDescriptors is None:
