@@ -19,12 +19,11 @@
 
 #include "../../include/orbx.h"
 #include "orbx_geom.h"
-#include "orbx_kernels.cuh"
-#include "orbx_match.cuh"
-#include "orbx_fast.cuh"
 #include "orbx_pyr.cuh"
-#include "orbx_desc.cuh"
+#include "orbx_fast.cuh"
 #include "orbx_select.cuh"
+#include "orbx_desc.cuh"
+#include "orbx_match.cuh"
 #include "orbx_map.cuh"
 #include "orbx_stage.h"
 #include <unordered_map>
@@ -455,10 +454,8 @@ int run_extract_range(orbx_ctx* c, cudaStream_t st, int lane_id, bool marks, int
     // Selection by problem size: one WARP per (frame, level) when the candidate lists are short and there are thousands of
     // them (256 VGA frames: 0.116 ms against 0.17 ms), one CTA per (frame, level) when the lists are long -- 512 threads wide
     // there (64 frames of 1920x1080: 0.30 ms against 0.43 ms with 128 threads and 0.65 ms with warps; 3840x2160: 1.21
-    // against 1.88 and 2.57 ms).  sel_cta_threads = 0: the warp trio k_select_fast, k_harris, k_select_harris.
-    const bool wide = (long)g.w * g.h > 600000L;
-    const bool cta_select = c->force_kernels >= 0 ? c->force_kernels != 0 : wide;
-    const int sel_cta_threads = !cta_select ? 0 : wide ? SEL_NT_WIDE : SEL_NT;
+    // against 1.88 and 2.57 ms).  cta_select = false: the warp trio k_select_fast, k_harris, k_select_harris.
+    const bool cta_select = c->force_kernels >= 0 ? c->force_kernels != 0 : (long)g.w * g.h > 600000L;
     // The small upper levels are a chain of short, latency-bound launches (at 640x480 levels 4..7 take as long as levels 1..3
     // for a fifth of the pixels).  They leave the critical path: from level `lt` on, the pyramid chain and the FAST bands of
     // those levels run on a HIGH-PRIORITY side stream (their few CTAs take the next free slots) underneath the FAST launch of the
@@ -526,9 +523,8 @@ int run_extract_range(orbx_ctx* c, cudaStream_t st, int lane_id, bool marks, int
     } else if (g.total_bands > 0) launch_fast(0, g.total_bands, st);
     nv.next("orbx:select_harris");
     if (marks) stage_mark(c, 3);
-    if (sel_cta_threads > 0) {
-        if (sel_cta_threads == SEL_NT_WIDE) k_select<SEL_NT_WIDE><<<dim3(B, (unsigned)g.nlevels), SEL_NT_WIDE, 0, st>>>(g, pyr, rowcnt, rowent, work, selpos, fincnt, status);
-        else                                k_select<SEL_NT><<<dim3(B, (unsigned)g.nlevels), SEL_NT, 0, st>>>(g, pyr, rowcnt, rowent, work, selpos, fincnt, status);
+    if (cta_select) {
+        k_select<<<dim3(B, (unsigned)g.nlevels), SEL_NT, 0, st>>>(g, pyr, rowcnt, rowent, work, selpos, fincnt);
         ++c->launches;
     } else {
         // (the warp going straight on to Harris and the second retainBest -- one launch instead of three -- was measured: 0.1435 ms
@@ -685,19 +681,18 @@ int run_match(orbx_ctx* c, const uint8_t* d_q, int nq, const uint8_t* d_t, int n
         ++c->launches;
     }
     const dim3 grd((unsigned)tiles_m, (unsigned)nsplit, (unsigned)zgroups);
-    if (pair && xchk) k_hamming_umma2_xc<><<<grd, MT_THREADS, MT_SMEM_BYTES_XC, st>>>(d_q, nq, d_t, nt, stride_rows, d_counts, nsets, rows_per_split, d_best, d_second, keys, d_status, col_keys);
-    else if (xchk) k_hamming_umma_xc<><<<grd, MT_THREADS, MT_SMEM_BYTES_XC, st>>>(d_q, nq, d_t, nt, stride_rows, d_counts, nsets, rows_per_split, d_best, d_second, keys, d_status, col_keys);
-    else if (pair && knn2) k_hamming_umma2<true><<<grd, MT_THREADS, MT_SMEM_BYTES, st>>>(d_q, nq, d_t, nt, stride_rows, d_counts, nsets, rows_per_split, d_best, d_second, keys, d_status);
-    else if (pair) k_hamming_umma2<false><<<grd, MT_THREADS, MT_SMEM_BYTES, st>>>(d_q, nq, d_t, nt, stride_rows, d_counts, nsets, rows_per_split, d_best, d_second, keys, d_status);
-    else if (knn2) k_hamming_umma<true><<<grd, MT_THREADS, MT_SMEM_BYTES, st>>>(d_q, nq, d_t, nt, stride_rows, d_counts, nsets, rows_per_split, d_best, d_second, keys, d_status);
-    else      k_hamming_umma<false><<<grd, MT_THREADS, MT_SMEM_BYTES, st>>>(d_q, nq, d_t, nt, stride_rows, d_counts, nsets, rows_per_split, d_best, d_second, keys, d_status);
+    // (knn2 and xchk never meet: the cross-check keeps the best match only)
+    auto* kernel = pair ? (xchk ? k_hamming_umma2<false, true> : knn2 ? k_hamming_umma2<true, false> : k_hamming_umma2<false, false>)
+                        : (xchk ? k_hamming_umma<false, true> : knn2 ? k_hamming_umma<true, false> : k_hamming_umma<false, false>);
+    kernel<<<grd, MT_THREADS, xchk ? MT_SMEM_BYTES_XC : MT_SMEM_BYTES, st>>>(d_q, nq, d_t, nt, stride_rows, d_counts, nsets, rows_per_split, d_best,
+                                                                          d_second, keys, d_status, col_keys);
     ++c->launches;
     if (nsplit > 1) {
         k_match_finalize<<<(unsigned)((nout + 255) / 256), 256, 0, st>>>(keys, nq, nout, d_best);
         ++c->launches;
     }
     if (xchk) {                                              // reads the finalised row winners
-        k_crosscheck_compact<><<<(unsigned)nsets, XC_NT, 0, st>>>(d_best, nq, col_keys, stride_rows, d_best, d_xc_count);
+        k_crosscheck_compact<<<(unsigned)nsets, XC_NT, 0, st>>>(d_best, nq, col_keys, stride_rows, d_best, d_xc_count);
         ++c->launches;
     }
     if (!lane_call) { stage_mark(c, 8); if (c->profiling) c->stage_valid[6] = true; }
@@ -807,12 +802,12 @@ int orbx_create(orbx_ctx** out, int device, int nfeatures, float scale_factor, i
         if (cudaMemcpy(c->pattern.p, pat, sizeof pat, cudaMemcpyHostToDevice) != cudaSuccess) return ORBX_E_CUDA;
     }
     if (cudaMemset(c->status.p, 0, sizeof(int) * B) != cudaSuccess) return ORBX_E_CUDA;
-    if (cudaFuncSetAttribute(k_hamming_umma2<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
-        cudaFuncSetAttribute(k_hamming_umma2<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
-        cudaFuncSetAttribute(k_hamming_umma<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
-        cudaFuncSetAttribute(k_hamming_umma<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
-        cudaFuncSetAttribute(k_hamming_umma2_xc<>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES_XC) != cudaSuccess ||
-        cudaFuncSetAttribute(k_hamming_umma_xc<>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES_XC) != cudaSuccess ||
+    if (cudaFuncSetAttribute(k_hamming_umma2<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
+        cudaFuncSetAttribute(k_hamming_umma2<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
+        cudaFuncSetAttribute(k_hamming_umma<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
+        cudaFuncSetAttribute(k_hamming_umma<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
+        cudaFuncSetAttribute(k_hamming_umma2<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES_XC) != cudaSuccess ||
+        cudaFuncSetAttribute(k_hamming_umma<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES_XC) != cudaSuccess ||
         cudaFuncSetAttribute(k_fast_warp<FAST_NWARP>, cudaFuncAttributeMaxDynamicSharedMemorySize, FAST_NWARP * FW_WARP_BYTES + 128) != cudaSuccess ||
         cudaFuncSetAttribute(k_pyr_tma, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024) != cudaSuccess ||
         cudaFuncSetAttribute(k_describe_tma, cudaFuncAttributeMaxDynamicSharedMemorySize, DS_NW * DS_WARP_BYTES + 128) != cudaSuccess ||

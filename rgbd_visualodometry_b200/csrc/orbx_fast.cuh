@@ -1,5 +1,6 @@
 // orbx_fast.cuh -- A.3 FAST-9/16 score + 3x3 NMS (the detector inside cv::ORB::detectAndCompute, src/frontend.cpp:153),
-// sm_100a.  WARP-PRIVATE tiles fed by TMA: no block barrier anywhere in the kernel.
+// sm_100a.  Two kernels, identical results: k_fast_bands (CTA-cooperative, small launches) and k_fast_warp (WARP-PRIVATE
+// tiles fed by TMA: no block barrier anywhere in the kernel), described here.
 //
 // Unit of work: one WARP owns one band of FW_R inner rows of one level of one frame and walks it left to right in chunks of
 // FW_CW output columns, so every row's survivors leave in x order and the per-row lists concatenate to OpenCV's raster
@@ -31,9 +32,287 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include "orbx_geom.h"
+#include "orbx_device.cuh"
 
 namespace orbx {
 
+__device__ __forceinline__ unsigned vmin2(unsigned a, unsigned b) { return __vminu2(a, b); }
+__device__ __forceinline__ unsigned vmax2(unsigned a, unsigned b) { return __vmaxu2(a, b); }
+__device__ __forceinline__ unsigned vmax3(unsigned a, unsigned b, unsigned c) { return __vimax3_u16x2(a, b, c); }
+__device__ __forceinline__ unsigned vmin3(unsigned a, unsigned b, unsigned c) { return __vimin3_u16x2(a, b, c); }
+__device__ __forceinline__ uint2 lds_v2(unsigned addr)
+{
+    uint2 v;
+    asm volatile("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(v.x), "=r"(v.y) : "r"(addr) : "memory");
+    return v;
+}
+__device__ __forceinline__ unsigned lds_u16(unsigned addr) { unsigned short v; asm volatile("ld.shared.u16 %0, [%1];" : "=h"(v) : "r"(addr) : "memory"); return v; }
+__device__ __forceinline__ void sts_u16(unsigned addr, unsigned v) { asm volatile("st.shared.u16 [%0], %1;" :: "r"(addr), "h"((unsigned short)v) : "memory"); }
+
+// ------------------------------------------------------------------------------------------------ A.3 FAST + NMS
+// One CTA = one band of R inner rows of one level of one frame, walked left to right in chunks of CWO = 248 output
+// columns, so every row's survivors come out in x order and the per-row lists concatenate to OpenCV's raster order.
+// Only the region that can survive the 31-px border filter is evaluated (SURVEY A.10).
+//
+// Per chunk (score tile = (R+2) rows x 256 columns, x = ox0-4 .. ox0+251), four block barriers:
+//   load      (R+8) x 288 pixels widened to u16 into smem with 128-bit global loads (16-byte aligned tile origin)
+//   phase A   per WARP, on its own (row, 128-pixel half) items: 4-compass-point rejection test of every pixel quad in
+//             u16x2 SIMD (native VIMNMX.U16x2) from five 64-bit shared loads; a quad with any passing pixel becomes one
+//             entry of the warp's private quad queue (one ballot per item, no atomics, no block scan, no barrier)
+//   phase A2  the same warp, on its queued quads: second rejection test on the two diagonal pairs of the circle, then the
+//             surviving pixels are expanded to pixel entries (bit-sliced warp prefix), in place
+//   phase B   the same warp runs the full 16-point test on its pixel queue.  Each circle pixel is packed
+//             (p | (255-p) << 16) so ONE sliding max over the 16 nine-long arcs (VIMNMX3.U16x2) yields both
+//             min-of-max(p) and max-of-min(p):  A = v - min_arcs max p,  -B = max_arcs min p - v,
+//             score = max(A, -B) - 1 (corner iff > t).  Corners inside the output region go to a private NMS queue.
+//   phase C   3x3 NMS (strict >) of the queued corners on the shared score tile -> per-row bit masks
+//   phase D   ordered extraction of the bit masks (popc prefix) -> global per-row lists
+// Measured and dropped (tools/stage_times.py, DESIGN.md section 8): register-prefetched next tile with three barriers per chunk,
+// persistent CTAs over (band, frame) items with static or ticket scheduling, a CTA-wide survivor queue that balances
+// phase B across warps, a u8 image tile (half the shared-memory wavefronts, more PRMT), 6-7 CTAs per SM by register cap.
+template <int R, int NT>
+__global__ void __launch_bounds__(NT) k_fast_bands(const __grid_constant__ Geom g, const uint8_t* __restrict__ pyr,
+                                                   uint32_t* __restrict__ rowcnt, uint32_t* __restrict__ rowent)
+{
+    constexpr int CWO = 248;               // output columns per chunk
+    constexpr int SP = 256;                // score tile pitch (bytes) = pixels evaluated per row
+    constexpr int SR = R + 2;              // score tile rows
+    constexpr int TP = SP + 32;            // image tile pitch (pixels, u16 each): 16-pixel aligned origin <= ox0-8, 18 x 16 pixels
+    constexpr int TPW = TP / 2;            // ... in 32-bit words
+    constexpr int TR = R + 8;              // image tile rows
+    constexpr int MW = 8;                  // mask words per row (248 bits used)
+    constexpr int T = ORBX_FAST_T;
+    constexpr int NWARP = NT / 32;
+    constexpr int ITEMS = (2 * SR + NWARP - 1) / NWARP;   // (row, half) items per warp
+    constexpr int QCAP = ITEMS * 128;      // private queue capacity: every pixel of the warp's items
+    static_assert(R * MW <= NT, "phase D needs one thread per mask word");
+    static_assert((R * MW) % 32 == 0, "phase D shuffles with a full-warp mask: its threads must be whole warps (R = 14 hangs)");
+
+    __shared__ __align__(16) uint16_t s_img[TR * TP];
+    __shared__ __align__(16) uint8_t s_score[SR * SP];
+    __shared__ uint16_t s_q[NWARP][QCAP];  // pass queues:   sy << 8 | sx; compacted IN PLACE to the corner queues (NMS candidates
+                                           // inside the output region) as phase B consumes them: a corner's slot index never
+                                           // passes the entries still to be read, so no second queue is needed
+    __shared__ uint32_t s_mask[R * MW];
+    __shared__ uint32_t s_rowcnt[R];
+
+    const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
+    const unsigned lt = lanemask_lt();
+    const int f = blockIdx.y;
+    int l = 0;
+#pragma unroll 1
+    for (int i = 1; i < g.nlevels; ++i) if ((int)blockIdx.x >= g.L[i].band0) l = i;
+    const LevelGeom& L = g.L[l];
+    const int band = blockIdx.x - L.band0;
+    if (band >= L.nbands) return;
+    const int y0 = ORBX_EDGE + band * R;
+    const int y1 = min(y0 + R, L.h - ORBX_EDGE);           // output rows [y0, y1)
+    const int nsr = y1 - y0 + 2;                            // score rows in use
+    const int xend = L.w - ORBX_EDGE;                       // output cols [31, xend)
+    const uint8_t* img = pyr + (size_t)f * g.pyr_frame + L.img_off;
+    uint32_t* cnt_out = rowcnt + (size_t)f * g.cnt_frame + L.cnt_off;
+    uint32_t* ent_out = rowent + (size_t)f * g.ent_frame + L.ent_off;
+
+    if (tid < R) s_rowcnt[tid] = 0;
+    uint16_t* myq = s_q[wid];
+    uint16_t* mycq = s_q[wid];
+
+    for (int ox0 = 28; ox0 < xend; ox0 += CWO) {
+        const int ox1 = min(ox0 + CWO, xend);
+        const int ix0 = (ox0 - 8) & ~15;                     // 16-byte aligned tile origin
+        const int xo = (ox0 - 8) - ix0;                      // 0, 4, 8 or 12: tile x of score column sx is sx + 4 + xo
+        const int need = min(ox1 - ox0 + 6, SP);             // score columns that matter: x = ox0-4 .. ox1+1
+        __syncthreads();                                     // previous chunk fully consumed
+        // ---- load tile rows [y0-4, y1+4): 128-bit loads, 16 pixels widened to u16 per thread and step
+        {
+            const int rows = y1 - y0 + 8;
+            constexpr int CPR = TP / 16;                     // 16-pixel columns per tile row
+            const int clast = (xo + need + 16) >> 4;         // last column holding a pixel phase A / B can touch
+            for (int i = tid; i < rows * CPR; i += NT) {
+                const int ty = i / CPR, col = i - ty * CPR;
+                if (col > clast) continue;
+                const int gx = ix0 + col * 16;
+                uint4 w = make_uint4(0, 0, 0, 0);
+                if (gx < L.pitch) w = __ldg(reinterpret_cast<const uint4*>(img + (size_t)(y0 - 4 + ty) * L.pitch + gx));
+                uint4* d = reinterpret_cast<uint4*>(&s_img[ty * TP + col * 16]);
+                d[0] = make_uint4(__byte_perm(w.x, 0, 0x4140), __byte_perm(w.x, 0, 0x4342), __byte_perm(w.y, 0, 0x4140), __byte_perm(w.y, 0, 0x4342));
+                d[1] = make_uint4(__byte_perm(w.z, 0, 0x4140), __byte_perm(w.z, 0, 0x4342), __byte_perm(w.w, 0, 0x4140), __byte_perm(w.w, 0, 0x4342));
+            }
+            for (int i = tid; i < SR * SP / 16; i += NT) reinterpret_cast<uint4*>(s_score)[i] = make_uint4(0, 0, 0, 0);
+            if (tid < R * MW) s_mask[tid] = 0;
+        }
+        __syncthreads();
+        // ---- phase A (per warp): compass rejection on (row, 128-pixel half) items -> private QUAD queue
+        // Shared memory is addressed through one precomputed 32-bit base per chunk (LDS with immediate offsets).  Only about
+        // one pixel in 13 passes, so the per-item bookkeeping is kept to ONE ballot: a lane whose quad has any passing
+        // pixel appends one 16-bit quad entry (sy << 10 | quad column << 4 | 4 pass flags).  The quad queue sits in the
+        // last quarter of the warp's queue region.
+        int qn4 = 0;
+        constexpr int QQ0 = QCAP - ITEMS * 32;               // first slot of the quad queue
+        {
+            constexpr unsigned K = ((511u - T) << 16) | (511u - T);
+            const unsigned qq_s = (unsigned)__cvta_generic_to_shared(myq + QQ0);
+            // 8-byte aligned: word index (sy+3)*TPW + 2q + 2 + xo/2 is even (TPW, xo/2 even)
+            const unsigned lane_s = (unsigned)__cvta_generic_to_shared(s_img) + (unsigned)(3 * TPW + 2 * lane + 2 + (xo >> 1)) * 4u;
+            for (int item = wid; item < 2 * nsr; item += NWARP) {
+                const int sy = item >> 1, half = item & 1;
+                if (half * 128 >= need) continue;            // warp-uniform: no needed pixel in this half
+                const int q = half * 32 + lane;              // quad column
+                unsigned m0 = 0, m1 = 0;
+                if (4 * q < need) {
+                    const unsigned ad = lane_s + (unsigned)(sy * TPW + half * 64) * 4u;
+                    const uint2 c = lds_v2(ad), n = lds_v2(ad - 3 * TPW * 4), s = lds_v2(ad + 3 * TPW * 4), e2 = lds_v2(ad + 8), w2 = lds_v2(ad - 8);
+                    const unsigned e0 = __byte_perm(c.y, e2.x, 0x5432), e1 = __byte_perm(e2.x, e2.y, 0x5432);
+                    const unsigned w0 = __byte_perm(w2.x, w2.y, 0x5432), w1 = __byte_perm(w2.y, c.x, 0x5432);
+                    const unsigned D0 = vmax2(vmin2(n.x, s.x), vmin2(e0, w0)), B0 = vmin2(vmax2(n.x, s.x), vmax2(e0, w0));
+                    const unsigned D1 = vmax2(vmin2(n.y, s.y), vmin2(e1, w1)), B1 = vmin2(vmax2(n.y, s.y), vmax2(e1, w1));
+                    m0 = (c.x + K - D0) | (B0 + K - c.x);
+                    m1 = (c.y + K - D1) | (B1 + K - c.y);
+                }
+                // pass flags of the quad's four pixels: bits 9 / 25 of m0 and (moved up one) bits 10 / 26 of m1, folded to
+                // a nibble: bit 0 = pixel 0, bit 1 = pixel 2, bit 2 = pixel 1, bit 3 = pixel 3
+                const unsigned pf = (m0 & 0x02000200u) | ((m1 << 1) & 0x04000400u);
+                const unsigned nib = ((pf | (pf >> 14)) >> 9) & 15u;
+                const unsigned any = __ballot_sync(0xffffffffu, nib != 0u);
+                if (nib) sts_u16(qq_s + 2u * (unsigned)(qn4 + __popc(any & lt)), (unsigned)(sy << 10) | (unsigned)(q << 4) | nib);
+                qn4 += __popc(any);
+            }
+        }
+        __syncwarp();
+        // ---- phase A2 (same warp): quad entries -> pixel entries (sy << 8 | sx), 32 quad entries at a time.
+        // First the SECOND rejection test, on the quads that survived only: the two diagonal opposite pairs of the circle
+        // ((+-2, +-2): points 2/10 and 6/14) must also hold a darker or a brighter pixel each -- same u16x2 arithmetic as
+        // phase A, from three loads per row +-2.  It roughly halves the pixels that reach the 16-point test, whose 17
+        // scattered 16-bit loads (bank conflicts) are the expensive part.  (The flags of the two tests are ANDed per pixel
+        // without their polarity: still a necessary condition.)
+        // Then each lane counts its 0..4 flagged pixels; the counts' three bit planes go through three ballots (prefix =
+        // popc of the lower lanes' bits, weighted 1 / 2 / 4) and the lane writes its entries back to back.  (Queue order is
+        // free: phase B scores every entry, the NMS works on bits.)  In place: after k quad entries at most
+        // 4k <= 3 * ITEMS * 32 + k pixel slots are written, which never reaches the unread part of the quad queue.
+        int qn = 0;
+        {
+            constexpr unsigned K = ((511u - T) << 16) | (511u - T);
+            const unsigned q_s = (unsigned)__cvta_generic_to_shared(myq);
+            const unsigned img_q = (unsigned)__cvta_generic_to_shared(s_img) + (unsigned)(3 * TPW + 2 + (xo >> 1)) * 4u;   // quad (sy, q) at + (sy * TPW + 2q) * 4
+            for (int i0 = 0; i0 < qn4; i0 += 32) {
+                const int i = i0 + lane;
+                unsigned e = 0;
+                if (i < qn4) {
+                    e = lds_u16(q_s + 2u * (unsigned)(QQ0 + i));
+                    const unsigned ad = img_q + ((e >> 10) * TPW + ((e >> 3) & 0x7Eu)) * 4u;
+                    const unsigned up = ad - 2 * TPW * 4, dn = ad + 2 * TPW * 4;
+                    const uint2 c = lds_v2(ad), u = lds_v2(up), d = lds_v2(dn);
+                    const unsigned um = lds_u32(up - 4), upp = lds_u32(up + 8), dm = lds_u32(dn - 4), dpp = lds_u32(dn + 8);
+                    // pixels 0,1: NW = um, NE = u.y, SW = dm, SE = d.y;   pixels 2,3: NW = u.x, NE = upp, SW = d.x, SE = dpp
+                    const unsigned D0 = vmax2(vmin2(um, d.y), vmin2(u.y, dm)), B0 = vmin2(vmax2(um, d.y), vmax2(u.y, dm));
+                    const unsigned D1 = vmax2(vmin2(u.x, dpp), vmin2(upp, d.x)), B1 = vmin2(vmax2(u.x, dpp), vmax2(upp, d.x));
+                    const unsigned m0 = (c.x + K - D0) | (B0 + K - c.x);
+                    const unsigned m1 = (c.y + K - D1) | (B1 + K - c.y);
+                    const unsigned pf = (m0 & 0x02000200u) | ((m1 << 1) & 0x04000400u);
+                    e &= 0xFFF0u | (((pf | (pf >> 14)) >> 9) & 15u);
+                }
+                const unsigned cnt = (unsigned)__popc(e & 15u);      // 0 .. 4
+                const unsigned c0 = __ballot_sync(0xffffffffu, cnt & 1u), c1 = __ballot_sync(0xffffffffu, cnt & 2u), c2 = __ballot_sync(0xffffffffu, cnt & 4u);
+                const unsigned pos = (unsigned)qn + __popc(c0 & lt) + 2u * __popc(c1 & lt) + 4u * __popc(c2 & lt);
+                qn += __popc(c0) + 2 * __popc(c1) + 4 * __popc(c2);
+                const unsigned ent = (e >> 2) & 0x3FFCu;             // sy << 8 | 4 * quad column
+                unsigned sa = q_s + 2u * pos;
+                if (e & 1u) { sts_u16(sa, ent); sa += 2u; }
+                if (e & 4u) { sts_u16(sa, ent + 1u); sa += 2u; }
+                if (e & 2u) { sts_u16(sa, ent + 2u); sa += 2u; }
+                if (e & 8u) sts_u16(sa, ent + 3u);
+            }
+        }
+        __syncwarp();
+        // ---- phase B (same warp): full segment test + score; corners inside the output region -> private NMS queue
+        int cn = 0;
+        {
+            const unsigned q_s = (unsigned)__cvta_generic_to_shared(myq);
+            const unsigned img_s = (unsigned)__cvta_generic_to_shared(s_img) + (unsigned)(3 * TP + 4 + xo) * 2u;   // pixel (sy, sx) at + (sy * TP + sx) * 2
+            const unsigned sc_s = (unsigned)__cvta_generic_to_shared(s_score);
+            // sx window of corners that belong to this chunk's output region: x = ox0 - 4 + sx in [max(ox0, EDGE), ox1)
+            const int sx_lo = max(ox0, ORBX_EDGE) - (ox0 - 4), sx_hi = ox1 - (ox0 - 4), sy_hi = y1 - y0;
+            for (int i0 = 0; i0 < qn; i0 += 32) {
+                const int i = i0 + lane;
+                bool corner = false;
+                unsigned e = 0;
+                if (i < qn) {
+                    e = lds_u16(q_s + 2u * (unsigned)i);
+                    const unsigned sy = e >> 8, sx = e & 255u;
+                    const unsigned c = img_s + (sy * TP + sx) * 2u;
+                    const int v = (int)lds_u16(c);
+                    unsigned q[16];
+#define ORBX_PK(k, dx, dy) q[k] = lds_u16(c + ((dy) * TP + (dx)) * 2) * 0xFFFF0001u + 0x00FF0000u
+                    ORBX_PK(0, 0, 3);   ORBX_PK(1, 1, 3);   ORBX_PK(2, 2, 2);    ORBX_PK(3, 3, 1);
+                    ORBX_PK(4, 3, 0);   ORBX_PK(5, 3, -1);  ORBX_PK(6, 2, -2);   ORBX_PK(7, 1, -3);
+                    ORBX_PK(8, 0, -3);  ORBX_PK(9, -1, -3); ORBX_PK(10, -2, -2); ORBX_PK(11, -3, -1);
+                    ORBX_PK(12, -3, 0); ORBX_PK(13, -3, 1); ORBX_PK(14, -2, 2);  ORBX_PK(15, -1, 3);
+#undef ORBX_PK
+                    unsigned m3[16], m9[16];
+#pragma unroll
+                    for (int k = 0; k < 16; ++k) m3[k] = vmax3(q[k], q[(k + 1) & 15], q[(k + 2) & 15]);
+#pragma unroll
+                    for (int k = 0; k < 16; ++k) m9[k] = vmax3(m3[k], m3[(k + 3) & 15], m3[(k + 6) & 15]);
+                    unsigned mm = vmin3(vmin3(vmin3(m9[0], m9[1], m9[2]), vmin3(m9[3], m9[4], m9[5]), vmin3(m9[6], m9[7], m9[8])),
+                                        vmin3(vmin3(m9[9], m9[10], m9[11]), vmin3(m9[12], m9[13], m9[14]), m9[15]),
+                                        0xFFFFFFFFu);
+                    const int A = v - (int)(mm & 0xffffu);
+                    const int nB = 255 - (int)(mm >> 16) - v;
+                    const int sc = max(A, nB);
+                    if (sc > T) {
+                        sts_u8(sc_s + sy * SP + sx, (unsigned)(sc - 1));
+                        corner = (int)sx >= sx_lo && (int)sx < sx_hi && sy - 1u < (unsigned)sy_hi;   // 1 <= sy <= y1 - y0
+                    }
+                }
+                const unsigned bc = __ballot_sync(0xffffffffu, corner);
+                __syncwarp();                                // every lane has read its entry of this batch before slots <= i0 + 31 are rewritten
+                if (corner) sts_u16(q_s + 2u * (unsigned)(cn + __popc(bc & lt)), e);
+                cn += __popc(bc);
+            }
+        }
+        __syncthreads();                                     // every score of the tile is in place
+        // ---- phase C (per warp): 3x3 NMS of its queued corners
+        for (int i = lane; i < cn; i += 32) {
+            const int e = mycq[i];
+            const int sy = e >> 8, sx = e & 255;
+            const uint8_t* p = &s_score[sy * SP + sx];
+            const int s = p[0];
+            if (s > p[-1] && s > p[1] && s > p[-SP - 1] && s > p[-SP] && s > p[-SP + 1] && s > p[SP - 1] && s > p[SP] && s > p[SP + 1]) {
+                const int bit = sx - 4;
+                atomicOr(&s_mask[(sy - 1) * MW + (bit >> 5)], 1u << (bit & 31));
+            }
+        }
+        __syncthreads();
+        // ---- phase D: ordered extraction; thread t owns mask word t (MW consecutive lanes = one row)
+        if (tid < R * MW) {
+            const int row = tid / MW, wi = tid - row * MW;
+            uint32_t m = s_mask[tid];
+            const int cnt = __popc(m);
+            int pre = cnt;                                   // inclusive prefix inside the row's MW-lane group
+#pragma unroll
+            for (int d = 1; d < MW; d <<= 1) {
+                const int o = __shfl_up_sync(0xffffffffu, pre, d, MW);
+                if (wi >= d) pre += o;
+            }
+            const uint32_t base = s_rowcnt[row];
+            __syncwarp();
+            uint32_t slot = base + pre - cnt;
+            uint32_t* dst = ent_out + (size_t)(y0 - ORBX_EDGE + row) * L.ent_pitch;
+            while (m) {
+                const int b = __ffs(m) - 1;
+                m &= m - 1;
+                const int bit = wi * 32 + b;
+                const uint32_t sc = s_score[(row + 1) * SP + bit + 4];
+                dst[slot++] = (uint32_t)(ox0 + bit) | (sc << 16);
+            }
+            if (wi == MW - 1) s_rowcnt[row] = base + pre;
+        }
+    }
+    __syncthreads();
+    if (tid < y1 - y0) cnt_out[y0 - ORBX_EDGE + tid] = s_rowcnt[tid];
+}
+
+// ------------------------------------------------------------------------------------------------ A.3 FAST + NMS, TMA-fed
 constexpr int FW_R = 16;                 // output rows per band
 constexpr int FW_CW = 124;               // output columns per chunk (score columns 3 .. 126 of 128)
 constexpr int FW_TP = 160;               // image tile pitch in bytes = TMA box width (16-byte aligned origin <= ox0 - 7, + 4 + 128 + 3)
@@ -56,16 +335,6 @@ static_assert(FW_CLR * 32 * 16 <= FW_OFF_CQ - FW_OFF_SCORE, "the score-tile clea
 static_assert(FW_OFF_SCORE % 16 == 0 && FW_OFF_MASK % 4 == 0 && FW_OFF_BAR % 8 == 0, "layout");
 
 struct FastMaps { CUtensorMap m[ORBX_LEVELS_MAX]; };   // one (x, y, frame) u8 tensor map per pyramid level
-
-__device__ __forceinline__ void tma_load_tile_3d(unsigned dst_s, const CUtensorMap* map, int x, int y, int z, unsigned bar_s)
-{
-    asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];"
-                 :: "r"(dst_s), "l"(map), "r"(x), "r"(y), "r"(z), "r"(bar_s) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(unsigned bar_s, unsigned bytes)
-{
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" :: "r"(bar_s), "r"(bytes) : "memory");
-}
 
 template <int NWARP>
 __global__ void __launch_bounds__(NWARP * 32, 28 / NWARP) k_fast_warp(const __grid_constant__ Geom g, const __grid_constant__ FastMaps maps, int f0,

@@ -32,6 +32,7 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include "orbx_device.cuh"
 
 namespace orbx {
 
@@ -70,27 +71,8 @@ constexpr int MT_MAX_QUERY_XC = 1 << MT_KEY_SHIFT;         // query rows represe
 
 // ---- PTX wrappers ------------------------------------------------------------------------------------------
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
 __device__ __forceinline__ void mbar_arrive(uint32_t bar) {
     asm volatile("{\n\t.reg .b64 st;\n\tmbarrier.arrive.shared::cta.b64 st, [%0];\n\t}" ::"r"(bar) : "memory");
-}
-// Bounded wait: returns false after ~0.25 s so that a protocol bug ends the kernel instead of hanging the GPU.
-__device__ __forceinline__ bool mbar_wait(uint32_t bar, uint32_t parity) {
-    unsigned long long t0 = 0;
-    for (uint32_t it = 0;; ++it) {
-        uint32_t ok;
-        asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.b32 %0, 1, 0, p;\n\t}"
-                     : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-        if (ok) return true;
-        if ((it & 1023u) == 1023u) {
-            unsigned long long t;
-            asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-            if (t0 == 0) t0 = t;
-            else if (t - t0 > 250000000ull) return false;
-        }
-    }
 }
 __device__ __forceinline__ bool elect_one() {
     uint32_t pred;
@@ -709,38 +691,33 @@ hamming_umma_body(const uint8_t* __restrict__ query, int nq, const uint8_t* __re
 }
 
 
-#define ORBX_MATCH_PARAMS const uint8_t* __restrict__ query, int nq, const uint8_t* __restrict__ train, int nt, int train_stride_rows, \
-               const int* __restrict__ train_counts, int nsets, int rows_per_split, int4* __restrict__ best, \
-               int4* __restrict__ second, int* __restrict__ keys, int* __restrict__ status
-#define ORBX_MATCH_ARGS query, nq, train, nt, train_stride_rows, train_counts, nsets, rows_per_split, best, second, keys, status
+// XCHK = true (BFMatcher crossCheck = true): the best match plus every train row's nearest query, merged into
+// col_keys[set][train_stride_rows] (INT_MIN-initialised) by atomicMax; launched with MT_SMEM_BYTES_XC.  col_keys is unused otherwise.
 // single CTA per query tile (small problems: independent CTAs, train rows can be split across them)
-template <bool KNN2>
-__global__ void __launch_bounds__(MT_THREADS, 1) k_hamming_umma(ORBX_MATCH_PARAMS) { hamming_umma_body<KNN2, false, false>(ORBX_MATCH_ARGS, nullptr); }
+template <bool KNN2, bool XCHK>
+__global__ void __launch_bounds__(MT_THREADS, 1) k_hamming_umma(const uint8_t* __restrict__ query, int nq, const uint8_t* __restrict__ train, int nt,
+                                                                int train_stride_rows, const int* __restrict__ train_counts, int nsets, int rows_per_split,
+                                                                int4* __restrict__ best, int4* __restrict__ second, int* __restrict__ keys,
+                                                                int* __restrict__ status, int* __restrict__ col_keys)
+{
+    hamming_umma_body<KNN2, false, XCHK>(query, nq, train, nt, train_stride_rows, train_counts, nsets, rows_per_split, best, second, keys, status, col_keys);
+}
 // CTA pair on the two SMs of a TPC (tcgen05 cta_group::2): blockIdx.x = 2 * pair + rank
-template <bool KNN2>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(MT_THREADS, 1) k_hamming_umma2(ORBX_MATCH_PARAMS) { hamming_umma_body<KNN2, true, false>(ORBX_MATCH_ARGS, nullptr); }
-// cross-check (BFMatcher crossCheck = true): the best-match kernels above plus every train row's nearest query, merged into
-// col_keys[set][train_stride_rows] (INT_MIN-initialised) by atomicMax; launched with MT_SMEM_BYTES_XC.
-// The cross-check kernels are templates (instantiated with <>) only so that they are emitted after the kernels instantiated
-// earlier in orbx.cu: as plain __global__ functions they change the module's function order, and with it NVVM's code for
-// k_select<512>, which they do not touch.
-template <int = 0> __global__ void __launch_bounds__(MT_THREADS, 1) k_hamming_umma_xc(ORBX_MATCH_PARAMS, int* __restrict__ col_keys)
+template <bool KNN2, bool XCHK>
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(MT_THREADS, 1) k_hamming_umma2(const uint8_t* __restrict__ query, int nq, const uint8_t* __restrict__ train,
+                                                                                          int nt, int train_stride_rows, const int* __restrict__ train_counts, int nsets,
+                                                                                          int rows_per_split, int4* __restrict__ best, int4* __restrict__ second,
+                                                                                          int* __restrict__ keys, int* __restrict__ status, int* __restrict__ col_keys)
 {
-    hamming_umma_body<false, false, true>(ORBX_MATCH_ARGS, col_keys);
+    hamming_umma_body<KNN2, true, XCHK>(query, nq, train, nt, train_stride_rows, train_counts, nsets, rows_per_split, best, second, keys, status, col_keys);
 }
-template <int = 0> __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(MT_THREADS, 1) k_hamming_umma2_xc(ORBX_MATCH_PARAMS, int* __restrict__ col_keys)
-{
-    hamming_umma_body<false, true, true>(ORBX_MATCH_ARGS, col_keys);
-}
-#undef ORBX_MATCH_PARAMS
-#undef ORBX_MATCH_ARGS
 
 // ONE CTA per set: query i keeps its best match (i, j) iff column j's key names i, i.e. i is also train row j's nearest
 // query (lowest index on ties); the kept records are compacted stably in query order to out[set][0 .. n_out[set]).
 // best and out may be the same buffer: a record only moves to a lower or equal index, and a chunk is read before it is written.
 constexpr int XC_NT = 1024;
-template <int = 0> __global__ void __launch_bounds__(XC_NT) k_crosscheck_compact(const int4* best, int nq, const int* __restrict__ col_keys, int stride_rows,
-                                                              int4* out, int* __restrict__ n_out)
+__global__ void __launch_bounds__(XC_NT) k_crosscheck_compact(const int4* best, int nq, const int* __restrict__ col_keys, int stride_rows,
+                                                                           int4* out, int* __restrict__ n_out)
 {
     __shared__ int s_warp[XC_NT / 32];
     __shared__ int s_base;

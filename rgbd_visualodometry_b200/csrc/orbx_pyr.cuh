@@ -1,5 +1,11 @@
-// orbx_pyr.cuh -- A.2 INTER_LINEAR_EXACT pyramid level l from level l-1 (cv::resize inside cv::ORB::detectAndCompute,
-// src/frontend.cpp:153), sm_100a, warp-private source tiles fed by TMA.
+// orbx_pyr.cuh -- A.1 BGR -> gray and A.2 INTER_LINEAR_EXACT pyramid (cv::cvtColor and the cv::resize inside
+// cv::ORB::detectAndCompute, src/frontend.cpp:153), sm_100a.
+//
+//   k_gray          A.1   BGR -> gray (level 0)                         HBM-bound, 16 px / thread
+//   k_pyr_down      A.2   level l from level l-1, CTA-cooperative       thread = 8 output columns x 16 rows, source rows streamed by cp.async
+//   k_pyr_tma       A.2   level l from level l-1, warp-private          warp = 128 output columns x a stack of strips, source rows by TMA
+//
+// k_pyr_tma (large launches):
 //
 //   dst(x, y) = (h0 * (256 - cy) + h1 * cy + 32768) >> 16,   h = p[i0] * (256 - cx) + p[i0 + 1] * cx     (8.8 taps, host tables)
 //
@@ -14,15 +20,220 @@
 //                    two IMADs per pixel (h <= 255 * 256, so byte 2 of the 24-bit sum IS the rounded pixel) and three PRMTs per quad.
 // ALU pipe (SHF, PRMT) and FMA pipe (IDP, IMAD) carry about the same number of instructions.
 // Levels whose scale factor makes a lane's 4 outputs span more than 7 source bytes, or whose boxes would not fit, keep the
-// register-window kernel k_pyr_down (orbx_kernels.cuh).
+// register-window kernel k_pyr_down.
 #pragma once
 #include <cuda.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include "orbx_geom.h"
+#include "orbx_device.cuh"
 
 namespace orbx {
 
+__device__ __forceinline__ void cp_async_4(unsigned dst, const void* src) { asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" :: "r"(dst), "l"(src) : "memory"); }
+
+// ------------------------------------------------------------------------------------------------ A.1 gray
+// g = (3735 B + 19235 G + 9798 R + 16384) >> 15.
+// 4 gray pixels from 12 BGR bytes: coefficients split into high / low bytes so each pixel is two IDP.4A
+//   3735 B + 19235 G + 9798 R + 16384 = 256 (14 B + 75 G + 38 R) + (151 B + 35 G + 70 R) + 16384      (exact)
+__device__ __forceinline__ uint32_t gray4(uint32_t w0, uint32_t w1, uint32_t w2)
+{
+    constexpr uint32_t CH_ = 14u | (75u << 8) | (38u << 16), CL_ = 151u | (35u << 8) | (70u << 16);
+    const uint32_t p0 = w0, p1 = __byte_perm(w0, w1, 0x0543), p2 = __byte_perm(w1, w2, 0x0432), p3 = w2 >> 8;
+    const uint32_t g0 = (__dp4a(p0, CH_, 0u) * 256u + __dp4a(p0, CL_, 16384u)) >> 15;
+    const uint32_t g1 = (__dp4a(p1, CH_, 0u) * 256u + __dp4a(p1, CL_, 16384u)) >> 15;
+    const uint32_t g2 = (__dp4a(p2, CH_, 0u) * 256u + __dp4a(p2, CL_, 16384u)) >> 15;
+    const uint32_t g3 = (__dp4a(p3, CH_, 0u) * 256u + __dp4a(p3, CL_, 16384u)) >> 15;
+    return g0 | (g1 << 8) | (g2 << 16) | (g3 << 24);
+}
+
+// One thread = 16 consecutive pixels of one row: three 128-bit loads (48 BGR bytes), one 128-bit store -- the kernel
+// is a pure HBM stream (3 bytes in, 1 byte out per pixel).  Unaligned inputs / row tails fall back to byte loads.
+template <int CH>
+__global__ void __launch_bounds__(256) k_gray(const uint8_t* __restrict__ in, unsigned long long frame_stride,
+                                              unsigned long long step, int aligned16, const __grid_constant__ Geom g,
+                                              uint8_t* __restrict__ pyr)
+{
+    const LevelGeom& L = g.L[0];
+    const int x = (blockIdx.x * blockDim.x + threadIdx.x) * 16;
+    const int y = blockIdx.y * blockDim.y + threadIdx.y;
+    const int f = blockIdx.z;
+    if (y >= L.h || x >= L.pitch) return;
+    const uint8_t* src = in + (size_t)f * frame_stride + (size_t)y * step + (size_t)x * CH;
+    uint4 out = make_uint4(0u, 0u, 0u, 0u);
+    if (aligned16 && x + 15 < L.w) {
+        const uint4* s4 = reinterpret_cast<const uint4*>(src);
+        if (CH == 3) {
+            const uint4 a = __ldg(s4), b = __ldg(s4 + 1), c = __ldg(s4 + 2);
+            out = make_uint4(gray4(a.x, a.y, a.z), gray4(a.w, b.x, b.y), gray4(b.z, b.w, c.x), gray4(c.y, c.z, c.w));
+        } else {
+            out = __ldg(s4);
+        }
+    } else {
+        uint32_t o[4] = {0u, 0u, 0u, 0u};
+#pragma unroll
+        for (int k = 0; k < 16; ++k)
+            if (x + k < L.w) {
+                const uint8_t* s = src + (size_t)k * CH;
+                const uint32_t p = CH == 3 ? (3735u * __ldg(s) + 19235u * __ldg(s + 1) + 9798u * __ldg(s + 2) + 16384u) >> 15 : (uint32_t)__ldg(s);
+                o[k >> 2] |= p << (8 * (k & 3));
+            }
+        out = make_uint4(o[0], o[1], o[2], o[3]);
+    }
+    *reinterpret_cast<uint4*>(pyr + (size_t)f * g.pyr_frame + L.img_off + (size_t)y * L.pitch + x) = out;   // pitch, offsets: multiples of 16
+}
+
+// ------------------------------------------------------------------------------------------------ A.2 pyramid
+// dst(x,y) = (h0*(256-cy) + h1*cy + 32768) >> 16,  h = p[i0]*(256-cx) + p[i1]*cx  (8.8 taps from host tables).
+// A quad of 4 adjacent output columns keeps its taps, byte offsets and funnel-shift amounts in registers; a source row
+// costs it three (wide: four) aligned 32-bit words (the 4 outputs read <= 9 consecutive source bytes at the reference's
+// ratio 1.2); each output's horizontal pass is one funnel shift + one IDP.2A (u16 taps x u8 pixels), taken once per
+// source row and reused by the next output row that needs the same row.
+constexpr int PYR_RH = 16;          // output rows per thread
+struct PyrRow { uint32_t h[4]; };
+// One level per launch.  The kernel is organised around the SOURCE rows: the thread streams the source rows it needs, in order,
+// through a private shared-memory ring filled by cp.async (PYR_DEPTH rows in flight), takes the horizontal pass of
+// each once, and emits an output row as soon as its lower source row has passed.  Load latency sits under the
+// arithmetic of the rows already there instead of in front of every output row.
+// A thread owns PYR_NQ = 2 adjacent column quads (8 output columns) of a strip of PYR_RH rows: the per-row control work
+// (ring slot, emission test, tap prefetch, pointer updates -- more than half of the instructions of a one-quad thread) is
+// shared by both quads, each of which keeps its own 3- or 4-word source window.  Work items (column octet, strip) of a
+// level are flattened over the CTAs, so warps stay full on narrow levels.
+constexpr int PYR_DEPTH = 8;
+constexpr int PYR_NT = 128;
+constexpr int PYR_NQ = 2;
+// WIDE = false: the 4 outputs of a quad reach at most 7 bytes past its aligned first source byte (scale factors up to
+// ~1.5, the reference's 1.2 included): 3 source words, one predicated select per operand.  WIDE = true: up to 11 bytes
+// (scale factors up to ~2.6): 4 source words, two selects per operand.
+template <bool WIDE>
+__global__ void __launch_bounds__(PYR_NT) k_pyr_down(const __grid_constant__ Geom g, int l, uint8_t* pyr, const uint32_t* __restrict__ tabs)
+{
+    __shared__ __align__(16) uint8_t s_ring[PYR_DEPTH * PYR_NQ * PYR_NT * 16];
+    const LevelGeom& D = g.L[l];
+    const LevelGeom& S = g.L[l - 1];
+    const int noct = D.pitch >> 3;                           // column octets per row (pitch is a multiple of 16)
+    const int item = blockIdx.x * PYR_NT + threadIdx.x;
+    const int strip = item / noct, oct = item - strip * noct;
+    const int x = oct * 8;
+    const int ys = strip * PYR_RH, ye = min(ys + PYR_RH, D.h);
+    const int f = blockIdx.y;
+    if (ys >= ye) return;
+    uint8_t* dst = pyr + (size_t)f * g.pyr_frame + D.img_off + (size_t)ys * D.pitch + x;
+    if (x >= D.w) {                                          // row padding: keep it zero
+        for (int y = ys; y < ye; ++y, dst += D.pitch) *reinterpret_cast<uint2*>(dst) = make_uint2(0u, 0u);
+        return;
+    }
+    uint32_t coef[PYR_NQ][4], sh[PYR_NQ][4];
+    bool hi[PYR_NQ][4], hi2[PYR_NQ][4];
+    int a[PYR_NQ];                                           // aligned source byte each quad is addressed from
+    bool w2ok[PYR_NQ], w3ok[PYR_NQ];
+#pragma unroll
+    for (int q = 0; q < PYR_NQ; ++q) {
+        const int xq = x + 4 * q;
+        a[q] = xq < D.w ? ((int)(__ldg(tabs + D.xtab + xq) & 0xffffu) & ~3) : a[0];
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+            const uint32_t t = (xq + k < D.w) ? __ldg(tabs + D.xtab + xq + k) : (uint32_t)a[q];   // padding columns: taps 0 -> output 0
+            const int off = (int)(t & 0xffffu) - a[q];       // 0 .. 7 (narrow), 0 .. 11 (wide)
+            const uint32_t c1 = t >> 16;
+            coef[q][k] = (xq + k < D.w) ? ((256u - c1) | (c1 << 16)) : 0u;
+            hi[q][k] = off >= 4;
+            hi2[q][k] = off >= 8;
+            sh[q][k] = (uint32_t)(off & 3) * 8u;
+        }
+        w2ok[q] = a[q] + 8 < S.pitch;
+        w3ok[q] = WIDE && a[q] + 12 < S.pitch;
+    }
+    const uint32_t* ytab = tabs + D.ytab;
+    const int s0 = (int)(__ldg(ytab + ys) & 0xffffu);
+    const int s1 = min((int)(__ldg(ytab + ye - 1) & 0xffffu) + 1, S.h - 1);         // last source row needed
+    const uint8_t* src = pyr + (size_t)f * g.pyr_frame + S.img_off + (size_t)s0 * S.pitch;
+    // ring slot d: [quad 0: 16 B x PYR_NT threads][quad 1: 16 B x PYR_NT threads]  (each LDS.128 conflict-free)
+    const unsigned ring = (unsigned)__cvta_generic_to_shared(s_ring) + threadIdx.x * 16u;
+    constexpr unsigned SLOT = PYR_NQ * PYR_NT * 16u;
+    auto fetch = [&](unsigned slot_addr, const uint8_t* row) {
+#pragma unroll
+        for (int q = 0; q < PYR_NQ; ++q) {
+            const unsigned sa = slot_addr + q * (PYR_NT * 16u);
+            const uint8_t* p = row + a[q];
+            cp_async_4(sa, p); cp_async_4(sa + 4u, p + 4);
+            if (w2ok[q]) cp_async_4(sa + 8u, p + 8);
+            if (w3ok[q]) cp_async_4(sa + 12u, p + 12);
+        }
+    };
+#pragma unroll
+    for (int d = 0; d < PYR_DEPTH; ++d) {
+        if (s0 + d <= s1) fetch(ring + d * SLOT, src + (size_t)d * S.pitch);
+        cp_async_commit();
+    }
+    src += (size_t)PYR_DEPTH * S.pitch;
+    // Output-row bookkeeping: `emit_at` is the source row at which the pending output row y can be produced
+    // (y1 = min(y0 + 1, S.h - 1)); the taps of row y + 1 are fetched one row ahead.
+    int y = ys;
+    uint32_t ty = __ldg(ytab + y), ty_next = y + 1 < ye ? __ldg(ytab + y + 1) : 0u;
+    int emit_at = min((int)(ty & 0xffffu) + 1, S.h - 1);
+    int to_fetch = (s1 - s0 + 1) - PYR_DEPTH;               // source rows not yet requested
+    unsigned sa = ring;
+    const unsigned ring_end = ring + PYR_DEPTH * SLOT;
+    PyrRow hA[PYR_NQ], hB[PYR_NQ];                           // horizontal passes of the last two source rows (ping-pong)
+#pragma unroll
+    for (int q = 0; q < PYR_NQ; ++q)
+#pragma unroll
+        for (int k = 0; k < 4; ++k) { hA[q].h[k] = 0; hB[q].h[k] = 0; }
+    // one source row: wait, read, refill the slot, horizontal pass into `hc`, emit what became complete
+    auto step = [&](int s, const PyrRow* hp, PyrRow* hc) {
+        cp_async_wait<PYR_DEPTH - 1>();
+        uint4 w[PYR_NQ];
+#pragma unroll
+        for (int q = 0; q < PYR_NQ; ++q) w[q] = lds_v4(sa + q * (PYR_NT * 16u));
+        if (to_fetch > 0) fetch(sa, src);
+        cp_async_commit();
+        --to_fetch;
+        src += S.pitch;
+        sa += SLOT;
+        if (sa == ring_end) sa = ring;
+#pragma unroll
+        for (int q = 0; q < PYR_NQ; ++q) {
+            const uint32_t w2 = w2ok[q] ? w[q].z : 0u, w3 = w3ok[q] ? w[q].w : 0u;
+#pragma unroll
+            for (int k = 0; k < 4; ++k) {
+                uint32_t lo = hi[q][k] ? w[q].y : w[q].x, up = hi[q][k] ? w2 : w[q].y;
+                if (WIDE) { lo = hi2[q][k] ? w2 : lo; up = hi2[q][k] ? w3 : up; }
+                hc[q].h[k] = __dp2a_lo(coef[q][k], __funnelshift_r(lo, up, sh[q][k]), 0u);
+            }
+        }
+        while (emit_at == s && y < ye) {                     // (two outputs per source row only when the bottom row clamps)
+            const bool clamped = (int)(ty & 0xffffu) == s;   // y1 == y0: both taps read the last source row
+            const uint32_t cy1 = ty >> 16, cy0 = 256u - cy1;
+            uint32_t out[PYR_NQ];
+            // vertical pass: h <= 255 * 256, so top * cy0 + cur * cy1 + 2^15 < 2^24 and its byte 2 IS the rounded pixel
+            // (never above 255): two IMADs per pixel on the FMA pipe and three PRMTs per quad to gather the bytes
+            auto blend = [&](const PyrRow* top) {
+#pragma unroll
+                for (int q = 0; q < PYR_NQ; ++q) {
+                    uint32_t v[4];
+#pragma unroll
+                    for (int k = 0; k < 4; ++k) v[k] = top[q].h[k] * cy0 + (hc[q].h[k] * cy1 + 32768u);
+                    out[q] = __byte_perm(__byte_perm(v[0], v[1], 0x0062), __byte_perm(v[2], v[3], 0x0062), 0x5410);
+                }
+            };
+            if (clamped) blend(hc); else blend(hp);
+            *reinterpret_cast<uint2*>(dst) = make_uint2(out[0], out[1]);
+            dst += D.pitch;
+            ++y;
+            ty = ty_next;
+            emit_at = min((int)(ty & 0xffffu) + 1, S.h - 1);
+            if (y + 1 < ye) ty_next = __ldg(ytab + y + 1);
+        }
+    };
+#pragma unroll 1
+    for (int s = s0; s <= s1; s += 2) {
+        step(s, hA, hB);
+        if (s + 1 <= s1) step(s + 1, hB, hA);
+    }
+}
+
+// ------------------------------------------------------------------------------------------------ A.2 pyramid, TMA-fed
 constexpr int PT_RH = 16;                // output rows per strip
 constexpr int PT_CW = 128;               // output columns per column tile
 constexpr int PT_NWARP = 4;              // warps per CTA (independent units)
