@@ -156,6 +156,25 @@ int orbx_match_hamming_crosscheck(orbx_ctx* ctx, const uint8_t* query, int nq, c
 int orbx_match_hamming_device_crosscheck(orbx_ctx* ctx, const uint8_t* d_query, int nq, const uint8_t* d_train,
                                          int train_stride_rows, const int* d_train_counts, int nsets,
                                          orbx_match* d_out, int* d_n_out);
+/* PAIRWISE batch, DEVICE-resident, asynchronous: pair p matches query set p against train set p (per-frame candidate
+ * sets, frame-to-frame, stereo or keyframe pairs), all pairs in one launch.  Query set p: min(d_query_counts[p],
+ * query_stride_rows) rows at d_query + p*query_stride_rows*32 (a negative count is 0); train set p likewise with
+ * d_train / train_stride_rows / d_train_counts.  These are exactly the layouts orbx_detect_and_compute_device writes, so
+ * frame-to-frame matching of a batch is d_query = desc, d_train = desc + cap*32, d_query_counts = counts,
+ * d_train_counts = counts + 1, both strides cap, npairs = batch - 1.  An arbitrary list of pairs is gathered into such
+ * sets first.  Per pair the results equal BFMatcher(NORM_HAMMING).match (and knnMatch(k = 2) with d_second) of that
+ * pair's rows: queryIdx / trainIdx index the pair's own sets, imgIdx = 0.  d_best / d_second (NULL: no second) are
+ * [npairs][query_stride_rows]; record i of pair p is written for i < that pair's query count only; an empty train set
+ * gives trainIdx = -1, distance = 0.  npairs = 0 or a stride of 0 launches nothing.  Null pointers, negative sizes or
+ * npairs > 65535 -> ORBX_E_ARG; a stride of 2^20 rows or more -> ORBX_E_UNSUPPORTED. */
+int orbx_match_hamming_device_pairwise(orbx_ctx* ctx, const uint8_t* d_query, int query_stride_rows, const int* d_query_counts,
+                                       const uint8_t* d_train, int train_stride_rows, const int* d_train_counts, int npairs,
+                                       orbx_match* d_best, orbx_match* d_second);
+/* As above with crossCheck = true: pair p's mutual pairs compacted to d_out + p*query_stride_rows (ascending queryIdx),
+ * their count in d_n_out[p].  A stride of 0 zeroes d_n_out[0 .. npairs). */
+int orbx_match_hamming_device_pairwise_crosscheck(orbx_ctx* ctx, const uint8_t* d_query, int query_stride_rows,
+                                                  const int* d_query_counts, const uint8_t* d_train, int train_stride_rows,
+                                                  const int* d_train_counts, int npairs, orbx_match* d_out, int* d_n_out);
 /* The front-end's whole per-frame pattern on HOST frames in one call (src/frontend.cpp:98-108: one detectAndCompute,
  * then match() of map-point candidates against the frame's descriptors, src/frontend.cpp:153 + :187), for a batch:
  * extraction as orbx_detect_and_compute_batch, then for each of the `nmaps` query sets (queries[j]: nq[j] x 32 host

@@ -70,6 +70,8 @@ SYMBOLS = {
     "orbx_match_hamming_sets": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, _P, C.c_int, _P, _P]),
     "orbx_match_hamming_crosscheck": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, _P, C.POINTER(C.c_int)]),
     "orbx_match_hamming_device_crosscheck": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, _P, C.c_int, _P, _P]),
+    "orbx_match_hamming_device_pairwise": (C.c_int, [_P, _P, C.c_int, _P, _P, C.c_int, _P, C.c_int, _P, _P]),
+    "orbx_match_hamming_device_pairwise_crosscheck": (C.c_int, [_P, _P, C.c_int, _P, _P, C.c_int, _P, C.c_int, _P, _P]),
     "orbx_extract_match_batch": (C.c_int, [_P, C.POINTER(_P), C.c_int, C.c_int, C.c_int, C.c_size_t, C.c_int, _P, _P, C.c_int, _P,
                                           C.POINTER(_P), C.POINTER(C.c_int), C.c_int, C.POINTER(_P)]),
     "orbx_host_register": (C.c_int, [_P, _P, C.c_size_t]),

@@ -621,8 +621,10 @@ int sync_match_words(orbx_ctx* c, int slot, int n)
 // whose key scratch is shared.
 // Cross-check (d_xc_count set, d_second null, not a lane call): set s's mutual pairs are compacted in place to d_best + s * nq,
 // their count to d_xc_count[s].
+// Pairwise (d_qcounts set, not a lane call): set s matches its own min(d_qcounts[s], nq) query rows at d_q + s * nq * 32, so nq
+// is the query stride (and the record pitch); one CTA per (set, query tile), and record slots past a set's count stay untouched.
 int run_match(orbx_ctx* c, const uint8_t* d_q, int nq, const uint8_t* d_t, int nt, int stride_rows, const int* d_counts, int nsets,
-              int4* d_best, int4* d_second, cudaStream_t st = nullptr, int slot = 0, int* d_xc_count = nullptr)
+              int4* d_best, int4* d_second, cudaStream_t st = nullptr, int slot = 0, int* d_xc_count = nullptr, const int* d_qcounts = nullptr)
 {
     NvtxRange nvr("orbx:match_hamming");
     const bool lane_call = st != nullptr;
@@ -649,9 +651,12 @@ int run_match(orbx_ctx* c, const uint8_t* d_q, int nq, const uint8_t* d_t, int n
     nsplit = (nt + rows_per_split - 1) / rows_per_split;
     // Many sets: each CTA keeps its expanded query tile and walks sets z, z + zgroups, ... (persistent pipelines).
     // zgroups: waves(z) * sets-per-CTA(z) is the time in units of one (query tile, set) pass; a CTA's setup (TMEM
-    // allocation, query expansion, pipeline fill) costs about a third of such a pass for ~1000-row sets, less for longer ones
-    int zgroups = 1;
-    {
+    // allocation, query expansion, pipeline fill) costs about a third of such a pass for ~1000-row sets, less for longer ones.
+    // Pairwise: every set has its own query tile, so every set gets its own CTAs.
+    const bool pairwise = d_qcounts != nullptr;
+    int zgroups = nsets;
+    if (!pairwise) {
+        zgroups = 1;
         const long per_z = (long)tiles_m * nsplit;
         const long setup20 = std::max<long>(1, std::min<long>(20, 20L * 4 / std::max(1, tiles_per_split)));   // in 1/20 passes
         long best_cost = -1;
@@ -681,18 +686,28 @@ int run_match(orbx_ctx* c, const uint8_t* d_q, int nq, const uint8_t* d_t, int n
         ++c->launches;
     }
     const dim3 grd((unsigned)tiles_m, (unsigned)nsplit, (unsigned)zgroups);
+    const int smem = xchk ? MT_SMEM_BYTES_XC : MT_SMEM_BYTES;
     // (knn2 and xchk never meet: the cross-check keeps the best match only)
-    auto* kernel = pair ? (xchk ? k_hamming_umma2<false, true> : knn2 ? k_hamming_umma2<true, false> : k_hamming_umma2<false, false>)
-                        : (xchk ? k_hamming_umma<false, true> : knn2 ? k_hamming_umma<true, false> : k_hamming_umma<false, false>);
-    kernel<<<grd, MT_THREADS, xchk ? MT_SMEM_BYTES_XC : MT_SMEM_BYTES, st>>>(d_q, nq, d_t, nt, stride_rows, d_counts, nsets, rows_per_split, d_best,
-                                                                          d_second, keys, d_status, col_keys);
+    if (pairwise) {
+        auto* kernel = pair ? (xchk ? k_hamming_umma2_pw<false, true> : knn2 ? k_hamming_umma2_pw<true, false> : k_hamming_umma2_pw<false, false>)
+                            : (xchk ? k_hamming_umma_pw<false, true> : knn2 ? k_hamming_umma_pw<true, false> : k_hamming_umma_pw<false, false>);
+        kernel<<<grd, MT_THREADS, smem, st>>>(d_q, nq, d_t, nt, stride_rows, d_counts, nsets, rows_per_split, d_best, d_second, keys, d_status,
+                                              col_keys, d_qcounts);
+    } else {
+        auto* kernel = pair ? (xchk ? k_hamming_umma2<false, true> : knn2 ? k_hamming_umma2<true, false> : k_hamming_umma2<false, false>)
+                            : (xchk ? k_hamming_umma<false, true> : knn2 ? k_hamming_umma<true, false> : k_hamming_umma<false, false>);
+        kernel<<<grd, MT_THREADS, smem, st>>>(d_q, nq, d_t, nt, stride_rows, d_counts, nsets, rows_per_split, d_best, d_second, keys, d_status,
+                                              col_keys);
+    }
     ++c->launches;
     if (nsplit > 1) {
-        k_match_finalize<<<(unsigned)((nout + 255) / 256), 256, 0, st>>>(keys, nq, nout, d_best);
+        if (pairwise) k_match_finalize_pw<<<(unsigned)((nout + 255) / 256), 256, 0, st>>>(keys, nq, d_qcounts, nout, d_best);
+        else          k_match_finalize<<<(unsigned)((nout + 255) / 256), 256, 0, st>>>(keys, nq, nout, d_best);
         ++c->launches;
     }
     if (xchk) {                                              // reads the finalised row winners
-        k_crosscheck_compact<<<(unsigned)nsets, XC_NT, 0, st>>>(d_best, nq, col_keys, stride_rows, d_best, d_xc_count);
+        if (pairwise) k_crosscheck_compact_pw<<<(unsigned)nsets, XC_NT, 0, st>>>(d_best, nq, d_qcounts, col_keys, stride_rows, d_best, d_xc_count);
+        else          k_crosscheck_compact<<<(unsigned)nsets, XC_NT, 0, st>>>(d_best, nq, col_keys, stride_rows, d_best, d_xc_count);
         ++c->launches;
     }
     if (!lane_call) { stage_mark(c, 8); if (c->profiling) c->stage_valid[6] = true; }
@@ -808,6 +823,12 @@ int orbx_create(orbx_ctx** out, int device, int nfeatures, float scale_factor, i
         cudaFuncSetAttribute(k_hamming_umma<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
         cudaFuncSetAttribute(k_hamming_umma2<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES_XC) != cudaSuccess ||
         cudaFuncSetAttribute(k_hamming_umma<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES_XC) != cudaSuccess ||
+        cudaFuncSetAttribute(k_hamming_umma2_pw<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
+        cudaFuncSetAttribute(k_hamming_umma2_pw<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
+        cudaFuncSetAttribute(k_hamming_umma_pw<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
+        cudaFuncSetAttribute(k_hamming_umma_pw<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
+        cudaFuncSetAttribute(k_hamming_umma2_pw<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES_XC) != cudaSuccess ||
+        cudaFuncSetAttribute(k_hamming_umma_pw<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES_XC) != cudaSuccess ||
         cudaFuncSetAttribute(k_fast_warp<FAST_NWARP>, cudaFuncAttributeMaxDynamicSharedMemorySize, FAST_NWARP * FW_WARP_BYTES + 128) != cudaSuccess ||
         cudaFuncSetAttribute(k_pyr_tma, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024) != cudaSuccess ||
         cudaFuncSetAttribute(k_describe_tma, cudaFuncAttributeMaxDynamicSharedMemorySize, DS_NW * DS_WARP_BYTES + 128) != cudaSuccess ||
@@ -1147,6 +1168,48 @@ int orbx_match_hamming_device_crosscheck(orbx_ctx* c, const uint8_t* d_query, in
     }
     if (!d_query || !d_train || !d_out || !d_train_counts) return fail(c, ORBX_E_ARG, "null pointer");
     return run_match(c, d_query, nq, d_train, train_stride_rows, train_stride_rows, d_train_counts, nsets, (int4*)d_out, nullptr, nullptr, 0, d_n_out);
+}
+
+// orbx_match_hamming_device_pairwise[_crosscheck]: pair p = query set p against train set p.  Argument checks common to both.
+static int check_args_pairwise(orbx_ctx* c, const uint8_t* d_query, int query_stride_rows, const int* d_query_counts, const uint8_t* d_train,
+                               int train_stride_rows, const int* d_train_counts, int npairs, const void* d_out)
+{
+    if (query_stride_rows < 0 || train_stride_rows < 0 || npairs < 0 || npairs > 65535) return fail(c, ORBX_E_ARG, "bad sizes");
+    if (query_stride_rows >= MT_MAX_TRAIN || train_stride_rows >= MT_MAX_TRAIN)
+        return fail(c, ORBX_E_UNSUPPORTED, "pairwise set stride of 2^20 rows or more");
+    if (!d_query || !d_query_counts || !d_train || !d_train_counts || !d_out) return fail(c, ORBX_E_ARG, "null pointer");
+    return ORBX_OK;
+}
+
+int orbx_match_hamming_device_pairwise(orbx_ctx* c, const uint8_t* d_query, int query_stride_rows, const int* d_query_counts,
+                                       const uint8_t* d_train, int train_stride_rows, const int* d_train_counts, int npairs,
+                                       orbx_match* d_best, orbx_match* d_second)
+{
+    if (!c) return ORBX_E_ARG;
+    int rc = check_args_pairwise(c, d_query, query_stride_rows, d_query_counts, d_train, train_stride_rows, d_train_counts, npairs, d_best);
+    if (rc) return rc;
+    if (npairs == 0 || query_stride_rows == 0 || train_stride_rows == 0) return ORBX_OK;
+    CU(cudaSetDevice(c->device));
+    return run_match(c, d_query, query_stride_rows, d_train, train_stride_rows, train_stride_rows, d_train_counts, npairs, (int4*)d_best,
+                     (int4*)d_second, nullptr, 0, nullptr, d_query_counts);
+}
+
+int orbx_match_hamming_device_pairwise_crosscheck(orbx_ctx* c, const uint8_t* d_query, int query_stride_rows, const int* d_query_counts,
+                                                  const uint8_t* d_train, int train_stride_rows, const int* d_train_counts, int npairs,
+                                                  orbx_match* d_out, int* d_n_out)
+{
+    if (!c) return ORBX_E_ARG;
+    int rc = check_args_pairwise(c, d_query, query_stride_rows, d_query_counts, d_train, train_stride_rows, d_train_counts, npairs, d_out);
+    if (rc) return rc;
+    if (!d_n_out) return fail(c, ORBX_E_ARG, "null pointer");
+    if (npairs == 0) return ORBX_OK;
+    CU(cudaSetDevice(c->device));
+    if (query_stride_rows == 0 || train_stride_rows == 0) {  // no pairs in any set
+        CU(cudaMemsetAsync(d_n_out, 0, sizeof(int) * (size_t)npairs, c->stream));
+        return ORBX_OK;
+    }
+    return run_match(c, d_query, query_stride_rows, d_train, train_stride_rows, train_stride_rows, d_train_counts, npairs, (int4*)d_out, nullptr,
+                     nullptr, 0, d_n_out, d_query_counts);
 }
 
 int orbx_filter_matches(orbx_match* m, int n, float ratio)

@@ -29,6 +29,9 @@
 // Pipelines: smem stages (expanders <-> issuer) and TMEM accumulators (issuer <-> epilogue), all mbarrier based,
 // running continuously across set boundaries (persistent CTAs).  Train-row ranges can be split across CTAs (small
 // problems); partial results merge with atomicMax on the packed key.
+// Pairwise batches (SETQ: query set s against train set s, e.g. frame i against frame i + 1) cannot keep one A operand
+// across sets, so there a CTA owns ONE (set, query tile) unit: gridDim.z = number of sets, the A tile is expanded at setup
+// as above, and CTAs whose query tile is empty for their set exit before any setup.  Few units keep the train-row split.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -315,13 +318,25 @@ __device__ __forceinline__ void xc_warp_columns(const uint32_t* rp, bool valid, 
 }
 __device__ __forceinline__ void xc_epilogue_sync() { asm volatile("bar.sync 1, 256;" ::: "memory"); }   // the 8 epilogue warps only
 
-template <bool KNN2, bool PAIR, bool XCHK>
+// SETQ = false: one query set (the map) shared by every train set; nq is its row count.
+// SETQ = true (pairwise): set s has its own query rows, min(query_counts[s], nq) of them at query + s * nq * 32, so nq is
+// the query stride and the pitch of the outputs and of the split keys.  The A tile then belongs to ONE set: the grid has
+// gridDim.z = nsets (one (set, query tile) unit per CTA), and a CTA whose query tile is empty for its set exits before
+// any setup -- in a CTA pair only when the leader's (lower) tile is empty too, because the peer holds half of every B tile.
+template <bool KNN2, bool PAIR, bool XCHK, bool SETQ>
 __device__ __forceinline__ void
 hamming_umma_body(const uint8_t* __restrict__ query, int nq, const uint8_t* __restrict__ train, int nt, int train_stride_rows,
                const int* __restrict__ train_counts, int nsets, int rows_per_split, int4* __restrict__ best,
-               int4* __restrict__ second, int* __restrict__ keys, int* __restrict__ status, int* __restrict__ col_keys)
+               int4* __restrict__ second, int* __restrict__ keys, int* __restrict__ status, int* __restrict__ col_keys,
+               const int* __restrict__ query_counts)
 {
     static_assert(!(KNN2 && XCHK), "cross-check keeps the best match only");
+    int nqv = nq;                                            // query rows present (padded rows q >= nqv are excluded)
+    if constexpr (SETQ) {
+        nqv = max(0, min(__ldg(query_counts + blockIdx.z), nq));
+        if ((PAIR ? (int)(blockIdx.x & ~1u) : (int)blockIdx.x) * MT_QROWS >= nqv) return;
+        query += (size_t)blockIdx.z * nq * 32;
+    }
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
     const uint32_t sbase = smem_u32(smem);
@@ -362,7 +377,7 @@ hamming_umma_body(const uint8_t* __restrict__ query, int nq, const uint8_t* __re
     if (warp >= MT_EPI_WARP0 && warp < MT_EPI_WARP0 + 8) {   // thread <-> query row <-> TMEM lane (same mapping as the epilogue)
         const int q = q0 + ((warp - MT_EPI_WARP0) >> 2) * 128 + (warp & 3) * 32 + lane;
         uint4 lo = make_uint4(0, 0, 0, 0), hi = lo;
-        if (q < nq) {
+        if (q < nqv) {
             const uint4* p = reinterpret_cast<const uint4*>(query + (size_t)q * 32);
             lo = __ldg(p); hi = __ldg(p + 1);
         }
@@ -571,7 +586,7 @@ hamming_umma_body(const uint8_t* __restrict__ query, int nq, const uint8_t* __re
                     const unsigned pk = __vimax3_s16x2(__vimax3_s16x2(p[0], p[1], p[2]), __vimax3_s16x2(p[3], p[4], p[5]), __vmaxs2(p[6], p[7]));
                     k1 = max((int)(pk << 16) >> 16, (int)pk >> 16);
                     if constexpr (XCHK)
-                        xc_warp_columns(rp, qrow < nq, qrow - q0, reinterpret_cast<int*>(smem + MT_SMEM_XC) + (b * 8 + warp - MT_EPI_WARP0) * MT_BN);
+                        xc_warp_columns(rp, qrow < nqv, qrow - q0, reinterpret_cast<int*>(smem + MT_SMEM_XC) + (b * 8 + warp - MT_EPI_WARP0) * MT_BN);
                 } else if (!KNN2) {
                     // a set's partial last tile was issued with N = 32, 64 (or 96) columns, its rows past the set's end are
                     // copies of the last row (never the maximum): same packed path, 32-column chunks as far as N goes
@@ -599,7 +614,7 @@ hamming_umma_body(const uint8_t* __restrict__ query, int nq, const uint8_t* __re
                     const unsigned pk = __vimax3_s16x2(__vimax3_s16x2(p[0], p[1], p[2]), __vimax3_s16x2(p[3], p[4], p[5]), __vmaxs2(p[6], p[7]));
                     k1 = max((int)(pk << 16) >> 16, (int)pk >> 16);
                     if constexpr (XCHK)                      // (chunks past N hold -32768: no column there)
-                        xc_warp_columns(rp, qrow < nq, qrow - q0, reinterpret_cast<int*>(smem + MT_SMEM_XC) + (b * 8 + warp - MT_EPI_WARP0) * MT_BN);
+                        xc_warp_columns(rp, qrow < nqv, qrow - q0, reinterpret_cast<int*>(smem + MT_SMEM_XC) + (b * 8 + warp - MT_EPI_WARP0) * MT_BN);
                 } else {
 #pragma unroll
                     for (int ch = 0; ch < NCH; ++ch) tc_ld32(tacc + (uint32_t)(ch * 32), r[ch]);
@@ -659,7 +674,7 @@ hamming_umma_body(const uint8_t* __restrict__ query, int nq, const uint8_t* __re
                     }
                 }
             }
-            if (ok && qrow < nq) {
+            if (ok && qrow < nqv) {
                 const size_t o = (size_t)set * nq + qrow;
                 if (keys) {
                     if (m1 != INT_MIN) atomicMax(&keys[o], m1);
@@ -700,7 +715,8 @@ __global__ void __launch_bounds__(MT_THREADS, 1) k_hamming_umma(const uint8_t* _
                                                                 int4* __restrict__ best, int4* __restrict__ second, int* __restrict__ keys,
                                                                 int* __restrict__ status, int* __restrict__ col_keys)
 {
-    hamming_umma_body<KNN2, false, XCHK>(query, nq, train, nt, train_stride_rows, train_counts, nsets, rows_per_split, best, second, keys, status, col_keys);
+    hamming_umma_body<KNN2, false, XCHK, false>(query, nq, train, nt, train_stride_rows, train_counts, nsets, rows_per_split, best, second, keys, status,
+                                                col_keys, nullptr);
 }
 // CTA pair on the two SMs of a TPC (tcgen05 cta_group::2): blockIdx.x = 2 * pair + rank
 template <bool KNN2, bool XCHK>
@@ -709,21 +725,43 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(MT_THREADS, 1) k_ham
                                                                                           int rows_per_split, int4* __restrict__ best, int4* __restrict__ second,
                                                                                           int* __restrict__ keys, int* __restrict__ status, int* __restrict__ col_keys)
 {
-    hamming_umma_body<KNN2, true, XCHK>(query, nq, train, nt, train_stride_rows, train_counts, nsets, rows_per_split, best, second, keys, status, col_keys);
+    hamming_umma_body<KNN2, true, XCHK, false>(query, nq, train, nt, train_stride_rows, train_counts, nsets, rows_per_split, best, second, keys, status,
+                                               col_keys, nullptr);
+}
+// Pairwise (SETQ): set s's own query rows against train set s; nq = query stride, query_counts[nsets]; gridDim.z = nsets
+template <bool KNN2, bool XCHK>
+__global__ void __launch_bounds__(MT_THREADS, 1) k_hamming_umma_pw(const uint8_t* __restrict__ query, int nq, const uint8_t* __restrict__ train, int nt,
+                                                                   int train_stride_rows, const int* __restrict__ train_counts, int nsets, int rows_per_split,
+                                                                   int4* __restrict__ best, int4* __restrict__ second, int* __restrict__ keys,
+                                                                   int* __restrict__ status, int* __restrict__ col_keys, const int* __restrict__ query_counts)
+{
+    hamming_umma_body<KNN2, false, XCHK, true>(query, nq, train, nt, train_stride_rows, train_counts, nsets, rows_per_split, best, second, keys, status,
+                                               col_keys, query_counts);
+}
+template <bool KNN2, bool XCHK>
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(MT_THREADS, 1) k_hamming_umma2_pw(const uint8_t* __restrict__ query, int nq, const uint8_t* __restrict__ train,
+                                                                                             int nt, int train_stride_rows, const int* __restrict__ train_counts, int nsets,
+                                                                                             int rows_per_split, int4* __restrict__ best, int4* __restrict__ second,
+                                                                                             int* __restrict__ keys, int* __restrict__ status, int* __restrict__ col_keys,
+                                                                                             const int* __restrict__ query_counts)
+{
+    hamming_umma_body<KNN2, true, XCHK, true>(query, nq, train, nt, train_stride_rows, train_counts, nsets, rows_per_split, best, second, keys, status,
+                                              col_keys, query_counts);
 }
 
 // ONE CTA per set: query i keeps its best match (i, j) iff column j's key names i, i.e. i is also train row j's nearest
 // query (lowest index on ties); the kept records are compacted stably in query order to out[set][0 .. n_out[set]).
 // best and out may be the same buffer: a record only moves to a lower or equal index, and a chunk is read before it is written.
+// nq rows of the set are read; pitch is the record distance between sets (nq, or the query stride of a pairwise call).
 constexpr int XC_NT = 1024;
-__global__ void __launch_bounds__(XC_NT) k_crosscheck_compact(const int4* best, int nq, const int* __restrict__ col_keys, int stride_rows,
-                                                                           int4* out, int* __restrict__ n_out)
+__device__ __forceinline__ void crosscheck_compact_set(const int4* best, int nq, int pitch, const int* __restrict__ col_keys, int stride_rows,
+                                                       int4* out, int* __restrict__ n_out)
 {
     __shared__ int s_warp[XC_NT / 32];
     __shared__ int s_base;
     const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
     const size_t set = blockIdx.x;
-    best += set * nq; out += set * nq; col_keys += set * stride_rows;
+    best += set * pitch; out += set * pitch; col_keys += set * stride_rows;
     if (tid == 0) s_base = 0;
     __syncthreads();
     for (int base = 0; base < nq; base += XC_NT) {
@@ -744,6 +782,11 @@ __global__ void __launch_bounds__(XC_NT) k_crosscheck_compact(const int4* best, 
     }
     if (tid == 0) n_out[set] = s_base;
 }
+__global__ void __launch_bounds__(XC_NT) k_crosscheck_compact(const int4* best, int nq, const int* __restrict__ col_keys, int stride_rows,
+                                                                           int4* out, int* __restrict__ n_out)
+{
+    crosscheck_compact_set(best, nq, nq, col_keys, stride_rows, out, n_out);
+}
 
 __global__ void k_match_keys_init(int* __restrict__ keys, size_t n)
 {
@@ -751,14 +794,35 @@ __global__ void k_match_keys_init(int* __restrict__ keys, size_t n)
     if (i < n) keys[i] = INT_MIN;
 }
 
-__global__ void k_match_finalize(const int* __restrict__ keys, int nq, size_t n, int4* __restrict__ best)
+// split keys -> DMatch record i of [n / nq][nq]
+__device__ __forceinline__ void match_finalize_record(const int* __restrict__ keys, int nq, size_t i, int4* __restrict__ best)
 {
-    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
     const int k = keys[i];
     if (k == INT_MIN) { best[i] = make_int4((int)(i % (size_t)nq), -1, 0, 0); return; }
     const int dot = k >> MT_KEY_SHIFT, j = (MT_MAX_TRAIN - 1) - (k & (MT_MAX_TRAIN - 1));
     best[i] = make_int4((int)(i % (size_t)nq), j, 0, __float_as_int((float)((256 - dot) >> 1)));
+}
+
+__global__ void k_match_finalize(const int* __restrict__ keys, int nq, size_t n, int4* __restrict__ best)
+{
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    match_finalize_record(keys, nq, i, best);
+}
+
+// ---- pairwise (SETQ) finishing kernels: set s holds min(query_counts[s], nq) queries at records s * nq ...; the record
+// slots past that count are left as they are
+__global__ void k_match_finalize_pw(const int* __restrict__ keys, int nq, const int* __restrict__ query_counts, size_t n, int4* __restrict__ best)
+{
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n || (int)(i % (size_t)nq) >= __ldg(query_counts + i / (size_t)nq)) return;
+    match_finalize_record(keys, nq, i, best);
+}
+
+__global__ void __launch_bounds__(XC_NT) k_crosscheck_compact_pw(const int4* best, int nq, const int* __restrict__ query_counts,
+                                                                 const int* __restrict__ col_keys, int stride_rows, int4* out, int* __restrict__ n_out)
+{
+    crosscheck_compact_set(best, max(0, min(__ldg(query_counts + blockIdx.x), nq)), nq, col_keys, stride_rows, out, n_out);
 }
 
 }  // namespace orbx

@@ -183,6 +183,20 @@ class Context:
         self._check(self.lib.orbx_match_hamming_device_ragged(self.h, d_query_ptr, nq, d_train_ptr, stride_rows, d_counts_ptr, nsets,
                                                               d_best_ptr, d_second_ptr or None))
 
+    def match_device_pairwise(self, d_query_ptr: int, query_stride_rows: int, d_query_counts_ptr: int, d_train_ptr: int,
+                              train_stride_rows: int, d_train_counts_ptr: int, npairs: int, d_best_ptr: int, d_second_ptr: int = 0):
+        """Asynchronous, device-resident: pair p's own query set against its own train set ([npairs, query_stride_rows] records;
+        slots past a pair's query count are not written)."""
+        self._check(self.lib.orbx_match_hamming_device_pairwise(self.h, d_query_ptr, query_stride_rows, d_query_counts_ptr, d_train_ptr,
+                                                                train_stride_rows, d_train_counts_ptr, npairs, d_best_ptr, d_second_ptr or None))
+
+    def match_device_pairwise_crosscheck(self, d_query_ptr: int, query_stride_rows: int, d_query_counts_ptr: int, d_train_ptr: int,
+                                         train_stride_rows: int, d_train_counts_ptr: int, npairs: int, d_out_ptr: int, d_n_out_ptr: int):
+        """As match_device_pairwise with crossCheck: pair p's mutual pairs to d_out[p, :d_n_out[p]]."""
+        self._check(self.lib.orbx_match_hamming_device_pairwise_crosscheck(self.h, d_query_ptr, query_stride_rows, d_query_counts_ptr,
+                                                                           d_train_ptr, train_stride_rows, d_train_counts_ptr, npairs,
+                                                                           d_out_ptr, d_n_out_ptr))
+
     def match_sets(self, query: np.ndarray, train: np.ndarray, counts: np.ndarray, knn2: bool = False):
         """One map (query [M,32]) against nsets frames' descriptor sets (train [S,cap,32], counts [S]); host buffers."""
         q = np.ascontiguousarray(query, np.uint8).reshape(-1, 32)
