@@ -39,6 +39,7 @@ extern "C" {
 
 #define ORBX_MAX_LEVELS 16
 #define ORBX_DESC_BYTES 32
+#define ORBX_MAX_KNN 32   /* largest k of the knnMatch entry points (orbx_match_hamming_*knn) */
 
 typedef struct orbx_ctx orbx_ctx; /* opaque */
 
@@ -129,6 +130,12 @@ int orbx_match_hamming(orbx_ctx* ctx, const uint8_t* query, int nq, const uint8_
  * when nt == 1 the second record has trainIdx = -1. */
 int orbx_match_hamming_knn2(orbx_ctx* ctx, const uint8_t* query, int nq, const uint8_t* train, int nt,
                             orbx_match* out, int* n_out);
+/* knnMatch(query, train, k) for any 1 <= k <= ORBX_MAX_KNN, HOST buffers: out holds [nq][k] records; record r of query i
+ * is its r-th nearest train row by (distance, trainIdx), exactly cv's list; records r >= nt have trainIdx = -1, distance 0.
+ * *n_out = nq (0 if either set is empty).  k = 1 gives orbx_match_hamming's records, k = 2 orbx_match_hamming_knn2's.
+ * k < 1 -> ORBX_E_ARG; k > ORBX_MAX_KNN or nt >= 2^20 -> ORBX_E_UNSUPPORTED. */
+int orbx_match_hamming_knn(orbx_ctx* ctx, const uint8_t* query, int nq, const uint8_t* train, int nt, int k,
+                           orbx_match* out, int* n_out);
 /* DEVICE-resident, asynchronous, batched over `nsets` independent train sets (frames) that share one
  * query set (the map): d_train is [nsets][nt][32], d_best / d_second are [nsets][nq] (d_second may be NULL). */
 int orbx_match_hamming_device(orbx_ctx* ctx, const uint8_t* d_query, int nq, const uint8_t* d_train, int nt,
@@ -139,6 +146,12 @@ int orbx_match_hamming_device(orbx_ctx* ctx, const uint8_t* d_query, int nq, con
 int orbx_match_hamming_device_ragged(orbx_ctx* ctx, const uint8_t* d_query, int nq, const uint8_t* d_train,
                                      int train_stride_rows, const int* d_train_counts, int nsets,
                                      orbx_match* d_best, orbx_match* d_second);
+/* knnMatch form of the ragged batch (layout as orbx_match_hamming_device_ragged): d_out is [nsets][nq][k], set s's records
+ * of query i at d_out + (s*nq + i)*k, as orbx_match_hamming_knn; an empty set gives k records with trainIdx = -1,
+ * distance 0.  nq = 0, train_stride_rows = 0 or nsets = 0 launches nothing.  k < 1, null pointers, negative sizes or
+ * nsets > 65535 -> ORBX_E_ARG; k > ORBX_MAX_KNN or a stride of 2^20 rows or more -> ORBX_E_UNSUPPORTED. */
+int orbx_match_hamming_device_knn(orbx_ctx* ctx, const uint8_t* d_query, int nq, const uint8_t* d_train, int train_stride_rows,
+                                  const int* d_train_counts, int nsets, int k, orbx_match* d_out);
 /* HOST-buffer form of the ragged batched match: one map (query) against `nsets` frames' descriptor sets
  * ([nsets][train_stride_rows][32] with train_counts[nsets]); best / second are [nsets][nq] (second may be NULL). */
 int orbx_match_hamming_sets(orbx_ctx* ctx, const uint8_t* query, int nq, const uint8_t* train, int train_stride_rows,
@@ -175,6 +188,12 @@ int orbx_match_hamming_device_pairwise(orbx_ctx* ctx, const uint8_t* d_query, in
 int orbx_match_hamming_device_pairwise_crosscheck(orbx_ctx* ctx, const uint8_t* d_query, int query_stride_rows,
                                                   const int* d_query_counts, const uint8_t* d_train, int train_stride_rows,
                                                   const int* d_train_counts, int npairs, orbx_match* d_out, int* d_n_out);
+/* knnMatch form of the pairwise batch (layouts and count rules as orbx_match_hamming_device_pairwise): d_out is
+ * [npairs][query_stride_rows][k]; the k records of query i of pair p are written for i < that pair's query count only.
+ * k < 1 -> ORBX_E_ARG; k > ORBX_MAX_KNN -> ORBX_E_UNSUPPORTED; other argument rules as the pairwise call. */
+int orbx_match_hamming_device_pairwise_knn(orbx_ctx* ctx, const uint8_t* d_query, int query_stride_rows, const int* d_query_counts,
+                                           const uint8_t* d_train, int train_stride_rows, const int* d_train_counts, int npairs,
+                                           int k, orbx_match* d_out);
 /* The front-end's whole per-frame pattern on HOST frames in one call (src/frontend.cpp:98-108: one detectAndCompute,
  * then match() of map-point candidates against the frame's descriptors, src/frontend.cpp:153 + :187), for a batch:
  * extraction as orbx_detect_and_compute_batch, then for each of the `nmaps` query sets (queries[j]: nq[j] x 32 host

@@ -65,6 +65,9 @@ SYMBOLS = {
     "orbx_detect_and_compute_device": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_int, _P, _P, C.c_int, _P]),
     "orbx_match_hamming": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, _P, C.POINTER(C.c_int)]),
     "orbx_match_hamming_knn2": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, _P, C.POINTER(C.c_int)]),
+    "orbx_match_hamming_knn": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, C.c_int, _P, C.POINTER(C.c_int)]),
+    "orbx_match_hamming_device_knn": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, _P, C.c_int, C.c_int, _P]),
+    "orbx_match_hamming_device_pairwise_knn": (C.c_int, [_P, _P, C.c_int, _P, _P, C.c_int, _P, C.c_int, C.c_int, _P]),
     "orbx_match_hamming_device": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, C.c_int, _P, _P]),
     "orbx_match_hamming_device_ragged": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, _P, C.c_int, _P, _P]),
     "orbx_match_hamming_sets": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, _P, C.c_int, _P, _P]),

@@ -623,8 +623,11 @@ int sync_match_words(orbx_ctx* c, int slot, int n)
 // their count to d_xc_count[s].
 // Pairwise (d_qcounts set, not a lane call): set s matches its own min(d_qcounts[s], nq) query rows at d_q + s * nq * 32, so nq
 // is the query stride (and the record pitch); one CTA per (set, query tile), and record slots past a set's count stay untouched.
+// Top-k (knn_k >= 2, d_second null, not a lane call, no cross-check): d_best receives knnMatch's k records per (set, query row),
+// [nsets][nq][k], from the single-CTA top-k kernel of the smallest list bucket that holds k (no train-row split).
 int run_match(orbx_ctx* c, const uint8_t* d_q, int nq, const uint8_t* d_t, int nt, int stride_rows, const int* d_counts, int nsets,
-              int4* d_best, int4* d_second, cudaStream_t st = nullptr, int slot = 0, int* d_xc_count = nullptr, const int* d_qcounts = nullptr)
+              int4* d_best, int4* d_second, cudaStream_t st = nullptr, int slot = 0, int* d_xc_count = nullptr, const int* d_qcounts = nullptr,
+              int knn_k = 0)
 {
     NvtxRange nvr("orbx:match_hamming");
     const bool lane_call = st != nullptr;
@@ -633,16 +636,17 @@ int run_match(orbx_ctx* c, const uint8_t* d_q, int nq, const uint8_t* d_t, int n
     const bool xchk = d_xc_count != nullptr;
     if (xchk && nq >= MT_MAX_QUERY_XC) return fail(c, ORBX_E_UNSUPPORTED, "cross-check query set larger than 2^20 - 1 rows");
     const bool knn2 = d_second != nullptr;
+    const bool topk = knn_k > 0;
     // CTA-pair kernel (tcgen05 cta_group::2, query tiles in twos) whenever the (query tile, set) pairs alone fill the GPU;
     // small problems keep the single-CTA kernel, whose CTAs are independent units for the train-row split.
     const int tiles_1 = (nq + MT_QROWS - 1) / MT_QROWS, tiles_2 = (tiles_1 + 1) & ~1;
-    const bool pair = tiles_1 >= 2 && (long)tiles_2 * nsets >= 148;
+    const bool pair = !topk && tiles_1 >= 2 && (long)tiles_2 * nsets >= 148;
     const int tiles_m = pair ? tiles_2 : tiles_1;
     const int ntile_n = (nt + MT_BN - 1) / MT_BN;
     constexpr int kSMs = 148;                                // one CTA per SM (163 KB of shared memory each)
     // Few (query tile, set) pairs: split the train rows across CTAs and merge with atomicMax on the packed key.
     int nsplit = 1;
-    if (!knn2 && !lane_call) {
+    if (!knn2 && !topk && !lane_call) {
         const long base = (long)tiles_m * nsets;
         if (base < kSMs) nsplit = (int)std::min<long>(ntile_n, std::max<long>(1, (kSMs + base - 1) / base));
     }
@@ -688,7 +692,18 @@ int run_match(orbx_ctx* c, const uint8_t* d_q, int nq, const uint8_t* d_t, int n
     const dim3 grd((unsigned)tiles_m, (unsigned)nsplit, (unsigned)zgroups);
     const int smem = xchk ? MT_SMEM_BYTES_XC : MT_SMEM_BYTES;
     // (knn2 and xchk never meet: the cross-check keeps the best match only)
-    if (pairwise) {
+    if (topk) {                                              // list buckets of 4, 8, 16 and 32 keys
+        static_assert(ORBX_MAX_KNN <= 32, "the largest list bucket holds 32 keys");
+        const int kb = knn_k <= 4 ? 0 : knn_k <= 8 ? 1 : knn_k <= 16 ? 2 : 3;
+        if (pairwise) {
+            auto* kernel = kb == 0 ? k_hamming_umma_pw_topk<4> : kb == 1 ? k_hamming_umma_pw_topk<8> : kb == 2 ? k_hamming_umma_pw_topk<16>
+                                                                                                           : k_hamming_umma_pw_topk<32>;
+            kernel<<<grd, MT_THREADS, smem, st>>>(d_q, nq, d_t, nt, stride_rows, d_counts, nsets, rows_per_split, d_best, d_status, d_qcounts, knn_k);
+        } else {
+            auto* kernel = kb == 0 ? k_hamming_umma_topk<4> : kb == 1 ? k_hamming_umma_topk<8> : kb == 2 ? k_hamming_umma_topk<16> : k_hamming_umma_topk<32>;
+            kernel<<<grd, MT_THREADS, smem, st>>>(d_q, nq, d_t, nt, stride_rows, d_counts, nsets, rows_per_split, d_best, d_status, knn_k);
+        }
+    } else if (pairwise) {
         auto* kernel = pair ? (xchk ? k_hamming_umma2_pw<false, true> : knn2 ? k_hamming_umma2_pw<true, false> : k_hamming_umma2_pw<false, false>)
                             : (xchk ? k_hamming_umma_pw<false, true> : knn2 ? k_hamming_umma_pw<true, false> : k_hamming_umma_pw<false, false>);
         kernel<<<grd, MT_THREADS, smem, st>>>(d_q, nq, d_t, nt, stride_rows, d_counts, nsets, rows_per_split, d_best, d_second, keys, d_status,
@@ -719,10 +734,11 @@ int run_match(orbx_ctx* c, const uint8_t* d_q, int nq, const uint8_t* d_t, int n
 // each (all of them, or as many as the host `counts` give per set).  best and second (when not null) receive [nsets][nq]
 // records each; with `pairs` (the second-best of one set), `best` receives [nq][2] {best, second} records instead.
 // With `xc_count` (cross-check of one set), `best` receives the mutual pairs and *xc_count their number.
+// With knn_k (top-k, k >= 2), `best` receives [nsets][nq][knn_k] records.
 int match_host(orbx_ctx* c, const uint8_t* query, int nq, const uint8_t* train, int stride_rows, const int* counts, int nsets,
-               orbx_match* best, orbx_match* second, bool pairs, int* xc_count = nullptr)
+               orbx_match* best, orbx_match* second, bool pairs, int* xc_count = nullptr, int knn_k = 0)
 {
-    const size_t tbytes = (size_t)nsets * stride_rows * 32, obytes = (size_t)nsets * nq * 16;
+    const size_t tbytes = (size_t)nsets * stride_rows * 32, obytes = (size_t)nsets * nq * 16 * (size_t)std::max(1, knn_k);
     const bool knn2 = pairs || second;
     int rc;
     if ((rc = ensure(c, c->mq, (size_t)nq * 32)) || (rc = ensure(c, c->mt, tbytes)) || (rc = ensure(c, c->mbest, obytes)) ||
@@ -733,7 +749,8 @@ int match_host(orbx_ctx* c, const uint8_t* query, int nq, const uint8_t* train, 
     CU(cudaMemcpyAsync(c->mt.p, train, tbytes, cudaMemcpyHostToDevice, c->stream));
     if (counts) CU(cudaMemcpyAsync(c->mcounts.p, counts, sizeof(int) * (size_t)nsets, cudaMemcpyHostToDevice, c->stream));
     if ((rc = run_match(c, (const uint8_t*)c->mq.p, nq, (const uint8_t*)c->mt.p, stride_rows, stride_rows, counts ? (const int*)c->mcounts.p : nullptr,
-                        nsets, (int4*)c->mbest.p, knn2 ? (int4*)c->msecond.p : nullptr, nullptr, 0, xc_count ? (int*)c->mxcount.p : nullptr)))
+                        nsets, (int4*)c->mbest.p, knn2 ? (int4*)c->msecond.p : nullptr, nullptr, 0, xc_count ? (int*)c->mxcount.p : nullptr,
+                        nullptr, knn_k)))
         return rc;
     if (xc_count) CU(cudaMemcpyAsync(xc_count, c->mxcount.p, sizeof(int) * (size_t)nsets, cudaMemcpyDeviceToHost, c->stream));
     if (pairs) {
@@ -746,8 +763,9 @@ int match_host(orbx_ctx* c, const uint8_t* query, int nq, const uint8_t* train, 
     return sync_match_words(c, 0, 1);
 }
 
-// orbx_match_hamming / orbx_match_hamming_knn2: one train set of nt rows
-int match_one_set(orbx_ctx* c, const uint8_t* query, int nq, const uint8_t* train, int nt, orbx_match* out, int* n_out, bool knn2)
+// orbx_match_hamming / _knn2 / _knn: one train set of nt rows, k records per query row ([nq][k]): k = 1 the plain matcher,
+// k = 2 the knn2 one (interleaved {best, second}), larger k the top-k one
+int match_one_set(orbx_ctx* c, const uint8_t* query, int nq, const uint8_t* train, int nt, orbx_match* out, int* n_out, int k)
 {
     if (!c) return ORBX_E_ARG;
     if (n_out) *n_out = 0;
@@ -755,7 +773,7 @@ int match_one_set(orbx_ctx* c, const uint8_t* query, int nq, const uint8_t* trai
     if (nq == 0 || nt == 0) return ORBX_OK;                 // cv: empty query or train -> no matches, no throw
     if (!query || !train || !out) return fail(c, ORBX_E_ARG, "null pointer");
     CU(cudaSetDevice(c->device));
-    const int rc = match_host(c, query, nq, train, nt, nullptr, 1, out, nullptr, knn2);
+    const int rc = match_host(c, query, nq, train, nt, nullptr, 1, out, nullptr, k == 2, nullptr, k > 2 ? k : 0);
     if (rc) return rc;
     if (n_out) *n_out = nq;
     return ORBX_OK;
@@ -829,6 +847,14 @@ int orbx_create(orbx_ctx** out, int device, int nfeatures, float scale_factor, i
         cudaFuncSetAttribute(k_hamming_umma_pw<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
         cudaFuncSetAttribute(k_hamming_umma2_pw<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES_XC) != cudaSuccess ||
         cudaFuncSetAttribute(k_hamming_umma_pw<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES_XC) != cudaSuccess ||
+        cudaFuncSetAttribute(k_hamming_umma_topk<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
+        cudaFuncSetAttribute(k_hamming_umma_topk<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
+        cudaFuncSetAttribute(k_hamming_umma_topk<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
+        cudaFuncSetAttribute(k_hamming_umma_topk<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
+        cudaFuncSetAttribute(k_hamming_umma_pw_topk<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
+        cudaFuncSetAttribute(k_hamming_umma_pw_topk<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
+        cudaFuncSetAttribute(k_hamming_umma_pw_topk<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
+        cudaFuncSetAttribute(k_hamming_umma_pw_topk<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
         cudaFuncSetAttribute(k_fast_warp<FAST_NWARP>, cudaFuncAttributeMaxDynamicSharedMemorySize, FAST_NWARP * FW_WARP_BYTES + 128) != cudaSuccess ||
         cudaFuncSetAttribute(k_pyr_tma, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024) != cudaSuccess ||
         cudaFuncSetAttribute(k_describe_tma, cudaFuncAttributeMaxDynamicSharedMemorySize, DS_NW * DS_WARP_BYTES + 128) != cudaSuccess ||
@@ -1096,11 +1122,19 @@ int orbx_detect_and_compute(orbx_ctx* c, const uint8_t* img, int w, int h, size_
 
 int orbx_match_hamming(orbx_ctx* c, const uint8_t* q, int nq, const uint8_t* t, int nt, orbx_match* out, int* n_out)
 {
-    return match_one_set(c, q, nq, t, nt, out, n_out, false);
+    return match_one_set(c, q, nq, t, nt, out, n_out, 1);
 }
 int orbx_match_hamming_knn2(orbx_ctx* c, const uint8_t* q, int nq, const uint8_t* t, int nt, orbx_match* out, int* n_out)
 {
-    return match_one_set(c, q, nq, t, nt, out, n_out, true);
+    return match_one_set(c, q, nq, t, nt, out, n_out, 2);
+}
+int orbx_match_hamming_knn(orbx_ctx* c, const uint8_t* q, int nq, const uint8_t* t, int nt, int k, orbx_match* out, int* n_out)
+{
+    if (!c) return ORBX_E_ARG;
+    if (n_out) *n_out = 0;
+    if (k < 1) return fail(c, ORBX_E_ARG, "k < 1");
+    if (k > ORBX_MAX_KNN) return fail(c, ORBX_E_UNSUPPORTED, "k larger than ORBX_MAX_KNN");
+    return match_one_set(c, q, nq, t, nt, out, n_out, k);
 }
 
 int orbx_match_hamming_device(orbx_ctx* c, const uint8_t* d_query, int nq, const uint8_t* d_train, int nt, int nsets,
@@ -1170,7 +1204,21 @@ int orbx_match_hamming_device_crosscheck(orbx_ctx* c, const uint8_t* d_query, in
     return run_match(c, d_query, nq, d_train, train_stride_rows, train_stride_rows, d_train_counts, nsets, (int4*)d_out, nullptr, nullptr, 0, d_n_out);
 }
 
-// orbx_match_hamming_device_pairwise[_crosscheck]: pair p = query set p against train set p.  Argument checks common to both.
+int orbx_match_hamming_device_knn(orbx_ctx* c, const uint8_t* d_query, int nq, const uint8_t* d_train, int train_stride_rows,
+                                  const int* d_train_counts, int nsets, int k, orbx_match* d_out)
+{
+    if (!c) return ORBX_E_ARG;
+    if (nq < 0 || train_stride_rows < 0 || nsets < 0 || nsets > 65535 || k < 1) return fail(c, ORBX_E_ARG, "bad sizes");
+    if (k > ORBX_MAX_KNN) return fail(c, ORBX_E_UNSUPPORTED, "k larger than ORBX_MAX_KNN");
+    if (nq == 0 || train_stride_rows == 0 || nsets == 0) return ORBX_OK;
+    if (!d_query || !d_train || !d_out || !d_train_counts) return fail(c, ORBX_E_ARG, "null pointer");
+    CU(cudaSetDevice(c->device));
+    // k = 1: the plain matcher's [nsets][nq] records are the [nsets][nq][1] layout
+    return run_match(c, d_query, nq, d_train, train_stride_rows, train_stride_rows, d_train_counts, nsets, (int4*)d_out, nullptr, nullptr, 0,
+                     nullptr, nullptr, k > 1 ? k : 0);
+}
+
+// orbx_match_hamming_device_pairwise[_crosscheck|_knn]: pair p = query set p against train set p.  Argument checks common to all.
 static int check_args_pairwise(orbx_ctx* c, const uint8_t* d_query, int query_stride_rows, const int* d_query_counts, const uint8_t* d_train,
                                int train_stride_rows, const int* d_train_counts, int npairs, const void* d_out)
 {
@@ -1210,6 +1258,21 @@ int orbx_match_hamming_device_pairwise_crosscheck(orbx_ctx* c, const uint8_t* d_
     }
     return run_match(c, d_query, query_stride_rows, d_train, train_stride_rows, train_stride_rows, d_train_counts, npairs, (int4*)d_out, nullptr,
                      nullptr, 0, d_n_out, d_query_counts);
+}
+
+int orbx_match_hamming_device_pairwise_knn(orbx_ctx* c, const uint8_t* d_query, int query_stride_rows, const int* d_query_counts,
+                                           const uint8_t* d_train, int train_stride_rows, const int* d_train_counts, int npairs, int k,
+                                           orbx_match* d_out)
+{
+    if (!c) return ORBX_E_ARG;
+    if (k < 1) return fail(c, ORBX_E_ARG, "k < 1");
+    int rc = check_args_pairwise(c, d_query, query_stride_rows, d_query_counts, d_train, train_stride_rows, d_train_counts, npairs, d_out);
+    if (rc) return rc;
+    if (k > ORBX_MAX_KNN) return fail(c, ORBX_E_UNSUPPORTED, "k larger than ORBX_MAX_KNN");
+    if (npairs == 0 || query_stride_rows == 0 || train_stride_rows == 0) return ORBX_OK;
+    CU(cudaSetDevice(c->device));
+    return run_match(c, d_query, query_stride_rows, d_train, train_stride_rows, train_stride_rows, d_train_counts, npairs, (int4*)d_out,
+                     nullptr, nullptr, 0, nullptr, d_query_counts, k > 1 ? k : 0);
 }
 
 int orbx_filter_matches(orbx_match* m, int n, float ratio)

@@ -32,6 +32,8 @@
 // Pairwise batches (SETQ: query set s against train set s, e.g. frame i against frame i + 1) cannot keep one A operand
 // across sets, so there a CTA owns ONE (set, query tile) unit: gridDim.z = number of sets, the A tile is expanded at setup
 // as above, and CTAs whose query tile is empty for their set exit before any setup.  Few units keep the train-row split.
+// knnMatch for k > 2 (TOP-K, KB = list capacity 4 / 8 / 16 / 32): the single-CTA body, shared-query or pairwise, whose epilogue
+// keeps each query row's KB best keys in registers (see topk_tile); no CTA pair and no train-row split, as for knn2.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -318,19 +320,64 @@ __device__ __forceinline__ void xc_warp_columns(const uint32_t* rp, bool valid, 
 }
 __device__ __forceinline__ void xc_epilogue_sync() { asm volatile("bar.sync 1, 256;" ::: "memory"); }   // the 8 epilogue warps only
 
+// ---- top-k (KB > 0, BFMatcher knnMatch for any k <= KB): each epilogue thread keeps its query row's KB largest keys
+// dot << 20 | (0xFFFFF - j) in registers, in descending order (INT_MIN = empty slot).  Keys are distinct per train row, so
+// the first k of them are exactly cv's k nearest by (distance, trainIdx).  A tile's columns are tested against the list's
+// last key in accumulator form (one compare per column; the whole tile is skipped when its packed maximum fails); only a
+// column that enters the list is decoded and inserted by a branchless shift chain.
+// The smallest accumulator of the tile at train row j0 whose key beats key t.  Every earlier tile holds lower train indices,
+// so a row of such a tile is beaten by a strictly larger dot only; a row of this tile by a larger 127 * dot + code.
+// An empty slot admits every column but the -32768 fill of chunks past the tile's UMMA N.
+__device__ __forceinline__ int topk_threshold(int t, int j0)
+{
+    if (t == INT_MIN) return -32767;
+    const int dot = t >> MT_KEY_SHIFT, j = (MT_MAX_TRAIN - 1) - (t & (MT_MAX_TRAIN - 1));
+    return j < j0 ? MT_ASCALE * (dot + 1) : MT_ASCALE * dot + ((MT_BN - 1) - (j - j0)) + 1;
+}
+template <int KB>
+__device__ __forceinline__ void topk_insert(int (&list)[KB], int x)   // x > list[KB - 1] or x == INT_MIN (no-op)
+{
+#pragma unroll
+    for (int i = KB - 1; i > 0; --i) list[i] = x > list[i - 1] ? list[i - 1] : max(list[i], x);
+    list[0] = max(list[0], x);
+}
+// One tile's packed accumulators (tmax: their maximum) of train rows j0 .. into the list; columns decoding to j >= n1 are the
+// copies of the set's last row that pad a partial tile.
+template <int KB>
+__device__ __forceinline__ void topk_tile(const uint32_t* rp, int tmax, int j0, int n1, int (&list)[KB])
+{
+    int thr = topk_threshold(list[KB - 1], j0);
+    if (tmax < thr) return;
+#pragma unroll
+    for (int u = 0; u < MT_BN / 2; ++u)
+#pragma unroll
+        for (int h = 0; h < 2; ++h) {
+            const int v = h ? (int)rp[u] >> 16 : (int)(rp[u] << 16) >> 16;
+            if (v >= thr) {
+                const unsigned kk = (unsigned)(v + MT_ASCALE * 256);
+                const unsigned q = kk / (unsigned)MT_ASCALE;          // dot + 256
+                const int j = j0 + (MT_BN - 1) - (int)(kk - q * (unsigned)MT_ASCALE);
+                topk_insert<KB>(list, j < n1 ? ((int)q - 256) * (1 << MT_KEY_SHIFT) + ((MT_MAX_TRAIN - 1) - j) : INT_MIN);
+                thr = topk_threshold(list[KB - 1], j0);
+            }
+        }
+}
+
 // SETQ = false: one query set (the map) shared by every train set; nq is its row count.
 // SETQ = true (pairwise): set s has its own query rows, min(query_counts[s], nq) of them at query + s * nq * 32, so nq is
 // the query stride and the pitch of the outputs and of the split keys.  The A tile then belongs to ONE set: the grid has
 // gridDim.z = nsets (one (set, query tile) unit per CTA), and a CTA whose query tile is empty for its set exits before
 // any setup -- in a CTA pair only when the leader's (lower) tile is empty too, because the peer holds half of every B tile.
-template <bool KNN2, bool PAIR, bool XCHK, bool SETQ>
+// KB > 0 (top-k, k = knn_k <= KB): best receives k records per (set, query row), [nsets][nq][k]; single CTA, no split.
+template <bool KNN2, bool PAIR, bool XCHK, bool SETQ, int KB = 0>
 __device__ __forceinline__ void
 hamming_umma_body(const uint8_t* __restrict__ query, int nq, const uint8_t* __restrict__ train, int nt, int train_stride_rows,
                const int* __restrict__ train_counts, int nsets, int rows_per_split, int4* __restrict__ best,
                int4* __restrict__ second, int* __restrict__ keys, int* __restrict__ status, int* __restrict__ col_keys,
-               const int* __restrict__ query_counts)
+               const int* __restrict__ query_counts, int knn_k = 0)
 {
     static_assert(!(KNN2 && XCHK), "cross-check keeps the best match only");
+    static_assert(KB == 0 || (!KNN2 && !PAIR && !XCHK), "top-k runs on the single-CTA kernel alone");
     int nqv = nq;                                            // query rows present (padded rows q >= nqv are excluded)
     if constexpr (SETQ) {
         nqv = max(0, min(__ldg(query_counts + blockIdx.z), nq));
@@ -549,6 +596,9 @@ hamming_umma_body(const uint8_t* __restrict__ query, int nq, const uint8_t* __re
             const MatchSetRange rg = match_set_range_n(cnt_next, nt, split, rows_per_split);   // (next set's row count loaded a set ahead, as in the issuer)
             if (set + (int)gridDim.z < nsets) cnt_next = match_set_count(train_counts, set + (int)gridDim.z, nt);
             int m1 = INT_MIN, m2 = INT_MIN;
+            int list[KB > 0 ? KB : 1];                       // top-k: this row's best keys, descending
+#pragma unroll
+            for (int r = 0; r < (KB > 0 ? KB : 1); ++r) list[r] = INT_MIN;
             for (int i = 0; i < rg.ntiles; ++i, ++t) {
                 const int b = t & 1;
                 const uint32_t bph = (uint32_t)(t >> 1) & 1u;
@@ -585,6 +635,7 @@ hamming_umma_body(const uint8_t* __restrict__ query, int nq, const uint8_t* __re
                     }
                     const unsigned pk = __vimax3_s16x2(__vimax3_s16x2(p[0], p[1], p[2]), __vimax3_s16x2(p[3], p[4], p[5]), __vmaxs2(p[6], p[7]));
                     k1 = max((int)(pk << 16) >> 16, (int)pk >> 16);
+                    if constexpr (KB > 0) topk_tile<KB>(rp, k1, j0, rg.n1, list);
                     if constexpr (XCHK)
                         xc_warp_columns(rp, qrow < nqv, qrow - q0, reinterpret_cast<int*>(smem + MT_SMEM_XC) + (b * 8 + warp - MT_EPI_WARP0) * MT_BN);
                 } else if (!KNN2) {
@@ -613,6 +664,7 @@ hamming_umma_body(const uint8_t* __restrict__ query, int nq, const uint8_t* __re
                     }
                     const unsigned pk = __vimax3_s16x2(__vimax3_s16x2(p[0], p[1], p[2]), __vimax3_s16x2(p[3], p[4], p[5]), __vmaxs2(p[6], p[7]));
                     k1 = max((int)(pk << 16) >> 16, (int)pk >> 16);
+                    if constexpr (KB > 0) topk_tile<KB>(rp, k1, j0, rg.n1, list);
                     if constexpr (XCHK)                      // (chunks past N hold -32768: no column there)
                         xc_warp_columns(rp, qrow < nqv, qrow - q0, reinterpret_cast<int*>(smem + MT_SMEM_XC) + (b * 8 + warp - MT_EPI_WARP0) * MT_BN);
                 } else {
@@ -636,7 +688,7 @@ hamming_umma_body(const uint8_t* __restrict__ query, int nq, const uint8_t* __re
                 }
                 // decode the tile winner(s) into the global key  dot << 20 | (0xFFFFF - j)
 #pragma unroll
-                for (int w = 0; w < (KNN2 ? 2 : 1); ++w) {
+                for (int w = 0; w < (KB > 0 ? 0 : KNN2 ? 2 : 1); ++w) {   // (top-k: already in the list)
                     const int k = w == 0 ? k1 : k2;
                     if (k != INT_MIN) {
                         const unsigned kk = (unsigned)(k + MT_ASCALE * 256);
@@ -676,7 +728,16 @@ hamming_umma_body(const uint8_t* __restrict__ query, int nq, const uint8_t* __re
             }
             if (ok && qrow < nqv) {
                 const size_t o = (size_t)set * nq + qrow;
-                if (keys) {
+                if constexpr (KB > 0) {                     // the k records of this row, once per set
+                    int4* out = best + o * knn_k;
+#pragma unroll
+                    for (int r = 0; r < KB; ++r) {
+                        if (r >= knn_k) break;
+                        const int key = list[r];
+                        const int dot = key >> MT_KEY_SHIFT, j = (MT_MAX_TRAIN - 1) - (key & (MT_MAX_TRAIN - 1));
+                        out[r] = key == INT_MIN ? make_int4(qrow, -1, 0, 0) : make_int4(qrow, j, 0, __float_as_int((float)((256 - dot) >> 1)));
+                    }
+                } else if (keys) {
                     if (m1 != INT_MIN) atomicMax(&keys[o], m1);
                 } else if (m1 == INT_MIN) {                   // empty train set: no match (trainIdx -1)
                     best[o] = make_int4(qrow, -1, 0, 0);
@@ -747,6 +808,25 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(MT_THREADS, 1) k_ham
 {
     hamming_umma_body<KNN2, true, XCHK, true>(query, nq, train, nt, train_stride_rows, train_counts, nsets, rows_per_split, best, second, keys, status,
                                               col_keys, query_counts);
+}
+// top-k (knnMatch, k = knn_k <= KB): best receives [nsets][nq][k] records (train-row split and second are unused)
+template <int KB>
+__global__ void __launch_bounds__(MT_THREADS, 1) k_hamming_umma_topk(const uint8_t* __restrict__ query, int nq, const uint8_t* __restrict__ train, int nt,
+                                                                     int train_stride_rows, const int* __restrict__ train_counts, int nsets, int rows_per_split,
+                                                                     int4* __restrict__ best, int* __restrict__ status, int knn_k)
+{
+    hamming_umma_body<false, false, false, false, KB>(query, nq, train, nt, train_stride_rows, train_counts, nsets, rows_per_split, best, nullptr, nullptr,
+                                                      status, nullptr, nullptr, knn_k);
+}
+// pairwise top-k: best receives [nsets][nq][k] records, those of query i of set s for i < query_counts[s] only
+template <int KB>
+__global__ void __launch_bounds__(MT_THREADS, 1) k_hamming_umma_pw_topk(const uint8_t* __restrict__ query, int nq, const uint8_t* __restrict__ train, int nt,
+                                                                        int train_stride_rows, const int* __restrict__ train_counts, int nsets, int rows_per_split,
+                                                                        int4* __restrict__ best, int* __restrict__ status, const int* __restrict__ query_counts,
+                                                                        int knn_k)
+{
+    hamming_umma_body<false, false, false, true, KB>(query, nq, train, nt, train_stride_rows, train_counts, nsets, rows_per_split, best, nullptr, nullptr,
+                                                     status, nullptr, query_counts, knn_k);
 }
 
 // ONE CTA per set: query i keeps its best match (i, j) iff column j's key names i, i.e. i is also train row j's nearest

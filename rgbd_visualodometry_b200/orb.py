@@ -7,7 +7,7 @@
   orb_->detectAndCompute(color_, Mat(), kps, desc)            ORB.detectAndCompute(image, None) -> (kps, desc)
       src/frontend.cpp:153
   matcher.match(query, train, matches)                        BFMatcher(NORM_HAMMING).match(query, train)
-      src/frontend.cpp:187                                    (+ knnMatch(query, train, k=2), crossCheck=True)
+      src/frontend.cpp:187                                    (+ knnMatch(query, train, k <= 32), crossCheck=True)
   max(min_dis * match_ratio, 30) filter                       filter_matches(matches, match_ratio)
       src/frontend.cpp:190-211
 
@@ -28,6 +28,7 @@ KP_DTYPE = np.dtype([("x", "<f4"), ("y", "<f4"), ("size", "<f4"), ("angle", "<f4
                      ("octave", "<i4"), ("class_id", "<i4")])
 DMATCH_DTYPE = np.dtype([("queryIdx", "<i4"), ("trainIdx", "<i4"), ("imgIdx", "<i4"), ("distance", "<f4")])
 NORM_HAMMING = 6  # == cv2.NORM_HAMMING
+MAX_KNN = 32      # == ORBX_MAX_KNN: the largest k of knnMatch
 
 OK, E_ARG, E_CAPACITY, E_CUDA, E_NOMEM, E_UNSUPPORTED, E_INTERNAL, E_ORDER = 0, -1, -2, -3, -4, -5, -6, -7
 
@@ -159,6 +160,16 @@ class Context:
         self._check(self.lib.orbx_match_hamming_knn2(self.h, _ptr(q), len(q), _ptr(t), len(t), _ptr(out), C.byref(n)))
         return out[:n.value]
 
+    def knn_match(self, query: np.ndarray, train: np.ndarray, k: int) -> np.ndarray:
+        """knnMatch(query, train, k), 1 <= k <= MAX_KNN: [nq, k] records, row i = query i's k nearest train rows by
+        (distance, trainIdx); slots past the train set's size hold trainIdx = -1.  [0, k] when either set is empty."""
+        q = np.ascontiguousarray(query, np.uint8).reshape(-1, 32)
+        t = np.ascontiguousarray(train, np.uint8).reshape(-1, 32)
+        out = np.zeros((max(len(q), 1), max(int(k), 1)), DMATCH_DTYPE)
+        n = C.c_int(0)
+        self._check(self.lib.orbx_match_hamming_knn(self.h, _ptr(q), len(q), _ptr(t), len(t), int(k), _ptr(out), C.byref(n)))
+        return out[:n.value]
+
     def match_crosscheck(self, query: np.ndarray, train: np.ndarray) -> np.ndarray:
         """BFMatcher(NORM_HAMMING, crossCheck=True).match: the mutual nearest pairs, ascending queryIdx."""
         q = np.ascontiguousarray(query, np.uint8).reshape(-1, 32)
@@ -196,6 +207,19 @@ class Context:
         self._check(self.lib.orbx_match_hamming_device_pairwise_crosscheck(self.h, d_query_ptr, query_stride_rows, d_query_counts_ptr,
                                                                            d_train_ptr, train_stride_rows, d_train_counts_ptr, npairs,
                                                                            d_out_ptr, d_n_out_ptr))
+
+    def match_device_knn(self, d_query_ptr: int, nq: int, d_train_ptr: int, stride_rows: int, d_counts_ptr: int, nsets: int, k: int,
+                         d_out_ptr: int):
+        """Asynchronous, device-resident, ragged batch: knnMatch of the query set against every set, [nsets, nq, k] records."""
+        self._check(self.lib.orbx_match_hamming_device_knn(self.h, d_query_ptr, nq, d_train_ptr, stride_rows, d_counts_ptr, nsets, int(k),
+                                                           d_out_ptr))
+
+    def match_device_pairwise_knn(self, d_query_ptr: int, query_stride_rows: int, d_query_counts_ptr: int, d_train_ptr: int,
+                                  train_stride_rows: int, d_train_counts_ptr: int, npairs: int, k: int, d_out_ptr: int):
+        """As match_device_pairwise with knnMatch: [npairs, query_stride_rows, k] records (slots past a pair's query count are
+        not written)."""
+        self._check(self.lib.orbx_match_hamming_device_pairwise_knn(self.h, d_query_ptr, query_stride_rows, d_query_counts_ptr, d_train_ptr,
+                                                                    train_stride_rows, d_train_counts_ptr, npairs, int(k), d_out_ptr))
 
     def match_sets(self, query: np.ndarray, train: np.ndarray, counts: np.ndarray, knn2: bool = False):
         """One map (query [M,32]) against nsets frames' descriptor sets (train [S,cap,32], counts [S]); host buffers."""
@@ -378,13 +402,31 @@ class BFMatcher:
         return self._ctx.match(queryDescriptors, trainDescriptors)
 
     def knnMatch(self, queryDescriptors, trainDescriptors, k=2):
-        if self.crossCheck:
-            raise OrbxError(E_UNSUPPORTED, "knnMatch with crossCheck is not implemented")
-        if k != 2:
-            raise OrbxError(E_UNSUPPORTED, "knnMatch is implemented for k = 2")
+        """[nq, k] records, row i = query i's k nearest train rows by (distance, trainIdx) as cv2's list for query i, padded
+        with trainIdx = -1 records where cv2's list is shorter (k > number of train rows).  With crossCheck (k = 1 only, as
+        cv2): the mutual pair, or a trainIdx = -1 record where cv2 gives []."""
+        k = int(k)
+        if k < 1:
+            raise OrbxError(E_ARG, "knnMatch needs k >= 1")
+        if k > MAX_KNN:
+            raise OrbxError(E_UNSUPPORTED, f"knnMatch is implemented for k <= {MAX_KNN}")
+        if self.crossCheck and k != 1:
+            raise OrbxError(E_UNSUPPORTED, "knnMatch with crossCheck is implemented for k = 1 (cv2 asserts otherwise)")
         if queryDescriptors is None or trainDescriptors is None:
-            return np.zeros((0, 2), DMATCH_DTYPE)
-        return self._ctx.knn_match2(queryDescriptors, trainDescriptors)
+            return np.zeros((0, k), DMATCH_DTYPE)
+        if self.crossCheck:
+            nq = len(np.ascontiguousarray(queryDescriptors, np.uint8).reshape(-1, 32))
+            pairs = self._ctx.match_crosscheck(queryDescriptors, trainDescriptors)
+            if len(np.ascontiguousarray(trainDescriptors, np.uint8).reshape(-1, 32)) == 0:
+                nq = 0                                      # an empty train set: no lists (as knn_match)
+            out = np.zeros((nq, 1), DMATCH_DTYPE)
+            out["queryIdx"][:, 0] = np.arange(nq)
+            out["trainIdx"] = -1
+            out[pairs["queryIdx"], 0] = pairs
+            return out
+        if k == 2:
+            return self._ctx.knn_match2(queryDescriptors, trainDescriptors)
+        return self._ctx.knn_match(queryDescriptors, trainDescriptors, k)
 
 
 def filter_matches(matches: np.ndarray, match_ratio: float = 2.0) -> np.ndarray:
