@@ -194,6 +194,33 @@ int orbx_match_hamming_device_pairwise_crosscheck(orbx_ctx* ctx, const uint8_t* 
 int orbx_match_hamming_device_pairwise_knn(orbx_ctx* ctx, const uint8_t* d_query, int query_stride_rows, const int* d_query_counts,
                                            const uint8_t* d_train, int train_stride_rows, const int* d_train_counts, int npairs,
                                            int k, orbx_match* d_out);
+/* radiusMatch(query, train, maxDistance): for every query row, every train row at Hamming distance <= maxDistance, in
+ * cv::BFMatcher(NORM_HAMMING).radiusMatch's exact list order.  That order is libstdc++'s std::sort by distance alone (an
+ * unstable introsort) of the rows in ascending trainIdx, NOT (distance, trainIdx): equal distances can come out in any
+ * index order once a list holds more than 16 entries.  Output is CSR: list L occupies out[offsets[L] .. offsets[L + 1])
+ * (offsets are 64-bit), records {queryIdx, trainIdx, 0, distance} with indices local to the set or pair.  The integer radius
+ * is R = min(256, floor(max_distance)), so +inf or any value >= 256 keeps every row.  max_distance <= FLT_EPSILON or NaN
+ * (cv asserts), null pointers or negative sizes -> ORBX_E_ARG; a train set (stride) of 2^20 rows or more ->
+ * ORBX_E_UNSUPPORTED.  cv's crossCheck does not apply to radiusMatch: its lists are these.
+ * HOST buffers: lists [nq], offsets has nq + 1 entries; *n_out = offsets[nq] = the number of records.  If that exceeds cap
+ * the call returns ORBX_E_CAPACITY with *n_out = the number needed.  An empty train set gives nq empty lists (all offsets
+ * 0), an empty query set none. */
+int orbx_match_hamming_radius(orbx_ctx* ctx, const uint8_t* query, int nq, const uint8_t* train, int nt, float max_distance,
+                              orbx_match* out, int cap, int64_t* offsets, int* n_out);
+/* Ragged DEVICE batch (layout as orbx_match_hamming_device_ragged), asynchronous: list L = s*nq + i is query i against set
+ * s, d_offsets has nsets*nq + 1 entries.  d_offsets is always written in full; list L's records are written only when
+ * d_offsets[L + 1] <= cap (as orbx_detect_and_compute_device, records beyond cap are not written), so a caller reads
+ * d_offsets[nsets*nq] and calls again with a larger buffer.  nq = 0, train_stride_rows = 0 or nsets = 0 launches nothing
+ * and zeroes d_offsets; nsets > 65535 or cap < 0 -> ORBX_E_ARG. */
+int orbx_match_hamming_device_radius(orbx_ctx* ctx, const uint8_t* d_query, int nq, const uint8_t* d_train, int train_stride_rows,
+                                     const int* d_train_counts, int nsets, float max_distance, orbx_match* d_out, int64_t cap,
+                                     int64_t* d_offsets);
+/* PAIRWISE DEVICE batch (layouts and count rules as orbx_match_hamming_device_pairwise), asynchronous: list
+ * L = p*query_stride_rows + i is query i of pair p against train set p; d_offsets has npairs*query_stride_rows + 1 entries.
+ * Query rows past a pair's count have empty lists.  cap and d_offsets as the ragged form. */
+int orbx_match_hamming_device_pairwise_radius(orbx_ctx* ctx, const uint8_t* d_query, int query_stride_rows, const int* d_query_counts,
+                                              const uint8_t* d_train, int train_stride_rows, const int* d_train_counts, int npairs,
+                                              float max_distance, orbx_match* d_out, int64_t cap, int64_t* d_offsets);
 /* The front-end's whole per-frame pattern on HOST frames in one call (src/frontend.cpp:98-108: one detectAndCompute,
  * then match() of map-point candidates against the frame's descriptors, src/frontend.cpp:153 + :187), for a batch:
  * extraction as orbx_detect_and_compute_batch, then for each of the `nmaps` query sets (queries[j]: nq[j] x 32 host

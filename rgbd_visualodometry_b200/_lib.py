@@ -68,6 +68,9 @@ SYMBOLS = {
     "orbx_match_hamming_knn": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, C.c_int, _P, C.POINTER(C.c_int)]),
     "orbx_match_hamming_device_knn": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, _P, C.c_int, C.c_int, _P]),
     "orbx_match_hamming_device_pairwise_knn": (C.c_int, [_P, _P, C.c_int, _P, _P, C.c_int, _P, C.c_int, C.c_int, _P]),
+    "orbx_match_hamming_radius": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, C.c_float, _P, C.c_int, _P, C.POINTER(C.c_int)]),
+    "orbx_match_hamming_device_radius": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, _P, C.c_int, C.c_float, _P, C.c_int64, _P]),
+    "orbx_match_hamming_device_pairwise_radius": (C.c_int, [_P, _P, C.c_int, _P, _P, C.c_int, _P, C.c_int, C.c_float, _P, C.c_int64, _P]),
     "orbx_match_hamming_device": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, C.c_int, _P, _P]),
     "orbx_match_hamming_device_ragged": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, _P, C.c_int, _P, _P]),
     "orbx_match_hamming_sets": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, _P, C.c_int, _P, _P]),

@@ -6,6 +6,8 @@
 // There is no CPU fallback anywhere in this file: every entry point either runs the sm_100a kernels or fails.
 #include <cuda_runtime.h>
 #include <nvtx3/nvToolsExt.h>
+#include <float.h>
+#include <limits.h>
 #include <math.h>
 #include <stdint.h>
 #include <stdio.h>
@@ -24,6 +26,7 @@
 #include "orbx_select.cuh"
 #include "orbx_desc.cuh"
 #include "orbx_match.cuh"
+#include "orbx_radius.cuh"
 #include "orbx_map.cuh"
 #include "orbx_stage.h"
 #include <unordered_map>
@@ -120,6 +123,7 @@ struct orbx_ctx {
     int view_frames = 0;
     Buf mq, mt, mbest, msecond, mkeys, mstatus, mcounts;
     Buf mcolkeys, mxcount;                   // cross-check: column keys [nsets][stride_rows], the host form's pair count
+    Buf mradoff, mradsums;                   // radius: the host form's offsets, the offsets scan's tile sums
     int last_batch = 0;
 
     // device-resident map-point table (SURVEY 8(f).1): slot-addressed columns + the host's id -> slot index
@@ -625,9 +629,17 @@ int sync_match_words(orbx_ctx* c, int slot, int n)
 // is the query stride (and the record pitch); one CTA per (set, query tile), and record slots past a set's count stay untouched.
 // Top-k (knn_k >= 2, d_second null, not a lane call, no cross-check): d_best receives knnMatch's k records per (set, query row),
 // [nsets][nq][k], from the single-CTA top-k kernel of the smallest list bucket that holds k (no train-row split).
+// Radius (rad set, d_second null, not a lane call, no cross-check, no top-k): one pass of the single-CTA radius kernel (no
+// train-row split); see run_radius.
+struct RadiusPass {
+    int pass;                // 1: list lengths to offsets[1 + L]; 2: hits of lists ending at or below cap to d_best
+    int thr;                 // 127 * (256 - 2R)
+    long long* offsets;
+    long long cap;
+};
 int run_match(orbx_ctx* c, const uint8_t* d_q, int nq, const uint8_t* d_t, int nt, int stride_rows, const int* d_counts, int nsets,
               int4* d_best, int4* d_second, cudaStream_t st = nullptr, int slot = 0, int* d_xc_count = nullptr, const int* d_qcounts = nullptr,
-              int knn_k = 0)
+              int knn_k = 0, const RadiusPass* rad = nullptr)
 {
     NvtxRange nvr("orbx:match_hamming");
     const bool lane_call = st != nullptr;
@@ -637,16 +649,17 @@ int run_match(orbx_ctx* c, const uint8_t* d_q, int nq, const uint8_t* d_t, int n
     if (xchk && nq >= MT_MAX_QUERY_XC) return fail(c, ORBX_E_UNSUPPORTED, "cross-check query set larger than 2^20 - 1 rows");
     const bool knn2 = d_second != nullptr;
     const bool topk = knn_k > 0;
+    const bool unsplit = topk || rad;                       // top-k and radius: single-CTA kernels, no train-row split
     // CTA-pair kernel (tcgen05 cta_group::2, query tiles in twos) whenever the (query tile, set) pairs alone fill the GPU;
     // small problems keep the single-CTA kernel, whose CTAs are independent units for the train-row split.
     const int tiles_1 = (nq + MT_QROWS - 1) / MT_QROWS, tiles_2 = (tiles_1 + 1) & ~1;
-    const bool pair = !topk && tiles_1 >= 2 && (long)tiles_2 * nsets >= 148;
+    const bool pair = !unsplit && tiles_1 >= 2 && (long)tiles_2 * nsets >= 148;
     const int tiles_m = pair ? tiles_2 : tiles_1;
     const int ntile_n = (nt + MT_BN - 1) / MT_BN;
     constexpr int kSMs = 148;                                // one CTA per SM (163 KB of shared memory each)
     // Few (query tile, set) pairs: split the train rows across CTAs and merge with atomicMax on the packed key.
     int nsplit = 1;
-    if (!knn2 && !topk && !lane_call) {
+    if (!knn2 && !unsplit && !lane_call) {
         const long base = (long)tiles_m * nsets;
         if (base < kSMs) nsplit = (int)std::min<long>(ntile_n, std::max<long>(1, (kSMs + base - 1) / base));
     }
@@ -692,7 +705,18 @@ int run_match(orbx_ctx* c, const uint8_t* d_q, int nq, const uint8_t* d_t, int n
     const dim3 grd((unsigned)tiles_m, (unsigned)nsplit, (unsigned)zgroups);
     const int smem = xchk ? MT_SMEM_BYTES_XC : MT_SMEM_BYTES;
     // (knn2 and xchk never meet: the cross-check keeps the best match only)
-    if (topk) {                                              // list buckets of 4, 8, 16 and 32 keys
+    if (rad) {
+        const bool count = rad->pass == 1;
+        if (pairwise) {
+            auto* kernel = count ? k_hamming_umma_pw_radius<1> : k_hamming_umma_pw_radius<2>;
+            kernel<<<grd, MT_THREADS, smem, st>>>(d_q, nq, d_t, nt, stride_rows, d_counts, nsets, rows_per_split, d_best, d_status, d_qcounts,
+                                                  rad->thr, rad->offsets, rad->cap);
+        } else {
+            auto* kernel = count ? k_hamming_umma_radius<1> : k_hamming_umma_radius<2>;
+            kernel<<<grd, MT_THREADS, smem, st>>>(d_q, nq, d_t, nt, stride_rows, d_counts, nsets, rows_per_split, d_best, d_status, rad->thr,
+                                                  rad->offsets, rad->cap);
+        }
+    } else if (topk) {                                       // list buckets of 4, 8, 16 and 32 keys
         static_assert(ORBX_MAX_KNN <= 32, "the largest list bucket holds 32 keys");
         const int kb = knn_k <= 4 ? 0 : knn_k <= 8 ? 1 : knn_k <= 16 ? 2 : 3;
         if (pairwise) {
@@ -779,6 +803,55 @@ int match_one_set(orbx_ctx* c, const uint8_t* query, int nq, const uint8_t* trai
     return ORBX_OK;
 }
 
+// radiusMatch, first half: list L = set * nq + query row (run_match's operands; d_qcounts: pairwise).  The count pass writes
+// every list's length to d_offsets[1 + L], and the scan turns d_offsets[0 .. nsets * nq] into the 64-bit CSR offsets.
+// Asynchronous on the context's stream.
+int radius_count(orbx_ctx* c, const uint8_t* d_q, int nq, const uint8_t* d_t, int stride_rows, const int* d_counts, int nsets,
+                 const int* d_qcounts, int thr, long long* d_offsets)
+{
+    const long long nlists = (long long)nsets * nq;
+    const long long ntiles = (nlists + RS_SCAN_TILE - 1) / RS_SCAN_TILE;
+    int rc;
+    if ((rc = ensure(c, c->mradsums, sizeof(long long) * (size_t)ntiles))) return rc;
+    CU(cudaMemsetAsync(d_offsets, 0, sizeof(long long) * (size_t)(nlists + 1), c->stream));   // (pairwise: rows past a count stay 0)
+    const RadiusPass count{1, thr, d_offsets, 0};
+    if ((rc = run_match(c, d_q, nq, d_t, stride_rows, stride_rows, d_counts, nsets, nullptr, nullptr, nullptr, 0, nullptr, d_qcounts, 0, &count)))
+        return rc;
+    long long* sums = (long long*)c->mradsums.p;
+    k_radius_tile_sums<<<(unsigned)ntiles, RS_SCAN_NT, 0, c->stream>>>(d_offsets + 1, nlists, sums);
+    k_radius_scan_sums<<<1, RS_SCAN_NT, 0, c->stream>>>(sums, ntiles);
+    k_radius_scan_tiles<<<(unsigned)ntiles, RS_SCAN_NT, 0, c->stream>>>(d_offsets + 1, nlists, sums);
+    c->launches += 3;
+    CU(cudaGetLastError());
+    return ORBX_OK;
+}
+
+// radiusMatch, second half (behind radius_count on the context's stream): the emit pass writes every list that ends at or
+// below cap to d_out in ascending trainIdx, and k_radius_order puts each into std::sort's order.
+int radius_emit(orbx_ctx* c, const uint8_t* d_q, int nq, const uint8_t* d_t, int stride_rows, const int* d_counts, int nsets,
+                const int* d_qcounts, int thr, long long* d_offsets, int4* d_out, long long cap)
+{
+    const long long nlists = (long long)nsets * nq;
+    const RadiusPass emit{2, thr, d_offsets, cap};
+    int rc;
+    if ((rc = run_match(c, d_q, nq, d_t, stride_rows, stride_rows, d_counts, nsets, d_out, nullptr, nullptr, 0, nullptr, d_qcounts, 0, &emit)))
+        return rc;
+    k_radius_order<<<(unsigned)((nlists + RS_WARPS - 1) / RS_WARPS), RS_WARPS * 32, 0, c->stream>>>(d_out, d_offsets, nlists, nq, cap);
+    ++c->launches;
+    CU(cudaGetLastError());
+    return ORBX_OK;
+}
+
+// The matcher's threshold of the integer radius R = min(256, floor(max_distance)): distance <= R <=> accumulator >= thr
+int radius_threshold(float max_distance)
+{
+    const int r = max_distance >= 256.0f ? 256 : (int)floorf(max_distance);
+    return MT_ASCALE * (256 - 2 * r);
+}
+
+// cv's CV_Assert(maxDistance > FLT_EPSILON) (false for NaN too)
+bool bad_radius(float max_distance) { return !(max_distance > FLT_EPSILON); }
+
 }  // namespace
 
 // =================================================================================================== C-ABI
@@ -855,6 +928,10 @@ int orbx_create(orbx_ctx** out, int device, int nfeatures, float scale_factor, i
         cudaFuncSetAttribute(k_hamming_umma_pw_topk<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
         cudaFuncSetAttribute(k_hamming_umma_pw_topk<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
         cudaFuncSetAttribute(k_hamming_umma_pw_topk<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
+        cudaFuncSetAttribute(k_hamming_umma_radius<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
+        cudaFuncSetAttribute(k_hamming_umma_radius<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
+        cudaFuncSetAttribute(k_hamming_umma_pw_radius<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
+        cudaFuncSetAttribute(k_hamming_umma_pw_radius<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
         cudaFuncSetAttribute(k_fast_warp<FAST_NWARP>, cudaFuncAttributeMaxDynamicSharedMemorySize, FAST_NWARP * FW_WARP_BYTES + 128) != cudaSuccess ||
         cudaFuncSetAttribute(k_pyr_tma, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024) != cudaSuccess ||
         cudaFuncSetAttribute(k_describe_tma, cudaFuncAttributeMaxDynamicSharedMemorySize, DS_NW * DS_WARP_BYTES + 128) != cudaSuccess ||
@@ -1273,6 +1350,85 @@ int orbx_match_hamming_device_pairwise_knn(orbx_ctx* c, const uint8_t* d_query, 
     CU(cudaSetDevice(c->device));
     return run_match(c, d_query, query_stride_rows, d_train, train_stride_rows, train_stride_rows, d_train_counts, npairs, (int4*)d_out,
                      nullptr, nullptr, 0, nullptr, d_query_counts, k > 1 ? k : 0);
+}
+
+int orbx_match_hamming_radius(orbx_ctx* c, const uint8_t* q, int nq, const uint8_t* t, int nt, float max_distance, orbx_match* out, int cap,
+                              int64_t* offsets, int* n_out)
+{
+    if (!c) return ORBX_E_ARG;
+    if (!n_out || !offsets) return fail(c, ORBX_E_ARG, "null pointer");
+    *n_out = 0;
+    if (nq < 0 || nt < 0 || cap < 0) return fail(c, ORBX_E_ARG, "negative size");
+    if (bad_radius(max_distance)) return fail(c, ORBX_E_ARG, "maxDistance must be larger than FLT_EPSILON");
+    if (nt >= MT_MAX_TRAIN) return fail(c, ORBX_E_UNSUPPORTED, "train set larger than 2^20 - 1 rows");
+    if (nq == 0 || nt == 0) {                                // one empty list per query (cv), or none
+        memset(offsets, 0, sizeof(int64_t) * ((size_t)nq + 1));
+        return ORBX_OK;
+    }
+    if (!q || !t || !out) return fail(c, ORBX_E_ARG, "null pointer");
+    CU(cudaSetDevice(c->device));
+    const int thr = radius_threshold(max_distance);
+    int rc;
+    if ((rc = ensure(c, c->mq, (size_t)nq * 32)) || (rc = ensure(c, c->mt, (size_t)nt * 32)) ||
+        (rc = ensure(c, c->mradoff, sizeof(long long) * ((size_t)nq + 1))))
+        return rc;
+    long long* d_off = (long long*)c->mradoff.p;
+    CU(cudaMemcpyAsync(c->mq.p, q, (size_t)nq * 32, cudaMemcpyHostToDevice, c->stream));
+    CU(cudaMemcpyAsync(c->mt.p, t, (size_t)nt * 32, cudaMemcpyHostToDevice, c->stream));
+    if ((rc = radius_count(c, (const uint8_t*)c->mq.p, nq, (const uint8_t*)c->mt.p, nt, nullptr, 1, nullptr, thr, d_off))) return rc;
+    long long total = 0;
+    CU(cudaMemcpyAsync(&total, d_off + nq, sizeof total, cudaMemcpyDeviceToHost, c->stream));
+    if ((rc = sync_match_words(c, 0, 1))) return rc;
+    if (total > INT_MAX) return fail(c, ORBX_E_UNSUPPORTED, "more than 2^31 - 1 records");
+    *n_out = (int)total;
+    if (total > cap) return fail(c, ORBX_E_CAPACITY, "output capacity below the number of records");
+    if ((rc = ensure(c, c->mbest, 16 * (size_t)total))) return rc;
+    if ((rc = radius_emit(c, (const uint8_t*)c->mq.p, nq, (const uint8_t*)c->mt.p, nt, nullptr, 1, nullptr, thr, d_off, (int4*)c->mbest.p, total)))
+        return rc;
+    CU(cudaMemcpyAsync(out, c->mbest.p, 16 * (size_t)total, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaMemcpyAsync(offsets, d_off, sizeof(int64_t) * ((size_t)nq + 1), cudaMemcpyDeviceToHost, c->stream));
+    return sync_match_words(c, 0, 1);
+}
+
+int orbx_match_hamming_device_radius(orbx_ctx* c, const uint8_t* d_query, int nq, const uint8_t* d_train, int train_stride_rows,
+                                     const int* d_train_counts, int nsets, float max_distance, orbx_match* d_out, int64_t cap, int64_t* d_offsets)
+{
+    if (!c) return ORBX_E_ARG;
+    if (nq < 0 || train_stride_rows < 0 || nsets < 0 || nsets > 65535 || cap < 0) return fail(c, ORBX_E_ARG, "bad sizes");
+    if (bad_radius(max_distance)) return fail(c, ORBX_E_ARG, "maxDistance must be larger than FLT_EPSILON");
+    if (!d_query || !d_train || !d_train_counts || !d_out || !d_offsets) return fail(c, ORBX_E_ARG, "null pointer");
+    if (train_stride_rows >= MT_MAX_TRAIN) return fail(c, ORBX_E_UNSUPPORTED, "train set stride of 2^20 rows or more");
+    CU(cudaSetDevice(c->device));
+    long long* d_off = (long long*)d_offsets;
+    if (nq == 0 || train_stride_rows == 0 || nsets == 0) {   // every list empty
+        CU(cudaMemsetAsync(d_off, 0, sizeof(int64_t) * ((size_t)nsets * nq + 1), c->stream));
+        return ORBX_OK;
+    }
+    const int thr = radius_threshold(max_distance);
+    const int rc = radius_count(c, d_query, nq, d_train, train_stride_rows, d_train_counts, nsets, nullptr, thr, d_off);
+    return rc ? rc : radius_emit(c, d_query, nq, d_train, train_stride_rows, d_train_counts, nsets, nullptr, thr, d_off, (int4*)d_out, cap);
+}
+
+int orbx_match_hamming_device_pairwise_radius(orbx_ctx* c, const uint8_t* d_query, int query_stride_rows, const int* d_query_counts,
+                                              const uint8_t* d_train, int train_stride_rows, const int* d_train_counts, int npairs,
+                                              float max_distance, orbx_match* d_out, int64_t cap, int64_t* d_offsets)
+{
+    if (!c) return ORBX_E_ARG;
+    if (cap < 0) return fail(c, ORBX_E_ARG, "bad sizes");
+    if (bad_radius(max_distance)) return fail(c, ORBX_E_ARG, "maxDistance must be larger than FLT_EPSILON");
+    if (!d_offsets) return fail(c, ORBX_E_ARG, "null pointer");
+    int rc = check_args_pairwise(c, d_query, query_stride_rows, d_query_counts, d_train, train_stride_rows, d_train_counts, npairs, d_out);
+    if (rc) return rc;
+    CU(cudaSetDevice(c->device));
+    long long* d_off = (long long*)d_offsets;
+    if (npairs == 0 || query_stride_rows == 0 || train_stride_rows == 0) {   // every list empty
+        CU(cudaMemsetAsync(d_off, 0, sizeof(int64_t) * ((size_t)npairs * query_stride_rows + 1), c->stream));
+        return ORBX_OK;
+    }
+    const int thr = radius_threshold(max_distance);
+    rc = radius_count(c, d_query, query_stride_rows, d_train, train_stride_rows, d_train_counts, npairs, d_query_counts, thr, d_off);
+    return rc ? rc : radius_emit(c, d_query, query_stride_rows, d_train, train_stride_rows, d_train_counts, npairs, d_query_counts, thr, d_off,
+                                 (int4*)d_out, cap);
 }
 
 int orbx_filter_matches(orbx_match* m, int n, float ratio)

@@ -34,6 +34,8 @@
 // as above, and CTAs whose query tile is empty for their set exit before any setup.  Few units keep the train-row split.
 // knnMatch for k > 2 (TOP-K, KB = list capacity 4 / 8 / 16 / 32): the single-CTA body, shared-query or pairwise, whose epilogue
 // keeps each query row's KB best keys in registers (see topk_tile); no CTA pair and no train-row split, as for knn2.
+// radiusMatch (RAD = 1 count, 2 emit): the same single-CTA body, whose epilogue counts, then writes, each query row's columns
+// at or above the radius threshold (see radius_tile); orbx_radius.cuh scans the counts and orders the lists.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -363,21 +365,53 @@ __device__ __forceinline__ void topk_tile(const uint32_t* rp, int tmax, int j0, 
         }
 }
 
+// ---- radius (RAD = 1 count pass, 2 emit pass; BFMatcher radiusMatch): distance h <= R  <=>  127 * dot + code >= thr =
+// 127 * (256 - 2R), because the index code is below 127.  A tile whose packed maximum is below thr has no hit.  Count: n
+// grows by the hits of train rows j < n1 (columns past the set's end are copies of its last row, with the same dot).  Emit
+// (out != nullptr): the hits are also written to out[n], in ascending train row, the row decoded from the column's code.
+template <bool EMIT>
+__device__ __forceinline__ void radius_tile(const uint32_t* rp, int tmax, int thr, int j0, int n1, int qrow, int4* out, int& n)
+{
+    if (tmax < thr) return;
+#pragma unroll
+    for (int u = 0; u < MT_BN / 2; ++u) {
+        if (__vcmpges2(rp[u], (uint32_t)(thr & 0xFFFF) * 0x10001u) == 0u) continue;   // neither column of the pair is a hit
+#pragma unroll
+        for (int h = 0; h < 2; ++h) {
+            const int v = h ? (int)rp[u] >> 16 : (int)(rp[u] << 16) >> 16;
+            if (v >= thr) {
+                const unsigned kk = (unsigned)(v + MT_ASCALE * 256);
+                const unsigned q = kk / (unsigned)MT_ASCALE;          // dot + 256
+                const int j = j0 + (MT_BN - 1) - (int)(kk - q * (unsigned)MT_ASCALE);
+                if (j < n1) {
+                    if (EMIT && out) out[n] = make_int4(qrow, j, 0, __float_as_int((float)((512 - (int)q) >> 1)));
+                    ++n;
+                }
+            }
+        }
+    }
+}
+
 // SETQ = false: one query set (the map) shared by every train set; nq is its row count.
 // SETQ = true (pairwise): set s has its own query rows, min(query_counts[s], nq) of them at query + s * nq * 32, so nq is
 // the query stride and the pitch of the outputs and of the split keys.  The A tile then belongs to ONE set: the grid has
 // gridDim.z = nsets (one (set, query tile) unit per CTA), and a CTA whose query tile is empty for its set exits before
 // any setup -- in a CTA pair only when the leader's (lower) tile is empty too, because the peer holds half of every B tile.
 // KB > 0 (top-k, k = knn_k <= KB): best receives k records per (set, query row), [nsets][nq][k]; single CTA, no split.
-template <bool KNN2, bool PAIR, bool XCHK, bool SETQ, int KB = 0>
+// RAD > 0 (radius, distance <= R with rad_thr = 127 * (256 - 2R)), list L = set * nq + query row; single CTA, no split.
+// RAD = 1: rad_offsets[1 + L] = list L's length.  RAD = 2: rad_offsets holds the scanned offsets, and list L's hits go to
+// best[rad_offsets[L] ..] in ascending train row when rad_offsets[L + 1] <= rad_cap.
+template <bool KNN2, bool PAIR, bool XCHK, bool SETQ, int KB = 0, int RAD = 0>
 __device__ __forceinline__ void
 hamming_umma_body(const uint8_t* __restrict__ query, int nq, const uint8_t* __restrict__ train, int nt, int train_stride_rows,
                const int* __restrict__ train_counts, int nsets, int rows_per_split, int4* __restrict__ best,
                int4* __restrict__ second, int* __restrict__ keys, int* __restrict__ status, int* __restrict__ col_keys,
-               const int* __restrict__ query_counts, int knn_k = 0)
+               const int* __restrict__ query_counts, int knn_k = 0, int rad_thr = 0, long long* __restrict__ rad_offsets = nullptr,
+               long long rad_cap = 0)
 {
     static_assert(!(KNN2 && XCHK), "cross-check keeps the best match only");
     static_assert(KB == 0 || (!KNN2 && !PAIR && !XCHK), "top-k runs on the single-CTA kernel alone");
+    static_assert(RAD == 0 || (KB == 0 && !KNN2 && !PAIR && !XCHK), "radius runs on the single-CTA kernel alone");
     int nqv = nq;                                            // query rows present (padded rows q >= nqv are excluded)
     if constexpr (SETQ) {
         nqv = max(0, min(__ldg(query_counts + blockIdx.z), nq));
@@ -599,6 +633,14 @@ hamming_umma_body(const uint8_t* __restrict__ query, int nq, const uint8_t* __re
             int list[KB > 0 ? KB : 1];                       // top-k: this row's best keys, descending
 #pragma unroll
             for (int r = 0; r < (KB > 0 ? KB : 1); ++r) list[r] = INT_MIN;
+            int rad_n = 0;                                   // radius: this row's hits so far in the set
+            int4* rad_out = nullptr;                         // emit pass: where they go (null: the list is past the cap)
+            if constexpr (RAD == 2) {
+                if (qrow < nqv) {
+                    const size_t o = (size_t)set * nq + qrow;
+                    if (rad_offsets[o + 1] <= rad_cap) rad_out = best + rad_offsets[o];
+                }
+            }
             for (int i = 0; i < rg.ntiles; ++i, ++t) {
                 const int b = t & 1;
                 const uint32_t bph = (uint32_t)(t >> 1) & 1u;
@@ -636,6 +678,7 @@ hamming_umma_body(const uint8_t* __restrict__ query, int nq, const uint8_t* __re
                     const unsigned pk = __vimax3_s16x2(__vimax3_s16x2(p[0], p[1], p[2]), __vimax3_s16x2(p[3], p[4], p[5]), __vmaxs2(p[6], p[7]));
                     k1 = max((int)(pk << 16) >> 16, (int)pk >> 16);
                     if constexpr (KB > 0) topk_tile<KB>(rp, k1, j0, rg.n1, list);
+                    if constexpr (RAD > 0) radius_tile<RAD == 2>(rp, k1, rad_thr, j0, rg.n1, qrow, rad_out, rad_n);
                     if constexpr (XCHK)
                         xc_warp_columns(rp, qrow < nqv, qrow - q0, reinterpret_cast<int*>(smem + MT_SMEM_XC) + (b * 8 + warp - MT_EPI_WARP0) * MT_BN);
                 } else if (!KNN2) {
@@ -665,6 +708,7 @@ hamming_umma_body(const uint8_t* __restrict__ query, int nq, const uint8_t* __re
                     const unsigned pk = __vimax3_s16x2(__vimax3_s16x2(p[0], p[1], p[2]), __vimax3_s16x2(p[3], p[4], p[5]), __vmaxs2(p[6], p[7]));
                     k1 = max((int)(pk << 16) >> 16, (int)pk >> 16);
                     if constexpr (KB > 0) topk_tile<KB>(rp, k1, j0, rg.n1, list);
+                    if constexpr (RAD > 0) radius_tile<RAD == 2>(rp, k1, rad_thr, j0, rg.n1, qrow, rad_out, rad_n);
                     if constexpr (XCHK)                      // (chunks past N hold -32768: no column there)
                         xc_warp_columns(rp, qrow < nqv, qrow - q0, reinterpret_cast<int*>(smem + MT_SMEM_XC) + (b * 8 + warp - MT_EPI_WARP0) * MT_BN);
                 } else {
@@ -688,7 +732,7 @@ hamming_umma_body(const uint8_t* __restrict__ query, int nq, const uint8_t* __re
                 }
                 // decode the tile winner(s) into the global key  dot << 20 | (0xFFFFF - j)
 #pragma unroll
-                for (int w = 0; w < (KB > 0 ? 0 : KNN2 ? 2 : 1); ++w) {   // (top-k: already in the list)
+                for (int w = 0; w < (KB > 0 || RAD > 0 ? 0 : KNN2 ? 2 : 1); ++w) {   // (top-k: already in the list; radius: nothing to keep)
                     const int k = w == 0 ? k1 : k2;
                     if (k != INT_MIN) {
                         const unsigned kk = (unsigned)(k + MT_ASCALE * 256);
@@ -728,7 +772,9 @@ hamming_umma_body(const uint8_t* __restrict__ query, int nq, const uint8_t* __re
             }
             if (ok && qrow < nqv) {
                 const size_t o = (size_t)set * nq + qrow;
-                if constexpr (KB > 0) {                     // the k records of this row, once per set
+                if constexpr (RAD > 0) {                    // count pass: the list's length (the emit pass has written its hits)
+                    if constexpr (RAD == 1) rad_offsets[1 + o] = rad_n;
+                } else if constexpr (KB > 0) {                     // the k records of this row, once per set
                     int4* out = best + o * knn_k;
 #pragma unroll
                     for (int r = 0; r < KB; ++r) {
@@ -827,6 +873,26 @@ __global__ void __launch_bounds__(MT_THREADS, 1) k_hamming_umma_pw_topk(const ui
 {
     hamming_umma_body<false, false, false, true, KB>(query, nq, train, nt, train_stride_rows, train_counts, nsets, rows_per_split, best, nullptr, nullptr,
                                                      status, nullptr, query_counts, knn_k);
+}
+// radius (radiusMatch): RAD = 1 writes list lengths to offsets[1 + L], RAD = 2 the hits of lists ending at or below cap to out
+template <int RAD>
+__global__ void __launch_bounds__(MT_THREADS, 1) k_hamming_umma_radius(const uint8_t* __restrict__ query, int nq, const uint8_t* __restrict__ train, int nt,
+                                                                       int train_stride_rows, const int* __restrict__ train_counts, int nsets, int rows_per_split,
+                                                                       int4* __restrict__ out, int* __restrict__ status, int thr, long long* __restrict__ offsets,
+                                                                       long long cap)
+{
+    hamming_umma_body<false, false, false, false, 0, RAD>(query, nq, train, nt, train_stride_rows, train_counts, nsets, rows_per_split, out, nullptr,
+                                                          nullptr, status, nullptr, nullptr, 0, thr, offsets, cap);
+}
+// pairwise radius: lists [nsets][nq] (nq = query stride); rows past a set's query count are not visited (their lengths stay 0)
+template <int RAD>
+__global__ void __launch_bounds__(MT_THREADS, 1) k_hamming_umma_pw_radius(const uint8_t* __restrict__ query, int nq, const uint8_t* __restrict__ train, int nt,
+                                                                          int train_stride_rows, const int* __restrict__ train_counts, int nsets, int rows_per_split,
+                                                                          int4* __restrict__ out, int* __restrict__ status, const int* __restrict__ query_counts,
+                                                                          int thr, long long* __restrict__ offsets, long long cap)
+{
+    hamming_umma_body<false, false, false, true, 0, RAD>(query, nq, train, nt, train_stride_rows, train_counts, nsets, rows_per_split, out, nullptr,
+                                                         nullptr, status, nullptr, query_counts, 0, thr, offsets, cap);
 }
 
 // ONE CTA per set: query i keeps its best match (i, j) iff column j's key names i, i.e. i is also train row j's nearest

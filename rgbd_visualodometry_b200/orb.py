@@ -7,7 +7,8 @@
   orb_->detectAndCompute(color_, Mat(), kps, desc)            ORB.detectAndCompute(image, None) -> (kps, desc)
       src/frontend.cpp:153
   matcher.match(query, train, matches)                        BFMatcher(NORM_HAMMING).match(query, train)
-      src/frontend.cpp:187                                    (+ knnMatch(query, train, k <= 32), crossCheck=True)
+      src/frontend.cpp:187                                    (+ knnMatch(query, train, k <= 32), crossCheck=True,
+                                                              radiusMatch(query, train, maxDistance))
   max(min_dis * match_ratio, 30) filter                       filter_matches(matches, match_ratio)
       src/frontend.cpp:190-211
 
@@ -170,6 +171,24 @@ class Context:
         self._check(self.lib.orbx_match_hamming_knn(self.h, _ptr(q), len(q), _ptr(t), len(t), int(k), _ptr(out), C.byref(n)))
         return out[:n.value]
 
+    def radius_match(self, query: np.ndarray, train: np.ndarray, max_distance: float):
+        """radiusMatch(query, train, maxDistance): (records, offsets), query i's list = records[offsets[i]:offsets[i + 1]] in cv2's
+        order (libstdc++ std::sort by distance of the rows in ascending trainIdx).  offsets is int64 [nq + 1]."""
+        q = np.ascontiguousarray(query, np.uint8).reshape(-1, 32)
+        t = np.ascontiguousarray(train, np.uint8).reshape(-1, 32)
+        offsets = np.zeros(len(q) + 1, np.int64)
+        n = C.c_int(0)
+        cap = min(len(q) * len(t), max(1024, 16 * len(q)))
+        while True:
+            out = np.zeros(max(cap, 1), DMATCH_DTYPE)
+            rc = self.lib.orbx_match_hamming_radius(self.h, _ptr(q), len(q), _ptr(t), len(t), float(max_distance), _ptr(out), cap,
+                                                    _ptr(offsets), C.byref(n))
+            if rc == E_CAPACITY:
+                cap = n.value
+                continue
+            self._check(rc)
+            return out[:n.value], offsets
+
     def match_crosscheck(self, query: np.ndarray, train: np.ndarray) -> np.ndarray:
         """BFMatcher(NORM_HAMMING, crossCheck=True).match: the mutual nearest pairs, ascending queryIdx."""
         q = np.ascontiguousarray(query, np.uint8).reshape(-1, 32)
@@ -220,6 +239,22 @@ class Context:
         not written)."""
         self._check(self.lib.orbx_match_hamming_device_pairwise_knn(self.h, d_query_ptr, query_stride_rows, d_query_counts_ptr, d_train_ptr,
                                                                     train_stride_rows, d_train_counts_ptr, npairs, int(k), d_out_ptr))
+
+    def match_device_radius(self, d_query_ptr: int, nq: int, d_train_ptr: int, stride_rows: int, d_counts_ptr: int, nsets: int,
+                            max_distance: float, d_out_ptr: int, cap: int, d_offsets_ptr: int):
+        """Asynchronous, device-resident, ragged batch: radiusMatch of the query set against every set.  List s * nq + i at
+        d_out[d_offsets[L] : d_offsets[L + 1]] (d_offsets: int64 [nsets * nq + 1], always complete); lists ending past cap
+        records are not written."""
+        self._check(self.lib.orbx_match_hamming_device_radius(self.h, d_query_ptr, nq, d_train_ptr, stride_rows, d_counts_ptr, nsets,
+                                                              float(max_distance), d_out_ptr, int(cap), d_offsets_ptr))
+
+    def match_device_pairwise_radius(self, d_query_ptr: int, query_stride_rows: int, d_query_counts_ptr: int, d_train_ptr: int,
+                                     train_stride_rows: int, d_train_counts_ptr: int, npairs: int, max_distance: float, d_out_ptr: int,
+                                     cap: int, d_offsets_ptr: int):
+        """As match_device_radius, pairwise: list p * query_stride_rows + i (empty past pair p's query count)."""
+        self._check(self.lib.orbx_match_hamming_device_pairwise_radius(self.h, d_query_ptr, query_stride_rows, d_query_counts_ptr,
+                                                                       d_train_ptr, train_stride_rows, d_train_counts_ptr, npairs,
+                                                                       float(max_distance), d_out_ptr, int(cap), d_offsets_ptr))
 
     def match_sets(self, query: np.ndarray, train: np.ndarray, counts: np.ndarray, knn2: bool = False):
         """One map (query [M,32]) against nsets frames' descriptor sets (train [S,cap,32], counts [S]); host buffers."""
@@ -427,6 +462,15 @@ class BFMatcher:
         if k == 2:
             return self._ctx.knn_match2(queryDescriptors, trainDescriptors)
         return self._ctx.knn_match(queryDescriptors, trainDescriptors, k)
+
+    def radiusMatch(self, queryDescriptors, trainDescriptors, maxDistance):
+        """A list of nq DMATCH_DTYPE arrays (views of one buffer): query i's train rows at distance <= maxDistance, in cv2's
+        order.  crossCheck does not apply, as in cv2.  maxDistance <= FLT_EPSILON or NaN raises (E_ARG) unless the query set is
+        empty (cv2 returns no lists before it checks)."""
+        if queryDescriptors is None or trainDescriptors is None or np.asarray(queryDescriptors).size == 0:
+            return []
+        rec, off = self._ctx.radius_match(queryDescriptors, trainDescriptors, maxDistance)
+        return [rec[off[i]:off[i + 1]] for i in range(len(off) - 1)]
 
 
 def filter_matches(matches: np.ndarray, match_ratio: float = 2.0) -> np.ndarray:
