@@ -620,36 +620,91 @@ int sync_match_words(orbx_ctx* c, int slot, int n)
     return ORBX_OK;
 }
 
-// The matcher on device-resident operands, asynchronous on `st` (default: the context's stream).  `slot` selects the
-// status word (one per lane, so concurrent lanes never reset each other's); lanes never take the split-train path,
-// whose key scratch is shared.
-// Cross-check (d_xc_count set, d_second null, not a lane call): set s's mutual pairs are compacted in place to d_best + s * nq,
-// their count to d_xc_count[s].
-// Pairwise (d_qcounts set, not a lane call): set s matches its own min(d_qcounts[s], nq) query rows at d_q + s * nq * 32, so nq
-// is the query stride (and the record pitch); one CTA per (set, query tile), and record slots past a set's count stay untouched.
-// Top-k (knn_k >= 2, d_second null, not a lane call, no cross-check): d_best receives knnMatch's k records per (set, query row),
-// [nsets][nq][k], from the single-CTA top-k kernel of the smallest list bucket that holds k (no train-row split).
-// Radius (rad set, d_second null, not a lane call, no cross-check, no top-k): one pass of the single-CTA radius kernel (no
-// train-row split); see run_radius.
-struct RadiusPass {
-    int pass;                // 1: list lengths to offsets[1 + L]; 2: hits of lists ending at or below cap to d_best
-    int thr;                 // 127 * (256 - 2R)
-    long long* offsets;
-    long long cap;
+// One matcher job on device-resident operands: nq query rows (shared by every set, or pairwise: set s's own
+// min(query_counts[s], nq) rows at query + s * nq * 32, nq being the query stride and the record pitch) against nsets train
+// sets of min(train_counts[s], train_stride) rows (null train_counts: all) at train + s * train_stride * 32.
+struct MatchJob {
+    MatchOp op = MatchOp::Best;
+    const uint8_t* query = nullptr;
+    int nq = 0;
+    const int* query_counts = nullptr;       // pairwise; one CTA per (set, query tile), record slots past a set's count untouched
+    const uint8_t* train = nullptr;
+    int train_stride = 0;                    // rows per set
+    const int* train_counts = nullptr;
+    int nsets = 1;
+    int4* best = nullptr;                    // [nsets][nq] records; TopK: [nsets][nq][k]; CrossCheck: set s's mutual pairs
+                                             // compacted in place to best + s * nq; RadiusEmit: the lists
+    int4* second = nullptr;                  // Knn2
+    int* xc_count = nullptr;                 // CrossCheck: set s's pair count
+    int k = 0;                               // TopK: k >= 2 (the single-CTA kernel of the smallest list bucket that holds k)
+    int rad_thr = 0;                         // radius passes: see radius_pass
+    long long* rad_offsets = nullptr;
+    long long rad_cap = 0;
+    // a lane of host_batch: its own stream and status word (concurrent lanes never reset each other's), no train-row split
+    // (its key scratch is shared) and no stage marks; otherwise the context's stream and status word 0
+    bool lane = false;
+    cudaStream_t lane_stream = nullptr;
+    int lane_slot = 0;
 };
-int run_match(orbx_ctx* c, const uint8_t* d_q, int nq, const uint8_t* d_t, int nt, int stride_rows, const int* d_counts, int nsets,
-              int4* d_best, int4* d_second, cudaStream_t st = nullptr, int slot = 0, int* d_xc_count = nullptr, const int* d_qcounts = nullptr,
-              int knn_k = 0, const RadiusPass* rad = nullptr)
+// The job of an operation on nsets train sets of train_stride rows each, train_counts[s] of them present (null: all), and
+// one query set of nq rows; the other fields keep their defaults
+MatchJob match_job(MatchOp op, const uint8_t* query, int nq, const uint8_t* train, int train_stride, const int* train_counts, int nsets, void* best)
+{
+    MatchJob job;
+    job.op = op;
+    job.query = query; job.nq = nq;
+    job.train = train; job.train_stride = train_stride; job.train_counts = train_counts; job.nsets = nsets;
+    job.best = (int4*)best;
+    return job;
+}
+
+// The kernel of an operation: CTA pair or not, shared query or pairwise (SETQ), TopK's list bucket (4, 8, 16 or 32 keys).
+using MatchKernel = void (*)(MatchArgs);
+template <bool SETQ>
+MatchKernel match_kernel(MatchOp op, bool pair, int k)
+{
+    static_assert(ORBX_MAX_KNN <= 32, "the largest list bucket holds 32 keys");
+    switch (op) {
+    case MatchOp::Best:       return pair ? k_hamming_umma2<MatchOp::Best, SETQ> : k_hamming_umma<MatchOp::Best, SETQ>;
+    case MatchOp::Knn2:       return pair ? k_hamming_umma2<MatchOp::Knn2, SETQ> : k_hamming_umma<MatchOp::Knn2, SETQ>;
+    case MatchOp::CrossCheck: return pair ? k_hamming_umma2<MatchOp::CrossCheck, SETQ> : k_hamming_umma<MatchOp::CrossCheck, SETQ>;
+    case MatchOp::TopK:       return k <= 4 ? k_hamming_umma<MatchOp::TopK, SETQ, 4> : k <= 8 ? k_hamming_umma<MatchOp::TopK, SETQ, 8>
+                                   : k <= 16 ? k_hamming_umma<MatchOp::TopK, SETQ, 16> : k_hamming_umma<MatchOp::TopK, SETQ, 32>;
+    case MatchOp::RadiusCount: return k_hamming_umma<MatchOp::RadiusCount, SETQ>;
+    case MatchOp::RadiusEmit:  return k_hamming_umma<MatchOp::RadiusEmit, SETQ>;
+    }
+    return nullptr;
+}
+MatchKernel match_kernel(MatchOp op, bool pair, bool pairwise, int k)
+{
+    return pairwise ? match_kernel<true>(op, pair, k) : match_kernel<false>(op, pair, k);
+}
+int match_smem(MatchOp op) { return op == MatchOp::CrossCheck ? MT_SMEM_BYTES_XC : MT_SMEM_BYTES; }
+
+// Every matcher kernel may use its dynamic shared memory (once per context)
+bool match_kernels_allow_smem()
+{
+    constexpr MatchOp ops[] = {MatchOp::Best, MatchOp::Knn2, MatchOp::CrossCheck, MatchOp::TopK, MatchOp::RadiusCount, MatchOp::RadiusEmit};
+    for (MatchOp op : ops)
+        for (int pairwise = 0; pairwise < 2; ++pairwise)
+            for (int pair = 0; pair < 2; ++pair)
+                for (int k : {4, 8, 16, 32})
+                    if (cudaFuncSetAttribute(match_kernel(op, pair, pairwise, k), cudaFuncAttributeMaxDynamicSharedMemorySize, match_smem(op)) != cudaSuccess)
+                        return false;
+    return true;
+}
+
+// Runs a job, asynchronous on its stream.
+int run_match(orbx_ctx* c, const MatchJob& job)
 {
     NvtxRange nvr("orbx:match_hamming");
-    const bool lane_call = st != nullptr;
-    if (!st) st = c->stream;
+    const int nq = job.nq, nt = job.train_stride, nsets = job.nsets;
+    const cudaStream_t st = job.lane ? job.lane_stream : c->stream;
     if (nt >= MT_MAX_TRAIN) return fail(c, ORBX_E_UNSUPPORTED, "train set larger than 2^20 - 1 rows");
-    const bool xchk = d_xc_count != nullptr;
+    const bool xchk = job.op == MatchOp::CrossCheck;
     if (xchk && nq >= MT_MAX_QUERY_XC) return fail(c, ORBX_E_UNSUPPORTED, "cross-check query set larger than 2^20 - 1 rows");
-    const bool knn2 = d_second != nullptr;
-    const bool topk = knn_k > 0;
-    const bool unsplit = topk || rad;                       // top-k and radius: single-CTA kernels, no train-row split
+    const bool knn2 = job.op == MatchOp::Knn2;
+    const bool unsplit = !match_op_pairs(job.op);            // top-k and radius: single-CTA kernels, no train-row split
     // CTA-pair kernel (tcgen05 cta_group::2, query tiles in twos) whenever the (query tile, set) pairs alone fill the GPU;
     // small problems keep the single-CTA kernel, whose CTAs are independent units for the train-row split.
     const int tiles_1 = (nq + MT_QROWS - 1) / MT_QROWS, tiles_2 = (tiles_1 + 1) & ~1;
@@ -659,7 +714,7 @@ int run_match(orbx_ctx* c, const uint8_t* d_q, int nq, const uint8_t* d_t, int n
     constexpr int kSMs = 148;                                // one CTA per SM (163 KB of shared memory each)
     // Few (query tile, set) pairs: split the train rows across CTAs and merge with atomicMax on the packed key.
     int nsplit = 1;
-    if (!knn2 && !unsplit && !lane_call) {
+    if (!knn2 && !unsplit && !job.lane) {
         const long base = (long)tiles_m * nsets;
         if (base < kSMs) nsplit = (int)std::min<long>(ntile_n, std::max<long>(1, (kSMs + base - 1) / base));
     }
@@ -670,7 +725,7 @@ int run_match(orbx_ctx* c, const uint8_t* d_q, int nq, const uint8_t* d_t, int n
     // zgroups: waves(z) * sets-per-CTA(z) is the time in units of one (query tile, set) pass; a CTA's setup (TMEM
     // allocation, query expansion, pipeline fill) costs about a third of such a pass for ~1000-row sets, less for longer ones.
     // Pairwise: every set has its own query tile, so every set gets its own CTAs.
-    const bool pairwise = d_qcounts != nullptr;
+    const bool pairwise = job.query_counts != nullptr;
     int zgroups = nsets;
     if (!pairwise) {
         zgroups = 1;
@@ -683,87 +738,53 @@ int run_match(orbx_ctx* c, const uint8_t* d_q, int nq, const uint8_t* d_t, int n
             if (best_cost < 0 || cost < best_cost) { best_cost = cost; zgroups = z; }
         }
     }
-    int* keys = nullptr;
+    // (status words: zero since orbx_create; re-zeroed by match_timed_out() after a failure)
+    MatchArgs a = {job.query, nq, job.query_counts, job.train, nt, nt, job.train_counts, nsets, rows_per_split, job.best,
+                   job.second, nullptr, nullptr, (int*)c->mstatus.p + (job.lane ? job.lane_slot : 0), job.k, job.rad_thr, job.rad_offsets,
+                   job.rad_cap};
     const size_t nout = (size_t)nq * nsets;
     int rc;
-    int* d_status = (int*)c->mstatus.p + slot;               // zero since orbx_create; re-zeroed by match_timed_out() after a failure
-    if (!lane_call) stage_mark(c, 7);
+    if (!job.lane) stage_mark(c, 7);
     if (nsplit > 1) {
         if ((rc = ensure(c, c->mkeys, nout * sizeof(int)))) return rc;
-        keys = (int*)c->mkeys.p;
-        k_match_keys_init<<<(unsigned)((nout + 255) / 256), 256, 0, st>>>(keys, nout);
+        a.keys = (int*)c->mkeys.p;
+        k_match_keys_init<<<(unsigned)((nout + 255) / 256), 256, 0, st>>>(a.keys, nout);
         ++c->launches;
     }
-    int* col_keys = nullptr;
     if (xchk) {
-        const size_t ncol = (size_t)nsets * stride_rows;
+        const size_t ncol = (size_t)nsets * job.train_stride;
         if ((rc = ensure(c, c->mcolkeys, ncol * sizeof(int)))) return rc;
-        col_keys = (int*)c->mcolkeys.p;
-        k_match_keys_init<<<(unsigned)((ncol + 255) / 256), 256, 0, st>>>(col_keys, ncol);
+        a.col_keys = (int*)c->mcolkeys.p;
+        k_match_keys_init<<<(unsigned)((ncol + 255) / 256), 256, 0, st>>>(a.col_keys, ncol);
         ++c->launches;
     }
     const dim3 grd((unsigned)tiles_m, (unsigned)nsplit, (unsigned)zgroups);
-    const int smem = xchk ? MT_SMEM_BYTES_XC : MT_SMEM_BYTES;
-    // (knn2 and xchk never meet: the cross-check keeps the best match only)
-    if (rad) {
-        const bool count = rad->pass == 1;
-        if (pairwise) {
-            auto* kernel = count ? k_hamming_umma_pw_radius<1> : k_hamming_umma_pw_radius<2>;
-            kernel<<<grd, MT_THREADS, smem, st>>>(d_q, nq, d_t, nt, stride_rows, d_counts, nsets, rows_per_split, d_best, d_status, d_qcounts,
-                                                  rad->thr, rad->offsets, rad->cap);
-        } else {
-            auto* kernel = count ? k_hamming_umma_radius<1> : k_hamming_umma_radius<2>;
-            kernel<<<grd, MT_THREADS, smem, st>>>(d_q, nq, d_t, nt, stride_rows, d_counts, nsets, rows_per_split, d_best, d_status, rad->thr,
-                                                  rad->offsets, rad->cap);
-        }
-    } else if (topk) {                                       // list buckets of 4, 8, 16 and 32 keys
-        static_assert(ORBX_MAX_KNN <= 32, "the largest list bucket holds 32 keys");
-        const int kb = knn_k <= 4 ? 0 : knn_k <= 8 ? 1 : knn_k <= 16 ? 2 : 3;
-        if (pairwise) {
-            auto* kernel = kb == 0 ? k_hamming_umma_pw_topk<4> : kb == 1 ? k_hamming_umma_pw_topk<8> : kb == 2 ? k_hamming_umma_pw_topk<16>
-                                                                                                           : k_hamming_umma_pw_topk<32>;
-            kernel<<<grd, MT_THREADS, smem, st>>>(d_q, nq, d_t, nt, stride_rows, d_counts, nsets, rows_per_split, d_best, d_status, d_qcounts, knn_k);
-        } else {
-            auto* kernel = kb == 0 ? k_hamming_umma_topk<4> : kb == 1 ? k_hamming_umma_topk<8> : kb == 2 ? k_hamming_umma_topk<16> : k_hamming_umma_topk<32>;
-            kernel<<<grd, MT_THREADS, smem, st>>>(d_q, nq, d_t, nt, stride_rows, d_counts, nsets, rows_per_split, d_best, d_status, knn_k);
-        }
-    } else if (pairwise) {
-        auto* kernel = pair ? (xchk ? k_hamming_umma2_pw<false, true> : knn2 ? k_hamming_umma2_pw<true, false> : k_hamming_umma2_pw<false, false>)
-                            : (xchk ? k_hamming_umma_pw<false, true> : knn2 ? k_hamming_umma_pw<true, false> : k_hamming_umma_pw<false, false>);
-        kernel<<<grd, MT_THREADS, smem, st>>>(d_q, nq, d_t, nt, stride_rows, d_counts, nsets, rows_per_split, d_best, d_second, keys, d_status,
-                                              col_keys, d_qcounts);
-    } else {
-        auto* kernel = pair ? (xchk ? k_hamming_umma2<false, true> : knn2 ? k_hamming_umma2<true, false> : k_hamming_umma2<false, false>)
-                            : (xchk ? k_hamming_umma<false, true> : knn2 ? k_hamming_umma<true, false> : k_hamming_umma<false, false>);
-        kernel<<<grd, MT_THREADS, smem, st>>>(d_q, nq, d_t, nt, stride_rows, d_counts, nsets, rows_per_split, d_best, d_second, keys, d_status,
-                                              col_keys);
-    }
+    const MatchKernel kernel = match_kernel(job.op, pair, pairwise, job.k);
+    kernel<<<grd, MT_THREADS, match_smem(job.op), st>>>(a);
     ++c->launches;
     if (nsplit > 1) {
-        if (pairwise) k_match_finalize_pw<<<(unsigned)((nout + 255) / 256), 256, 0, st>>>(keys, nq, d_qcounts, nout, d_best);
-        else          k_match_finalize<<<(unsigned)((nout + 255) / 256), 256, 0, st>>>(keys, nq, nout, d_best);
+        k_match_finalize<<<(unsigned)((nout + 255) / 256), 256, 0, st>>>(a.keys, nq, job.query_counts, nout, job.best);
         ++c->launches;
     }
     if (xchk) {                                              // reads the finalised row winners
-        if (pairwise) k_crosscheck_compact_pw<<<(unsigned)nsets, XC_NT, 0, st>>>(d_best, nq, d_qcounts, col_keys, stride_rows, d_best, d_xc_count);
-        else          k_crosscheck_compact<<<(unsigned)nsets, XC_NT, 0, st>>>(d_best, nq, col_keys, stride_rows, d_best, d_xc_count);
+        k_crosscheck_compact<<<(unsigned)nsets, XC_NT, 0, st>>>(job.best, nq, job.query_counts, a.col_keys, job.train_stride, job.best,
+                                                               job.xc_count);
         ++c->launches;
     }
-    if (!lane_call) { stage_mark(c, 8); if (c->profiling) c->stage_valid[6] = true; }
+    if (!job.lane) { stage_mark(c, 8); if (c->profiling) c->stage_valid[6] = true; }
     CU(cudaGetLastError());
     return ORBX_OK;
 }
 
 // The host-buffer matcher, synchronous on the context's stream: nq query rows against nsets train sets of stride_rows rows
-// each (all of them, or as many as the host `counts` give per set).  best and second (when not null) receive [nsets][nq]
-// records each; with `pairs` (the second-best of one set), `best` receives [nq][2] {best, second} records instead.
-// With `xc_count` (cross-check of one set), `best` receives the mutual pairs and *xc_count their number.
-// With knn_k (top-k, k >= 2), `best` receives [nsets][nq][knn_k] records.
-int match_host(orbx_ctx* c, const uint8_t* query, int nq, const uint8_t* train, int stride_rows, const int* counts, int nsets,
-               orbx_match* best, orbx_match* second, bool pairs, int* xc_count = nullptr, int knn_k = 0)
+// each (all of them, or as many as the host `counts` give per set).  Best: `best` receives [nsets][nq] records.  Knn2: best
+// and `second` the same, or without `second` (one set) `best` receives [nq][2] {best, second} records.  TopK: `best` receives
+// [nsets][nq][k] records.  CrossCheck (one set): `best` receives the mutual pairs and *xc_count their number.
+int match_host(orbx_ctx* c, MatchOp op, const uint8_t* query, int nq, const uint8_t* train, int stride_rows, const int* counts, int nsets,
+               orbx_match* best, orbx_match* second = nullptr, int* xc_count = nullptr, int k = 0)
 {
-    const size_t tbytes = (size_t)nsets * stride_rows * 32, obytes = (size_t)nsets * nq * 16 * (size_t)std::max(1, knn_k);
-    const bool knn2 = pairs || second;
+    const size_t tbytes = (size_t)nsets * stride_rows * 32, obytes = (size_t)nsets * nq * 16 * (size_t)(op == MatchOp::TopK ? k : 1);
+    const bool knn2 = op == MatchOp::Knn2, pairs = knn2 && !second;
     int rc;
     if ((rc = ensure(c, c->mq, (size_t)nq * 32)) || (rc = ensure(c, c->mt, tbytes)) || (rc = ensure(c, c->mbest, obytes)) ||
         (knn2 && (rc = ensure(c, c->msecond, obytes))) || (counts && (rc = ensure(c, c->mcounts, sizeof(int) * (size_t)nsets))) ||
@@ -772,10 +793,10 @@ int match_host(orbx_ctx* c, const uint8_t* query, int nq, const uint8_t* train, 
     CU(cudaMemcpyAsync(c->mq.p, query, (size_t)nq * 32, cudaMemcpyHostToDevice, c->stream));
     CU(cudaMemcpyAsync(c->mt.p, train, tbytes, cudaMemcpyHostToDevice, c->stream));
     if (counts) CU(cudaMemcpyAsync(c->mcounts.p, counts, sizeof(int) * (size_t)nsets, cudaMemcpyHostToDevice, c->stream));
-    if ((rc = run_match(c, (const uint8_t*)c->mq.p, nq, (const uint8_t*)c->mt.p, stride_rows, stride_rows, counts ? (const int*)c->mcounts.p : nullptr,
-                        nsets, (int4*)c->mbest.p, knn2 ? (int4*)c->msecond.p : nullptr, nullptr, 0, xc_count ? (int*)c->mxcount.p : nullptr,
-                        nullptr, knn_k)))
-        return rc;
+    MatchJob job = match_job(op, (const uint8_t*)c->mq.p, nq, (const uint8_t*)c->mt.p, stride_rows, counts ? (const int*)c->mcounts.p : nullptr,
+                             nsets, c->mbest.p);
+    job.second = knn2 ? (int4*)c->msecond.p : nullptr; job.xc_count = xc_count ? (int*)c->mxcount.p : nullptr; job.k = k;
+    if ((rc = run_match(c, job))) return rc;
     if (xc_count) CU(cudaMemcpyAsync(xc_count, c->mxcount.p, sizeof(int) * (size_t)nsets, cudaMemcpyDeviceToHost, c->stream));
     if (pairs) {
         CU(cudaMemcpy2DAsync(best, 32, c->mbest.p, 16, 16, (size_t)nq, cudaMemcpyDeviceToHost, c->stream));
@@ -797,49 +818,49 @@ int match_one_set(orbx_ctx* c, const uint8_t* query, int nq, const uint8_t* trai
     if (nq == 0 || nt == 0) return ORBX_OK;                 // cv: empty query or train -> no matches, no throw
     if (!query || !train || !out) return fail(c, ORBX_E_ARG, "null pointer");
     CU(cudaSetDevice(c->device));
-    const int rc = match_host(c, query, nq, train, nt, nullptr, 1, out, nullptr, k == 2, nullptr, k > 2 ? k : 0);
+    const MatchOp op = k == 1 ? MatchOp::Best : k == 2 ? MatchOp::Knn2 : MatchOp::TopK;
+    const int rc = match_host(c, op, query, nq, train, nt, nullptr, 1, out, nullptr, nullptr, k);
     if (rc) return rc;
     if (n_out) *n_out = nq;
     return ORBX_OK;
 }
 
-// radiusMatch, first half: list L = set * nq + query row (run_match's operands; d_qcounts: pairwise).  The count pass writes
-// every list's length to d_offsets[1 + L], and the scan turns d_offsets[0 .. nsets * nq] into the 64-bit CSR offsets.
-// Asynchronous on the context's stream.
-int radius_count(orbx_ctx* c, const uint8_t* d_q, int nq, const uint8_t* d_t, int stride_rows, const int* d_counts, int nsets,
-                 const int* d_qcounts, int thr, long long* d_offsets)
+// One pass of radiusMatch (job.op RadiusCount or RadiusEmit, rad_thr and rad_offsets set), list L = set * nq + query row,
+// asynchronous on the context's stream.  The count pass writes every list's length to rad_offsets[1 + L], and the scan turns
+// rad_offsets[0 .. nsets * nq] into the 64-bit CSR offsets.  The emit pass (behind it) writes every list that ends at or below
+// rad_cap to job.best in ascending trainIdx, and k_radius_order puts each into std::sort's order.
+int radius_pass(orbx_ctx* c, const MatchJob& job)
 {
-    const long long nlists = (long long)nsets * nq;
-    const long long ntiles = (nlists + RS_SCAN_TILE - 1) / RS_SCAN_TILE;
+    const long long nlists = (long long)job.nsets * job.nq;
+    long long* d_offsets = job.rad_offsets;
     int rc;
-    if ((rc = ensure(c, c->mradsums, sizeof(long long) * (size_t)ntiles))) return rc;
-    CU(cudaMemsetAsync(d_offsets, 0, sizeof(long long) * (size_t)(nlists + 1), c->stream));   // (pairwise: rows past a count stay 0)
-    const RadiusPass count{1, thr, d_offsets, 0};
-    if ((rc = run_match(c, d_q, nq, d_t, stride_rows, stride_rows, d_counts, nsets, nullptr, nullptr, nullptr, 0, nullptr, d_qcounts, 0, &count)))
-        return rc;
-    long long* sums = (long long*)c->mradsums.p;
-    k_radius_tile_sums<<<(unsigned)ntiles, RS_SCAN_NT, 0, c->stream>>>(d_offsets + 1, nlists, sums);
-    k_radius_scan_sums<<<1, RS_SCAN_NT, 0, c->stream>>>(sums, ntiles);
-    k_radius_scan_tiles<<<(unsigned)ntiles, RS_SCAN_NT, 0, c->stream>>>(d_offsets + 1, nlists, sums);
-    c->launches += 3;
+    if (job.op == MatchOp::RadiusCount) {
+        const long long ntiles = (nlists + RS_SCAN_TILE - 1) / RS_SCAN_TILE;
+        if ((rc = ensure(c, c->mradsums, sizeof(long long) * (size_t)ntiles))) return rc;
+        CU(cudaMemsetAsync(d_offsets, 0, sizeof(long long) * (size_t)(nlists + 1), c->stream));   // (pairwise: rows past a count stay 0)
+        if ((rc = run_match(c, job))) return rc;
+        long long* sums = (long long*)c->mradsums.p;
+        k_radius_tile_sums<<<(unsigned)ntiles, RS_SCAN_NT, 0, c->stream>>>(d_offsets + 1, nlists, sums);
+        k_radius_scan_sums<<<1, RS_SCAN_NT, 0, c->stream>>>(sums, ntiles);
+        k_radius_scan_tiles<<<(unsigned)ntiles, RS_SCAN_NT, 0, c->stream>>>(d_offsets + 1, nlists, sums);
+        c->launches += 3;
+    } else {
+        if ((rc = run_match(c, job))) return rc;
+        k_radius_order<<<(unsigned)((nlists + RS_WARPS - 1) / RS_WARPS), RS_WARPS * 32, 0, c->stream>>>(job.best, d_offsets, nlists, job.nq,
+                                                                                                        job.rad_cap);
+        ++c->launches;
+    }
     CU(cudaGetLastError());
     return ORBX_OK;
 }
 
-// radiusMatch, second half (behind radius_count on the context's stream): the emit pass writes every list that ends at or
-// below cap to d_out in ascending trainIdx, and k_radius_order puts each into std::sort's order.
-int radius_emit(orbx_ctx* c, const uint8_t* d_q, int nq, const uint8_t* d_t, int stride_rows, const int* d_counts, int nsets,
-                const int* d_qcounts, int thr, long long* d_offsets, int4* d_out, long long cap)
+// Both passes of radiusMatch on a job, the count's results on the device
+int radius_match(orbx_ctx* c, MatchJob job)
 {
-    const long long nlists = (long long)nsets * nq;
-    const RadiusPass emit{2, thr, d_offsets, cap};
-    int rc;
-    if ((rc = run_match(c, d_q, nq, d_t, stride_rows, stride_rows, d_counts, nsets, d_out, nullptr, nullptr, 0, nullptr, d_qcounts, 0, &emit)))
-        return rc;
-    k_radius_order<<<(unsigned)((nlists + RS_WARPS - 1) / RS_WARPS), RS_WARPS * 32, 0, c->stream>>>(d_out, d_offsets, nlists, nq, cap);
-    ++c->launches;
-    CU(cudaGetLastError());
-    return ORBX_OK;
+    job.op = MatchOp::RadiusCount;
+    const int rc = radius_pass(c, job);
+    job.op = MatchOp::RadiusEmit;
+    return rc ? rc : radius_pass(c, job);
 }
 
 // The matcher's threshold of the integer radius R = min(256, floor(max_distance)): distance <= R <=> accumulator >= thr
@@ -908,30 +929,7 @@ int orbx_create(orbx_ctx** out, int device, int nfeatures, float scale_factor, i
         if (cudaMemcpy(c->pattern.p, pat, sizeof pat, cudaMemcpyHostToDevice) != cudaSuccess) return ORBX_E_CUDA;
     }
     if (cudaMemset(c->status.p, 0, sizeof(int) * B) != cudaSuccess) return ORBX_E_CUDA;
-    if (cudaFuncSetAttribute(k_hamming_umma2<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
-        cudaFuncSetAttribute(k_hamming_umma2<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
-        cudaFuncSetAttribute(k_hamming_umma<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
-        cudaFuncSetAttribute(k_hamming_umma<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
-        cudaFuncSetAttribute(k_hamming_umma2<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES_XC) != cudaSuccess ||
-        cudaFuncSetAttribute(k_hamming_umma<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES_XC) != cudaSuccess ||
-        cudaFuncSetAttribute(k_hamming_umma2_pw<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
-        cudaFuncSetAttribute(k_hamming_umma2_pw<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
-        cudaFuncSetAttribute(k_hamming_umma_pw<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
-        cudaFuncSetAttribute(k_hamming_umma_pw<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
-        cudaFuncSetAttribute(k_hamming_umma2_pw<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES_XC) != cudaSuccess ||
-        cudaFuncSetAttribute(k_hamming_umma_pw<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES_XC) != cudaSuccess ||
-        cudaFuncSetAttribute(k_hamming_umma_topk<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
-        cudaFuncSetAttribute(k_hamming_umma_topk<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
-        cudaFuncSetAttribute(k_hamming_umma_topk<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
-        cudaFuncSetAttribute(k_hamming_umma_topk<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
-        cudaFuncSetAttribute(k_hamming_umma_pw_topk<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
-        cudaFuncSetAttribute(k_hamming_umma_pw_topk<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
-        cudaFuncSetAttribute(k_hamming_umma_pw_topk<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
-        cudaFuncSetAttribute(k_hamming_umma_pw_topk<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
-        cudaFuncSetAttribute(k_hamming_umma_radius<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
-        cudaFuncSetAttribute(k_hamming_umma_radius<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
-        cudaFuncSetAttribute(k_hamming_umma_pw_radius<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
-        cudaFuncSetAttribute(k_hamming_umma_pw_radius<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_BYTES) != cudaSuccess ||
+    if (!match_kernels_allow_smem() ||
         cudaFuncSetAttribute(k_fast_warp<FAST_NWARP>, cudaFuncAttributeMaxDynamicSharedMemorySize, FAST_NWARP * FW_WARP_BYTES + 128) != cudaSuccess ||
         cudaFuncSetAttribute(k_pyr_tma, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024) != cudaSuccess ||
         cudaFuncSetAttribute(k_describe_tma, cudaFuncAttributeMaxDynamicSharedMemorySize, DS_NW * DS_WARP_BYTES + 128) != cudaSuccess ||
@@ -1084,9 +1082,10 @@ static int host_batch(orbx_ctx* c, const uint8_t* const* imgs, int batch, int w,
             if (nq[j] > 0) {
                 int4* d_best = (int4*)c->mbest.p + moff + (size_t)f0 * nq[j];
                 // train sets = this lane's frames, straight from the extraction outputs ([frame][cap][32] + counts)
-                if ((rc = run_match(c, (const uint8_t*)c->mq.p + qoff * 32, nq[j], (const uint8_t*)c->desc.p + (size_t)f0 * cap * 32, cap, cap,
-                                    (const int*)c->counts.p + f0, (int)n, d_best, nullptr, st, k)))
-                    return rc;
+                MatchJob job = match_job(MatchOp::Best, (const uint8_t*)c->mq.p + qoff * 32, nq[j], (const uint8_t*)c->desc.p + (size_t)f0 * cap * 32,
+                                         cap, (const int*)c->counts.p + f0, (int)n, d_best);
+                job.lane = true; job.lane_stream = st; job.lane_slot = k;
+                if ((rc = run_match(c, job))) return rc;
                 orbx_match* dl = stage_out ? (orbx_match*)(c->h_stage_out.p + o_best) + moff + (size_t)f0 * nq[j] : best[j] + (size_t)f0 * nq[j];
                 CU(cudaMemcpyAsync(dl, d_best, (size_t)16 * nq[j] * n, cudaMemcpyDeviceToHost, st));
             }
@@ -1222,29 +1221,48 @@ int orbx_match_hamming_device(orbx_ctx* c, const uint8_t* d_query, int nq, const
     if (nq == 0 || nt == 0 || nsets == 0) return ORBX_OK;
     if (!d_query || !d_train || !d_best) return fail(c, ORBX_E_ARG, "null pointer");
     CU(cudaSetDevice(c->device));
-    return run_match(c, d_query, nq, d_train, nt, nt, nullptr, nsets, (int4*)d_best, (int4*)d_second);
+    MatchJob job = match_job(d_second ? MatchOp::Knn2 : MatchOp::Best, d_query, nq, d_train, nt, nullptr, nsets, d_best);
+    job.second = (int4*)d_second;
+    return run_match(c, job);
+}
+
+// Argument checks of the shared-query ragged family (_device_ragged, _sets, _device_crosscheck, _device_knn, _device_radius):
+// nq query rows against nsets train sets of train_stride_rows rows.  In order: the sizes and the caller's other invalid
+// arguments (`bad`) -> E_ARG; the caller's unsupported case (`unsupported`: its message, or null) -> E_UNSUPPORTED; the
+// pointers -> E_ARG.  With `empty`, an empty input (no query row, train row or set) is reported there, before the pointers
+// are checked; without it the pointers are checked whatever the sizes.
+static int check_args_ragged(orbx_ctx* c, const void* query, int nq, const void* train, int train_stride_rows, const int* train_counts,
+                             int nsets, const void* out, bool bad, const char* unsupported, bool* empty)
+{
+    if (bad || nq < 0 || train_stride_rows < 0 || nsets < 0 || nsets > 65535) return fail(c, ORBX_E_ARG, "bad sizes");
+    if (unsupported) return fail(c, ORBX_E_UNSUPPORTED, unsupported);
+    if (empty && (*empty = nq == 0 || train_stride_rows == 0 || nsets == 0)) return ORBX_OK;
+    if (!query || !train || !train_counts || !out) return fail(c, ORBX_E_ARG, "null pointer");
+    return ORBX_OK;
 }
 
 int orbx_match_hamming_device_ragged(orbx_ctx* c, const uint8_t* d_query, int nq, const uint8_t* d_train, int train_stride_rows,
                                      const int* d_train_counts, int nsets, orbx_match* d_best, orbx_match* d_second)
 {
     if (!c) return ORBX_E_ARG;
-    if (nq < 0 || train_stride_rows < 0 || nsets < 0 || nsets > 65535) return fail(c, ORBX_E_ARG, "bad sizes");
-    if (nq == 0 || train_stride_rows == 0 || nsets == 0) return ORBX_OK;
-    if (!d_query || !d_train || !d_best || !d_train_counts) return fail(c, ORBX_E_ARG, "null pointer");
+    bool empty;
+    const int rc = check_args_ragged(c, d_query, nq, d_train, train_stride_rows, d_train_counts, nsets, d_best, false, nullptr, &empty);
+    if (rc || empty) return rc;
     CU(cudaSetDevice(c->device));
-    return run_match(c, d_query, nq, d_train, train_stride_rows, train_stride_rows, d_train_counts, nsets, (int4*)d_best, (int4*)d_second);
+    MatchJob job = match_job(d_second ? MatchOp::Knn2 : MatchOp::Best, d_query, nq, d_train, train_stride_rows, d_train_counts, nsets, d_best);
+    job.second = (int4*)d_second;
+    return run_match(c, job);
 }
 
 int orbx_match_hamming_sets(orbx_ctx* c, const uint8_t* query, int nq, const uint8_t* train, int train_stride_rows,
                             const int* train_counts, int nsets, orbx_match* best, orbx_match* second)
 {
     if (!c) return ORBX_E_ARG;
-    if (nq < 0 || train_stride_rows < 0 || nsets < 0 || nsets > 65535) return fail(c, ORBX_E_ARG, "bad sizes");
-    if (nq == 0 || train_stride_rows == 0 || nsets == 0) return ORBX_OK;
-    if (!query || !train || !best || !train_counts) return fail(c, ORBX_E_ARG, "null pointer");
+    bool empty;
+    const int rc = check_args_ragged(c, query, nq, train, train_stride_rows, train_counts, nsets, best, false, nullptr, &empty);
+    if (rc || empty) return rc;
     CU(cudaSetDevice(c->device));
-    return match_host(c, query, nq, train, train_stride_rows, train_counts, nsets, best, second, false);
+    return match_host(c, second ? MatchOp::Knn2 : MatchOp::Best, query, nq, train, train_stride_rows, train_counts, nsets, best, second);
 }
 
 int orbx_match_hamming_crosscheck(orbx_ctx* c, const uint8_t* q, int nq, const uint8_t* t, int nt, orbx_match* out, int* n_out)
@@ -1258,7 +1276,7 @@ int orbx_match_hamming_crosscheck(orbx_ctx* c, const uint8_t* q, int nq, const u
     if (!q || !t || !out) return fail(c, ORBX_E_ARG, "null pointer");
     CU(cudaSetDevice(c->device));
     int n = 0;
-    const int rc = match_host(c, q, nq, t, nt, nullptr, 1, out, nullptr, false, &n);
+    const int rc = match_host(c, MatchOp::CrossCheck, q, nq, t, nt, nullptr, 1, out, nullptr, &n);
     if (rc) return rc;
     *n_out = n;
     return ORBX_OK;
@@ -1268,34 +1286,38 @@ int orbx_match_hamming_device_crosscheck(orbx_ctx* c, const uint8_t* d_query, in
                                          const int* d_train_counts, int nsets, orbx_match* d_out, int* d_n_out)
 {
     if (!c) return ORBX_E_ARG;
-    if (nq < 0 || train_stride_rows < 0 || nsets < 0 || nsets > 65535) return fail(c, ORBX_E_ARG, "bad sizes");
-    if (nq >= MT_MAX_QUERY_XC) return fail(c, ORBX_E_UNSUPPORTED, "cross-check query set larger than 2^20 - 1 rows");
-    if (nsets == 0) return ORBX_OK;
+    bool empty;
+    const int rc = check_args_ragged(c, d_query, nq, d_train, train_stride_rows, d_train_counts, nsets, d_out, false,
+                                     nq >= MT_MAX_QUERY_XC ? "cross-check query set larger than 2^20 - 1 rows" : nullptr, &empty);
+    if (rc || nsets == 0) return rc;
     if (!d_n_out) return fail(c, ORBX_E_ARG, "null pointer");
     CU(cudaSetDevice(c->device));
-    if (nq == 0 || train_stride_rows == 0) {                 // no pairs in any set
+    if (empty) {                                             // no pairs in any set
         CU(cudaMemsetAsync(d_n_out, 0, sizeof(int) * (size_t)nsets, c->stream));
         return ORBX_OK;
     }
-    if (!d_query || !d_train || !d_out || !d_train_counts) return fail(c, ORBX_E_ARG, "null pointer");
-    return run_match(c, d_query, nq, d_train, train_stride_rows, train_stride_rows, d_train_counts, nsets, (int4*)d_out, nullptr, nullptr, 0, d_n_out);
+    MatchJob job = match_job(MatchOp::CrossCheck, d_query, nq, d_train, train_stride_rows, d_train_counts, nsets, d_out);
+    job.xc_count = d_n_out;
+    return run_match(c, job);
 }
 
 int orbx_match_hamming_device_knn(orbx_ctx* c, const uint8_t* d_query, int nq, const uint8_t* d_train, int train_stride_rows,
                                   const int* d_train_counts, int nsets, int k, orbx_match* d_out)
 {
     if (!c) return ORBX_E_ARG;
-    if (nq < 0 || train_stride_rows < 0 || nsets < 0 || nsets > 65535 || k < 1) return fail(c, ORBX_E_ARG, "bad sizes");
-    if (k > ORBX_MAX_KNN) return fail(c, ORBX_E_UNSUPPORTED, "k larger than ORBX_MAX_KNN");
-    if (nq == 0 || train_stride_rows == 0 || nsets == 0) return ORBX_OK;
-    if (!d_query || !d_train || !d_out || !d_train_counts) return fail(c, ORBX_E_ARG, "null pointer");
+    bool empty;
+    const int rc = check_args_ragged(c, d_query, nq, d_train, train_stride_rows, d_train_counts, nsets, d_out, k < 1,
+                                     k > ORBX_MAX_KNN ? "k larger than ORBX_MAX_KNN" : nullptr, &empty);
+    if (rc || empty) return rc;
     CU(cudaSetDevice(c->device));
     // k = 1: the plain matcher's [nsets][nq] records are the [nsets][nq][1] layout
-    return run_match(c, d_query, nq, d_train, train_stride_rows, train_stride_rows, d_train_counts, nsets, (int4*)d_out, nullptr, nullptr, 0,
-                     nullptr, nullptr, k > 1 ? k : 0);
+    MatchJob job = match_job(k > 1 ? MatchOp::TopK : MatchOp::Best, d_query, nq, d_train, train_stride_rows, d_train_counts, nsets, d_out);
+    job.k = k > 1 ? k : 0;
+    return run_match(c, job);
 }
 
-// orbx_match_hamming_device_pairwise[_crosscheck|_knn]: pair p = query set p against train set p.  Argument checks common to all.
+// orbx_match_hamming_device_pairwise[_crosscheck|_knn|_radius]: pair p = query set p against train set p.  Argument checks
+// common to all.
 static int check_args_pairwise(orbx_ctx* c, const uint8_t* d_query, int query_stride_rows, const int* d_query_counts, const uint8_t* d_train,
                                int train_stride_rows, const int* d_train_counts, int npairs, const void* d_out)
 {
@@ -1315,8 +1337,10 @@ int orbx_match_hamming_device_pairwise(orbx_ctx* c, const uint8_t* d_query, int 
     if (rc) return rc;
     if (npairs == 0 || query_stride_rows == 0 || train_stride_rows == 0) return ORBX_OK;
     CU(cudaSetDevice(c->device));
-    return run_match(c, d_query, query_stride_rows, d_train, train_stride_rows, train_stride_rows, d_train_counts, npairs, (int4*)d_best,
-                     (int4*)d_second, nullptr, 0, nullptr, d_query_counts);
+    MatchJob job = match_job(d_second ? MatchOp::Knn2 : MatchOp::Best, d_query, query_stride_rows, d_train, train_stride_rows, d_train_counts, npairs, d_best);
+    job.query_counts = d_query_counts;
+    job.second = (int4*)d_second;
+    return run_match(c, job);
 }
 
 int orbx_match_hamming_device_pairwise_crosscheck(orbx_ctx* c, const uint8_t* d_query, int query_stride_rows, const int* d_query_counts,
@@ -1333,8 +1357,10 @@ int orbx_match_hamming_device_pairwise_crosscheck(orbx_ctx* c, const uint8_t* d_
         CU(cudaMemsetAsync(d_n_out, 0, sizeof(int) * (size_t)npairs, c->stream));
         return ORBX_OK;
     }
-    return run_match(c, d_query, query_stride_rows, d_train, train_stride_rows, train_stride_rows, d_train_counts, npairs, (int4*)d_out, nullptr,
-                     nullptr, 0, d_n_out, d_query_counts);
+    MatchJob job = match_job(MatchOp::CrossCheck, d_query, query_stride_rows, d_train, train_stride_rows, d_train_counts, npairs, d_out);
+    job.query_counts = d_query_counts;
+    job.xc_count = d_n_out;
+    return run_match(c, job);
 }
 
 int orbx_match_hamming_device_pairwise_knn(orbx_ctx* c, const uint8_t* d_query, int query_stride_rows, const int* d_query_counts,
@@ -1348,8 +1374,10 @@ int orbx_match_hamming_device_pairwise_knn(orbx_ctx* c, const uint8_t* d_query, 
     if (k > ORBX_MAX_KNN) return fail(c, ORBX_E_UNSUPPORTED, "k larger than ORBX_MAX_KNN");
     if (npairs == 0 || query_stride_rows == 0 || train_stride_rows == 0) return ORBX_OK;
     CU(cudaSetDevice(c->device));
-    return run_match(c, d_query, query_stride_rows, d_train, train_stride_rows, train_stride_rows, d_train_counts, npairs, (int4*)d_out,
-                     nullptr, nullptr, 0, nullptr, d_query_counts, k > 1 ? k : 0);
+    MatchJob job = match_job(k > 1 ? MatchOp::TopK : MatchOp::Best, d_query, query_stride_rows, d_train, train_stride_rows, d_train_counts, npairs, d_out);
+    job.query_counts = d_query_counts;
+    job.k = k > 1 ? k : 0;
+    return run_match(c, job);
 }
 
 int orbx_match_hamming_radius(orbx_ctx* c, const uint8_t* q, int nq, const uint8_t* t, int nt, float max_distance, orbx_match* out, int cap,
@@ -1367,7 +1395,6 @@ int orbx_match_hamming_radius(orbx_ctx* c, const uint8_t* q, int nq, const uint8
     }
     if (!q || !t || !out) return fail(c, ORBX_E_ARG, "null pointer");
     CU(cudaSetDevice(c->device));
-    const int thr = radius_threshold(max_distance);
     int rc;
     if ((rc = ensure(c, c->mq, (size_t)nq * 32)) || (rc = ensure(c, c->mt, (size_t)nt * 32)) ||
         (rc = ensure(c, c->mradoff, sizeof(long long) * ((size_t)nq + 1))))
@@ -1375,7 +1402,9 @@ int orbx_match_hamming_radius(orbx_ctx* c, const uint8_t* q, int nq, const uint8
     long long* d_off = (long long*)c->mradoff.p;
     CU(cudaMemcpyAsync(c->mq.p, q, (size_t)nq * 32, cudaMemcpyHostToDevice, c->stream));
     CU(cudaMemcpyAsync(c->mt.p, t, (size_t)nt * 32, cudaMemcpyHostToDevice, c->stream));
-    if ((rc = radius_count(c, (const uint8_t*)c->mq.p, nq, (const uint8_t*)c->mt.p, nt, nullptr, 1, nullptr, thr, d_off))) return rc;
+    MatchJob job = match_job(MatchOp::RadiusCount, (const uint8_t*)c->mq.p, nq, (const uint8_t*)c->mt.p, nt, nullptr, 1, nullptr);
+    job.rad_thr = radius_threshold(max_distance); job.rad_offsets = d_off;
+    if ((rc = radius_pass(c, job))) return rc;
     long long total = 0;
     CU(cudaMemcpyAsync(&total, d_off + nq, sizeof total, cudaMemcpyDeviceToHost, c->stream));
     if ((rc = sync_match_words(c, 0, 1))) return rc;
@@ -1383,8 +1412,8 @@ int orbx_match_hamming_radius(orbx_ctx* c, const uint8_t* q, int nq, const uint8
     *n_out = (int)total;
     if (total > cap) return fail(c, ORBX_E_CAPACITY, "output capacity below the number of records");
     if ((rc = ensure(c, c->mbest, 16 * (size_t)total))) return rc;
-    if ((rc = radius_emit(c, (const uint8_t*)c->mq.p, nq, (const uint8_t*)c->mt.p, nt, nullptr, 1, nullptr, thr, d_off, (int4*)c->mbest.p, total)))
-        return rc;
+    job.op = MatchOp::RadiusEmit; job.best = (int4*)c->mbest.p; job.rad_cap = total;
+    if ((rc = radius_pass(c, job))) return rc;
     CU(cudaMemcpyAsync(out, c->mbest.p, 16 * (size_t)total, cudaMemcpyDeviceToHost, c->stream));
     CU(cudaMemcpyAsync(offsets, d_off, sizeof(int64_t) * ((size_t)nq + 1), cudaMemcpyDeviceToHost, c->stream));
     return sync_match_words(c, 0, 1);
@@ -1394,19 +1423,19 @@ int orbx_match_hamming_device_radius(orbx_ctx* c, const uint8_t* d_query, int nq
                                      const int* d_train_counts, int nsets, float max_distance, orbx_match* d_out, int64_t cap, int64_t* d_offsets)
 {
     if (!c) return ORBX_E_ARG;
-    if (nq < 0 || train_stride_rows < 0 || nsets < 0 || nsets > 65535 || cap < 0) return fail(c, ORBX_E_ARG, "bad sizes");
+    const int rc = check_args_ragged(c, d_query, nq, d_train, train_stride_rows, d_train_counts, nsets, d_out, cap < 0, nullptr, nullptr);
+    if (rc) return rc;
     if (bad_radius(max_distance)) return fail(c, ORBX_E_ARG, "maxDistance must be larger than FLT_EPSILON");
-    if (!d_query || !d_train || !d_train_counts || !d_out || !d_offsets) return fail(c, ORBX_E_ARG, "null pointer");
+    if (!d_offsets) return fail(c, ORBX_E_ARG, "null pointer");
     if (train_stride_rows >= MT_MAX_TRAIN) return fail(c, ORBX_E_UNSUPPORTED, "train set stride of 2^20 rows or more");
     CU(cudaSetDevice(c->device));
-    long long* d_off = (long long*)d_offsets;
     if (nq == 0 || train_stride_rows == 0 || nsets == 0) {   // every list empty
-        CU(cudaMemsetAsync(d_off, 0, sizeof(int64_t) * ((size_t)nsets * nq + 1), c->stream));
+        CU(cudaMemsetAsync(d_offsets, 0, sizeof(int64_t) * ((size_t)nsets * nq + 1), c->stream));
         return ORBX_OK;
     }
-    const int thr = radius_threshold(max_distance);
-    const int rc = radius_count(c, d_query, nq, d_train, train_stride_rows, d_train_counts, nsets, nullptr, thr, d_off);
-    return rc ? rc : radius_emit(c, d_query, nq, d_train, train_stride_rows, d_train_counts, nsets, nullptr, thr, d_off, (int4*)d_out, cap);
+    MatchJob job = match_job(MatchOp::RadiusCount, d_query, nq, d_train, train_stride_rows, d_train_counts, nsets, d_out);
+    job.rad_thr = radius_threshold(max_distance); job.rad_offsets = (long long*)d_offsets; job.rad_cap = cap;
+    return radius_match(c, job);
 }
 
 int orbx_match_hamming_device_pairwise_radius(orbx_ctx* c, const uint8_t* d_query, int query_stride_rows, const int* d_query_counts,
@@ -1420,15 +1449,14 @@ int orbx_match_hamming_device_pairwise_radius(orbx_ctx* c, const uint8_t* d_quer
     int rc = check_args_pairwise(c, d_query, query_stride_rows, d_query_counts, d_train, train_stride_rows, d_train_counts, npairs, d_out);
     if (rc) return rc;
     CU(cudaSetDevice(c->device));
-    long long* d_off = (long long*)d_offsets;
     if (npairs == 0 || query_stride_rows == 0 || train_stride_rows == 0) {   // every list empty
-        CU(cudaMemsetAsync(d_off, 0, sizeof(int64_t) * ((size_t)npairs * query_stride_rows + 1), c->stream));
+        CU(cudaMemsetAsync(d_offsets, 0, sizeof(int64_t) * ((size_t)npairs * query_stride_rows + 1), c->stream));
         return ORBX_OK;
     }
-    const int thr = radius_threshold(max_distance);
-    rc = radius_count(c, d_query, query_stride_rows, d_train, train_stride_rows, d_train_counts, npairs, d_query_counts, thr, d_off);
-    return rc ? rc : radius_emit(c, d_query, query_stride_rows, d_train, train_stride_rows, d_train_counts, npairs, d_query_counts, thr, d_off,
-                                 (int4*)d_out, cap);
+    MatchJob job = match_job(MatchOp::RadiusCount, d_query, query_stride_rows, d_train, train_stride_rows, d_train_counts, npairs, d_out);
+    job.query_counts = d_query_counts;
+    job.rad_thr = radius_threshold(max_distance); job.rad_offsets = (long long*)d_offsets; job.rad_cap = cap;
+    return radius_match(c, job);
 }
 
 int orbx_filter_matches(orbx_match* m, int n, float ratio)
@@ -1713,7 +1741,7 @@ int orbx_track_match(orbx_ctx* c, const int64_t* ids, int m, const double* pose_
     // train set: host rows, or frame `nt_or_frame` of the last host-API extraction (still on the device)
     const uint8_t* d_train = nullptr;
     const int* d_tcount = nullptr;
-    int nt = 0, stride = 0;
+    int nt = 0;
     int rc;
     if (train) {
         nt = nt_or_frame;
@@ -1723,13 +1751,12 @@ int orbx_track_match(orbx_ctx* c, const int64_t* ids, int m, const double* pose_
             CU(cudaMemcpyAsync(c->mt.p, train, (size_t)nt * 32, cudaMemcpyHostToDevice, c->stream));
             d_train = (const uint8_t*)c->mt.p;
         }
-        stride = nt;
     } else {
         const int f = nt_or_frame;
         if (!c->view_desc || c->out_cap <= 0 || f < 0 || f >= c->view_frames) return fail(c, ORBX_E_ARG, "no host-API extraction holds that frame");
         d_train = c->view_desc + (size_t)f * c->out_cap * 32;
         d_tcount = c->view_counts + f;
-        nt = stride = c->out_cap;
+        nt = c->out_cap;
     }
     std::vector<int> slots;
     if ((rc = map_slots(c, ids, m, false, &slots))) return rc;
@@ -1752,7 +1779,8 @@ int orbx_track_match(orbx_ctx* c, const int64_t* ids, int m, const double* pose_
     k_gather_desc<<<(unsigned)((nc + 255) / 256), 256, 0, c->stream>>>((const int*)c->t_slots.p, (const int*)c->t_cand.p, nc, (const uint8_t*)c->t_desc.p,
                                                                        (uint8_t*)c->t_q.p);
     ++c->launches;
-    if ((rc = run_match(c, (const uint8_t*)c->t_q.p, nc, d_train, nt, stride, d_tcount, 1, (int4*)c->t_best.p, nullptr))) return rc;
+    const MatchJob job = match_job(MatchOp::Best, (const uint8_t*)c->t_q.p, nc, d_train, nt, d_tcount, 1, c->t_best.p);
+    if ((rc = run_match(c, job))) return rc;
     k_filter_matches<<<1, VIS_NT, 0, c->stream>>>((const int4*)c->t_best.p, nc, match_ratio, (int4*)c->t_filtered.p, (int*)c->t_ncand.p + 1,
                                                   (float*)c->t_minmax.p);
     ++c->launches;

@@ -32,9 +32,10 @@
 // Pairwise batches (SETQ: query set s against train set s, e.g. frame i against frame i + 1) cannot keep one A operand
 // across sets, so there a CTA owns ONE (set, query tile) unit: gridDim.z = number of sets, the A tile is expanded at setup
 // as above, and CTAs whose query tile is empty for their set exit before any setup.  Few units keep the train-row split.
-// knnMatch for k > 2 (TOP-K, KB = list capacity 4 / 8 / 16 / 32): the single-CTA body, shared-query or pairwise, whose epilogue
+// One body serves every operation (MatchOp): match, knnMatch k = 2, cross-check, top-k and the two radius passes.
+// knnMatch for k > 2 (TopK, KB = list capacity 4 / 8 / 16 / 32): the single-CTA body, shared-query or pairwise, whose epilogue
 // keeps each query row's KB best keys in registers (see topk_tile); no CTA pair and no train-row split, as for knn2.
-// radiusMatch (RAD = 1 count, 2 emit): the same single-CTA body, whose epilogue counts, then writes, each query row's columns
+// radiusMatch (RadiusCount, RadiusEmit): the same single-CTA body, whose epilogue counts, then writes, each query row's columns
 // at or above the radius threshold (see radius_tile); orbx_radius.cuh scans the counts and orders the lists.
 #pragma once
 #include <cuda_runtime.h>
@@ -199,9 +200,6 @@ __device__ __forceinline__ void expand_half_row(uint8_t* tile, int rows, int r, 
     }
 }
 
-// KNN2 = false: best match only (cv match);  true: best and second best (cv knnMatch k = 2; needs nsplit == 1).
-// Outputs: if keys != nullptr (split mode) atomicMax of the packed key, finalised by k_match_finalize;
-//          else DMatch records are written directly.
 // Persistent over train sets: CTA (x = query tile, y = train-row split, z = set group) expands its 256 query rows
 // ONCE and then walks sets z, z + gridDim.z, ... with all three pipelines running continuously across set
 // boundaries (the map is shared by every frame, so the A operand never has to be rebuilt).
@@ -294,7 +292,67 @@ template <bool PAIR> __device__ __forceinline__ void umma_i8(uint32_t d, uint64_
 }
 template <bool PAIR> __device__ __forceinline__ void umma_commit(uint32_t bar) { if (PAIR) tc_commit2(bar); else tc_commit(bar); }
 
-// ---- cross-check (XCHK): column maxima from the same accumulators ----------------------------------------------------
+// ---- what one launch computes -----------------------------------------------------------------------------------------
+// The operations of the body.  Best, Knn2 and CrossCheck run on the single-CTA kernel and on the CTA pair; TopK and the
+// two radius passes on the single-CTA kernel alone, without a train-row split (as Knn2).
+enum class MatchOp : int {
+    Best,           // cv match: each query row's nearest train row per set
+    Knn2,           // cv knnMatch k = 2: best and second best
+    CrossCheck,     // Best, plus every train row's nearest query (column keys) for BFMatcher crossCheck = true
+    TopK,           // cv knnMatch for any k <= KB
+    RadiusCount,    // cv radiusMatch, first pass: every list's length
+    RadiusEmit,     // cv radiusMatch, second pass: the hits of every list that fits the output
+};
+__host__ __device__ constexpr bool match_op_pairs(MatchOp op) { return op == MatchOp::Best || op == MatchOp::Knn2 || op == MatchOp::CrossCheck; }
+
+// The kernel parameters of one launch.  Record outputs are [nsets][nq] (list L = set * nq + query row).
+struct MatchArgs {
+    const uint8_t* query;        // nq rows, shared by every set; pairwise (SETQ): set s's own rows at query + s * nq * 32
+    int nq;                      // query rows, or the query stride of a pairwise launch (and then the record pitch)
+    const int* query_counts;     // pairwise: set s holds min(query_counts[s], nq) query rows; null otherwise
+    const uint8_t* train;        // set s at train + s * train_stride_rows * 32
+    int nt, train_stride_rows;   // rows per set, stride between sets
+    const int* train_counts;     // ragged sets: set s holds min(train_counts[s], nt) rows; null: nt each
+    int nsets, rows_per_split;   // train-row split: CTA y takes rows [y * rows_per_split, (y + 1) * rows_per_split) of a set
+    int4* best;                  // records (TopK: [nsets][nq][knn_k]; RadiusEmit: the lists, at rad_offsets)
+    int4* second;                // Knn2: the second-best records
+    int* keys;                   // train-row split: packed row keys merged by atomicMax, made records by k_match_finalize
+    int* col_keys;               // CrossCheck: [nsets][train_stride_rows] column keys, INT_MIN-initialised, merged by atomicMax
+    int* status;                 // |= 2 when an mbarrier wait timed out
+    int knn_k;                   // TopK: k
+    int rad_thr;                 // radius: distance <= R  <=>  accumulator >= rad_thr = 127 * (256 - 2R)
+    long long* rad_offsets;      // RadiusCount: list L's length to rad_offsets[1 + L]; RadiusEmit: the scanned offsets
+    long long rad_cap;           // RadiusEmit: list L is written when rad_offsets[L + 1] <= rad_cap
+};
+
+// A DMatch record {queryIdx, trainIdx, imgIdx 0, distance = (256 - dot) / 2}
+__device__ __forceinline__ int4 match_record(int qrow, int dot, int j)
+{
+    return make_int4(qrow, j, 0, __float_as_int((float)((256 - dot) >> 1)));
+}
+// packed row key  dot << 20 | (0xFFFFF - j)  (plain maximum = largest dot, lowest train index)
+__device__ __forceinline__ int row_key(int dot, int j) { return dot * (1 << MT_KEY_SHIFT) + ((MT_MAX_TRAIN - 1) - j); }
+// row key -> its record; INT_MIN (no train row) -> trainIdx -1
+__device__ __forceinline__ int4 key_record(int qrow, int key)
+{
+    if (key == INT_MIN) return make_int4(qrow, -1, 0, 0);
+    return match_record(qrow, key >> MT_KEY_SHIFT, (MT_MAX_TRAIN - 1) - (key & (MT_MAX_TRAIN - 1)));
+}
+// An accumulator 127 * dot + code of the tile at train row j0 -> dot and the global train row.  The code is MT_BN - 1 minus
+// the row's place in the tile; in a CTA pair places 48 .. 95 are the peer's local rows, which hold tile rows N/2 .. N - 1
+// (N: the tile's UMMA N, from the set's end n1).
+struct AccRow { int dot, j; };
+template <bool PAIR>
+__device__ __forceinline__ AccRow acc_row(int v, int j0, int n1)
+{
+    const unsigned kk = (unsigned)(v + MT_ASCALE * 256);
+    const unsigned q = kk / (unsigned)MT_ASCALE;             // dot + 256
+    const int place = (MT_BN - 1) - (int)(kk - q * (unsigned)MT_ASCALE);
+    const int nh = ((min(MT_BN, n1 - j0) + 31) & ~31) >> 1;
+    return {(int)q - 256, j0 + (PAIR && place >= MT2_HALF ? nh + place - MT2_HALF : place)};
+}
+
+// ---- cross-check (CrossCheck): column maxima from the same accumulators ----------------------------------------------
 // Every column of a tile holds one train row, and all its values carry that row's code, so the column maximum of the
 // accumulator is the row's largest dot.  Widened to (v << 8) | (255 - row of the CTA), its plain maximum is "largest
 // dot, lowest query row".  One PRMT widens a packed half (the selector's msb replicates the sign of the selected byte).
@@ -322,7 +380,7 @@ __device__ __forceinline__ void xc_warp_columns(const uint32_t* rp, bool valid, 
 }
 __device__ __forceinline__ void xc_epilogue_sync() { asm volatile("bar.sync 1, 256;" ::: "memory"); }   // the 8 epilogue warps only
 
-// ---- top-k (KB > 0, BFMatcher knnMatch for any k <= KB): each epilogue thread keeps its query row's KB largest keys
+// ---- top-k (TopK, KB > 0, BFMatcher knnMatch for any k <= KB): each epilogue thread keeps its query row's KB largest keys
 // dot << 20 | (0xFFFFF - j) in registers, in descending order (INT_MIN = empty slot).  Keys are distinct per train row, so
 // the first k of them are exactly cv's k nearest by (distance, trainIdx).  A tile's columns are tested against the list's
 // last key in accumulator form (one compare per column; the whole tile is skipped when its packed maximum fails); only a
@@ -356,16 +414,14 @@ __device__ __forceinline__ void topk_tile(const uint32_t* rp, int tmax, int j0, 
         for (int h = 0; h < 2; ++h) {
             const int v = h ? (int)rp[u] >> 16 : (int)(rp[u] << 16) >> 16;
             if (v >= thr) {
-                const unsigned kk = (unsigned)(v + MT_ASCALE * 256);
-                const unsigned q = kk / (unsigned)MT_ASCALE;          // dot + 256
-                const int j = j0 + (MT_BN - 1) - (int)(kk - q * (unsigned)MT_ASCALE);
-                topk_insert<KB>(list, j < n1 ? ((int)q - 256) * (1 << MT_KEY_SHIFT) + ((MT_MAX_TRAIN - 1) - j) : INT_MIN);
+                const AccRow d = acc_row<false>(v, j0, n1);
+                topk_insert<KB>(list, d.j < n1 ? row_key(d.dot, d.j) : INT_MIN);
                 thr = topk_threshold(list[KB - 1], j0);
             }
         }
 }
 
-// ---- radius (RAD = 1 count pass, 2 emit pass; BFMatcher radiusMatch): distance h <= R  <=>  127 * dot + code >= thr =
+// ---- radius (RadiusCount and RadiusEmit passes; BFMatcher radiusMatch): distance h <= R  <=>  127 * dot + code >= thr =
 // 127 * (256 - 2R), because the index code is below 127.  A tile whose packed maximum is below thr has no hit.  Count: n
 // grows by the hits of train rows j < n1 (columns past the set's end are copies of its last row, with the same dot).  Emit
 // (out != nullptr): the hits are also written to out[n], in ascending train row, the row decoded from the column's code.
@@ -380,11 +436,9 @@ __device__ __forceinline__ void radius_tile(const uint32_t* rp, int tmax, int th
         for (int h = 0; h < 2; ++h) {
             const int v = h ? (int)rp[u] >> 16 : (int)(rp[u] << 16) >> 16;
             if (v >= thr) {
-                const unsigned kk = (unsigned)(v + MT_ASCALE * 256);
-                const unsigned q = kk / (unsigned)MT_ASCALE;          // dot + 256
-                const int j = j0 + (MT_BN - 1) - (int)(kk - q * (unsigned)MT_ASCALE);
-                if (j < n1) {
-                    if (EMIT && out) out[n] = make_int4(qrow, j, 0, __float_as_int((float)((512 - (int)q) >> 1)));
+                const AccRow d = acc_row<false>(v, j0, n1);
+                if (d.j < n1) {
+                    if (EMIT && out) out[n] = match_record(qrow, d.dot, d.j);
                     ++n;
                 }
             }
@@ -392,29 +446,59 @@ __device__ __forceinline__ void radius_tile(const uint32_t* rp, int tmax, int th
     }
 }
 
+// The packed accumulators of one tile (chunks past its UMMA N hold -32768) -> their maximum, after the operation's consumers
+// have seen the tile: the top-k list, the radius hits, the cross-check column maxima (xc_slots: this warp's).
+template <MatchOp OP, int KB>
+__device__ __forceinline__ int epilogue_tile(const uint32_t* rp, int j0, int n1, int qrow, int (&list)[KB > 0 ? KB : 1], int rad_thr,
+                                             int4* rad_out, int& rad_n, bool qvalid, int row_cta, int* xc_slots)
+{
+    unsigned p[8];                                           // eight independent max chains (ILP), then a short tree
+#pragma unroll
+    for (int u = 0; u < 8; ++u) {
+        p[u] = __vimax3_s16x2(rp[u], rp[8 + u], rp[16 + u]);
+        p[u] = __vimax3_s16x2(p[u], rp[24 + u], rp[32 + u]);
+        p[u] = __vmaxs2(p[u], rp[40 + u]);
+    }
+    const unsigned pk = __vimax3_s16x2(__vimax3_s16x2(p[0], p[1], p[2]), __vimax3_s16x2(p[3], p[4], p[5]), __vmaxs2(p[6], p[7]));
+    const int k1 = max((int)(pk << 16) >> 16, (int)pk >> 16);
+    if constexpr (OP == MatchOp::TopK) topk_tile<KB>(rp, k1, j0, n1, list);
+    if constexpr (OP == MatchOp::RadiusCount || OP == MatchOp::RadiusEmit)
+        radius_tile<OP == MatchOp::RadiusEmit>(rp, k1, rad_thr, j0, n1, qrow, rad_out, rad_n);
+    if constexpr (OP == MatchOp::CrossCheck) xc_warp_columns(rp, qvalid, row_cta, xc_slots);
+    return k1;
+}
+
 // SETQ = false: one query set (the map) shared by every train set; nq is its row count.
 // SETQ = true (pairwise): set s has its own query rows, min(query_counts[s], nq) of them at query + s * nq * 32, so nq is
 // the query stride and the pitch of the outputs and of the split keys.  The A tile then belongs to ONE set: the grid has
 // gridDim.z = nsets (one (set, query tile) unit per CTA), and a CTA whose query tile is empty for its set exits before
 // any setup -- in a CTA pair only when the leader's (lower) tile is empty too, because the peer holds half of every B tile.
-// KB > 0 (top-k, k = knn_k <= KB): best receives k records per (set, query row), [nsets][nq][k]; single CTA, no split.
-// RAD > 0 (radius, distance <= R with rad_thr = 127 * (256 - 2R)), list L = set * nq + query row; single CTA, no split.
-// RAD = 1: rad_offsets[1 + L] = list L's length.  RAD = 2: rad_offsets holds the scanned offsets, and list L's hits go to
-// best[rad_offsets[L] ..] in ascending train row when rad_offsets[L + 1] <= rad_cap.
-template <bool KNN2, bool PAIR, bool XCHK, bool SETQ, int KB = 0, int RAD = 0>
-__device__ __forceinline__ void
-hamming_umma_body(const uint8_t* __restrict__ query, int nq, const uint8_t* __restrict__ train, int nt, int train_stride_rows,
-               const int* __restrict__ train_counts, int nsets, int rows_per_split, int4* __restrict__ best,
-               int4* __restrict__ second, int* __restrict__ keys, int* __restrict__ status, int* __restrict__ col_keys,
-               const int* __restrict__ query_counts, int knn_k = 0, int rad_thr = 0, long long* __restrict__ rad_offsets = nullptr,
-               long long rad_cap = 0)
+// Outputs: with keys (train-row split) atomicMax of the packed row key, finalised by k_match_finalize; else records directly.
+// TopK (k = knn_k <= KB): best receives k records per (set, query row), [nsets][nq][k].
+// RadiusCount: rad_offsets[1 + L] = list L's length.  RadiusEmit: rad_offsets holds the scanned offsets, and list L's hits
+// go to best[rad_offsets[L] ..] in ascending train row when rad_offsets[L + 1] <= rad_cap.
+template <MatchOp OP, bool PAIR, bool SETQ, int KB>
+__device__ __forceinline__ void hamming_umma_body(const MatchArgs& args)
 {
-    static_assert(!(KNN2 && XCHK), "cross-check keeps the best match only");
-    static_assert(KB == 0 || (!KNN2 && !PAIR && !XCHK), "top-k runs on the single-CTA kernel alone");
-    static_assert(RAD == 0 || (KB == 0 && !KNN2 && !PAIR && !XCHK), "radius runs on the single-CTA kernel alone");
+    static_assert(!PAIR || match_op_pairs(OP), "top-k and radius run on the single-CTA kernel alone");
+    static_assert((OP == MatchOp::TopK) == (KB > 0), "KB is the top-k list capacity");
+    constexpr bool KNN2 = OP == MatchOp::Knn2, XCHK = OP == MatchOp::CrossCheck;
+    constexpr int RAD = OP == MatchOp::RadiusCount ? 1 : OP == MatchOp::RadiusEmit ? 2 : 0;
+    const uint8_t* __restrict__ query = args.query;
+    const uint8_t* __restrict__ train = args.train;
+    const int* __restrict__ train_counts = args.train_counts;
+    int4* __restrict__ best = args.best;
+    int4* __restrict__ second = args.second;
+    int* __restrict__ keys = args.keys;
+    int* __restrict__ status = args.status;
+    int* __restrict__ col_keys = args.col_keys;
+    long long* __restrict__ rad_offsets = args.rad_offsets;
+    const int nq = args.nq, nt = args.nt, train_stride_rows = args.train_stride_rows, nsets = args.nsets;
+    const int rows_per_split = args.rows_per_split, knn_k = args.knn_k, rad_thr = args.rad_thr;
+    const long long rad_cap = args.rad_cap;
     int nqv = nq;                                            // query rows present (padded rows q >= nqv are excluded)
     if constexpr (SETQ) {
-        nqv = max(0, min(__ldg(query_counts + blockIdx.z), nq));
+        nqv = max(0, min(__ldg(args.query_counts + blockIdx.z), nq));
         if ((PAIR ? (int)(blockIdx.x & ~1u) : (int)blockIdx.x) * MT_QROWS >= nqv) return;
         query += (size_t)blockIdx.z * nq * 32;
     }
@@ -668,19 +752,8 @@ hamming_umma_body(const uint8_t* __restrict__ query, int nq, const uint8_t* __re
                     tc_fence_before();
                     __syncwarp();
                     if (lane == 0) bar_arrive_lead<PAIR>(lead_tempty + 8 * b);           // TMEM buffer back to the issuer BEFORE the reduction
-                    unsigned p[8];                           // eight independent max chains (ILP), then a short tree
-#pragma unroll
-                    for (int u = 0; u < 8; ++u) {
-                        p[u] = __vimax3_s16x2(rp[u], rp[8 + u], rp[16 + u]);
-                        p[u] = __vimax3_s16x2(p[u], rp[24 + u], rp[32 + u]);
-                        p[u] = __vmaxs2(p[u], rp[40 + u]);
-                    }
-                    const unsigned pk = __vimax3_s16x2(__vimax3_s16x2(p[0], p[1], p[2]), __vimax3_s16x2(p[3], p[4], p[5]), __vmaxs2(p[6], p[7]));
-                    k1 = max((int)(pk << 16) >> 16, (int)pk >> 16);
-                    if constexpr (KB > 0) topk_tile<KB>(rp, k1, j0, rg.n1, list);
-                    if constexpr (RAD > 0) radius_tile<RAD == 2>(rp, k1, rad_thr, j0, rg.n1, qrow, rad_out, rad_n);
-                    if constexpr (XCHK)
-                        xc_warp_columns(rp, qrow < nqv, qrow - q0, reinterpret_cast<int*>(smem + MT_SMEM_XC) + (b * 8 + warp - MT_EPI_WARP0) * MT_BN);
+                    k1 = epilogue_tile<OP, KB>(rp, j0, rg.n1, qrow, list, rad_thr, rad_out, rad_n, qrow < nqv, qrow - q0,
+                                               reinterpret_cast<int*>(smem + MT_SMEM_XC) + (b * 8 + warp - MT_EPI_WARP0) * MT_BN);
                 } else if (!KNN2) {
                     // a set's partial last tile was issued with N = 32, 64 (or 96) columns, its rows past the set's end are
                     // copies of the last row (never the maximum): same packed path, 32-column chunks as far as N goes
@@ -698,19 +771,8 @@ hamming_umma_body(const uint8_t* __restrict__ query, int nq, const uint8_t* __re
                     tc_fence_before();
                     __syncwarp();
                     if (lane == 0) bar_arrive_lead<PAIR>(lead_tempty + 8 * b);
-                    unsigned p[8];
-#pragma unroll
-                    for (int u = 0; u < 8; ++u) {
-                        p[u] = __vimax3_s16x2(rp[u], rp[8 + u], rp[16 + u]);
-                        p[u] = __vimax3_s16x2(p[u], rp[24 + u], rp[32 + u]);
-                        p[u] = __vmaxs2(p[u], rp[40 + u]);
-                    }
-                    const unsigned pk = __vimax3_s16x2(__vimax3_s16x2(p[0], p[1], p[2]), __vimax3_s16x2(p[3], p[4], p[5]), __vmaxs2(p[6], p[7]));
-                    k1 = max((int)(pk << 16) >> 16, (int)pk >> 16);
-                    if constexpr (KB > 0) topk_tile<KB>(rp, k1, j0, rg.n1, list);
-                    if constexpr (RAD > 0) radius_tile<RAD == 2>(rp, k1, rad_thr, j0, rg.n1, qrow, rad_out, rad_n);
-                    if constexpr (XCHK)                      // (chunks past N hold -32768: no column there)
-                        xc_warp_columns(rp, qrow < nqv, qrow - q0, reinterpret_cast<int*>(smem + MT_SMEM_XC) + (b * 8 + warp - MT_EPI_WARP0) * MT_BN);
+                    k1 = epilogue_tile<OP, KB>(rp, j0, rg.n1, qrow, list, rad_thr, rad_out, rad_n, qrow < nqv, qrow - q0,
+                                               reinterpret_cast<int*>(smem + MT_SMEM_XC) + (b * 8 + warp - MT_EPI_WARP0) * MT_BN);
                 } else {
 #pragma unroll
                     for (int ch = 0; ch < NCH; ++ch) tc_ld32(tacc + (uint32_t)(ch * 32), r[ch]);
@@ -730,17 +792,13 @@ hamming_umma_body(const uint8_t* __restrict__ query, int nq, const uint8_t* __re
                                 k1 = max(k1, k);
                             }
                 }
-                // decode the tile winner(s) into the global key  dot << 20 | (0xFFFFF - j)
+                // decode the tile winner(s) into the global row key (top-k: already in the list; radius: nothing to keep)
 #pragma unroll
-                for (int w = 0; w < (KB > 0 || RAD > 0 ? 0 : KNN2 ? 2 : 1); ++w) {   // (top-k: already in the list; radius: nothing to keep)
+                for (int w = 0; w < (KNN2 ? 2 : match_op_pairs(OP) ? 1 : 0); ++w) {
                     const int k = w == 0 ? k1 : k2;
                     if (k != INT_MIN) {
-                        const unsigned kk = (unsigned)(k + MT_ASCALE * 256);
-                        const unsigned q = kk / (unsigned)MT_ASCALE;          // dot + 256
-                        const int code = (MT_BN - 1) - (int)(kk - q * (unsigned)MT_ASCALE);   // 48 * (CTA holding the row) + local row
-                        const int nh = ((min(MT_BN, rg.n1 - j0) + 31) & ~31) >> 1;
-                        const int jl = PAIR && code >= MT2_HALF ? nh + code - MT2_HALF : code;
-                        const int gk = ((int)q - 256) * (1 << MT_KEY_SHIFT) + ((MT_MAX_TRAIN - 1) - (j0 + jl));
+                        const AccRow d = acc_row<PAIR>(k, j0, rg.n1);
+                        const int gk = row_key(d.dot, d.j);
                         if (KNN2) m2 = max(m2, min(m1, gk));
                         m1 = max(m1, gk);
                     }
@@ -758,14 +816,10 @@ hamming_umma_body(const uint8_t* __restrict__ query, int nq, const uint8_t* __re
                         for (int w = 1; w < 8; ++w) kx = max(kx, xcs[w * MT_BN]);
                         const int v = kx >> 8;
                         if (v != -32768) {                   // (only padded query rows, or a chunk past the tile's N)
-                            const unsigned kk = (unsigned)(v + MT_ASCALE * 256);
-                            const unsigned q = kk / (unsigned)MT_ASCALE;      // dot + 256
-                            const int code = (MT_BN - 1) - (int)(kk - q * (unsigned)MT_ASCALE);
-                            const int nh = ((min(MT_BN, rg.n1 - j0) + 31) & ~31) >> 1;
-                            const int j = j0 + (PAIR && code >= MT2_HALF ? nh + code - MT2_HALF : code);
-                            if (j < rg.n1)                   // columns past the set's end are copies of its last row
-                                atomicMax(&col_keys[(size_t)set * train_stride_rows + j],
-                                          ((int)q - 256) * (1 << MT_KEY_SHIFT) + ((MT_MAX_QUERY_XC - 1) - (q0 + 255 - (kx & 255))));
+                            const AccRow d = acc_row<PAIR>(v, j0, rg.n1);
+                            if (d.j < rg.n1)                 // columns past the set's end are copies of its last row
+                                atomicMax(&col_keys[(size_t)set * train_stride_rows + d.j],
+                                          d.dot * (1 << MT_KEY_SHIFT) + ((MT_MAX_QUERY_XC - 1) - (q0 + 255 - (kx & 255))));
                         }
                     }
                 }
@@ -774,31 +828,18 @@ hamming_umma_body(const uint8_t* __restrict__ query, int nq, const uint8_t* __re
                 const size_t o = (size_t)set * nq + qrow;
                 if constexpr (RAD > 0) {                    // count pass: the list's length (the emit pass has written its hits)
                     if constexpr (RAD == 1) rad_offsets[1 + o] = rad_n;
-                } else if constexpr (KB > 0) {                     // the k records of this row, once per set
+                } else if constexpr (KB > 0) {              // the k records of this row, once per set
                     int4* out = best + o * knn_k;
 #pragma unroll
                     for (int r = 0; r < KB; ++r) {
                         if (r >= knn_k) break;
-                        const int key = list[r];
-                        const int dot = key >> MT_KEY_SHIFT, j = (MT_MAX_TRAIN - 1) - (key & (MT_MAX_TRAIN - 1));
-                        out[r] = key == INT_MIN ? make_int4(qrow, -1, 0, 0) : make_int4(qrow, j, 0, __float_as_int((float)((256 - dot) >> 1)));
+                        out[r] = key_record(qrow, list[r]);
                     }
                 } else if (keys) {
                     if (m1 != INT_MIN) atomicMax(&keys[o], m1);
-                } else if (m1 == INT_MIN) {                   // empty train set: no match (trainIdx -1)
-                    best[o] = make_int4(qrow, -1, 0, 0);
-                    if (KNN2) second[o] = make_int4(qrow, -1, 0, 0);
-                } else {
-                    const int dot = m1 >> MT_KEY_SHIFT, j = (MT_MAX_TRAIN - 1) - (m1 & (MT_MAX_TRAIN - 1));
-                    best[o] = make_int4(qrow, j, 0, __float_as_int((float)((256 - dot) >> 1)));
-                    if (KNN2) {
-                        if (m2 != INT_MIN) {
-                            const int dot2 = m2 >> MT_KEY_SHIFT, j2 = (MT_MAX_TRAIN - 1) - (m2 & (MT_MAX_TRAIN - 1));
-                            second[o] = make_int4(qrow, j2, 0, __float_as_int((float)((256 - dot2) >> 1)));
-                        } else {
-                            second[o] = make_int4(qrow, -1, 0, 0);
-                        }
-                    }
+                } else {                                     // (an empty train set: trainIdx -1)
+                    best[o] = key_record(qrow, m1);
+                    if (KNN2) second[o] = key_record(qrow, m2);
                 }
             }
         }
@@ -813,107 +854,41 @@ hamming_umma_body(const uint8_t* __restrict__ query, int nq, const uint8_t* __re
 }
 
 
-// XCHK = true (BFMatcher crossCheck = true): the best match plus every train row's nearest query, merged into
-// col_keys[set][train_stride_rows] (INT_MIN-initialised) by atomicMax; launched with MT_SMEM_BYTES_XC.  col_keys is unused otherwise.
-// single CTA per query tile (small problems: independent CTAs, train rows can be split across them)
-template <bool KNN2, bool XCHK>
-__global__ void __launch_bounds__(MT_THREADS, 1) k_hamming_umma(const uint8_t* __restrict__ query, int nq, const uint8_t* __restrict__ train, int nt,
-                                                                int train_stride_rows, const int* __restrict__ train_counts, int nsets, int rows_per_split,
-                                                                int4* __restrict__ best, int4* __restrict__ second, int* __restrict__ keys,
-                                                                int* __restrict__ status, int* __restrict__ col_keys)
+// The matcher kernels: the body for one operation (see MatchOp; CrossCheck is launched with MT_SMEM_BYTES_XC), shared query
+// or pairwise (SETQ: set s's own query rows against train set s, gridDim.z = nsets), and KB: TopK's list capacity.
+// Single CTA per query tile (small problems: independent CTAs, train rows can be split across them): every operation.
+template <MatchOp OP, bool SETQ, int KB = 0>
+__global__ void __launch_bounds__(MT_THREADS, 1) k_hamming_umma(const __grid_constant__ MatchArgs args)
 {
-    hamming_umma_body<KNN2, false, XCHK, false>(query, nq, train, nt, train_stride_rows, train_counts, nsets, rows_per_split, best, second, keys, status,
-                                                col_keys, nullptr);
+    hamming_umma_body<OP, false, SETQ, KB>(args);
 }
-// CTA pair on the two SMs of a TPC (tcgen05 cta_group::2): blockIdx.x = 2 * pair + rank
-template <bool KNN2, bool XCHK>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(MT_THREADS, 1) k_hamming_umma2(const uint8_t* __restrict__ query, int nq, const uint8_t* __restrict__ train,
-                                                                                          int nt, int train_stride_rows, const int* __restrict__ train_counts, int nsets,
-                                                                                          int rows_per_split, int4* __restrict__ best, int4* __restrict__ second,
-                                                                                          int* __restrict__ keys, int* __restrict__ status, int* __restrict__ col_keys)
+// CTA pair on the two SMs of a TPC (tcgen05 cta_group::2): blockIdx.x = 2 * pair + rank; Best, Knn2 and CrossCheck
+template <MatchOp OP, bool SETQ>
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(MT_THREADS, 1) k_hamming_umma2(const __grid_constant__ MatchArgs args)
 {
-    hamming_umma_body<KNN2, true, XCHK, false>(query, nq, train, nt, train_stride_rows, train_counts, nsets, rows_per_split, best, second, keys, status,
-                                               col_keys, nullptr);
-}
-// Pairwise (SETQ): set s's own query rows against train set s; nq = query stride, query_counts[nsets]; gridDim.z = nsets
-template <bool KNN2, bool XCHK>
-__global__ void __launch_bounds__(MT_THREADS, 1) k_hamming_umma_pw(const uint8_t* __restrict__ query, int nq, const uint8_t* __restrict__ train, int nt,
-                                                                   int train_stride_rows, const int* __restrict__ train_counts, int nsets, int rows_per_split,
-                                                                   int4* __restrict__ best, int4* __restrict__ second, int* __restrict__ keys,
-                                                                   int* __restrict__ status, int* __restrict__ col_keys, const int* __restrict__ query_counts)
-{
-    hamming_umma_body<KNN2, false, XCHK, true>(query, nq, train, nt, train_stride_rows, train_counts, nsets, rows_per_split, best, second, keys, status,
-                                               col_keys, query_counts);
-}
-template <bool KNN2, bool XCHK>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(MT_THREADS, 1) k_hamming_umma2_pw(const uint8_t* __restrict__ query, int nq, const uint8_t* __restrict__ train,
-                                                                                             int nt, int train_stride_rows, const int* __restrict__ train_counts, int nsets,
-                                                                                             int rows_per_split, int4* __restrict__ best, int4* __restrict__ second,
-                                                                                             int* __restrict__ keys, int* __restrict__ status, int* __restrict__ col_keys,
-                                                                                             const int* __restrict__ query_counts)
-{
-    hamming_umma_body<KNN2, true, XCHK, true>(query, nq, train, nt, train_stride_rows, train_counts, nsets, rows_per_split, best, second, keys, status,
-                                              col_keys, query_counts);
-}
-// top-k (knnMatch, k = knn_k <= KB): best receives [nsets][nq][k] records (train-row split and second are unused)
-template <int KB>
-__global__ void __launch_bounds__(MT_THREADS, 1) k_hamming_umma_topk(const uint8_t* __restrict__ query, int nq, const uint8_t* __restrict__ train, int nt,
-                                                                     int train_stride_rows, const int* __restrict__ train_counts, int nsets, int rows_per_split,
-                                                                     int4* __restrict__ best, int* __restrict__ status, int knn_k)
-{
-    hamming_umma_body<false, false, false, false, KB>(query, nq, train, nt, train_stride_rows, train_counts, nsets, rows_per_split, best, nullptr, nullptr,
-                                                      status, nullptr, nullptr, knn_k);
-}
-// pairwise top-k: best receives [nsets][nq][k] records, those of query i of set s for i < query_counts[s] only
-template <int KB>
-__global__ void __launch_bounds__(MT_THREADS, 1) k_hamming_umma_pw_topk(const uint8_t* __restrict__ query, int nq, const uint8_t* __restrict__ train, int nt,
-                                                                        int train_stride_rows, const int* __restrict__ train_counts, int nsets, int rows_per_split,
-                                                                        int4* __restrict__ best, int* __restrict__ status, const int* __restrict__ query_counts,
-                                                                        int knn_k)
-{
-    hamming_umma_body<false, false, false, true, KB>(query, nq, train, nt, train_stride_rows, train_counts, nsets, rows_per_split, best, nullptr, nullptr,
-                                                     status, nullptr, query_counts, knn_k);
-}
-// radius (radiusMatch): RAD = 1 writes list lengths to offsets[1 + L], RAD = 2 the hits of lists ending at or below cap to out
-template <int RAD>
-__global__ void __launch_bounds__(MT_THREADS, 1) k_hamming_umma_radius(const uint8_t* __restrict__ query, int nq, const uint8_t* __restrict__ train, int nt,
-                                                                       int train_stride_rows, const int* __restrict__ train_counts, int nsets, int rows_per_split,
-                                                                       int4* __restrict__ out, int* __restrict__ status, int thr, long long* __restrict__ offsets,
-                                                                       long long cap)
-{
-    hamming_umma_body<false, false, false, false, 0, RAD>(query, nq, train, nt, train_stride_rows, train_counts, nsets, rows_per_split, out, nullptr,
-                                                          nullptr, status, nullptr, nullptr, 0, thr, offsets, cap);
-}
-// pairwise radius: lists [nsets][nq] (nq = query stride); rows past a set's query count are not visited (their lengths stay 0)
-template <int RAD>
-__global__ void __launch_bounds__(MT_THREADS, 1) k_hamming_umma_pw_radius(const uint8_t* __restrict__ query, int nq, const uint8_t* __restrict__ train, int nt,
-                                                                          int train_stride_rows, const int* __restrict__ train_counts, int nsets, int rows_per_split,
-                                                                          int4* __restrict__ out, int* __restrict__ status, const int* __restrict__ query_counts,
-                                                                          int thr, long long* __restrict__ offsets, long long cap)
-{
-    hamming_umma_body<false, false, false, true, 0, RAD>(query, nq, train, nt, train_stride_rows, train_counts, nsets, rows_per_split, out, nullptr,
-                                                         nullptr, status, nullptr, query_counts, 0, thr, offsets, cap);
+    hamming_umma_body<OP, true, SETQ, 0>(args);
 }
 
 // ONE CTA per set: query i keeps its best match (i, j) iff column j's key names i, i.e. i is also train row j's nearest
 // query (lowest index on ties); the kept records are compacted stably in query order to out[set][0 .. n_out[set]).
 // best and out may be the same buffer: a record only moves to a lower or equal index, and a chunk is read before it is written.
-// nq rows of the set are read; pitch is the record distance between sets (nq, or the query stride of a pairwise call).
+// Sets are nq records apart; set s holds min(query_counts[s], nq) query rows (pairwise), or all nq (query_counts null).
 constexpr int XC_NT = 1024;
-__device__ __forceinline__ void crosscheck_compact_set(const int4* best, int nq, int pitch, const int* __restrict__ col_keys, int stride_rows,
-                                                       int4* out, int* __restrict__ n_out)
+__global__ void __launch_bounds__(XC_NT) k_crosscheck_compact(const int4* best, int nq, const int* __restrict__ query_counts,
+                                                              const int* __restrict__ col_keys, int stride_rows, int4* out, int* __restrict__ n_out)
 {
     __shared__ int s_warp[XC_NT / 32];
     __shared__ int s_base;
     const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
     const size_t set = blockIdx.x;
-    best += set * pitch; out += set * pitch; col_keys += set * stride_rows;
+    const int nrows = query_counts ? max(0, min(__ldg(query_counts + set), nq)) : nq;
+    best += set * nq; out += set * nq; col_keys += set * stride_rows;
     if (tid == 0) s_base = 0;
     __syncthreads();
-    for (int base = 0; base < nq; base += XC_NT) {
+    for (int base = 0; base < nrows; base += XC_NT) {
         const int i = base + tid;
         int4 r = make_int4(0, -1, 0, 0);
-        if (i < nq) r = best[i];
+        if (i < nrows) r = best[i];
         const bool keep = r.y >= 0 && (MT_MAX_QUERY_XC - 1) - (col_keys[r.y] & (MT_MAX_QUERY_XC - 1)) == i;
         const unsigned bal = __ballot_sync(0xffffffffu, keep);
         if (lane == 0) s_warp[wid] = __popc(bal);
@@ -928,11 +903,6 @@ __device__ __forceinline__ void crosscheck_compact_set(const int4* best, int nq,
     }
     if (tid == 0) n_out[set] = s_base;
 }
-__global__ void __launch_bounds__(XC_NT) k_crosscheck_compact(const int4* best, int nq, const int* __restrict__ col_keys, int stride_rows,
-                                                                           int4* out, int* __restrict__ n_out)
-{
-    crosscheck_compact_set(best, nq, nq, col_keys, stride_rows, out, n_out);
-}
 
 __global__ void k_match_keys_init(int* __restrict__ keys, size_t n)
 {
@@ -940,35 +910,13 @@ __global__ void k_match_keys_init(int* __restrict__ keys, size_t n)
     if (i < n) keys[i] = INT_MIN;
 }
 
-// split keys -> DMatch record i of [n / nq][nq]
-__device__ __forceinline__ void match_finalize_record(const int* __restrict__ keys, int nq, size_t i, int4* __restrict__ best)
-{
-    const int k = keys[i];
-    if (k == INT_MIN) { best[i] = make_int4((int)(i % (size_t)nq), -1, 0, 0); return; }
-    const int dot = k >> MT_KEY_SHIFT, j = (MT_MAX_TRAIN - 1) - (k & (MT_MAX_TRAIN - 1));
-    best[i] = make_int4((int)(i % (size_t)nq), j, 0, __float_as_int((float)((256 - dot) >> 1)));
-}
-
-__global__ void k_match_finalize(const int* __restrict__ keys, int nq, size_t n, int4* __restrict__ best)
+// split keys -> DMatch record i of [n / nq][nq]; with query_counts (pairwise) only the min(query_counts[s], nq) rows of set
+// s, the record slots past that count left as they are
+__global__ void k_match_finalize(const int* __restrict__ keys, int nq, const int* __restrict__ query_counts, size_t n, int4* __restrict__ best)
 {
     const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    match_finalize_record(keys, nq, i, best);
-}
-
-// ---- pairwise (SETQ) finishing kernels: set s holds min(query_counts[s], nq) queries at records s * nq ...; the record
-// slots past that count are left as they are
-__global__ void k_match_finalize_pw(const int* __restrict__ keys, int nq, const int* __restrict__ query_counts, size_t n, int4* __restrict__ best)
-{
-    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n || (int)(i % (size_t)nq) >= __ldg(query_counts + i / (size_t)nq)) return;
-    match_finalize_record(keys, nq, i, best);
-}
-
-__global__ void __launch_bounds__(XC_NT) k_crosscheck_compact_pw(const int4* best, int nq, const int* __restrict__ query_counts,
-                                                                 const int* __restrict__ col_keys, int stride_rows, int4* out, int* __restrict__ n_out)
-{
-    crosscheck_compact_set(best, max(0, min(__ldg(query_counts + blockIdx.x), nq)), nq, col_keys, stride_rows, out, n_out);
+    if (i >= n || (query_counts && (int)(i % (size_t)nq) >= __ldg(query_counts + i / (size_t)nq))) return;
+    best[i] = key_record((int)(i % (size_t)nq), keys[i]);
 }
 
 }  // namespace orbx

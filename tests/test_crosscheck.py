@@ -227,7 +227,16 @@ def test_argument_errors(orbmod):
     assert dev(h, dp, 1, dp, 1, None, 1, dp, dp) == orbmod.E_ARG
     assert dev(h, dp, 1, dp, 1, dp, 1, None, dp) == orbmod.E_ARG
     assert dev(h, dp, 1, dp, 1, dp, 1, dp, None) == orbmod.E_ARG
+    # empty sizes: no sets returns before every pointer; no query or train rows still needs d_n_out, and zeroes it
+    n.value = 7
+    assert lib.orbx_match_hamming_crosscheck(h, None, 0, None, 1, None, C.byref(n)) == orbmod.OK and n.value == 0
+    assert dev(h, None, 1, None, 1, None, 0, None, None) == orbmod.OK
+    assert dev(h, None, 0, dp, 1, dp, 1, dp, None) == orbmod.E_ARG
+    d.fill_(5)
+    assert dev(h, None, 0, None, 4, None, 3, None, dp) == orbmod.OK
+    assert dev(h, dp, 4, dp, 0, dp, 3, dp, dp + 12) == orbmod.OK
     ctx.synchronize()
+    assert d[:7].tolist() == [0] * 6 + [5]
     ctx.close()
 
 

@@ -246,7 +246,7 @@ def _check_knn2(got_best, got_second, q, train, oracle, what):
 
 
 def test_match_pair_kernel_knn2_ragged_sets(orbmod, oracle):
-    """The CTA-pair kernel WITH the fused second-minimum (k_hamming_umma2<true>, knnMatch k = 2): 42 ragged train sets x 1203
+    """The CTA-pair kernel WITH the fused second-minimum (k_hamming_umma2<Knn2, ...>, knnMatch k = 2): 42 ragged train sets x 1203
     queries (6 padded query tiles x 42 sets >= 148 pairs selects it), sizes on every tile / chunk boundary, the set's last row
     duplicated earlier (ties across the padded last tile -> lowest index first, the copy second)."""
     import torch

@@ -334,6 +334,10 @@ def test_argument_errors(orbmod, ctx):
     assert pw(a6=65536) == orbmod.E_ARG and pw(a7=0) == orbmod.E_ARG and pw(a7=33) == orbmod.E_UNSUPPORTED
     assert pw(a1=1 << 20) == orbmod.E_UNSUPPORTED and pw(a4=1 << 20) == orbmod.E_UNSUPPORTED
     assert pw(a6=0) == orbmod.OK and pw(a1=0) == orbmod.OK and pw(a4=0) == orbmod.OK
+    # empty sizes with null pointers: the host and ragged forms return first, the pairwise one checks its pointers first
+    assert lib.orbx_match_hamming_knn(h, None, 0, None, 4, 3, None, orbmod.C.byref(n)) == orbmod.OK and n.value == 0
+    assert dev(a1=0, a0=None, a7=None) == orbmod.OK
+    assert pw(a6=0, a8=None) == orbmod.E_ARG
     ctx.synchronize()
     bf = orbmod.BFMatcher()
     for k, code in ((0, orbmod.E_ARG), (33, orbmod.E_UNSUPPORTED)):

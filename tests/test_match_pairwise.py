@@ -261,6 +261,16 @@ def test_argument_errors(orbmod):
     assert lib.orbx_match_hamming_device_pairwise_crosscheck(h, p, 0, p, p, 4, p, 5, p, nout.data_ptr()) == orbmod.OK
     ctx.synchronize()
     assert (nout.cpu().numpy() == 0).all() and ctx.launch_count == n0
+    # an empty size does not excuse a null pointer here: the pairwise forms check their pointers first
+    assert lib.orbx_match_hamming_device_pairwise(h, None, 0, p, p, 1, p, 1, p, None) == orbmod.E_ARG
+    assert lib.orbx_match_hamming_device_pairwise_crosscheck(h, p, 1, p, p, 0, p, 1, None, p) == orbmod.E_ARG
+    # the shared-query forms return before their pointers on an empty input
+    n = orbmod.C.c_int(7)
+    for fn in (lib.orbx_match_hamming, lib.orbx_match_hamming_knn2):
+        assert fn(h, None, 0, None, 4, None, orbmod.C.byref(n)) == orbmod.OK and n.value == 0
+    assert lib.orbx_match_hamming_device(h, None, 4, None, 4, 0, None, None) == orbmod.OK
+    assert lib.orbx_match_hamming_device_ragged(h, p, 4, None, 0, None, 2, None, None) == orbmod.OK
+    assert lib.orbx_match_hamming_sets(h, None, 0, None, 4, None, 2, None, None) == orbmod.OK
     ctx.close()
 
 

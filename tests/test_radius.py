@@ -317,6 +317,15 @@ def test_argument_errors(orbmod, ctx):
     assert dev(a5=3, a1=0) == orbmod.OK
     ctx.synchronize()
     assert int(d[0]) == 0
+    # empty sizes with null pointers: the host form returns first, the device forms check their pointers first
+    assert host(nq=0, qp=None, op=None) == orbmod.OK and n.value == 0
+    assert dev(a1=0, a0=None) == orbmod.E_ARG
+    assert pw(a6=0, a0=None) == orbmod.E_ARG
+    # an empty pairwise batch zeroes every list's offset: 3 pairs of query stride 2, no train rows
+    d.fill_(5)
+    assert pw(a1=2, a4=0, a6=3) == orbmod.OK
+    ctx.synchronize()
+    assert d[:8].tolist() == [0] * 7 + [5]
     with pytest.raises(orbmod.OrbxError) as e:
         orbmod.BFMatcher().radiusMatch(q, q, 0.0)
     assert e.value.code == orbmod.E_ARG

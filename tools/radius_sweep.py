@@ -5,8 +5,8 @@ context's stream after a warm-up, at radii 30, 64 and 128.  Shapes:
   bench_2048x1000x256   the bench's batch: 2048 map rows against 256 sets of 1000 rows
   frame_to_frame        255 pairs of extracted 640x480 / 1000-feature frames (pairwise calls)
 Each call is made once with cap = 0 (offsets only) to size the output, then timed with the full buffer.  A separate
-torch.profiler run of a few calls splits the device time into the count pass (k_hamming_umma*_radius<1>), the offsets
-scan, the emit pass (<2>) and the ordering (k_radius_order).  cv2's BFMatcher.radiusMatch on the host is timed for the VO
+torch.profiler run of a few calls splits the device time into the count pass (k_hamming_umma<RadiusCount, ...>), the
+offsets scan, the emit pass (<RadiusEmit, ...>) and the ordering (k_radius_order).  cv2's BFMatcher.radiusMatch on the host is timed for the VO
 call.  The VO call's output is compared with cv2's lists (`vo_mismatched_lists` must be 0).  Prints the card, its power
 limit and SM clock with the numbers and writes them as JSON.
 
@@ -31,7 +31,8 @@ from rgbd_visualodometry_b200 import orb  # noqa: E402
 from rgbd_visualodometry_b200.synth import synth_descriptors, synth_map_queries, synth_sequence  # noqa: E402
 
 RADII = (30, 64, 128)
-PARTS = (("count", "radius<1>"), ("emit", "radius<2>"), ("scan", "k_radius_scan"), ("scan", "k_radius_tile_sums"), ("order", "k_radius_order"))
+PARTS = (("count", "MatchOp)4"), ("emit", "MatchOp)5"),   # k_hamming_umma<MatchOp::RadiusCount / RadiusEmit, ...>
+          ("scan", "k_radius_scan"), ("scan", "k_radius_tile_sums"), ("order", "k_radius_order"))
 
 
 def breakdown(fn, calls=3):
