@@ -776,55 +776,6 @@ int run_match(orbx_ctx* c, const MatchJob& job)
     return ORBX_OK;
 }
 
-// The host-buffer matcher, synchronous on the context's stream: nq query rows against nsets train sets of stride_rows rows
-// each (all of them, or as many as the host `counts` give per set).  Best: `best` receives [nsets][nq] records.  Knn2: best
-// and `second` the same, or without `second` (one set) `best` receives [nq][2] {best, second} records.  TopK: `best` receives
-// [nsets][nq][k] records.  CrossCheck (one set): `best` receives the mutual pairs and *xc_count their number.
-int match_host(orbx_ctx* c, MatchOp op, const uint8_t* query, int nq, const uint8_t* train, int stride_rows, const int* counts, int nsets,
-               orbx_match* best, orbx_match* second = nullptr, int* xc_count = nullptr, int k = 0)
-{
-    const size_t tbytes = (size_t)nsets * stride_rows * 32, obytes = (size_t)nsets * nq * 16 * (size_t)(op == MatchOp::TopK ? k : 1);
-    const bool knn2 = op == MatchOp::Knn2, pairs = knn2 && !second;
-    int rc;
-    if ((rc = ensure(c, c->mq, (size_t)nq * 32)) || (rc = ensure(c, c->mt, tbytes)) || (rc = ensure(c, c->mbest, obytes)) ||
-        (knn2 && (rc = ensure(c, c->msecond, obytes))) || (counts && (rc = ensure(c, c->mcounts, sizeof(int) * (size_t)nsets))) ||
-        (xc_count && (rc = ensure(c, c->mxcount, sizeof(int) * (size_t)nsets))))
-        return rc;
-    CU(cudaMemcpyAsync(c->mq.p, query, (size_t)nq * 32, cudaMemcpyHostToDevice, c->stream));
-    CU(cudaMemcpyAsync(c->mt.p, train, tbytes, cudaMemcpyHostToDevice, c->stream));
-    if (counts) CU(cudaMemcpyAsync(c->mcounts.p, counts, sizeof(int) * (size_t)nsets, cudaMemcpyHostToDevice, c->stream));
-    MatchJob job = match_job(op, (const uint8_t*)c->mq.p, nq, (const uint8_t*)c->mt.p, stride_rows, counts ? (const int*)c->mcounts.p : nullptr,
-                             nsets, c->mbest.p);
-    job.second = knn2 ? (int4*)c->msecond.p : nullptr; job.xc_count = xc_count ? (int*)c->mxcount.p : nullptr; job.k = k;
-    if ((rc = run_match(c, job))) return rc;
-    if (xc_count) CU(cudaMemcpyAsync(xc_count, c->mxcount.p, sizeof(int) * (size_t)nsets, cudaMemcpyDeviceToHost, c->stream));
-    if (pairs) {
-        CU(cudaMemcpy2DAsync(best, 32, c->mbest.p, 16, 16, (size_t)nq, cudaMemcpyDeviceToHost, c->stream));
-        CU(cudaMemcpy2DAsync(best + 1, 32, c->msecond.p, 16, 16, (size_t)nq, cudaMemcpyDeviceToHost, c->stream));
-    } else {
-        CU(cudaMemcpyAsync(best, c->mbest.p, obytes, cudaMemcpyDeviceToHost, c->stream));
-        if (second) CU(cudaMemcpyAsync(second, c->msecond.p, obytes, cudaMemcpyDeviceToHost, c->stream));
-    }
-    return sync_match_words(c, 0, 1);
-}
-
-// orbx_match_hamming / _knn2 / _knn: one train set of nt rows, k records per query row ([nq][k]): k = 1 the plain matcher,
-// k = 2 the knn2 one (interleaved {best, second}), larger k the top-k one
-int match_one_set(orbx_ctx* c, const uint8_t* query, int nq, const uint8_t* train, int nt, orbx_match* out, int* n_out, int k)
-{
-    if (!c) return ORBX_E_ARG;
-    if (n_out) *n_out = 0;
-    if (nq < 0 || nt < 0) return fail(c, ORBX_E_ARG, "negative row count");
-    if (nq == 0 || nt == 0) return ORBX_OK;                 // cv: empty query or train -> no matches, no throw
-    if (!query || !train || !out) return fail(c, ORBX_E_ARG, "null pointer");
-    CU(cudaSetDevice(c->device));
-    const MatchOp op = k == 1 ? MatchOp::Best : k == 2 ? MatchOp::Knn2 : MatchOp::TopK;
-    const int rc = match_host(c, op, query, nq, train, nt, nullptr, 1, out, nullptr, nullptr, k);
-    if (rc) return rc;
-    if (n_out) *n_out = nq;
-    return ORBX_OK;
-}
-
 // One pass of radiusMatch (job.op RadiusCount or RadiusEmit, rad_thr and rad_offsets set), list L = set * nq + query row,
 // asynchronous on the context's stream.  The count pass writes every list's length to rad_offsets[1 + L], and the scan turns
 // rad_offsets[0 .. nsets * nq] into the 64-bit CSR offsets.  The emit pass (behind it) writes every list that ends at or below
@@ -854,15 +805,6 @@ int radius_pass(orbx_ctx* c, const MatchJob& job)
     return ORBX_OK;
 }
 
-// Both passes of radiusMatch on a job, the count's results on the device
-int radius_match(orbx_ctx* c, MatchJob job)
-{
-    job.op = MatchOp::RadiusCount;
-    const int rc = radius_pass(c, job);
-    job.op = MatchOp::RadiusEmit;
-    return rc ? rc : radius_pass(c, job);
-}
-
 // The matcher's threshold of the integer radius R = min(256, floor(max_distance)): distance <= R <=> accumulator >= thr
 int radius_threshold(float max_distance)
 {
@@ -872,6 +814,105 @@ int radius_threshold(float max_distance)
 
 // cv's CV_Assert(maxDistance > FLT_EPSILON) (false for NaN too)
 bool bad_radius(float max_distance) { return !(max_distance > FLT_EPSILON); }
+
+// One matcher request, on host buffers (match_on_host) or device memory (match_on_device).
+// in: nq query rows shared by every set, or pairwise (query_counts set) set s's own min(query_counts[s], nq) rows at
+//     query + s * nq * 32; against nsets train sets of min(train_counts[s], train_stride) rows (null: all) at
+//     train + s * train_stride * 32.
+// what: k for TopK; max_distance and cap (the records `best` holds) for radius.  RadiusEmit is radiusMatch: the count
+//     pass, then the lists (the emit pass alone once `counted`, the offsets holding the count); RadiusCount the count alone.
+// out: best [nsets][nq] records (TopK [nsets][nq][k]; CrossCheck set s's mutual pairs at best + s * nq; radius the lists);
+//     second for Knn2 (on the host without it, best receives [nq][2] {best, second}); n_out each set's CrossCheck pair count
+//     (on the host: the pairs, radius's records, otherwise nq); offsets radius's nsets * nq + 1 CSR offsets.
+struct MatchRequest {
+    struct { const uint8_t* query; int nq; const int* query_counts; const uint8_t* train; int train_stride; const int* train_counts; int nsets; } in;
+    struct { MatchOp op; int k; float max_distance; long long cap; bool counted; } what;
+    struct { orbx_match* best; orbx_match* second; int* n_out; int64_t* offsets; } out;
+};
+
+// A request on device memory, asynchronous on the context's stream.  An empty input (no query row, train row or set)
+// launches nothing: CrossCheck zeroes every set's pair count and radius every list's offset.
+int match_on_device(orbx_ctx* c, const MatchRequest& r)
+{
+    CU(cudaSetDevice(c->device));
+    const MatchOp op = r.what.op;
+    const bool radius = op == MatchOp::RadiusCount || op == MatchOp::RadiusEmit;
+    if (r.in.nq == 0 || r.in.train_stride == 0 || r.in.nsets == 0) {
+        if (op == MatchOp::CrossCheck) CU(cudaMemsetAsync(r.out.n_out, 0, sizeof(int) * (size_t)r.in.nsets, c->stream));
+        if (radius) CU(cudaMemsetAsync(r.out.offsets, 0, sizeof(int64_t) * ((size_t)r.in.nsets * r.in.nq + 1), c->stream));
+        return ORBX_OK;
+    }
+    MatchJob job = match_job(op, r.in.query, r.in.nq, r.in.train, r.in.train_stride, r.in.train_counts, r.in.nsets, r.out.best);
+    job.query_counts = r.in.query_counts; job.second = (int4*)r.out.second; job.k = r.what.k;
+    job.xc_count = op == MatchOp::CrossCheck ? r.out.n_out : nullptr;
+    if (!radius) return run_match(c, job);
+    job.rad_thr = radius_threshold(r.what.max_distance); job.rad_offsets = (long long*)r.out.offsets; job.rad_cap = r.what.cap;
+    if (op == MatchOp::RadiusEmit && !r.what.counted) {      // the count pass first
+        job.op = MatchOp::RadiusCount;
+        const int rc = radius_pass(c, job);
+        if (rc) return rc;
+        job.op = MatchOp::RadiusEmit;
+    }
+    return radius_pass(c, job);
+}
+
+// A request on host buffers (not empty), synchronous on the context's stream: the operands go to the context's staging
+// buffers, match_on_device runs there (radius: the count pass, the capacity check, then the lists), and the results come
+// back.
+int match_on_host(orbx_ctx* c, const MatchRequest& r)
+{
+    CU(cudaSetDevice(c->device));
+    const MatchOp op = r.what.op;
+    const bool knn2 = op == MatchOp::Knn2, xchk = op == MatchOp::CrossCheck, radius = op == MatchOp::RadiusEmit;
+    const int nq = r.in.nq, nsets = r.in.nsets;
+    const size_t tbytes = (size_t)nsets * r.in.train_stride * 32, nlists = (size_t)nsets * nq;
+    const size_t obytes = nlists * 16 * (size_t)(op == MatchOp::TopK ? r.what.k : 1);
+    int rc;
+    if ((rc = ensure(c, c->mq, (size_t)nq * 32)) || (rc = ensure(c, c->mt, tbytes)) ||
+        (r.in.train_counts && (rc = ensure(c, c->mcounts, sizeof(int) * (size_t)nsets))) ||
+        (radius && (rc = ensure(c, c->mradoff, sizeof(long long) * (nlists + 1)))) || (!radius && (rc = ensure(c, c->mbest, obytes))) ||
+        (knn2 && (rc = ensure(c, c->msecond, obytes))) || (xchk && (rc = ensure(c, c->mxcount, sizeof(int) * (size_t)nsets))))
+        return rc;
+    CU(cudaMemcpyAsync(c->mq.p, r.in.query, (size_t)nq * 32, cudaMemcpyHostToDevice, c->stream));
+    CU(cudaMemcpyAsync(c->mt.p, r.in.train, tbytes, cudaMemcpyHostToDevice, c->stream));
+    if (r.in.train_counts)
+        CU(cudaMemcpyAsync(c->mcounts.p, r.in.train_counts, sizeof(int) * (size_t)nsets, cudaMemcpyHostToDevice, c->stream));
+    MatchRequest d = r;                                      // the same request on the staging buffers
+    d.in.query = (const uint8_t*)c->mq.p;
+    d.in.train = (const uint8_t*)c->mt.p;
+    d.in.train_counts = r.in.train_counts ? (const int*)c->mcounts.p : nullptr;
+    d.out = {(orbx_match*)c->mbest.p, knn2 ? (orbx_match*)c->msecond.p : nullptr, xchk ? (int*)c->mxcount.p : nullptr,
+             radius ? (int64_t*)c->mradoff.p : nullptr};
+    if (radius) {                                            // the lists are made only once they are known to fit
+        d.what.op = MatchOp::RadiusCount;
+        if ((rc = match_on_device(c, d))) return rc;
+        long long total = 0;
+        CU(cudaMemcpyAsync(&total, d.out.offsets + nlists, sizeof total, cudaMemcpyDeviceToHost, c->stream));
+        if ((rc = sync_match_words(c, 0, 1))) return rc;
+        if (total > INT_MAX) return fail(c, ORBX_E_UNSUPPORTED, "more than 2^31 - 1 records");
+        *r.out.n_out = (int)total;
+        if (total > r.what.cap) return fail(c, ORBX_E_CAPACITY, "output capacity below the number of records");
+        if ((rc = ensure(c, c->mbest, 16 * (size_t)total))) return rc;
+        d.what = {MatchOp::RadiusEmit, 0, r.what.max_distance, total, true};
+        d.out.best = (orbx_match*)c->mbest.p;
+    }
+    if ((rc = match_on_device(c, d))) return rc;
+    int pairs = 0;
+    if (xchk) CU(cudaMemcpyAsync(&pairs, d.out.n_out, sizeof(int), cudaMemcpyDeviceToHost, c->stream));   // (one set)
+    if (radius) {
+        CU(cudaMemcpyAsync(r.out.best, d.out.best, 16 * (size_t)d.what.cap, cudaMemcpyDeviceToHost, c->stream));
+        CU(cudaMemcpyAsync(r.out.offsets, d.out.offsets, sizeof(int64_t) * (nlists + 1), cudaMemcpyDeviceToHost, c->stream));
+    } else if (knn2 && !r.out.second) {
+        CU(cudaMemcpy2DAsync(r.out.best, 32, d.out.best, 16, 16, (size_t)nq, cudaMemcpyDeviceToHost, c->stream));
+        CU(cudaMemcpy2DAsync(r.out.best + 1, 32, d.out.second, 16, 16, (size_t)nq, cudaMemcpyDeviceToHost, c->stream));
+    } else {
+        CU(cudaMemcpyAsync(r.out.best, d.out.best, obytes, cudaMemcpyDeviceToHost, c->stream));
+        if (r.out.second) CU(cudaMemcpyAsync(r.out.second, d.out.second, obytes, cudaMemcpyDeviceToHost, c->stream));
+    }
+    if ((rc = sync_match_words(c, 0, 1))) return rc;
+    if (r.out.n_out && !radius) *r.out.n_out = xchk ? pairs : nq;
+    return ORBX_OK;
+}
 
 }  // namespace
 
@@ -1196,13 +1237,26 @@ int orbx_detect_and_compute(orbx_ctx* c, const uint8_t* img, int w, int h, size_
     return orbx_detect_and_compute_batch(c, one, 1, w, h, step, channels, kps, desc, cap, n_out);
 }
 
+// Argument checks of the one-set host forms (orbx_match_hamming, _knn2, _knn, _crosscheck, _radius), after their own: the
+// row counts and the caller's other invalid arguments (`bad`) -> E_ARG; the caller's unsupported case (`unsupported`: its
+// message, or null) -> E_UNSUPPORTED; an empty input (no query or train row) -> *empty, before the pointers -> E_ARG.
+static int check_args_one_set(orbx_ctx* c, const void* q, int nq, const void* t, int nt, const void* out, bool bad, const char* unsupported,
+                              bool* empty)
+{
+    if (bad || nq < 0 || nt < 0) return fail(c, ORBX_E_ARG, "bad sizes");
+    if (unsupported) return fail(c, ORBX_E_UNSUPPORTED, unsupported);
+    if ((*empty = nq == 0 || nt == 0)) return ORBX_OK;       // cv: empty query or train -> no matches, no throw
+    if (!q || !t || !out) return fail(c, ORBX_E_ARG, "null pointer");
+    return ORBX_OK;
+}
+
 int orbx_match_hamming(orbx_ctx* c, const uint8_t* q, int nq, const uint8_t* t, int nt, orbx_match* out, int* n_out)
 {
-    return match_one_set(c, q, nq, t, nt, out, n_out, 1);
+    return orbx_match_hamming_knn(c, q, nq, t, nt, 1, out, n_out);
 }
 int orbx_match_hamming_knn2(orbx_ctx* c, const uint8_t* q, int nq, const uint8_t* t, int nt, orbx_match* out, int* n_out)
 {
-    return match_one_set(c, q, nq, t, nt, out, n_out, 2);
+    return orbx_match_hamming_knn(c, q, nq, t, nt, 2, out, n_out);
 }
 int orbx_match_hamming_knn(orbx_ctx* c, const uint8_t* q, int nq, const uint8_t* t, int nt, int k, orbx_match* out, int* n_out)
 {
@@ -1210,7 +1264,12 @@ int orbx_match_hamming_knn(orbx_ctx* c, const uint8_t* q, int nq, const uint8_t*
     if (n_out) *n_out = 0;
     if (k < 1) return fail(c, ORBX_E_ARG, "k < 1");
     if (k > ORBX_MAX_KNN) return fail(c, ORBX_E_UNSUPPORTED, "k larger than ORBX_MAX_KNN");
-    return match_one_set(c, q, nq, t, nt, out, n_out, k);
+    bool empty;
+    const int rc = check_args_one_set(c, q, nq, t, nt, out, false, nullptr, &empty);
+    if (rc || empty) return rc;
+    // k records per query row ([nq][k]): k = 1 the plain matcher, k = 2 the knn2 one (interleaved {best, second})
+    const MatchOp op = k == 1 ? MatchOp::Best : k == 2 ? MatchOp::Knn2 : MatchOp::TopK;
+    return match_on_host(c, {{q, nq, nullptr, t, nt, nullptr, 1}, {op, k}, {out, nullptr, n_out}});
 }
 
 int orbx_match_hamming_device(orbx_ctx* c, const uint8_t* d_query, int nq, const uint8_t* d_train, int nt, int nsets,
@@ -1220,10 +1279,7 @@ int orbx_match_hamming_device(orbx_ctx* c, const uint8_t* d_query, int nq, const
     if (nq < 0 || nt < 0 || nsets < 0 || nsets > 65535) return fail(c, ORBX_E_ARG, "bad sizes");
     if (nq == 0 || nt == 0 || nsets == 0) return ORBX_OK;
     if (!d_query || !d_train || !d_best) return fail(c, ORBX_E_ARG, "null pointer");
-    CU(cudaSetDevice(c->device));
-    MatchJob job = match_job(d_second ? MatchOp::Knn2 : MatchOp::Best, d_query, nq, d_train, nt, nullptr, nsets, d_best);
-    job.second = (int4*)d_second;
-    return run_match(c, job);
+    return match_on_device(c, {{d_query, nq, nullptr, d_train, nt, nullptr, nsets}, {d_second ? MatchOp::Knn2 : MatchOp::Best}, {d_best, d_second}});
 }
 
 // Argument checks of the shared-query ragged family (_device_ragged, _sets, _device_crosscheck, _device_knn, _device_radius):
@@ -1248,10 +1304,8 @@ int orbx_match_hamming_device_ragged(orbx_ctx* c, const uint8_t* d_query, int nq
     bool empty;
     const int rc = check_args_ragged(c, d_query, nq, d_train, train_stride_rows, d_train_counts, nsets, d_best, false, nullptr, &empty);
     if (rc || empty) return rc;
-    CU(cudaSetDevice(c->device));
-    MatchJob job = match_job(d_second ? MatchOp::Knn2 : MatchOp::Best, d_query, nq, d_train, train_stride_rows, d_train_counts, nsets, d_best);
-    job.second = (int4*)d_second;
-    return run_match(c, job);
+    return match_on_device(c, {{d_query, nq, nullptr, d_train, train_stride_rows, d_train_counts, nsets},
+                               {d_second ? MatchOp::Knn2 : MatchOp::Best}, {d_best, d_second}});
 }
 
 int orbx_match_hamming_sets(orbx_ctx* c, const uint8_t* query, int nq, const uint8_t* train, int train_stride_rows,
@@ -1261,8 +1315,8 @@ int orbx_match_hamming_sets(orbx_ctx* c, const uint8_t* query, int nq, const uin
     bool empty;
     const int rc = check_args_ragged(c, query, nq, train, train_stride_rows, train_counts, nsets, best, false, nullptr, &empty);
     if (rc || empty) return rc;
-    CU(cudaSetDevice(c->device));
-    return match_host(c, second ? MatchOp::Knn2 : MatchOp::Best, query, nq, train, train_stride_rows, train_counts, nsets, best, second);
+    return match_on_host(c, {{query, nq, nullptr, train, train_stride_rows, train_counts, nsets}, {second ? MatchOp::Knn2 : MatchOp::Best},
+                             {best, second}});
 }
 
 int orbx_match_hamming_crosscheck(orbx_ctx* c, const uint8_t* q, int nq, const uint8_t* t, int nt, orbx_match* out, int* n_out)
@@ -1270,16 +1324,11 @@ int orbx_match_hamming_crosscheck(orbx_ctx* c, const uint8_t* q, int nq, const u
     if (!c) return ORBX_E_ARG;
     if (!n_out) return fail(c, ORBX_E_ARG, "null n_out");
     *n_out = 0;
-    if (nq < 0 || nt < 0) return fail(c, ORBX_E_ARG, "negative row count");
-    if (nq >= MT_MAX_QUERY_XC) return fail(c, ORBX_E_UNSUPPORTED, "cross-check query set larger than 2^20 - 1 rows");
-    if (nq == 0 || nt == 0) return ORBX_OK;                 // empty query or train -> no pairs (cv2 raises on an empty train)
-    if (!q || !t || !out) return fail(c, ORBX_E_ARG, "null pointer");
-    CU(cudaSetDevice(c->device));
-    int n = 0;
-    const int rc = match_host(c, MatchOp::CrossCheck, q, nq, t, nt, nullptr, 1, out, nullptr, &n);
-    if (rc) return rc;
-    *n_out = n;
-    return ORBX_OK;
+    bool empty;                                              // empty query or train -> no pairs (cv2 raises on an empty train)
+    const int rc = check_args_one_set(c, q, nq, t, nt, out, false,
+                                      nq >= MT_MAX_QUERY_XC ? "cross-check query set larger than 2^20 - 1 rows" : nullptr, &empty);
+    if (rc || empty) return rc;
+    return match_on_host(c, {{q, nq, nullptr, t, nt, nullptr, 1}, {MatchOp::CrossCheck}, {out, nullptr, n_out}});
 }
 
 int orbx_match_hamming_device_crosscheck(orbx_ctx* c, const uint8_t* d_query, int nq, const uint8_t* d_train, int train_stride_rows,
@@ -1291,14 +1340,8 @@ int orbx_match_hamming_device_crosscheck(orbx_ctx* c, const uint8_t* d_query, in
                                      nq >= MT_MAX_QUERY_XC ? "cross-check query set larger than 2^20 - 1 rows" : nullptr, &empty);
     if (rc || nsets == 0) return rc;
     if (!d_n_out) return fail(c, ORBX_E_ARG, "null pointer");
-    CU(cudaSetDevice(c->device));
-    if (empty) {                                             // no pairs in any set
-        CU(cudaMemsetAsync(d_n_out, 0, sizeof(int) * (size_t)nsets, c->stream));
-        return ORBX_OK;
-    }
-    MatchJob job = match_job(MatchOp::CrossCheck, d_query, nq, d_train, train_stride_rows, d_train_counts, nsets, d_out);
-    job.xc_count = d_n_out;
-    return run_match(c, job);
+    return match_on_device(c, {{d_query, nq, nullptr, d_train, train_stride_rows, d_train_counts, nsets}, {MatchOp::CrossCheck},
+                               {d_out, nullptr, d_n_out}});
 }
 
 int orbx_match_hamming_device_knn(orbx_ctx* c, const uint8_t* d_query, int nq, const uint8_t* d_train, int train_stride_rows,
@@ -1309,11 +1352,9 @@ int orbx_match_hamming_device_knn(orbx_ctx* c, const uint8_t* d_query, int nq, c
     const int rc = check_args_ragged(c, d_query, nq, d_train, train_stride_rows, d_train_counts, nsets, d_out, k < 1,
                                      k > ORBX_MAX_KNN ? "k larger than ORBX_MAX_KNN" : nullptr, &empty);
     if (rc || empty) return rc;
-    CU(cudaSetDevice(c->device));
     // k = 1: the plain matcher's [nsets][nq] records are the [nsets][nq][1] layout
-    MatchJob job = match_job(k > 1 ? MatchOp::TopK : MatchOp::Best, d_query, nq, d_train, train_stride_rows, d_train_counts, nsets, d_out);
-    job.k = k > 1 ? k : 0;
-    return run_match(c, job);
+    return match_on_device(c, {{d_query, nq, nullptr, d_train, train_stride_rows, d_train_counts, nsets}, {k > 1 ? MatchOp::TopK : MatchOp::Best, k},
+                               {d_out}});
 }
 
 // orbx_match_hamming_device_pairwise[_crosscheck|_knn|_radius]: pair p = query set p against train set p.  Argument checks
@@ -1335,12 +1376,8 @@ int orbx_match_hamming_device_pairwise(orbx_ctx* c, const uint8_t* d_query, int 
     if (!c) return ORBX_E_ARG;
     int rc = check_args_pairwise(c, d_query, query_stride_rows, d_query_counts, d_train, train_stride_rows, d_train_counts, npairs, d_best);
     if (rc) return rc;
-    if (npairs == 0 || query_stride_rows == 0 || train_stride_rows == 0) return ORBX_OK;
-    CU(cudaSetDevice(c->device));
-    MatchJob job = match_job(d_second ? MatchOp::Knn2 : MatchOp::Best, d_query, query_stride_rows, d_train, train_stride_rows, d_train_counts, npairs, d_best);
-    job.query_counts = d_query_counts;
-    job.second = (int4*)d_second;
-    return run_match(c, job);
+    return match_on_device(c, {{d_query, query_stride_rows, d_query_counts, d_train, train_stride_rows, d_train_counts, npairs},
+                               {d_second ? MatchOp::Knn2 : MatchOp::Best}, {d_best, d_second}});
 }
 
 int orbx_match_hamming_device_pairwise_crosscheck(orbx_ctx* c, const uint8_t* d_query, int query_stride_rows, const int* d_query_counts,
@@ -1351,16 +1388,8 @@ int orbx_match_hamming_device_pairwise_crosscheck(orbx_ctx* c, const uint8_t* d_
     int rc = check_args_pairwise(c, d_query, query_stride_rows, d_query_counts, d_train, train_stride_rows, d_train_counts, npairs, d_out);
     if (rc) return rc;
     if (!d_n_out) return fail(c, ORBX_E_ARG, "null pointer");
-    if (npairs == 0) return ORBX_OK;
-    CU(cudaSetDevice(c->device));
-    if (query_stride_rows == 0 || train_stride_rows == 0) {  // no pairs in any set
-        CU(cudaMemsetAsync(d_n_out, 0, sizeof(int) * (size_t)npairs, c->stream));
-        return ORBX_OK;
-    }
-    MatchJob job = match_job(MatchOp::CrossCheck, d_query, query_stride_rows, d_train, train_stride_rows, d_train_counts, npairs, d_out);
-    job.query_counts = d_query_counts;
-    job.xc_count = d_n_out;
-    return run_match(c, job);
+    return match_on_device(c, {{d_query, query_stride_rows, d_query_counts, d_train, train_stride_rows, d_train_counts, npairs},
+                               {MatchOp::CrossCheck}, {d_out, nullptr, d_n_out}});
 }
 
 int orbx_match_hamming_device_pairwise_knn(orbx_ctx* c, const uint8_t* d_query, int query_stride_rows, const int* d_query_counts,
@@ -1372,12 +1401,8 @@ int orbx_match_hamming_device_pairwise_knn(orbx_ctx* c, const uint8_t* d_query, 
     int rc = check_args_pairwise(c, d_query, query_stride_rows, d_query_counts, d_train, train_stride_rows, d_train_counts, npairs, d_out);
     if (rc) return rc;
     if (k > ORBX_MAX_KNN) return fail(c, ORBX_E_UNSUPPORTED, "k larger than ORBX_MAX_KNN");
-    if (npairs == 0 || query_stride_rows == 0 || train_stride_rows == 0) return ORBX_OK;
-    CU(cudaSetDevice(c->device));
-    MatchJob job = match_job(k > 1 ? MatchOp::TopK : MatchOp::Best, d_query, query_stride_rows, d_train, train_stride_rows, d_train_counts, npairs, d_out);
-    job.query_counts = d_query_counts;
-    job.k = k > 1 ? k : 0;
-    return run_match(c, job);
+    return match_on_device(c, {{d_query, query_stride_rows, d_query_counts, d_train, train_stride_rows, d_train_counts, npairs},
+                               {k > 1 ? MatchOp::TopK : MatchOp::Best, k}, {d_out}});
 }
 
 int orbx_match_hamming_radius(orbx_ctx* c, const uint8_t* q, int nq, const uint8_t* t, int nt, float max_distance, orbx_match* out, int cap,
@@ -1386,37 +1411,15 @@ int orbx_match_hamming_radius(orbx_ctx* c, const uint8_t* q, int nq, const uint8
     if (!c) return ORBX_E_ARG;
     if (!n_out || !offsets) return fail(c, ORBX_E_ARG, "null pointer");
     *n_out = 0;
-    if (nq < 0 || nt < 0 || cap < 0) return fail(c, ORBX_E_ARG, "negative size");
-    if (bad_radius(max_distance)) return fail(c, ORBX_E_ARG, "maxDistance must be larger than FLT_EPSILON");
-    if (nt >= MT_MAX_TRAIN) return fail(c, ORBX_E_UNSUPPORTED, "train set larger than 2^20 - 1 rows");
-    if (nq == 0 || nt == 0) {                                // one empty list per query (cv), or none
+    bool empty;
+    const int rc = check_args_one_set(c, q, nq, t, nt, out, cap < 0 || bad_radius(max_distance),
+                                      nt >= MT_MAX_TRAIN ? "train set larger than 2^20 - 1 rows" : nullptr, &empty);
+    if (rc) return rc;
+    if (empty) {                                             // one empty list per query (cv), or none
         memset(offsets, 0, sizeof(int64_t) * ((size_t)nq + 1));
         return ORBX_OK;
     }
-    if (!q || !t || !out) return fail(c, ORBX_E_ARG, "null pointer");
-    CU(cudaSetDevice(c->device));
-    int rc;
-    if ((rc = ensure(c, c->mq, (size_t)nq * 32)) || (rc = ensure(c, c->mt, (size_t)nt * 32)) ||
-        (rc = ensure(c, c->mradoff, sizeof(long long) * ((size_t)nq + 1))))
-        return rc;
-    long long* d_off = (long long*)c->mradoff.p;
-    CU(cudaMemcpyAsync(c->mq.p, q, (size_t)nq * 32, cudaMemcpyHostToDevice, c->stream));
-    CU(cudaMemcpyAsync(c->mt.p, t, (size_t)nt * 32, cudaMemcpyHostToDevice, c->stream));
-    MatchJob job = match_job(MatchOp::RadiusCount, (const uint8_t*)c->mq.p, nq, (const uint8_t*)c->mt.p, nt, nullptr, 1, nullptr);
-    job.rad_thr = radius_threshold(max_distance); job.rad_offsets = d_off;
-    if ((rc = radius_pass(c, job))) return rc;
-    long long total = 0;
-    CU(cudaMemcpyAsync(&total, d_off + nq, sizeof total, cudaMemcpyDeviceToHost, c->stream));
-    if ((rc = sync_match_words(c, 0, 1))) return rc;
-    if (total > INT_MAX) return fail(c, ORBX_E_UNSUPPORTED, "more than 2^31 - 1 records");
-    *n_out = (int)total;
-    if (total > cap) return fail(c, ORBX_E_CAPACITY, "output capacity below the number of records");
-    if ((rc = ensure(c, c->mbest, 16 * (size_t)total))) return rc;
-    job.op = MatchOp::RadiusEmit; job.best = (int4*)c->mbest.p; job.rad_cap = total;
-    if ((rc = radius_pass(c, job))) return rc;
-    CU(cudaMemcpyAsync(out, c->mbest.p, 16 * (size_t)total, cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaMemcpyAsync(offsets, d_off, sizeof(int64_t) * ((size_t)nq + 1), cudaMemcpyDeviceToHost, c->stream));
-    return sync_match_words(c, 0, 1);
+    return match_on_host(c, {{q, nq, nullptr, t, nt, nullptr, 1}, {MatchOp::RadiusEmit, 0, max_distance, cap}, {out, nullptr, n_out, offsets}});
 }
 
 int orbx_match_hamming_device_radius(orbx_ctx* c, const uint8_t* d_query, int nq, const uint8_t* d_train, int train_stride_rows,
@@ -1428,14 +1431,8 @@ int orbx_match_hamming_device_radius(orbx_ctx* c, const uint8_t* d_query, int nq
     if (bad_radius(max_distance)) return fail(c, ORBX_E_ARG, "maxDistance must be larger than FLT_EPSILON");
     if (!d_offsets) return fail(c, ORBX_E_ARG, "null pointer");
     if (train_stride_rows >= MT_MAX_TRAIN) return fail(c, ORBX_E_UNSUPPORTED, "train set stride of 2^20 rows or more");
-    CU(cudaSetDevice(c->device));
-    if (nq == 0 || train_stride_rows == 0 || nsets == 0) {   // every list empty
-        CU(cudaMemsetAsync(d_offsets, 0, sizeof(int64_t) * ((size_t)nsets * nq + 1), c->stream));
-        return ORBX_OK;
-    }
-    MatchJob job = match_job(MatchOp::RadiusCount, d_query, nq, d_train, train_stride_rows, d_train_counts, nsets, d_out);
-    job.rad_thr = radius_threshold(max_distance); job.rad_offsets = (long long*)d_offsets; job.rad_cap = cap;
-    return radius_match(c, job);
+    return match_on_device(c, {{d_query, nq, nullptr, d_train, train_stride_rows, d_train_counts, nsets}, {MatchOp::RadiusEmit, 0, max_distance, cap},
+                               {d_out, nullptr, nullptr, d_offsets}});
 }
 
 int orbx_match_hamming_device_pairwise_radius(orbx_ctx* c, const uint8_t* d_query, int query_stride_rows, const int* d_query_counts,
@@ -1448,15 +1445,8 @@ int orbx_match_hamming_device_pairwise_radius(orbx_ctx* c, const uint8_t* d_quer
     if (!d_offsets) return fail(c, ORBX_E_ARG, "null pointer");
     int rc = check_args_pairwise(c, d_query, query_stride_rows, d_query_counts, d_train, train_stride_rows, d_train_counts, npairs, d_out);
     if (rc) return rc;
-    CU(cudaSetDevice(c->device));
-    if (npairs == 0 || query_stride_rows == 0 || train_stride_rows == 0) {   // every list empty
-        CU(cudaMemsetAsync(d_offsets, 0, sizeof(int64_t) * ((size_t)npairs * query_stride_rows + 1), c->stream));
-        return ORBX_OK;
-    }
-    MatchJob job = match_job(MatchOp::RadiusCount, d_query, query_stride_rows, d_train, train_stride_rows, d_train_counts, npairs, d_out);
-    job.query_counts = d_query_counts;
-    job.rad_thr = radius_threshold(max_distance); job.rad_offsets = (long long*)d_offsets; job.rad_cap = cap;
-    return radius_match(c, job);
+    return match_on_device(c, {{d_query, query_stride_rows, d_query_counts, d_train, train_stride_rows, d_train_counts, npairs},
+                               {MatchOp::RadiusEmit, 0, max_distance, cap}, {d_out, nullptr, nullptr, d_offsets}});
 }
 
 int orbx_filter_matches(orbx_match* m, int n, float ratio)
